@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA)
     python bench.py --impl reference --gpus N --steps K ...  # CPU reference arm
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's result arrays, DIR/*.npy
 
 Workload (config 2): phi+DM fit, 512 chan x 2048 bin, 10k subints per GPU per
 step, synthetic portraits from example.gmodel (rotated model + white noise).
@@ -231,6 +232,27 @@ GATHER_KEYS = ("params", "param_errs", "nu_out", "cov", "chi2", "red_chi2", "snr
                "return_code", "lag_index")
 
 
+# --dump-outputs: array bytes written in all, leaving room under 64 MB for the .npy headers
+DUMP_BYTES = 60 * 10 ** 6
+
+
+def dump_outputs(res, nsub, outdir, seed=0):
+    """Write the arrays of one fit_batch call, every one indexed by subint first, as outdir/<name>.npy.
+    float32 arrays stay float32, everything else is written as float64 (integer codes are exact there).
+    When the batch does not fit DUMP_BYTES, every array keeps the same seeded sample of subints (sorted),
+    as many as fit: the rows depend only on nsub and seed, so two builds run with the same arguments
+    write arrays that compare element for element."""
+    arrs = {k: np.asarray(v) for k, v in res.items()}
+    dts = {k: np.float32 if a.dtype == np.float32 else np.float64 for k, a in arrs.items()}
+    row_bytes = sum(np.dtype(dts[k]).itemsize * (a.size // nsub) for k, a in arrs.items())
+    rows = min(nsub, DUMP_BYTES // row_bytes)
+    idx = np.arange(nsub) if rows == nsub else np.sort(np.random.default_rng(seed).choice(nsub, rows, replace=False))
+    os.makedirs(outdir, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(outdir, k + ".npy"), a[idx].astype(dts[k]))
+    return rows
+
+
 def pack_toa_level(res, n):
     cols = [np.asarray(res[k][:n], dtype=np.float64).reshape(n, -1) for k in GATHER_KEYS]
     return np.ascontiguousarray(np.concatenate(cols, axis=1))
@@ -362,6 +384,9 @@ def run_ours(args):
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        # res still holds the last timed step's arrays: the next fit_batch call on this plan overwrites them
+        dump_outputs(res, nsub, args.dump_outputs)
     tt = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -707,7 +732,14 @@ def main():
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--facade-nsub", type=int, default=256)
     ap.add_argument("--c3-nsub", type=int, default=512)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result arrays of the last timed step as DIR/<name>.npy (a seeded sample of "
+                         "subints where the batch exceeds 60 MB; with several ranks, rank 0's shard)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the arrays of --impl ours")
     # stdout carries exactly one JSON line: anything libraries write to fd 1 (e.g. NCCL's version
     # banner under NCCL_DEBUG=VERSION) is sent to stderr, the line goes to the saved descriptor
     global _JSON_FD
