@@ -1,6 +1,6 @@
-// Radix-16 register butterflies for the N = 1024 row transform of k_spectra:
-// 1024 = 16 * 16 * 4, two shared-memory passes of 64 threads (16 points per
-// thread) and a last radix-4 pass fused into the real-FFT split.  Compared with
+// Radix-16 register butterflies of k_spectra16 (spectra16.cuh), the N = 1024 row
+// transform: 1024 = 16 * 16 * 4, two shared-memory passes of 64 threads (16 points
+// per thread) and a last radix-4 pass fused into the real-FFT split.  Compared with
 // the radix-8 plan (8 * 8 * 8 * 2) one full shared-memory round trip per row
 // disappears; shared-memory bandwidth is what bounds the radix-8 passes.
 #pragma once
@@ -11,32 +11,6 @@ namespace ppb {
 // 16 B elements: the radix-16 passes read stride-64 / write stride-16 (pass 1) and
 // stride-16 within 256 (pass 2); XOR the column with bits 4..6 of the position.
 __device__ __forceinline__ int phys16(int i) { return i ^ ((i >> 4) & 7); }
-
-// float -> double by integer operations (ALU pipe; F2F runs on the XU pipe): exact for normal floats
-// and zero, subnormals flush towards zero, Inf/NaN come out as huge finite values (callers that must
-// keep them non-finite test the biased exponent themselves).
-__device__ __forceinline__ double f2d_bits(float f) {
-  const unsigned b = __float_as_uint(f);
-  const unsigned a = b & 0x7fffffffu;
-  unsigned hi = (a >> 3) + (a >= 0x00800000u ? 0x38000000u : 0u);
-  hi |= b & 0x80000000u;
-  return __hiloint2double((int)hi, (int)(b << 29));
-}
-// double -> float, round to nearest even, by integer operations: |d| below the float normal range
-// gives zero; |d| >= 2^128 (and Inf/NaN) is not handled (the caller's values are bounded).
-__device__ __forceinline__ float d2f_bits(double d) {
-  const unsigned hi = (unsigned)__double2hiint(d), lo = (unsigned)__double2loint(d);
-  const unsigned a = hi & 0x7fffffffu;
-  unsigned f = __funnelshift_l(lo, a - 0x38000000u, 3);
-  const unsigned t = (lo & 0x1fffffffu) + 0x0fffffffu + (f & 1u);   // bit 29: round up (ties to even)
-  f += t >> 29;
-  if (a < 0x38100000u) f = 0u;
-  return __uint_as_float(f | (hi & 0x80000000u));
-}
-
-template <typename F> __device__ __forceinline__ cx<F> mul_c(cx<F> a, F c, F s) {   // a * (c - i s)
-  return mk<F>(fma(a.x, c, a.y * s), fma(a.y, c, -a.x * s));
-}
 
 // In-register forward DFT of 16 points.  Input natural order; output X[k] is left
 // in v[(k >> 2) + 4 (k & 3)] (read it through dft16_at()).
@@ -81,24 +55,6 @@ template <typename F> __device__ __forceinline__ void dft16(cx<F> (&v)[16]) {
   }
   dft16_group13(v[12], v[13], v[14], v[15], true);                         // q = 3: X[3 + 4s] -> v[12 + s]
 }
-// the textbook form (twiddle multiplications, then the second stage): kept for the probes
-template <typename F> __device__ __forceinline__ void dft16_plain(cx<F> (&v)[16]) {
-#pragma unroll
-  for (int r = 0; r < 4; ++r) dft4(v[r], v[r + 4], v[r + 8], v[r + 12]);   // A_r[q] -> v[r + 4q]
-  const F h = F(0.70710678118654752440), c1 = F(0.92387953251128675613), s1 = F(0.38268343236508977173);
-  // v[r + 4q] *= W16^(r q)
-  v[5] = mul_c(v[5], c1, s1);                                        // W16^1
-  v[6] = mk<F>(h * (v[6].x + v[6].y), h * (v[6].y - v[6].x));        // W16^2
-  v[7] = mul_c(v[7], s1, c1);                                        // W16^3
-  v[9] = mk<F>(h * (v[9].x + v[9].y), h * (v[9].y - v[9].x));        // W16^2
-  v[10] = mk<F>(v[10].y, -v[10].x);                                  // W16^4 = -i
-  v[11] = mk<F>(h * (v[11].y - v[11].x), -h * (v[11].x + v[11].y));  // W16^6
-  v[13] = mul_c(v[13], s1, c1);                                      // W16^3
-  v[14] = mk<F>(h * (v[14].y - v[14].x), -h * (v[14].x + v[14].y));  // W16^6
-  v[15] = mul_c(v[15], -c1, -s1);                                    // W16^9 = -c1 + i s1
-#pragma unroll
-  for (int q = 0; q < 4; ++q) dft4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);  // X[q + 4s] -> v[s + 4q]
-}
 __host__ __device__ constexpr int dft16_at(int k) { return (k >> 2) + 4 * (k & 3); }
 
 // v[r] *= w^r, r = 1..15
@@ -114,74 +70,17 @@ template <typename F> __device__ __forceinline__ void twiddle16(cx<F> (&v)[16], 
   v[13] = cmul(v[13], cmul(w12, w1)); v[14] = cmul(v[14], cmul(w12, w2)); v[15] = cmul(v[15], cmul(w12, w3));
 }
 
-// v[r] *= tab[16 r + k], r = 1..15: the powers come from a table (r-major, so that the 16 values of k a
-// warp holds are consecutive 16-byte words: two wavefronts per load)
-template <typename F> __device__ __forceinline__ void twiddle16_tab(cx<F> (&v)[16], const cx<F>* __restrict__ tabk) {
-#pragma unroll
-  for (int r = 1; r < 16; ++r) v[r] = cmul(v[r], tabk[16 * r]);
-}
-
-// The two radix-16 passes of a 1024-point row, 64 threads (t = 0..63), in place in
-// `buf` (phys16 layout).  `g`: the staged packed real row (RowSrcF32 / RowSrcI16); `tw16`: 16
-// factors e^{-2 pi i k/256}.  sync(): barrier over the 64 threads of the row.
-// Afterwards buf[p + 256 c] (c = 0..3, p < 256) is the input of the last radix-4 pass.
-template <typename F, bool TWTAB = false, bool ICVT = false, typename Src, typename Sync, typename Fn, typename Fn2>
-__device__ __forceinline__ void fft16_rows1024(cx<F>* __restrict__ buf, const cx<F>* __restrict__ tw16,
-                                               const cx<F>* __restrict__ tab, int t,
-                                               const Src g, bool gvalid, Sync sync,
-                                               Fn after_first_reads, Fn2 in_last_pass) {
-  cx<F> v[16];
-  if (gvalid) {      // uniform over the row
-    if constexpr (ICVT) {
-      unsigned amax = 0u;
-#pragma unroll
-      for (int r = 0; r < 16; ++r) {
-        const float2 x = g(t + 64 * r);
-        amax = max(amax, max(__float_as_uint(x.x) & 0x7fffffffu, __float_as_uint(x.y) & 0x7fffffffu));
-        v[r] = mk<F>((F)f2d_bits(x.x), (F)f2d_bits(x.y));
-      }
-      if (amax >= 0x7f800000u) v[0].x = F(__longlong_as_double(0x7ff8000000000000LL));   // Inf/NaN sample: poison the row
-    } else {
-#pragma unroll
-      for (int r = 0; r < 16; ++r) {
-        const float2 x = g(t + 64 * r);
-        v[r] = mk<F>((F)x.x, (F)x.y);
-      }
-    }
-  } else {
-#pragma unroll
-    for (int r = 0; r < 16; ++r) v[r] = mk<F>(F(0), F(0));
-  }
-  sync();   // staged row consumed; the previous row's split reads of buf are done
-  after_first_reads();
-  dft16_plain(v);
-#pragma unroll
-  for (int k = 0; k < 16; ++k) buf[phys16(16 * t + k)] = v[dft16_at(k)];
-  sync();
-  const int k = t & 15;
-#pragma unroll
-  for (int r = 0; r < 16; ++r) v[r] = buf[phys16(t + 64 * r)];
-  sync();
-  in_last_pass();
-  if constexpr (TWTAB) twiddle16_tab(v, tab + k);
-  else twiddle16(v, tw16[k]);
-  dft16_plain(v);
-  const int j0 = (t - k) * 16 + k;
-#pragma unroll
-  for (int r = 0; r < 16; ++r) buf[phys16(j0 + 16 * r)] = v[dft16_at(r)];
-  sync();
-}
-
 // Last radix-4 pass fused with the real-FFT split (N = 1024).  The butterflies p and
 // 256 - p (1 <= p <= 127) give Z[p + 256 j] and Z[256 - p + 256 j], i.e. the four
 // conjugate pairs (p + 256 j, N - p - 256 j): d[2j] = harmonic p + 256 j,
-// d[2j + 1] = harmonic N - p - 256 j.  w2s[p] = e^{-2 pi i p/2048}, p <= 128.
+// d[2j + 1] = harmonic N - p - 256 j.  pa = &buf[phys16(p)], pb = &buf[phys16(256 - p)]
+// (phys16 moves an element within its 16-element block, so the other three inputs of
+// each butterfly sit 256, 512 and 768 elements further on); w2 = e^{-2 pi i p/2048}.
 template <typename F>
-__device__ __forceinline__ void split_oct16(const cx<F>* __restrict__ buf, const cx<F>* __restrict__ w2s, int p, cx<F> (&d)[8]) {
+__device__ __forceinline__ void split16_general(const cx<F>* __restrict__ pa, const cx<F>* __restrict__ pb, cx<F> w2, cx<F> (&d)[8]) {
   const F h = F(0.70710678118654752440);
-  const cx<F> w2 = w2s[p];
-  cx<F> a0 = buf[phys16(p)], a1 = buf[phys16(p + 256)], a2 = buf[phys16(p + 512)], a3 = buf[phys16(p + 768)];
-  cx<F> b0 = buf[phys16(256 - p)], b1 = buf[phys16(512 - p)], b2 = buf[phys16(768 - p)], b3 = buf[phys16(1024 - p)];
+  cx<F> a0 = pa[0], a1 = pa[256], a2 = pa[512], a3 = pa[768];
+  cx<F> b0 = pb[0], b1 = pb[256], b2 = pb[512], b3 = pb[768];
   const cx<F> wn1 = csqr(w2), wn2 = csqr(wn1), wn3 = cmul(wn1, wn2);     // e^{-2 pi i c p/N}
   a1 = cmul(a1, wn1); a2 = cmul(a2, wn2); a3 = cmul(a3, wn3);
   dft4(a0, a1, a2, a3);                                                  // Z[p + 256 j]

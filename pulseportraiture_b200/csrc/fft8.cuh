@@ -93,12 +93,10 @@ template <int N> struct Plan8 {
   __host__ __device__ static constexpr int radix(int i) { return (int)((code >> (4 * i)) & 0xFu); }
 };
 
-#ifndef PP_SPECTRA_THREADS
-#define PP_SPECTRA_THREADS 128
-#endif
 template <int N> struct Slot8 {
   static constexpr int kT = N / 8;                     // threads per row slot
-  static constexpr int kSlots = (PP_SPECTRA_THREADS / kT) > 0 ? (PP_SPECTRA_THREADS / kT) : 1;  // row slots per CTA
+  static constexpr int kCtaThreads = 128;              // CTA size asked for; a row of more threads takes a CTA alone
+  static constexpr int kSlots = (kCtaThreads / kT) > 0 ? (kCtaThreads / kT) : 1;  // row slots per CTA
   static constexpr int kThreads = kSlots * kT;         // CTA size
   static constexpr int kQuads = (N / 4) / kT;          // = 2 split quads (4 harmonics each) per thread
   static constexpr int kBufElems = Padded<N>::value;   // padded complex elements per slot

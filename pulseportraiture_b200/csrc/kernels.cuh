@@ -21,6 +21,8 @@
 #include <math_constants.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "fft.cuh"
 #include "spectra_plan.cuh"
 #include "bluestein.cuh"
@@ -29,9 +31,6 @@ namespace ppb {
 
 constexpr double kDconst = 1.0 / 0.000241;  // pplib.py:48-51
 constexpr double kTwoPi = 6.283185307179586476925286766559;
-#ifndef PP_SPECTRA_MINB
-#define PP_SPECTRA_MINB 4
-#endif
 constexpr int kNCsum = 9;                   // per-channel sums kept per subint
 // The first kLoK slots of every X row also keep the float32 rounding residual
 // ("lo" part): the low harmonics carry almost all of |X|^2, so their float
@@ -83,11 +82,6 @@ __device__ __noinline__ float2 rot2pi(float vx, float vy, double x) {
   cis2pi(x, c, sn);
   const float cf = (float)c, sf = (float)sn;
   return make_float2(vx * cf - vy * sf, vx * sf + vy * cf);
-}
-
-// fire-and-forget float2 add in L2 (sm_90+: red.global.add.v2.f32); no destination registers
-__device__ __forceinline__ void red_add_f32x2(float2* p, float x, float y) {
-  asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(p), "f"(x), "f"(y) : "memory");
 }
 
 __device__ __forceinline__ double wrap_phase(double phi) {
@@ -309,7 +303,8 @@ __global__ void k_prep(PrepArgs a) {
 // PL::kSlots row slots of PL::kT threads and walks G channel rows (row plan PL:
 // spectra_plan.cuh).  Rows arrive by TMA bulk copies into a double-buffered
 // staging area; the FFT runs in double (DESIGN.md "precision"); X is stored as
-// float2 plus the float32 residual of the first LoK slots.
+// float2 plus the float32 residual of the first LoK slots.  Rows of nbin = 2048
+// are transformed by k_spectra16 (spectra16.cuh) instead.
 // ----------------------------------------------------------------------------
 struct SpectraArgs {
   const void* data;          // [nsub,nchan,2N] float32 (or int16: k_spectra<N, PL, true>), global subint index
@@ -350,16 +345,13 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
   using F = double;
   constexpr int T = PL::kT, NS = PL::kSlots, NUNIT = PL::kUnits, NOUT = PL::kOut, NACC = NUNIT * NOUT;
   static_assert(NACC * T == N, "every harmonic slot has one owner");
+  static_assert(FROMSPEC || !std::is_same<PL, SpecPlan16>::value, "nbin 2048 rows are transformed by k_spectra16");
   constexpr unsigned kRowBytes = 2 * N * (I16 ? sizeof(short) : sizeof(float));   // raw row as stored
   constexpr int NSTG = PL::kStages;   // staged raw rows per slot (TMA prefetch depth)
   extern __shared__ __align__(16) unsigned char smem_raw[];
   cx<F>* tw = reinterpret_cast<cx<F>*>(smem_raw);                       // [PL::kTwTotal] (+pad)
   cx<F>* bufs = tw + ((PL::kTwTotal + 1) & ~1);                         // [NS][N]
   float* stage_all = reinterpret_cast<float*>(bufs + (size_t)NS * N);   // [NS][NSTG][2N]
-  constexpr int kAcc = PL::kAcc;                  // where the guess profile accumulates (spectra_plan.cuh)
-  constexpr bool kMcLate = PL::kMcLate;
-  static_assert(kAcc == 0 || NS == 1, "shared / global guess accumulators: one row slot per CTA");
-  float2* acc_sh = reinterpret_cast<float2*>(stage_all + (size_t)NS * PL::kStages * 2 * N);   // [N] (kAcc == 2)
   __shared__ double red[2][NS][(T >= 32 ? T / 32 : 1)][2];   // per-warp power sums, by row parity
   __shared__ __align__(8) unsigned long long mbar[NS][2];
   const int tid = threadIdx.x, slot = tid / T, t = tid % T;
@@ -382,22 +374,10 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
   const double numean = a.nu_mean[s];
   const double numean2 = 1.0 / (numean * numean);
 
-  float2 acc[kAcc == 0 ? NACC : 1];
+  float2 acc[NACC];
   float2* const part_row = want_guess ? a.partial + ((size_t)sl * a.nparts + blockIdx.x * NS + slot) * N : nullptr;
-  if constexpr (kAcc == 0) {
 #pragma unroll
-    for (int i = 0; i < NACC; ++i) acc[i] = make_float2(0.f, 0.f);
-  } else if (want_guess) {   // every slot of the CTA's partial row has one owner thread: zero it, then add row by row
-#pragma unroll
-    for (int i = 0; i < NUNIT; ++i) {
-#pragma unroll
-      for (int q = 0; q < NOUT; ++q) {
-        const int sk = PL::slot_of(t, i, q, t == 0);
-        if constexpr (kAcc == 1) part_row[sk] = make_float2(0.f, 0.f);
-        else acc_sh[sk] = make_float2(0.f, 0.f);
-      }
-    }
-  }
+  for (int i = 0; i < NACC; ++i) acc[i] = make_float2(0.f, 0.f);
   double keep_all = 0.0, keep_top = 0.0;
   // thread r of a slot collects the power sums of row r (T > 32: from the per-warp totals)
   auto latch = [&](int r) {
@@ -463,39 +443,25 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
     const int kcut = (a.njn && inrange) ? 16 * a.njn[ch] : N;
     const cx<F>* mc = a.mconj64 + (size_t)(inrange ? ch : 0) * N;
     const cx<float>* mcf = a.mconj32 + (size_t)(inrange ? ch : 0) * N;
-    static_assert(!kMcLate || kMix, "late conj(model) loads: mixed-precision plans only");
     cx<F> mc64[kMix ? 1 : NACC];
-    cx<float> mc32[kMix ? (kMcLate ? NOUT : NACC) : 1];
-    auto load_mc_unit = [&](int i) {   // kMcLate: the loads of unit i, issued right before its split
-      if (doX && used) {
-        if (i == 0) mc64[0] = mc[t];
-#pragma unroll
-        for (int q = 0; q < NOUT; ++q) mc32[q] = mcf[slot_of(i, q)];
-      } else {
-        if (i == 0) mc64[0] = mk<F>(0.0, 0.0);
-#pragma unroll
-        for (int q = 0; q < NOUT; ++q) mc32[q] = mk<float>(0.f, 0.f);
-      }
-    };
+    cx<float> mc32[kMix ? NACC : 1];
     auto load_mc = [&]() {
-      if constexpr (!kMcLate) {
-        if (doX && used) {
-          if constexpr (kMix) mc64[0] = mc[t];
+      if (doX && used) {
+        if constexpr (kMix) mc64[0] = mc[t];
 #pragma unroll
-          for (int i = 0; i < NUNIT; ++i) {
+        for (int i = 0; i < NUNIT; ++i) {
 #pragma unroll
-            for (int q = 0; q < NOUT; ++q) {
-              if constexpr (kMix) mc32[NOUT * i + q] = mcf[slot_of(i, q)];
-              else mc64[NOUT * i + q] = mc[slot_of(i, q)];
-            }
+          for (int q = 0; q < NOUT; ++q) {
+            if constexpr (kMix) mc32[NOUT * i + q] = mcf[slot_of(i, q)];
+            else mc64[NOUT * i + q] = mc[slot_of(i, q)];
           }
-        } else {   // unused rows store zeros
-          if constexpr (kMix) mc64[0] = mk<F>(0.0, 0.0);
+        }
+      } else {   // unused rows store zeros
+        if constexpr (kMix) mc64[0] = mk<F>(0.0, 0.0);
 #pragma unroll
-          for (int i = 0; i < NACC; ++i) {
-            if constexpr (kMix) mc32[i] = mk<float>(0.f, 0.f);
-            else mc64[i] = mk<F>(0.0, 0.0);
-          }
+        for (int i = 0; i < NACC; ++i) {
+          if constexpr (kMix) mc32[i] = mk<float>(0.f, 0.f);
+          else mc64[i] = mk<F>(0.0, 0.0);
         }
       }
     };
@@ -521,7 +487,6 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
 #pragma unroll
     for (int i = 0; i < NUNIT; ++i) {
       cx<F> d[NOUT];
-      if constexpr (kMcLate) load_mc_unit(i);
       F dc_term = F(0);
       if constexpr (FROMSPEC) {
 #pragma unroll
@@ -550,8 +515,7 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
           sa = fma(d[q].x, d[q].x, sa);
           sa = fma(d[q].y, d[q].y, sa);
         }
-        if constexpr ((PL::kCvt & 2) != 0) { vx[q] = d2f_bits(d[q].x); vy[q] = d2f_bits(d[q].y); }
-        else { vx[q] = (float)d[q].x; vy[q] = (float)d[q].y; }
+        vx[q] = (float)d[q].x; vy[q] = (float)d[q].y;
       }
       s_all += sa0 + sa1;
       if (doX) {        // uniform over the row
@@ -564,7 +528,7 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
           if constexpr (kMix) lo = (i == 0 && q == 0) && (t < kLo);
           else lo = true;
           if (!lo) {
-            const cx<float> m = mc32[kMix ? (kMcLate ? q : idx) : 0];
+            const cx<float> m = mc32[kMix ? idx : 0];
             Xrow[sk] = make_float2(fmaf(vx[q], m.x, -vy[q] * m.y), fmaf(vx[q], m.y, vy[q] * m.x));
           } else {
             const cx<F> pr = cmul(d[q], mc64[kMix ? 0 : idx]);
@@ -590,16 +554,8 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
       if (wrow != 0.f) {   // uniform: 0 when no guess is wanted, the row is unused or not finite
 #pragma unroll
         for (int q = 0; q < NOUT; ++q) {
-          if constexpr (kAcc == 0) {
-            acc[NOUT * i + q].x = fmaf(wrow, vx[q], acc[NOUT * i + q].x);
-            acc[NOUT * i + q].y = fmaf(wrow, vy[q], acc[NOUT * i + q].y);
-          } else if constexpr (kAcc == 1) {
-            red_add_f32x2(part_row + slot_of(i, q), wrow * vx[q], wrow * vy[q]);
-          } else {
-            float2* const p = acc_sh + slot_of(i, q);
-            const float2 o = *p;
-            *p = make_float2(fmaf(wrow, vx[q], o.x), fmaf(wrow, vy[q], o.y));
-          }
+          acc[NOUT * i + q].x = fmaf(wrow, vx[q], acc[NOUT * i + q].x);
+          acc[NOUT * i + q].y = fmaf(wrow, vy[q], acc[NOUT * i + q].y);
         }
       }
     }
@@ -637,16 +593,12 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
       a.Sdn[o] = ok ? keep_all / sF2 : 0.0;
     }
   }
-  if (want_guess && kAcc != 1) {
+  if (want_guess) {
     const bool first = (t == 0);
 #pragma unroll
     for (int i = 0; i < NUNIT; ++i) {
 #pragma unroll
-      for (int q = 0; q < NOUT; ++q) {
-        const int sk = PL::slot_of(t, i, q, first);
-        if constexpr (kAcc == 0) part_row[sk] = acc[NOUT * i + q];
-        else part_row[sk] = acc_sh[sk];
-      }
+      for (int q = 0; q < NOUT; ++q) part_row[PL::slot_of(t, i, q, first)] = acc[NOUT * i + q];
     }
   }
 }
@@ -890,12 +842,9 @@ struct PassArgs {
 };
 
 // streaming 16-byte load: read-only path, do not keep in L1
-#ifndef PP_LD_STREAM_QUAL
-#define PP_LD_STREAM_QUAL "ld.global.nc.L1::no_allocate.v4.f32"
-#endif
 __device__ __forceinline__ float4 ld_stream(const float4* p) {
   float4 v;
-  asm volatile(PP_LD_STREAM_QUAL " {%0,%1,%2,%3}, [%4];"
+  asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
                : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
   return v;
 }
@@ -917,12 +866,10 @@ template <int N> struct Pass2Ring {
   static constexpr int D = NJ < 8 ? NJ : 8;
   static constexpr int KJ = LoK<N>::value / 16;
   static constexpr size_t kBytes = sizeof(float4) * 256 * (D + KJ);
+  static constexpr int kMinBlocks = 4;   // CTAs per SM asked of the compiler
 };
-#ifndef PP_PASS2_MINB
-#define PP_PASS2_MINB 4
-#endif
 template <int N>
-__global__ void __launch_bounds__(256, PP_PASS2_MINB) k_pass2(PassArgs a) {
+__global__ void __launch_bounds__(256, Pass2Ring<N>::kMinBlocks) k_pass2(PassArgs a) {
   const int sl = blockIdx.y, s = a.s0 + sl;
   if (a.st.done[s] == 1) return;
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -1508,9 +1455,6 @@ struct Pass5Args {
   const int* njn;          // [nchan] groups of 16 harmonics where the model has power (k_model_cutoff)
 };
 
-#ifndef PP_PASS5_MINB
-#define PP_PASS5_MINB 2
-#endif
 // k_pass5 keeps D iterations of loads (X row piece + |m|^2 piece, 16 bytes each per thread) in flight through a
 // thread-private ring in shared memory: the kernel is FP64-bound with 128 registers per thread and 16 warps per SM,
 // too few to cover the load latency from registers.
@@ -1519,10 +1463,11 @@ template <int N> struct Pass5Ring {
   static constexpr int D = NJ < 8 ? NJ : 8;
   static constexpr int KJ = LoK<N>::value / 16;
   static constexpr size_t kBytes = sizeof(float4) * 256 * (2 * D + KJ);
+  static constexpr int kMinBlocks = 2;   // CTAs per SM asked of the compiler
 };
 
 template <int N>
-__global__ void __launch_bounds__(256, PP_PASS5_MINB) k_pass5(Pass5Args a) {
+__global__ void __launch_bounds__(256, Pass5Ring<N>::kMinBlocks) k_pass5(Pass5Args a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int sl = blockIdx.y, s = a.s0 + sl;
   constexpr int NJ = N / 16;

@@ -10,7 +10,6 @@
 
 #include <algorithm>
 #include <chrono>
-#include <type_traits>
 #include <string>
 #include <thread>
 #include <vector>
@@ -275,6 +274,13 @@ static void launch_spectra16(bool i16, bool guess, bool keepd, dim3 grid, cudaSt
   }
 #undef L16_
 }
+// the generic kernel on the other power-of-two nbin (N = 1024 is launch_spectra16's)
+template <int N> static void launch_spectra(bool i16, dim3 grid, cudaStream_t st, const SpectraArgs& a) {
+  if constexpr (N != 1024) {
+    if (i16) k_spectra<N, SpecPlan<N>, true><<<grid, SpecPlan<N>::kThreads, spectra_smem_bytes<N>(), st>>>(a);
+    else k_spectra<N><<<grid, SpecPlan<N>::kThreads, spectra_smem_bytes<N>(), st>>>(a);
+  }
+}
 
 // ---- arbitrary nbin: Bluestein row transforms (bluestein.cuh) ----------------------------------------------
 #define DISPATCH_M(Mval, ...)                                   \
@@ -307,8 +313,10 @@ template <int N> static cudaError_t setup_attrs() {
   const int b32 = (int)fft_smem_bytes<N, float>(), b64 = (int)fft_smem_bytes<N, double>();
   cudaError_t e;
 #define SET_(fn, bytes) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); if (e != cudaSuccess) return e;
-  SET_((k_spectra<N>), (int)spectra_smem_bytes<N>())
-  SET_((k_spectra<N, SpecPlan<N>, true>), (int)spectra_smem_bytes<N>())
+  if constexpr (N != 1024) {   // nbin 2048 rows go to k_spectra16 (spectra16_attrs)
+    SET_((k_spectra<N>), (int)spectra_smem_bytes<N>())
+    SET_((k_spectra<N, SpecPlan<N>, true>), (int)spectra_smem_bytes<N>())
+  }
   SET_((k_model<N>), b64)
   SET_((k_pass5<N>), (int)Pass5Ring<N>::kBytes)
   SET_((k_pass2<N>), (int)Pass2Ring<N>::kBytes)
@@ -843,16 +851,17 @@ static int pick_chunk(pp_plan* pl, int nsub, bool data_on_host, double bytes_per
   return (int)std::min<long>(c, nsub);
 }
 
+constexpr int kSpectraGMax = 32;   // most channel rows per spectra CTA
+// nbin 2048 has one row slot per CTA, so its G never exceeds kSpectraGMax: k_spectra16 takes every such launch
+static_assert(SpecPlan<1024>::kSlots == 1 && kSpectraGMax <= kSpec16MaxRows, "nbin 2048: G <= kSpec16MaxRows");
+
 static int rows_per_cta(pp_plan* pl, int chunk) {
   // Channel rows handled by one k_spectra CTA.  It fixes how the partial profile spectra of
   // the FFTFIT guess are grouped, so it must NOT depend on the batch or chunk size (results
   // are bit-identical for any chunking): a function of nchan only, ~16 CTAs per subint.
   (void)chunk;
   const int rows_conc = spectra_slots(pl->N);
-#ifndef PP_SPECTRA_GMAX
-#define PP_SPECTRA_GMAX 32
-#endif
-  int g = std::max(rows_conc, std::min(PP_SPECTRA_GMAX, pl->nchan / (512 / PP_SPECTRA_GMAX)));
+  int g = std::max(rows_conc, std::min(kSpectraGMax, pl->nchan / (512 / kSpectraGMax)));
   g = ((g + rows_conc - 1) / rows_conc) * rows_conc;
   // k_spectra finalises one row per thread of a row slot: rows per slot <= N/8 (32 <= 128 here)
   return g;
@@ -1138,12 +1147,10 @@ extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_f
         a.dspec = pl->any_spec.as<cx<double>>(); a.ddc = pl->any_dc.as<double>();
         a.nhalf = pl->L; a.kc_true = (3 * (pl->L + 1)) / 4;
         DISPATCH_N(N, (k_spectra<NN, SpecPlan<NN>, false, true><<<dim3(gx, ns), SpecPlan<NN>::kThreads, 0, pl->stream>>>(a)));
-      } else if (N == 1024 && G <= kSpec16MaxRows && std::is_same<SpecPlan<1024>, SpecPlan16>::value) {
+      } else if (N == 1024) {
         launch_spectra16(i16, want_guess, want_align, dim3(gx, ns), pl->stream, a);
-      } else if (i16) {
-        DISPATCH_N(N, (k_spectra<NN, SpecPlan<NN>, true><<<dim3(gx, ns), SpecPlan<NN>::kThreads, spectra_smem_bytes<NN>(), pl->stream>>>(a)));
       } else {
-        DISPATCH_N(N, k_spectra<NN><<<dim3(gx, ns), SpecPlan<NN>::kThreads, spectra_smem_bytes<NN>(), pl->stream>>>(a));
+        DISPATCH_N(N, launch_spectra<NN>(i16, dim3(gx, ns), pl->stream, a));
       }
       pl->stats.launches++;
     }

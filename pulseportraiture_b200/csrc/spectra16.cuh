@@ -1,9 +1,10 @@
-// k_spectra16: K1 + K2 for nbin = 2048 (N = 1024), the configuration the headline metric is quoted on.
-// Same arithmetic and outputs as k_spectra<1024, SpecPlan16> (kernels.cuh), restructured around what bounds
-// that kernel on B200: the warp schedulers' issue slots.  An FP64 instruction holds the dispatch port of its
-// SM sub-partition for two cycles and every other instruction for one (tools/micro/cvt_probe.cu), so
-// a row costs 2 * n_fp64 + n_other slots per thread; the generic kernel spends ~790 non-FP64 instructions per
-// thread and row, a third of them on shared-memory addresses and on predicated-off code.  Here
+// k_spectra16: K1 + K2 for nbin = 2048 (N = 1024), the configuration the headline metric is quoted on, and the
+// only kernel that transforms rows of that size.  The same work as k_spectra (kernels.cuh) on the radix-16 plan
+// of fft16.cuh, written around what bounds it on B200: the warp schedulers' issue slots.  An FP64 instruction
+// holds the dispatch port of its SM sub-partition for two cycles and every other instruction for one
+// (tools/micro/cvt_probe.cu), so a row costs 2 * n_fp64 + n_other slots per thread.  Run inside the generic
+// k_spectra, this plan spent ~790 non-FP64 instructions per thread and row, a third of them on shared-memory
+// addresses and on predicated-off code.  Here
 //   * every shared-memory address is a per-thread base plus an immediate: the XOR swizzle of a pass is split
 //     into its per-thread part (folded into a handful of base offsets, recomputed once per row) and its
 //     compile-time part,
@@ -29,27 +30,8 @@ constexpr int kSpec16MaxRows = 32;   // rows per CTA (host: rows_per_cta <= 32)
 //   pass 2 writes  i = 256 b + k + 16 r (b = t >> 4, k = t & 15) -> 256 b + 16 r + (k ^ (r & 7))
 //   split reads    i = p + 256 c       -> (p ^ ((p >> 4) & 7)) + 256 c
 
-template <typename F>
-__device__ __forceinline__ void split16_general(const cx<F>* __restrict__ pa, const cx<F>* __restrict__ pb, cx<F> w2, cx<F> (&d)[8]) {
-  // as split_oct16(): pa = &buf[phys16(p)], pb = &buf[phys16(256 - p)], w2 = e^{-2 pi i p/2048}
-  const F h = F(0.70710678118654752440);
-  cx<F> a0 = pa[0], a1 = pa[256], a2 = pa[512], a3 = pa[768];
-  cx<F> b0 = pb[0], b1 = pb[256], b2 = pb[512], b3 = pb[768];
-  const cx<F> wn1 = csqr(w2), wn2 = csqr(wn1), wn3 = cmul(wn1, wn2);
-  a1 = cmul(a1, wn1); a2 = cmul(a2, wn2); a3 = cmul(a3, wn3);
-  dft4(a0, a1, a2, a3);
-  b1 = cmul(b1, mk<F>(-wn1.y, -wn1.x)); b2 = cmul(b2, mk<F>(-wn2.x, wn2.y)); b3 = cmul(b3, mk<F>(wn3.y, wn3.x));
-  dft4(b0, b1, b2, b3);
-  const F hh = F(0.5) * h;
-  const cx<F> wh = chalf(w2);
-  real_pair_h(a0, b3, wh, d[0], d[1]);
-  real_pair_h(a1, b2, mk<F>(hh * (w2.x + w2.y), hh * (w2.y - w2.x)), d[2], d[3]);
-  real_pair_h(a2, b1, mk<F>(wh.y, -wh.x), d[4], d[5]);
-  real_pair_h(a3, b0, mk<F>(hh * (w2.y - w2.x), -hh * (w2.x + w2.y)), d[6], d[7]);
-}
-
-template <bool I16, bool GUESS, bool KEEPD, int EXP = 0>   // EXP: timing experiments only (tools/micro/spectra_probe.cu)
-__global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs a) {
+template <bool I16, bool GUESS, bool KEEPD>
+__global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(SpectraArgs a) {
   using F = double;
   using PL = SpecPlan16;
   constexpr int N = 1024, T = 64, kLo = LoK<N>::value;
@@ -153,7 +135,7 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
     fetch(step + 1);
     const bool doX = a.X != nullptr;
     const int kcut = a.njn ? 16 * a.njn[ch] : N;
-    if (doX && !(EXP & 1)) fetch_model(ch);
+    if (doX) fetch_model(ch);
     dft16(v);
     {
       cx<F>* const w0 = buf + 16 * t;
@@ -180,7 +162,7 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
     // (p = t + 64 i; the special unit of thread 0 uses p = 0 / 128).
     cx<F> mc64 = mk<F>(0.5, 0.25);
     const int po0 = first ? 128 : t;           // the odd outputs of unit 0
-    if (doX && !(EXP & 1)) mc64 = a.mconj64[(size_t)ch * N + t];   // the one double-precision factor (lo slot t)
+    if (doX) mc64 = a.mconj64[(size_t)ch * N + t];   // the one double-precision factor (lo slot t)
     float wgt = 0.f;
     double shift = 0.0;
     if constexpr (GUESS) {
@@ -203,8 +185,7 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
     // ---- last radix-4 pass fused with the real-FFT split; power sums; X; guess accumulators -------------
     double s_all = 0.0, s_top = 0.0;
     float wrow = wgt;
-    float dummy = 0.f;
-    if (doX && !(EXP & 1)) { mbar_wait(&mbar[1], ph1); ph1 ^= 1u; }   // the model row has landed long ago
+    if (doX) { mbar_wait(&mbar[1], ph1); ph1 ^= 1u; }   // the model row has landed long ago
 #pragma unroll
     for (int i = 0; i < 2; ++i) {
       const int p = t + 64 * i;
@@ -231,8 +212,7 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
           sa = fma(d[q].x, d[q].x, sa);
           sa = fma(d[q].y, d[q].y, sa);
         }
-        if (EXP & 8) { vx[q] = __int_as_float(__double2hiint(d[q].x)); vy[q] = __int_as_float(__double2hiint(d[q].y)); }   // no F2F
-        else { vx[q] = (float)d[q].x; vy[q] = (float)d[q].y; }
+        vx[q] = (float)d[q].x; vy[q] = (float)d[q].y;
       }
       s_all += sa0 + sa1;
       const int po = (i == 0) ? po0 : p;
@@ -253,12 +233,8 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
             *dst = xv;
             a.Xlo[row * kLo + t] = make_float2((float)(pr.x - (double)xv.x), (float)(pr.y - (double)xv.y));
           } else {
-            const cx<float> m = (EXP & 1) ? mk<float>(0.5f + q, 0.25f) : *((q & 1) ? Mo - 256 * (q >> 1) : Me + 256 * (q >> 1));
-            float2 xv;
-            if (EXP & 4) xv = make_float2(vx[q], vy[q]);                                                 // no product
-            else xv = make_float2(fmaf(vx[q], m.x, -vy[q] * m.y), fmaf(vx[q], m.y, vy[q] * m.x));
-            if (EXP & 2) dummy += xv.x + xv.y;                                                           // no store
-            else *dst = xv;
+            const cx<float> m = *((q & 1) ? Mo - 256 * (q >> 1) : Me + 256 * (q >> 1));
+            *dst = make_float2(fmaf(vx[q], m.x, -vy[q] * m.y), fmaf(vx[q], m.y, vy[q] * m.x));
           }
         }
       }
@@ -287,7 +263,6 @@ __global__ void __launch_bounds__(64, PP_SPECTRA16_MINB) k_spectra16(SpectraArgs
         }
       }
     }
-    if (EXP & 2) s_all += (double)dummy * 1e-300;
     s_all = warp_sum(s_all); s_top = warp_sum(s_top);
     if ((t & 31) == 0) rowsum[step][t >> 5] = make_double2(s_all, s_top);
   }

@@ -1,33 +1,21 @@
-// Row-transform plans of k_spectra.  A plan fixes how many threads own a row, how
-// the N-point transform is split into register butterflies, and how the fused last
-// pass + real-FFT split hands harmonics to threads ("units" of kOut outputs):
+// Row plans of k_spectra.  A plan fixes how many threads own a row, how the N-point
+// transform is split into register butterflies, and how the fused last pass + real-FFT
+// split hands harmonics to threads ("units" of kOut outputs):
 //
 //   SpecPlan8<N>   N/8 threads per row, radix-8/4 passes + (radix-2 fused with the
 //                  split), units = quads: slots p, N-p, N/2-p, N/2+p
-//   SpecPlan16     N = 1024 only: 64 threads per row, two radix-16 passes + (radix-4
-//                  fused with the split), units = octs: slots p+256j, N-p-256j
+//   SpecPlan16     N = 1024 only: 64 threads per row, units = octs: slots p+256j, N-p-256j.
+//                  The layout of k_spectra16 (spectra16.cuh: two radix-16 passes + radix-4
+//                  fused with the split) and of its twiddle table.  k_spectra runs it only on
+//                  rows that arrive transformed (FROMSPEC, nbin 1026..2046): there it fixes
+//                  which thread sums which harmonic powers, and SpecPlan8<1024> would sum the
+//                  noise estimate in another order.
 //
 // In both, unit 0 of thread 0 is the special unit that holds the self-paired and
 // the Nyquist harmonic; its outputs are ordered so that the per-output rules
 // (slot formula, "is in the top quarter", "may carry a lo part") stay uniform.
 #pragma once
 #include "fft16.cuh"
-
-#ifndef PP_SPECTRA_MINB
-#define PP_SPECTRA_MINB 4
-#endif
-#ifndef PP_SPECTRA_MINB_2048
-#define PP_SPECTRA_MINB_2048 2
-#endif
-#ifndef PP_SPECTRA_R16
-#define PP_SPECTRA_R16 1
-#endif
-#ifndef PP_SPECTRA16_MINB
-#define PP_SPECTRA16_MINB 6
-#endif
-#ifndef PP_SPECTRA16_STAGES
-#define PP_SPECTRA16_STAGES 2
-#endif
 
 namespace ppb {
 
@@ -36,12 +24,8 @@ template <int N> struct SpecPlan8 {
   static constexpr int kT = S8::kT, kSlots = S8::kSlots, kThreads = S8::kThreads;
   static constexpr int kUnits = S8::kQuads, kOut = 4;
   static constexpr int kTwTotal = TwLayout<N>::kTotal;
-  static constexpr int kMinBlocks = (N >= 2048 ? PP_SPECTRA_MINB_2048 : PP_SPECTRA_MINB);
+  static constexpr int kMinBlocks = N >= 2048 ? 2 : 4;   // CTAs per SM, chosen by measurement (DESIGN.md §4)
   static constexpr int kStages = 2;
-  static constexpr int kAcc = 0;
-  static constexpr bool kMcLate = false;
-  static constexpr int kCvt = 0;
-  static constexpr int kAccSmemBytes = 0;
   __device__ static __forceinline__ void sync(int slot) { slot_sync<N>(slot); }
   template <typename F, typename Src, typename Fn, typename Fn2>
   __device__ static __forceinline__ void transform(cx<F>* buf, const cx<F>* tw, int t, int slot, const Src g, bool used,
@@ -65,42 +49,15 @@ template <int N> struct SpecPlan8 {
   __device__ static __forceinline__ bool top(int i, int q, bool first) { return q == 1 || (q == 0 && i == 0 && first); }
 };
 
-// Knobs of the radix-16 plan (template parameters so that variants can be timed side by side,
-// tools/micro/spectra_probe.cu):
-//   STAGES  staged raw rows per CTA (TMA prefetch depth)
-//   MINB    CTAs per SM asked of the compiler (register budget 65536 / (64 MINB))
-//   ACC     where the partial profile spectra of the FFTFIT guess accumulate over the CTA's rows:
-//           0 registers (32 per thread), 1 red.global.add.v2.f32 on the CTA's own partial row
-//           (one thread per address, program order: still deterministic), 2 shared memory
-//   MCLATE  conj(model) loads issued per split unit instead of inside the last transform pass
-//   TWTAB   pass-2 twiddle powers w^2..w^15 from a shared-memory table instead of registers
-//   CVT     bit 0: float -> double of the samples by integer operations (ALU pipe) instead of F2F (XU pipe);
-//           bit 1: double -> float of the spectra likewise (round to nearest even)
-template <int STAGES, int MINB, int ACC, bool MCLATE, bool TWTAB, int CVT = 0>
-struct SpecPlan16T {
+struct SpecPlan16 {
   static constexpr int N = 1024;
   static constexpr int kT = 64, kSlots = 1, kThreads = 64;
   static constexpr int kUnits = 2, kOut = 8;
   static constexpr int kSplitOff = 16;                    // tw[0..15] = e^{-2 pi i k/256}; then e^{-2 pi i p/2048}, p <= 128
-  static constexpr int kTabOff = kSplitOff + 130;         // TWTAB: tw[kTabOff + 16 r + k] = e^{-2 pi i k r/256}
-  static constexpr int kTwTotal = TWTAB ? kTabOff + 256 : kSplitOff + 129;
-  static constexpr int kMinBlocks = MINB;
-  static constexpr int kStages = STAGES;
-  static constexpr int kAcc = ACC;
-  static constexpr bool kMcLate = MCLATE;
-  static constexpr int kCvt = CVT;
-  static constexpr int kAccSmemBytes = ACC == 2 ? N * 8 : 0;
+  static constexpr int kTwTotal = kSplitOff + 129;
+  static constexpr int kMinBlocks = 6;                    // CTAs per SM (register budget 65536 / (64 kMinBlocks))
+  static constexpr int kStages = 2;                       // staging space of two raw rows (k_spectra16: raw + model row)
   __device__ static __forceinline__ void sync(int) { __syncthreads(); }
-  template <typename F, typename Src, typename Fn, typename Fn2>
-  __device__ static __forceinline__ void transform(cx<F>* buf, const cx<F>* tw, int t, int, const Src g, bool used,
-                                                   Fn after_first_reads, Fn2 in_last_pass) {
-    fft16_rows1024<F, TWTAB, (CVT & 1) != 0>(buf, tw, tw + kTabOff, t, g, used, []() { __syncthreads(); }, after_first_reads, in_last_pass);
-  }
-  template <typename F>
-  __device__ static __forceinline__ F split(const cx<F>* buf, const cx<F>* tw, int t, int i, bool first, cx<F> (&d)[kOut]) {
-    if (i > 0 || !first) { split_oct16<F>(buf, tw + kSplitOff, t + i * kT, d); return F(0); }
-    return split_oct0<F>(buf, tw + kSplitOff, d);   // the row's DC term
-  }
   // q = 2j: slot p + 256 j; q = 2j + 1: slot N - p - 256 j; the special unit uses p = 0 for
   // the even and p = 128 for the odd outputs
   __device__ static __forceinline__ int slot_of(int t, int i, int q, bool first) {
@@ -110,21 +67,9 @@ struct SpecPlan16T {
   }
   __device__ static __forceinline__ bool top(int i, int q, bool first) { return q == 1 || q == 6 || (q == 0 && i == 0 && first); }
 };
-#ifndef PP_SPECTRA16_ACC
-#define PP_SPECTRA16_ACC 0
-#endif
-#ifndef PP_SPECTRA16_MCLATE
-#define PP_SPECTRA16_MCLATE 0
-#endif
-#ifndef PP_SPECTRA16_TWTAB
-#define PP_SPECTRA16_TWTAB 0
-#endif
-using SpecPlan16 = SpecPlan16T<PP_SPECTRA16_STAGES, PP_SPECTRA16_MINB, PP_SPECTRA16_ACC, PP_SPECTRA16_MCLATE != 0, PP_SPECTRA16_TWTAB != 0>;
 
 template <int N> struct SpecPlanSel { using type = SpecPlan8<N>; };
-#if PP_SPECTRA_R16
 template <> struct SpecPlanSel<1024> { using type = SpecPlan16; };
-#endif
 template <int N> using SpecPlan = typename SpecPlanSel<N>::type;
 
 }  // namespace ppb

@@ -19,15 +19,12 @@ inline double2 unit_root(long num, long den) {   // e^{-2 pi i num/den} with exa
 }
 
 template <class PL> struct TwBuilder;
-template <int ST, int MB, int AC, bool ML, bool TT, int CV> struct TwBuilder<SpecPlan16T<ST, MB, AC, ML, TT, CV>> {
+template <> struct TwBuilder<SpecPlan16> {
   static void build(std::vector<double2>& out) {
-    using PL = SpecPlan16T<ST, MB, AC, ML, TT, CV>;
+    using PL = SpecPlan16;
     out.assign(PL::kTwTotal, make_double2(0.0, 0.0));
     for (int k = 0; k < 16; ++k) out[k] = unit_root(k, 256);
     for (int p2 = 0; p2 <= 128; ++p2) out[PL::kSplitOff + p2] = unit_root(p2, 2048);
-    if (TT)
-      for (int r = 0; r < 16; ++r)
-        for (int k = 0; k < 16; ++k) out[PL::kTabOff + 16 * r + k] = unit_root((long)k * r, 256);
   }
 };
 // per-pass twiddle tables in the layout of TwLayout<N> (fft8.cuh)
@@ -46,7 +43,7 @@ template <int N> struct TwBuilder<SpecPlan8<N>> {
 
 template <int N, class PL = SpecPlan<N>> constexpr size_t spectra_smem_bytes_of() {
   return (size_t)(((PL::kTwTotal + 1) & ~1) + PL::kSlots * N) * sizeof(cx<double>) +
-         (size_t)PL::kSlots * PL::kStages * (2 * N) * sizeof(float) + (size_t)PL::kAccSmemBytes;
+         (size_t)PL::kSlots * PL::kStages * (2 * N) * sizeof(float);
 }
 
 }  // namespace ppb
