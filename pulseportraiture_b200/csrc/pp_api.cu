@@ -10,6 +10,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -62,10 +63,14 @@ extern "C" int pp_abi_version(void) { return PPB200_ABI_VERSION; }
 struct DBuf {
   void* p = nullptr;
   size_t cap = 0;
+  DBuf() = default;
+  DBuf(const DBuf&) = delete;
+  DBuf& operator=(const DBuf&) = delete;
+  DBuf(DBuf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+  ~DBuf() { release(); }
   cudaError_t need(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
-    if (p) cudaFree(p);
-    p = nullptr; cap = 0;
+    release();
     cudaError_t e = cudaMalloc(&p, bytes);
     if (e == cudaSuccess) cap = bytes;
     return e;
@@ -124,6 +129,16 @@ struct pp_plan {
   struct Span { int kind; cudaEvent_t a, b; };
   std::vector<Span> spans;
   pp_stats_t stats;
+  // the DBuf members free themselves after this; `stream` may be the caller's (pp_plan_set_stream)
+  ~pp_plan() {
+    for (cudaEvent_t e : ev_pool) cudaEventDestroy(e);
+    for (cudaEvent_t e : ev_chunk) cudaEventDestroy(e);
+    for (cudaEvent_t e : {ev_copy[0], ev_copy[1], ev_free[0], ev_free[1], pin_ev[0], pin_ev[1], pin_ev[2], pin_ev[3]})
+      if (e) cudaEventDestroy(e);
+    for (void* h : pin_ring) if (h) cudaFreeHost(h);
+    if (own_stream) cudaStreamDestroy(own_stream);
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+  }
 };
 
 enum { SP_SPECTRA = 0, SP_GUESS = 1, SP_PASS = 2, SP_UPDATE = 3, SP_TOTAL = 4, SP_COARSE = 5 };
@@ -177,32 +192,27 @@ static void stats_end(pp_plan* pl) {
 // ----------------------------------------------------------------------------
 // pointer staging: returns a device pointer for host-or-device input
 // ----------------------------------------------------------------------------
-static bool is_device_ptr(const void* p) {
+enum MemKind { kMemPageable, kMemPinned, kMemDevice };
+static MemKind mem_kind(const void* p) {
   cudaPointerAttributes at;
   cudaError_t e = cudaPointerGetAttributes(&at, p);
-  if (e != cudaSuccess) { cudaGetLastError(); return false; }
-  return at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged;
+  if (e != cudaSuccess) { cudaGetLastError(); return kMemPageable; }
+  if (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) return kMemDevice;
+  return at.type == cudaMemoryTypeHost ? kMemPinned : kMemPageable;
 }
+static bool is_device_ptr(const void* p) { return mem_kind(p) == kMemDevice; }
 
-static bool is_pinned_host_ptr(const void* p);
 static cudaError_t h2d_any(pp_plan* pl, void* dst, const void* src, size_t bytes, bool src_pinned, cudaStream_t st, bool narrow);
 
 template <typename T>
 static int stage_in(pp_plan* pl, DBuf& buf, const T* src, size_t n, const T** out) {
   if (!src) { *out = nullptr; return 0; }
-  if (is_device_ptr(src)) { *out = src; return 0; }
+  const MemKind kind = mem_kind(src);
+  if (kind == kMemDevice) { *out = src; return 0; }
   CK(buf.need(n * sizeof(T)));
   const size_t bytes = n * sizeof(T);
-  CK(h2d_any(pl, buf.p, src, bytes, bytes < (8u << 20) || is_pinned_host_ptr(src), pl->stream, false));
+  CK(h2d_any(pl, buf.p, src, bytes, bytes < (8u << 20) || kind == kMemPinned, pl->stream, false));
   *out = buf.as<T>();
-  return 0;
-}
-
-template <typename T>
-static int copy_out(pp_plan* pl, T* dst, const T* dev, size_t n) {
-  if (!dst) return 0;
-  CK(cudaMemcpyAsync(dst, dev, n * sizeof(T), is_device_ptr(dst) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost,
-                     pl->stream));
   return 0;
 }
 
@@ -220,6 +230,8 @@ static int copy_out_at(cudaStream_t st, T* dst, const T* dev, size_t off, size_t
 template <int N, typename T> static size_t fft_smem_bytes() {
   return (size_t)(N + N / 2 + 2 + RowGeom<N>::kRows * 2 * N) * sizeof(cx<T>);
 }
+// CTAs of a row kernel (RowGeom<N>::kRows rows each) for nrows rows
+template <int N> static unsigned row_ctas(long nrows) { return (unsigned)((nrows + RowGeom<N>::kRows - 1) / RowGeom<N>::kRows); }
 
 #define DISPATCH_N(Nval, ...)                                   \
   switch (Nval) {                                               \
@@ -236,43 +248,25 @@ template <int N, typename T> static size_t fft_smem_bytes() {
 template <int N> static size_t spectra_smem_bytes() { return spectra_smem_bytes_of<N>(); }
 // row slots per k_spectra CTA for this nbin
 static int spectra_slots(int N) {
-  switch (N) {
-    case 32: return SpecPlan<32>::kSlots;
-    case 64: return SpecPlan<64>::kSlots;
-    case 128: return SpecPlan<128>::kSlots;
-    case 256: return SpecPlan<256>::kSlots;
-    case 512: return SpecPlan<512>::kSlots;
-    case 1024: return SpecPlan<1024>::kSlots;
-    default: return SpecPlan<2048>::kSlots;
-  }
+  DISPATCH_N(N, return SpecPlan<NN>::kSlots);
+  return 0;
 }
 
 template <int N> static void build_tw8(std::vector<double2>& out) { TwBuilder<SpecPlan<N>>::build(out); }
 
 // k_spectra16 (nbin = 2048): one instantiation per (16-bit samples, FFTFIT guess, kept data spectra)
-template <bool I16, bool GUESS, bool KEEPD> static cudaError_t spectra16_attr() {
-  return cudaFuncSetAttribute(k_spectra16<I16, GUESS, KEEPD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              (int)spectra_smem_bytes_of<1024, SpecPlan16>());
-}
+static void (*const kSpectra16[8])(SpectraArgs) = {
+    k_spectra16<false, false, false>, k_spectra16<false, false, true>, k_spectra16<false, true, false>, k_spectra16<false, true, true>,
+    k_spectra16<true, false, false>, k_spectra16<true, false, true>, k_spectra16<true, true, false>, k_spectra16<true, true, true>};
 static cudaError_t spectra16_attrs() {
-  cudaError_t e;
-#define S16_(a, b, c) e = spectra16_attr<a, b, c>(); if (e != cudaSuccess) return e;
-  S16_(false, false, false) S16_(false, false, true) S16_(false, true, false) S16_(false, true, true)
-  S16_(true, false, false) S16_(true, false, true) S16_(true, true, false) S16_(true, true, true)
-#undef S16_
+  for (auto k : kSpectra16) {
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)spectra_smem_bytes_of<1024, SpecPlan16>());
+    if (e != cudaSuccess) return e;
+  }
   return cudaSuccess;
 }
 static void launch_spectra16(bool i16, bool guess, bool keepd, dim3 grid, cudaStream_t st, const SpectraArgs& a) {
-  const size_t sm = spectra_smem_bytes_of<1024, SpecPlan16>();
-#define L16_(A, B, C) k_spectra16<A, B, C><<<grid, 64, sm, st>>>(a)
-  if (!i16) {
-    if (!guess) { if (!keepd) L16_(false, false, false); else L16_(false, false, true); }
-    else { if (!keepd) L16_(false, true, false); else L16_(false, true, true); }
-  } else {
-    if (!guess) { if (!keepd) L16_(true, false, false); else L16_(true, false, true); }
-    else { if (!keepd) L16_(true, true, false); else L16_(true, true, true); }
-  }
-#undef L16_
+  kSpectra16[4 * i16 + 2 * guess + keepd]<<<grid, 64, spectra_smem_bytes_of<1024, SpecPlan16>(), st>>>(a);
 }
 // the generic kernel on the other power-of-two nbin (N = 1024 is launch_spectra16's)
 template <int N> static void launch_spectra(bool i16, dim3 grid, cudaStream_t st, const SpectraArgs& a) {
@@ -303,12 +297,6 @@ template <int M> static cudaError_t any_attrs() {
 #undef A_
   return cudaSuccess;
 }
-struct pp_plan;
-static AnyPlan any_dev(pp_plan* pl);
-static int launch_fwd_any(pp_plan* pl, const void* in, bool i16, const float* scl, const float* offs, long nrows,
-                          cx<double>* spec, double* dc);
-static int launch_inv_any(pp_plan* pl, const cx<double>* spec, const double* dc, void* out, long nrows, bool out_double);
-
 template <int N> static cudaError_t setup_attrs() {
   const int b32 = (int)fft_smem_bytes<N, float>(), b64 = (int)fft_smem_bytes<N, double>();
   cudaError_t e;
@@ -343,7 +331,7 @@ extern "C" int pp_plan_create(int32_t nchan, int32_t nbin, int32_t device, pp_pl
   CK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) return fail(-1, "device %d not available (%d devices)", device, ndev);
   CK(cudaSetDevice(device));
-  pp_plan* pl = new pp_plan();
+  std::unique_ptr<pp_plan> pl(new pp_plan());   // freed with all it holds when a step below fails
   pl->nchan = nchan; pl->nbin = nbin; pl->N = nbin / 2; pl->device = device;
   if (!pow2) {   // any other even nbin: Npad slots per spectrum row, Bluestein transforms of length M (bluestein.cuh)
     pl->anyn = true;
@@ -440,32 +428,14 @@ extern "C" int pp_plan_create(int32_t nchan, int32_t nbin, int32_t device, pp_pl
     CK(pl->tw8.need(t8.size() * sizeof(double2)));
     CK(cudaMemcpy(pl->tw8.p, t8.data(), t8.size() * sizeof(double2), cudaMemcpyHostToDevice));
   }
-  *out = pl;
+  *out = pl.release();
   return 0;
 }
 
 extern "C" void pp_plan_destroy(pp_plan_t* pl) {
   if (!pl) return;
   cudaSetDevice(pl->device);
-  cudaStreamSynchronize(pl->stream);
-  DBuf* all[] = {&pl->any_chirp, &pl->any_B, &pl->any_twM, &pl->any_tw2n, &pl->any_twL, &pl->any_spec, &pl->any_dc, &pl->any_spec2, &pl->any_dc2, &pl->resp, &pl->rot_gm, &pl->rot_nugm, &pl->al_w, &pl->al_out, &pl->al_wsum, &pl->running, &pl->minfo, &pl->njn, &pl->in_scat, &pl->in_scl, &pl->in_offs, &pl->tw8, &pl->twN32, &pl->tw2N32, &pl->twN64, &pl->tw2N64, &pl->freqs, &pl->nu2, &pl->lgf, &pl->gm_params, &pl->gm_taus, &pl->gm_zero, &pl->gm_one, &pl->mconj32, &pl->mconj64, &pl->mpow,
-                 &pl->pn, &pl->mmean, &pl->mmean_sub, &pl->model_stage, &pl->model_stage64, &pl->ps_spec, &pl->ps_mspec, &pl->ps_noise, &pl->rot_in, &pl->rot_out,
-                 &pl->rot_phase, &pl->rot_dm, &pl->rot_P, &pl->rot_nuref,
-                 &pl->in_P, &pl->in_errs, &pl->in_mask, &pl->in_w, &pl->in_init, &pl->in_dmg, &pl->in_snrs, &pl->in_nufits,
-                 &pl->in_nuouts, &pl->in_noise, &pl->in_models, &pl->nu_fit, &pl->nu_mean, &pl->wsum, &pl->nok, &pl->sigma,
-                 &pl->Ssn, &pl->Sdn, &pl->csum, &pl->st_x, &pl->st_xprev, &pl->st_step, &pl->st_fprev, &pl->st_lam,
-                 &pl->st_iter, &pl->st_iterc, &pl->st_done, &pl->o_params, &pl->o_perrs, &pl->o_nuout, &pl->o_cov, &pl->o_chi2, &pl->o_rchi2,
-                 &pl->o_snr, &pl->o_nfev, &pl->o_rc, &pl->o_scales, &pl->o_serrs, &pl->o_csnr, &pl->o_lag, &pl->o_phig,
-                 &pl->ps_phase, &pl->ps_perr, &pl->ps_scale, &pl->ps_serr, &pl->ps_snr, &pl->ps_rchi2, &pl->ps_lag, &pl->Dspec, &pl->Ddc, &pl->al_acc, &pl->al_wparts, &pl->X, &pl->Xlo,
-                 &pl->partial, &pl->data_stage[0], &pl->data_stage[1], &pl->data_stage64[0], &pl->data_stage64[1]};
-  for (DBuf* b : all) b->release();
-  for (auto& gt : pl->grid_tables) gt.second.release();
-  for (cudaEvent_t e : pl->ev_pool) cudaEventDestroy(e);
-  for (cudaEvent_t e : pl->ev_chunk) cudaEventDestroy(e);
-  for (int i = 0; i < 2; ++i) { cudaEventDestroy(pl->ev_copy[i]); cudaEventDestroy(pl->ev_free[i]); }
-  for (int i = 0; i < pp_plan::kPinSlots; ++i) { if (pl->pin_ring[i]) cudaFreeHost(pl->pin_ring[i]); if (pl->pin_ev[i]) cudaEventDestroy(pl->pin_ev[i]); }
-  cudaStreamDestroy(pl->own_stream);
-  cudaStreamDestroy(pl->copy_stream);
+  cudaStreamSynchronize(pl->stream);   // nothing is freed under the plan's queued work
   delete pl;
 }
 
@@ -579,16 +549,10 @@ static int rotate_rows(pp_plan* pl, RotateArgs a, bool fp64) {
   }
   if (fp64) {
     a.twN = pl->twN64.p; a.tw2N = pl->tw2N64.p;
-    DISPATCH_N(N, {
-      const int rows = RowGeom<NN>::kRows;
-      k_rotate<NN, double><<<(unsigned)((nrows + rows - 1) / rows), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a);
-    });
+    DISPATCH_N(N, (k_rotate<NN, double><<<row_ctas<NN>(nrows), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a)));
   } else {
     a.twN = pl->twN32.p; a.tw2N = pl->tw2N32.p;
-    DISPATCH_N(N, {
-      const int rows = RowGeom<NN>::kRows;
-      k_rotate<NN, float><<<(unsigned)((nrows + rows - 1) / rows), 256, fft_smem_bytes<NN, float>(), pl->stream>>>(a);
-    });
+    DISPATCH_N(N, (k_rotate<NN, float><<<row_ctas<NN>(nrows), 256, fft_smem_bytes<NN, float>(), pl->stream>>>(a)));
   }
   pl->stats.launches++;
   return 0;
@@ -682,6 +646,12 @@ extern "C" int pp_plan_set_fft_precision(pp_plan_t* pl, int32_t bits) {
   return 0;
 }
 
+// float64 -> float32 (cvt.rn) of n2 pairs of samples on st
+static void cvt_f64_f32(const void* src, void* dst, size_t n2, cudaStream_t st) {
+  k_cvt_f64_f32<<<(unsigned)std::min<size_t>((n2 + 255) / 256, 148 * 32), 256, 0, st>>>(
+      static_cast<const double2*>(src), static_cast<float2*>(dst), n2);
+}
+
 static int set_model_impl(pp_plan* pl, const float* model, const double* model64, const double* freqs) {
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
@@ -693,9 +663,7 @@ static int set_model_impl(pp_plan* pl, const float* model, const double* model64
     if (stage_in(pl, pl->model_stage64, model64, nsamp, &dmodel64)) return -2;
     if (pl->anyn) {   // the arbitrary-nbin rows take float32 input: round on the device
       CK(pl->model_stage.need(sizeof(float) * nsamp));
-      const size_t n2 = nsamp / 2;
-      k_cvt_f64_f32<<<(unsigned)std::min<size_t>((n2 + 255) / 256, 148 * 32), 256, 0, pl->stream>>>(
-          reinterpret_cast<const double2*>(dmodel64), pl->model_stage.as<float2>(), n2);
+      cvt_f64_f32(dmodel64, pl->model_stage.p, nsamp / 2, pl->stream);
       dmodel = pl->model_stage.as<float>();
       dmodel64 = nullptr;
     }
@@ -715,10 +683,7 @@ static int set_model_impl(pp_plan* pl, const float* model, const double* model64
     if (launch_fwd_any(pl, dmodel, false, nullptr, nullptr, nchan, pl->any_spec2.as<cx<double>>(), nullptr)) return -2;
     k_model_from_spec<<<nchan, 256, 0, pl->stream>>>(pl->any_spec2.as<cx<double>>(), a.mconj32, a.mconj64, a.mpow, a.pn, N);
   } else {
-    DISPATCH_N(N, {
-      const int rows = RowGeom<NN>::kRows;
-      k_model<NN><<<(nchan + rows - 1) / rows, 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a);
-    });
+    DISPATCH_N(N, (k_model<NN><<<row_ctas<NN>(nchan), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a)));
   }
   k_model_mean<<<(N + 127) / 128, 128, 0, pl->stream>>>(pl->mconj64.as<cx<double>>(), pl->mmean.as<float2>(), nchan, N);
   pl->stats.launches += 2;
@@ -741,39 +706,29 @@ extern "C" int pp_set_model_f64(pp_plan_t* pl, const double* model, const double
 // ----------------------------------------------------------------------------
 // fit
 // ----------------------------------------------------------------------------
-static bool is_pinned_host_ptr(const void* p) {
-  cudaPointerAttributes at;
-  cudaError_t e = cudaPointerGetAttributes(&at, p);
-  if (e != cudaSuccess) { cudaGetLastError(); return false; }
-  return at.type == cudaMemoryTypeHost;
+// run(o, m) on elements [o, o + m) of [0, n) from nthreads host threads, in pieces of a multiple of `align` (a power of two)
+template <typename F> static void parallel_pieces(size_t n, size_t align, int nthreads, F run) {
+  std::vector<std::thread> th;
+  const size_t per = ((n / nthreads) + align - 1) & ~(align - 1);
+  for (int i = 1; i < nthreads; ++i) {
+    const size_t o = (size_t)i * per;
+    if (o >= n) break;
+    th.emplace_back([=]() { run(o, std::min(per, n - o)); });
+  }
+  run(0, std::min(per, n));
+  for (auto& t : th) t.join();
 }
 
 static void parallel_memcpy(void* dst, const void* src, size_t n, int nthreads) {
   if (nthreads <= 1 || n < (4u << 20)) { memcpy(dst, src, n); return; }
-  std::vector<std::thread> th;
-  const size_t per = ((n / nthreads) + 4095) & ~(size_t)4095;
-  for (int i = 1; i < nthreads; ++i) {
-    const size_t o = (size_t)i * per;
-    if (o >= n) break;
-    th.emplace_back([=]() { memcpy((char*)dst + o, (const char*)src + o, std::min(per, n - o)); });
-  }
-  memcpy(dst, src, std::min(per, n));
-  for (auto& t : th) t.join();
+  parallel_pieces(n, 4096, nthreads, [=](size_t o, size_t m) { memcpy((char*)dst + o, (const char*)src + o, m); });
 }
 
 // float64 -> float32 (round to nearest even, as the device's cvt.rn.f32.f64) while staging pageable rows
 static void parallel_narrow(float* dst, const double* src, size_t n, int nthreads) {
-  auto run = [](float* d, const double* s, size_t m) { for (size_t i = 0; i < m; ++i) d[i] = (float)s[i]; };
-  if (nthreads <= 1 || n < (1u << 20)) { run(dst, src, n); return; }
-  std::vector<std::thread> th;
-  const size_t per = ((n / nthreads) + 1023) & ~(size_t)1023;
-  for (int i = 1; i < nthreads; ++i) {
-    const size_t o = (size_t)i * per;
-    if (o >= n) break;
-    th.emplace_back([=]() { run(dst + o, src + o, std::min(per, n - o)); });
-  }
-  run(dst, src, std::min(per, n));
-  for (auto& t : th) t.join();
+  auto run = [=](size_t o, size_t m) { for (size_t i = o; i < o + m; ++i) dst[i] = (float)src[i]; };
+  if (nthreads <= 1 || n < (1u << 20)) { run(0, n); return; }
+  parallel_pieces(n, 1024, nthreads, run);
 }
 
 static bool h2d_stages(size_t bytes, bool src_pinned) { return !src_pinned && bytes >= (8u << 20); }
@@ -785,31 +740,11 @@ static cudaError_t h2d_any(pp_plan* pl, void* dst, const void* src, size_t bytes
                            bool narrow) {
   if (!h2d_stages(bytes, src_pinned)) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
   static const int nthreads = std::max(1, std::min(8, (int)std::thread::hardware_concurrency() / 2));
-  if (narrow) {
-    const size_t n = bytes / sizeof(double), per = pp_plan::kPinPiece / sizeof(float);
-    for (size_t off = 0; off < n; off += per) {
-      const size_t len = std::min(per, n - off);
-      const int slot = (int)(pl->pin_count++ % pp_plan::kPinSlots);
-      cudaError_t e;
-      if (!pl->pin_ring[slot]) {
-        e = cudaHostAlloc(&pl->pin_ring[slot], pp_plan::kPinPiece, cudaHostAllocDefault);
-        if (e != cudaSuccess) return e;
-        e = cudaEventCreateWithFlags(&pl->pin_ev[slot], cudaEventDisableTiming);
-        if (e != cudaSuccess) return e;
-      } else {
-        e = cudaEventSynchronize(pl->pin_ev[slot]);
-        if (e != cudaSuccess) return e;
-      }
-      parallel_narrow(static_cast<float*>(pl->pin_ring[slot]), static_cast<const double*>(src) + off, len, nthreads);
-      e = cudaMemcpyAsync(static_cast<float*>(dst) + off, pl->pin_ring[slot], len * sizeof(float), cudaMemcpyHostToDevice, st);
-      if (e != cudaSuccess) return e;
-      e = cudaEventRecord(pl->pin_ev[slot], st);
-      if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
-  }
-  for (size_t off = 0; off < bytes; off += pp_plan::kPinPiece) {
-    const size_t len = std::min(pp_plan::kPinPiece, bytes - off);
+  // pieces of kPinPiece bytes as they are sent: counted in source elements (float64 when narrowing, else bytes)
+  const size_t src_size = narrow ? sizeof(double) : 1, dst_size = narrow ? sizeof(float) : 1;
+  const size_t n = bytes / src_size, per = pp_plan::kPinPiece / dst_size;
+  for (size_t off = 0; off < n; off += per) {
+    const size_t len = std::min(per, n - off);
     const int slot = (int)(pl->pin_count++ % pp_plan::kPinSlots);
     cudaError_t e;
     if (!pl->pin_ring[slot]) {
@@ -821,8 +756,9 @@ static cudaError_t h2d_any(pp_plan* pl, void* dst, const void* src, size_t bytes
       e = cudaEventSynchronize(pl->pin_ev[slot]);      // the copy that last used this slot has left it
       if (e != cudaSuccess) return e;
     }
-    parallel_memcpy(pl->pin_ring[slot], (const char*)src + off, len, nthreads);
-    e = cudaMemcpyAsync((char*)dst + off, pl->pin_ring[slot], len, cudaMemcpyHostToDevice, st);
+    if (narrow) parallel_narrow(static_cast<float*>(pl->pin_ring[slot]), static_cast<const double*>(src) + off, len, nthreads);
+    else parallel_memcpy(pl->pin_ring[slot], (const char*)src + off, len, nthreads);
+    e = cudaMemcpyAsync((char*)dst + off * dst_size, pl->pin_ring[slot], len * dst_size, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) return e;
     e = cudaEventRecord(pl->pin_ev[slot], st);
     if (e != cudaSuccess) return e;
@@ -855,11 +791,10 @@ constexpr int kSpectraGMax = 32;   // most channel rows per spectra CTA
 // nbin 2048 has one row slot per CTA, so its G never exceeds kSpectraGMax: k_spectra16 takes every such launch
 static_assert(SpecPlan<1024>::kSlots == 1 && kSpectraGMax <= kSpec16MaxRows, "nbin 2048: G <= kSpec16MaxRows");
 
-static int rows_per_cta(pp_plan* pl, int chunk) {
+static int rows_per_cta(pp_plan* pl) {
   // Channel rows handled by one k_spectra CTA.  It fixes how the partial profile spectra of
   // the FFTFIT guess are grouped, so it must NOT depend on the batch or chunk size (results
   // are bit-identical for any chunking): a function of nchan only, ~16 CTAs per subint.
-  (void)chunk;
   const int rows_conc = spectra_slots(pl->N);
   int g = std::max(rows_conc, std::min(kSpectraGMax, pl->nchan / (512 / kSpectraGMax)));
   g = ((g + rows_conc - 1) / rows_conc) * rows_conc;
@@ -867,67 +802,62 @@ static int rows_per_cta(pp_plan* pl, int chunk) {
   return g;
 }
 
-extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_fit_out_t* out) {
-  if (!pl || !args || !out) return fail(-1, "NULL argument");
-  if (!pl->model_set) return fail(-1, "pp_set_model must be called before pp_fit_batch");
-  if (!args->data || !args->P) return fail(-1, "data and P are required");
-  const bool i16 = args->data_type == PP_DATA_I16, f64 = args->data_type == PP_DATA_F64;
-  if (args->data_type != PP_DATA_F32 && !i16 && !f64) return fail(-1, "unknown data_type %d", args->data_type);
-  if (i16 && (!args->dat_scl || !args->dat_offs)) return fail(-1, "int16 data need dat_scl and dat_offs");
-  if (args->nsub < 1) return fail(-1, "nsub must be >= 1");
-  const uint8_t* ff = args->fit_flags;
-  if (!ff[0] && !ff[1] && !ff[2] && !ff[3] && !ff[4]) return fail(-1, "nothing to fit");
-  // The (phi, DM) kernels apply when GM, tau, alpha are neither fit nor non-zero.
-  bool general = ff[2] || ff[3] || ff[4] || args->log10_tau;
-  if (!general && args->init) {
-    if (is_device_ptr(args->init)) general = true;   // cannot inspect cheaply: take the general path
-    else
-      for (int i = 0; i < args->nsub && !general; ++i)
-        if (args->init[(size_t)i * 5 + 2] != 0.0 || args->init[(size_t)i * 5 + 3] != 0.0) general = true;
-  }
-  if (!general && args->scat_guess) general = true;
-  if (general && args->semantics == PP_SEM_FIT_PORTRAIT)
-    return fail(-1, "PP_SEM_FIT_PORTRAIT is defined for the (phi, DM) fit only");
-  CK(cudaSetDevice(pl->device));
-  stats_begin(pl);
-  // PP_TRACE=1: host-side wall-clock marks of the call on stderr (where a step's time goes outside the kernels)
-  static const bool trace = getenv("PP_TRACE") != nullptr;
-  const auto tr0 = std::chrono::steady_clock::now();
-  auto mark = [&](const char* what) {
-    if (trace) fprintf(stderr, "[pp_fit_batch] %-22s %8.3f ms\n", what,
-                       std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tr0).count());
-  };
-  const int nsub = args->nsub, nchan = pl->nchan, N = pl->N;
-  const int Ns = args->Ns > 0 ? args->Ns : 100;
-  if (Ns < 2) return fail(-1, "Ns must be >= 2");
-  // passes are launched only while some subint is still running (polled), so a generous limit costs
-  // nothing for batches started from the FFTFIT guess (1-2 passes) and lets caller-supplied start
-  // values far from the optimum converge (10-14 passes from 0.05-0.08 turn away, tools/far_start_probe.py)
-  const int dflt_iter = 40;
-  const int max_iter = args->max_iter > 0 ? args->max_iter : (args->max_iter < 0 ? -1 : dflt_iter);
-  const int n_launch_iter = max_iter < 0 ? 1 : (general ? max_iter + 1 : max_iter);
-
-  // (phi, DM): the epilogue applies the last Newton step through a second-order Taylor update of
-  // the per-channel sums, so stopping at 1e-2 sigma leaves < 2e-5 sigma (measured, tools/gpu_tol.py);
-  // the general solver re-evaluates at the final point instead and keeps 1e-3.
-  const double tol = args->tol > 0 ? args->tol : (general ? 1e-3 : 1e-2);
-  const size_t nsc = (size_t)nsub * nchan;
-
-  // ---- stage small inputs ------------------------------------------------------
+// One pp_fit_batch call: the validated flags, the staged inputs, the chunk geometry and the kernel arguments.  The
+// pass and update arguments are built once per call: each chunk sets s0, the coarse stage its own fields.
+struct FitCall {
+  const pp_fit_args_t* args;
+  const pp_fit_out_t* out;
+  std::chrono::steady_clock::time_point tr0;
+  bool general, want_guess, want_align, i16, f64, data_on_device, data_pinned;
+  int nsub, Ns, max_iter, n_launch_iter;
+  double tol;
+  // device copies of the inputs (or the caller's device pointers)
   const double *dP, *derrs, *dw, *dinit, *ddmg, *dsnrs, *dnufits, *dnuouts, *dscat;
   const uint8_t* dmask;
-  if (stage_in(pl, pl->in_P, args->P, (size_t)nsub, &dP)) return -2;
-  if (stage_in(pl, pl->in_errs, args->errs, nsc, &derrs)) return -2;
-  if (stage_in(pl, pl->in_mask, args->chan_mask, nsc, &dmask)) return -2;
-  if (stage_in(pl, pl->in_w, args->weights, nsc, &dw)) return -2;
-  if (stage_in(pl, pl->in_init, args->init, (size_t)nsub * 5, &dinit)) return -2;
-  if (stage_in(pl, pl->in_dmg, args->DM_guess, (size_t)nsub, &ddmg)) return -2;
-  if (stage_in(pl, pl->in_snrs, args->snrs, nsc, &dsnrs)) return -2;
-  if (stage_in(pl, pl->in_nufits, args->nu_fits, (size_t)nsub * 3, &dnufits)) return -2;
-  if (stage_in(pl, pl->in_nuouts, args->nu_outs, (size_t)nsub * 3, &dnuouts)) return -2;
-  if (stage_in(pl, pl->in_scat, args->scat_guess, (size_t)nsub * 2, &dscat)) return -2;
-  const bool want_guess = (args->init == nullptr);
+  const float *dscl = nullptr, *doffs = nullptr;
+  const double2* table = nullptr;   // FFTFIT grid
+  const char* data;                 // the caller's rows
+  size_t sub_bytes, src_bytes;      // one subint as the kernels read it, and as the caller stores it
+  int chunk, G, gx, nparts, align_nsplit = 1;
+  std::vector<int> cstart;          // chunk c is subints cstart[c] .. cstart[c + 1] - 1
+  SolverState st;
   Box box;
+  PassArgs pa; UpdateArgs ua; Pass5Args p5; Update5Args u5;
+  // chunk loop
+  int coarse_nj = 0;                // harmonic groups of this chunk's coarse objective (0: no coarse stage)
+  int pending_out = -1;             // chunk whose result copies still have to be queued
+  bool expect_third = false;        // the previous chunk still had unfinished subints after two passes
+};
+
+// PP_TRACE=1: host-side wall-clock marks of the call on stderr (where a step's time goes outside the kernels)
+static void mark(const FitCall& f, const char* fmt, ...) {
+  static const bool trace = getenv("PP_TRACE") != nullptr;
+  if (!trace) return;
+  char what[128];
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(what, sizeof what, fmt, ap);
+  va_end(ap);
+  fprintf(stderr, "[pp_fit_batch] %-22s %8.3f ms\n", what,
+          std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - f.tr0).count());
+}
+
+static int fit_stage_inputs(pp_plan* pl, FitCall& f) {
+  const pp_fit_args_t* args = f.args;
+  const int nsub = f.nsub;
+  const size_t nsc = (size_t)nsub * pl->nchan;
+  if (stage_in(pl, pl->in_P, args->P, (size_t)nsub, &f.dP)) return -2;
+  if (stage_in(pl, pl->in_errs, args->errs, nsc, &f.derrs)) return -2;
+  if (stage_in(pl, pl->in_mask, args->chan_mask, nsc, &f.dmask)) return -2;
+  if (stage_in(pl, pl->in_w, args->weights, nsc, &f.dw)) return -2;
+  if (stage_in(pl, pl->in_init, args->init, (size_t)nsub * 5, &f.dinit)) return -2;
+  if (stage_in(pl, pl->in_dmg, args->DM_guess, (size_t)nsub, &f.ddmg)) return -2;
+  if (stage_in(pl, pl->in_snrs, args->snrs, nsc, &f.dsnrs)) return -2;
+  if (stage_in(pl, pl->in_nufits, args->nu_fits, (size_t)nsub * 3, &f.dnufits)) return -2;
+  if (stage_in(pl, pl->in_nuouts, args->nu_outs, (size_t)nsub * 3, &f.dnuouts)) return -2;
+  if (stage_in(pl, pl->in_scat, args->scat_guess, (size_t)nsub * 2, &f.dscat)) return -2;
+  f.want_guess = (args->init == nullptr);
+  Box& box = f.box;
   box.on = 0;
   for (int i = 0; i < 5; ++i) { box.lo[i] = -INFINITY; box.hi[i] = INFINITY; }
   if (args->bounds) {
@@ -939,8 +869,14 @@ extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_f
       if (box.lo[i] > box.hi[i]) return fail(-1, "bounds[%d]: lower %g > upper %g", i, lo, hi);
     }
   }
+  return 0;
+}
 
-  // ---- workspace -------------------------------------------------------------------
+// per-subint and per-channel workspace; chunk size, spectra grid, the chunk-sized buffers and the chunk boundaries
+static int fit_workspace(pp_plan* pl, FitCall& f) {
+  const pp_fit_args_t* args = f.args;
+  const int nsub = f.nsub, nchan = pl->nchan, N = pl->N;
+  const size_t nsc = (size_t)nsub * nchan;
   CK(pl->nu_fit.need(sizeof(double) * nsub * 3));
   CK(pl->nu_mean.need(sizeof(double) * nsub));
   CK(pl->wsum.need(sizeof(double) * nsub));
@@ -972,360 +908,463 @@ extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_f
   CK(pl->o_lag.need(sizeof(int) * nsub));
   CK(pl->o_phig.need(sizeof(double) * nsub));
   CK(pl->running.need(sizeof(int)));
+  mark(f, "inputs staged");
 
-  mark("inputs staged");
-  const int chunk = pick_chunk(pl, nsub, !is_device_ptr(args->data), f64 ? 8.0 : 4.0);
-  const int G = rows_per_cta(pl, chunk);
-  const int rows_conc = spectra_slots(N);
-  const int gx = (nchan + G - 1) / G;
-  const int nparts = gx * rows_conc;
+  const MemKind data_kind = mem_kind(args->data);
+  f.data_on_device = data_kind == kMemDevice;
+  f.data_pinned = data_kind == kMemPinned;
+  const int chunk = f.chunk = pick_chunk(pl, nsub, !f.data_on_device, f.f64 ? 8.0 : 4.0);
+  f.G = rows_per_cta(pl);
+  f.gx = (nchan + f.G - 1) / f.G;
+  f.nparts = f.gx * spectra_slots(N);
   pl->stats.chunk = chunk;
   CK(pl->X.need(sizeof(float2) * (size_t)chunk * nchan * N));
   // fused ppalign accumulation (ppalign.py:197-213): keep the data spectra of the chunk
-  const bool want_align = out->align_sum != nullptr;
-  int align_nsplit = 1;
-  if (want_align) {
-    if (!out->align_wsum) return fail(-1, "align_sum needs align_wsum");
+  f.want_align = f.out->align_sum != nullptr;
+  if (f.want_align) {
+    if (!f.out->align_wsum) return fail(-1, "align_sum needs align_wsum");
     CK(pl->Dspec.need(sizeof(float2) * (size_t)chunk * nchan * N));
     CK(pl->Ddc.need(sizeof(double) * (size_t)chunk * nchan));
     // partial sums per k_align_spec grid slice (each slice is owned by one CTA: no atomics, so the
     // result is reproducible); the slice count depends on nchan only
-    align_nsplit = std::max(1, (8 * 148 * 8) / std::max(1, nchan));   // ~8 CTAs per SM
-    CK(pl->al_acc.need(sizeof(double2) * (size_t)align_nsplit * nchan * N));
-    CK(pl->al_wparts.need(sizeof(double) * (size_t)align_nsplit * nchan));
+    const int nsplit = f.align_nsplit = std::max(1, (8 * 148 * 8) / std::max(1, nchan));   // ~8 CTAs per SM
+    CK(pl->al_acc.need(sizeof(double2) * (size_t)nsplit * nchan * N));
+    CK(pl->al_wparts.need(sizeof(double) * (size_t)nsplit * nchan));
     CK(pl->al_wsum.need(sizeof(double) * nchan));
     CK(pl->al_out.need(sizeof(double) * (size_t)nchan * pl->nbin));
-    CK(cudaMemsetAsync(pl->al_acc.p, 0, sizeof(double2) * (size_t)align_nsplit * nchan * N, pl->stream));
-    CK(cudaMemsetAsync(pl->al_wparts.p, 0, sizeof(double) * (size_t)align_nsplit * nchan, pl->stream));
+    CK(cudaMemsetAsync(pl->al_acc.p, 0, sizeof(double2) * (size_t)nsplit * nchan * N, pl->stream));
+    CK(cudaMemsetAsync(pl->al_wparts.p, 0, sizeof(double) * (size_t)nsplit * nchan, pl->stream));
   }
   CK(pl->Xlo.need(sizeof(float2) * (size_t)chunk * nchan * std::min(N, 64)));
-  if (want_guess) CK(pl->partial.need(sizeof(float2) * (size_t)chunk * nparts * N));
-  const bool data_on_device = is_device_ptr(args->data);
-  const bool data_pinned = !data_on_device && is_pinned_host_ptr(args->data);
-  if (data_on_device && !pl->anyn && (reinterpret_cast<uintptr_t>(args->data) & 15))
+  if (f.want_guess) CK(pl->partial.need(sizeof(float2) * (size_t)chunk * f.nparts * N));
+  if (f.data_on_device && !pl->anyn && (reinterpret_cast<uintptr_t>(args->data) & 15))
     return fail(-1, "device data pointer must be 16-byte aligned");
-  const size_t sub_bytes = (size_t)nchan * pl->nbin * (i16 ? sizeof(int16_t) : sizeof(float));   // one subint as the kernels read it
-  const size_t src_bytes = f64 ? (size_t)nchan * pl->nbin * sizeof(double) : sub_bytes;           // ... and as the caller stores it
-  const char* data_bytes = reinterpret_cast<const char*>(args->data);
-  if (!data_on_device || f64)
-    for (int i = 0; i < 2; ++i) CK(pl->data_stage[i].need((size_t)chunk * sub_bytes));
-  if (f64 && !data_on_device)
-    for (int i = 0; i < 2; ++i) CK(pl->data_stage64[i].need((size_t)chunk * src_bytes));
-  auto convert_f64 = [&](const void* src, void* dst, int ns, cudaStream_t st) {   // float64 rows -> float32 rows
-    const size_t n2 = (size_t)ns * nchan * (pl->nbin / 2);
-    k_cvt_f64_f32<<<(unsigned)std::min<size_t>((n2 + 255) / 256, 148 * 32), 256, 0, st>>>(
-        static_cast<const double2*>(src), static_cast<float2*>(dst), n2);
-    pl->stats.launches++;
-  };
-  const float *dscl = nullptr, *doffs = nullptr;
-  if (i16) {
-    if (stage_in(pl, pl->in_scl, args->dat_scl, (size_t)nsub * nchan, &dscl)) return -2;
-    if (stage_in(pl, pl->in_offs, args->dat_offs, (size_t)nsub * nchan, &doffs)) return -2;
+  f.sub_bytes = (size_t)nchan * pl->nbin * (f.i16 ? sizeof(int16_t) : sizeof(float));
+  f.src_bytes = f.f64 ? (size_t)nchan * pl->nbin * sizeof(double) : f.sub_bytes;
+  f.data = reinterpret_cast<const char*>(args->data);
+  if (!f.data_on_device || f.f64)
+    for (int i = 0; i < 2; ++i) CK(pl->data_stage[i].need((size_t)chunk * f.sub_bytes));
+  if (f.f64 && !f.data_on_device)
+    for (int i = 0; i < 2; ++i) CK(pl->data_stage64[i].need((size_t)chunk * f.src_bytes));
+  if (f.i16) {
+    if (stage_in(pl, pl->in_scl, args->dat_scl, (size_t)nsub * nchan, &f.dscl)) return -2;
+    if (stage_in(pl, pl->in_offs, args->dat_offs, (size_t)nsub * nchan, &f.doffs)) return -2;
   }
+  // chunk boundaries; with several chunks the last one is kept short (<= 256 subints) because its
+  // result copy is the only one that cannot hide under a following chunk's kernels
+  for (int s0 = 0; s0 < nsub; s0 += chunk) f.cstart.push_back(s0);
+  if (f.cstart.size() >= 2) {
+    const int tail = 256, last0 = f.cstart.back();
+    if (nsub - last0 > tail) f.cstart.push_back(nsub - tail);
+  }
+  f.cstart.push_back(nsub);
+  return 0;
+}
 
-  SolverState st;
+// the solver state and the pass / update kernel arguments of the call (s0 is set per chunk)
+static void fit_kernel_args(pp_plan* pl, FitCall& f) {
+  const pp_fit_args_t* args = f.args;
+  const uint8_t* ff = args->fit_flags;
+  const int nchan = pl->nchan, N = pl->N;
+  SolverState& st = f.st;
   st.x = pl->st_x.as<double>(); st.xprev = pl->st_xprev.as<double>(); st.step = pl->st_step.as<double>();
   st.fprev = pl->st_fprev.as<double>(); st.lam = pl->st_lam.as<double>(); st.iter = pl->st_iter.as<int>(); st.iterc = pl->st_iterc.as<int>();
   st.done = pl->st_done.as<int>();
+  PassArgs& pa = f.pa;
+  pa.X = pl->X.as<float2>(); pa.Xlo = pl->Xlo.as<float2>(); pa.nu2 = pl->nu2.as<double>(); pa.P = f.dP; pa.nu_fit = pl->nu_fit.as<double>();
+  pa.Ssn = pl->Ssn.as<double>(); pa.sigma = pl->sigma.as<double>(); pa.csum = pl->csum.as<double>(); pa.st = st;
+  pa.s0 = 0; pa.nchan = nchan; pa.N = N; pa.nhalf = pl->anyn ? pl->L : 0; pa.njn = pl->njn.as<int>();
+  UpdateArgs& ua = f.ua;
+  memset(&ua, 0, sizeof ua);
+  ua.csum = pl->csum.as<double>(); ua.Ssn = pl->Ssn.as<double>(); ua.Sdn = pl->Sdn.as<double>(); ua.nu2 = pl->nu2.as<double>();
+  ua.freqs = pl->freqs.as<double>(); ua.P = f.dP; ua.nu_fit = pl->nu_fit.as<double>(); ua.nu_outs = f.dnuouts;
+  ua.nok = pl->nok.as<int>(); ua.st = st;
+  ua.params = pl->o_params.as<double>(); ua.param_errs = pl->o_perrs.as<double>(); ua.nu_out = pl->o_nuout.as<double>();
+  ua.cov = pl->o_cov.as<double>(); ua.chi2 = pl->o_chi2.as<double>(); ua.red_chi2 = pl->o_rchi2.as<double>();
+  ua.snr = pl->o_snr.as<double>(); ua.nfeval = pl->o_nfev.as<int>(); ua.rc = pl->o_rc.as<int>();
+  ua.scales = pl->o_scales.as<double>(); ua.scale_errs = pl->o_serrs.as<double>(); ua.channel_snrs = pl->o_csnr.as<double>();
+  ua.s0 = 0; ua.nchan = nchan; ua.nbin = pl->nbin; ua.max_iter = f.max_iter; ua.semantics = args->semantics;
+  ua.fit_phi = ff[0] ? 1 : 0; ua.fit_dm = ff[1] ? 1 : 0; ua.is_toa = args->is_toa; ua.tol = f.tol; ua.box = f.box;
+  ua.model_steps = pl->model_steps; ua.tol_model = (args->tol > 0 && args->tol < 1e-4) ? args->tol : 1e-4;
+  if (!f.general) return;
+  Pass5Args& p5 = f.p5;
+  p5.X = pl->X.as<float2>(); p5.Xlo = pl->Xlo.as<float2>(); p5.mpow = pl->mpow.as<double>(); p5.nu2 = pl->nu2.as<double>(); p5.lgf = pl->lgf.as<double>();
+  p5.freqs = pl->freqs.as<double>(); p5.P = f.dP; p5.nu_fit = pl->nu_fit.as<double>(); p5.Ssn = pl->Ssn.as<double>();
+  p5.sigma = pl->sigma.as<double>(); p5.csum = pl->csum.as<double>(); p5.st = st; p5.s0 = 0; p5.nchan = nchan;
+  p5.log10_tau = args->log10_tau; p5.nhalf = pl->anyn ? pl->L : 0; p5.nj = N / 16; p5.cstride = 1; p5.njn = pl->njn.as<int>();
+  Update5Args& u5 = f.u5;
+  memset(&u5, 0, sizeof u5);
+  u5.csum = pl->csum.as<double>(); u5.Sdn = pl->Sdn.as<double>(); u5.nu2 = pl->nu2.as<double>(); u5.lgf = pl->lgf.as<double>();
+  u5.freqs = pl->freqs.as<double>(); u5.P = f.dP; u5.nu_fit = pl->nu_fit.as<double>(); u5.nu_outs = f.dnuouts;
+  u5.nok = pl->nok.as<int>(); u5.st = st;
+  u5.params = ua.params; u5.param_errs = ua.param_errs; u5.nu_out = ua.nu_out; u5.cov = ua.cov; u5.chi2 = ua.chi2;
+  u5.red_chi2 = ua.red_chi2; u5.snr = ua.snr; u5.nfeval = ua.nfeval; u5.rc = ua.rc; u5.scales = ua.scales;
+  u5.scale_errs = ua.scale_errs; u5.channel_snrs = ua.channel_snrs;
+  u5.s0 = 0; u5.nchan = nchan; u5.nbin = pl->nbin; u5.max_iter = f.max_iter; u5.log10_tau = args->log10_tau;
+  u5.option = args->option; u5.is_toa = args->is_toa; u5.tol = f.tol; u5.box = f.box;
+  u5.taylor_finish = pl->model_steps != 1;
+  for (int i = 0; i < 5; ++i) u5.flags[i] = ff[i] ? 1 : 0;
+  u5.coarse = 0; u5.ctol = 0.0; u5.cstride = 1;
+}
 
-  cudaEvent_t ev_t0 = nullptr;
-  if (pl->timing) { ev_t0 = get_event(pl); CK(cudaEventRecord(ev_t0, pl->stream)); }
-
-  // ---- per-subint scalars ----------------------------------------------------------
-  {
-    PrepArgs p;
-    p.freqs = pl->freqs.as<double>(); p.mask = dmask; p.weights = dw; p.snrs = dsnrs; p.nu_fits_in = dnufits;
-    p.nu_fit = pl->nu_fit.as<double>(); p.nu_mean = pl->nu_mean.as<double>(); p.wsum = pl->wsum.as<double>();
-    p.nok = pl->nok.as<int>(); p.nsub = nsub; p.nchan = nchan; p.nu_fit_mode = args->nu_fit_mode;
-    k_prep<<<(nsub + 3) / 4, 128, 0, pl->stream>>>(p);
-    pl->stats.launches++;
-  }
-  if (!want_guess) {
-    k_init_state<<<(nsub + 127) / 128, 128, 0, pl->stream>>>(st, dinit, 0, nsub);
-    if (box.on) k_clamp_state<<<(nsub + 127) / 128, 128, 0, pl->stream>>>(st, box, 0, nsub);
+// per-subint scalars, the start state of fits from caller-supplied values, the FFTFIT grid
+static int fit_prep(pp_plan* pl, FitCall& f) {
+  const int nsub = f.nsub;
+  PrepArgs p;
+  p.freqs = pl->freqs.as<double>(); p.mask = f.dmask; p.weights = f.dw; p.snrs = f.dsnrs; p.nu_fits_in = f.dnufits;
+  p.nu_fit = pl->nu_fit.as<double>(); p.nu_mean = pl->nu_mean.as<double>(); p.wsum = pl->wsum.as<double>();
+  p.nok = pl->nok.as<int>(); p.nsub = nsub; p.nchan = pl->nchan; p.nu_fit_mode = f.args->nu_fit_mode;
+  k_prep<<<(nsub + 3) / 4, 128, 0, pl->stream>>>(p);
+  pl->stats.launches++;
+  if (!f.want_guess) {
+    k_init_state<<<(nsub + 127) / 128, 128, 0, pl->stream>>>(f.st, f.dinit, 0, nsub);
+    if (f.box.on) k_clamp_state<<<(nsub + 127) / 128, 128, 0, pl->stream>>>(f.st, f.box, 0, nsub);
     pl->stats.launches++;
     CK(cudaMemsetAsync(pl->o_lag.p, 0xff, sizeof(int) * nsub, pl->stream));
   }
-  const double2* table = nullptr;
-  if (want_guess && grid_table(pl, Ns, &table)) return -2;
+  if (f.want_guess && grid_table(pl, f.Ns, &f.table)) return -2;
+  return 0;
+}
 
-  // when the data live on the host: the first chunk's copy starts right away
-  // chunk boundaries; with several chunks the last one is kept short (<= 256 subints) because its
-  // result copy is the only one that cannot hide under a following chunk's kernels
-  std::vector<int> cstart;
-  for (int s0 = 0; s0 < nsub; s0 += chunk) cstart.push_back(s0);
-  if (cstart.size() >= 2) {
-    const int tail = 256, last0 = cstart.back();
-    if (nsub - last0 > tail) cstart.push_back(nsub - tail);
+// host data: chunk c's rows into staging buffer c & 1 on the copy stream, once the kernels that read it last are done
+static cudaError_t issue_copy(pp_plan* pl, const FitCall& f, int c) {
+  const int b = c & 1;
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0;
+  cudaError_t e = cudaStreamWaitEvent(pl->copy_stream, pl->ev_free[b], 0);
+  if (e != cudaSuccess) return e;
+  // float64 rows from pageable memory are rounded to float32 by the host threads that stage them anyway (half
+  // the bytes over PCIe); from page-locked memory they cross as they are and a kernel on the copy stream rounds
+  const bool narrow = f.f64 && h2d_stages((size_t)ns * f.src_bytes, f.data_pinned);
+  void* dst = (f.f64 && !narrow) ? pl->data_stage64[b].p : pl->data_stage[b].p;
+  e = h2d_any(pl, dst, f.data + (size_t)s0 * f.src_bytes, (size_t)ns * f.src_bytes, f.data_pinned, pl->copy_stream, narrow);
+  if (e != cudaSuccess) return e;
+  if (f.f64 && !narrow) {
+    cvt_f64_f32(dst, pl->data_stage[b].p, (size_t)ns * pl->nchan * (pl->nbin / 2), pl->copy_stream);
+    pl->stats.launches++;
   }
-  cstart.push_back(nsub);
-  const int nchunks = (int)cstart.size() - 1;
-  auto issue_copy = [&](int c) -> cudaError_t {
-    const int b = c & 1;
-    const int s0 = cstart[c], ns = cstart[c + 1] - s0;
-    cudaError_t e = cudaStreamWaitEvent(pl->copy_stream, pl->ev_free[b], 0);
-    if (e != cudaSuccess) return e;
-    // float64 rows from pageable memory are rounded to float32 by the host threads that stage them anyway (half
-    // the bytes over PCIe); from page-locked memory they cross as they are and a kernel on the copy stream rounds
-    const bool narrow = f64 && h2d_stages((size_t)ns * src_bytes, data_pinned);
-    void* dst = (f64 && !narrow) ? pl->data_stage64[b].p : pl->data_stage[b].p;
-    e = h2d_any(pl, dst, data_bytes + (size_t)s0 * src_bytes, (size_t)ns * src_bytes, data_pinned, pl->copy_stream, narrow);
-    if (e != cudaSuccess) return e;
-    if (f64 && !narrow) convert_f64(dst, pl->data_stage[b].p, ns, pl->copy_stream);
-    return cudaEventRecord(pl->ev_copy[b], pl->copy_stream);
-  };
-  if (!data_on_device) {
-    // the staging buffers are free at the start
-    CK(cudaEventRecord(pl->ev_free[0], pl->stream));
-    CK(cudaEventRecord(pl->ev_free[1], pl->stream));
-    CK(issue_copy(0));
+  return cudaEventRecord(pl->ev_copy[b], pl->copy_stream);
+}
+
+// chunk c's spectra from the caller's device rows or from the staging buffer the copy stream fills (the next chunk's
+// copy is issued first)
+static int fit_spectra(pp_plan* pl, const FitCall& f, int c) {
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan, N = pl->N, nchunks = (int)f.cstart.size() - 1;
+  const char* dchunk = f.data;
+  if (f.data_on_device && f.f64) {   // round the chunk to float32 next to the kernels that read it
+    cvt_f64_f32(f.data + (size_t)s0 * f.src_bytes, pl->data_stage[c & 1].p, (size_t)ns * pl->nchan * (pl->nbin / 2), pl->stream);
+    pl->stats.launches++;
   }
+  if (!f.data_on_device) {
+    if (c + 1 < nchunks) CK(issue_copy(pl, f, c + 1));
+    CK(cudaStreamWaitEvent(pl->stream, pl->ev_copy[c & 1], 0));
+  }
+  // kernels index data with the global subint number: bias the base pointer of the staged chunk
+  if (!f.data_on_device || f.f64) dchunk = pl->data_stage[c & 1].as<char>() - (size_t)s0 * f.sub_bytes;
+  SpanGuard g(pl, SP_SPECTRA);
+  SpectraArgs a;
+  a.data = dchunk; a.dat_scl = f.dscl; a.dat_offs = f.doffs;
+  a.mconj64 = pl->mconj64.as<cx<double>>(); a.mconj32 = pl->mconj32.as<cx<float>>();
+  a.pn = pl->pn.as<double>(); a.nu2 = pl->nu2.as<double>();
+  a.errs = f.derrs; a.mask = f.dmask; a.weights = f.dw; a.P = f.dP; a.DMg = f.ddmg; a.nu_mean = pl->nu_mean.as<double>();
+  a.X = pl->X.as<float2>(); a.Xlo = pl->Xlo.as<float2>(); a.partial = f.want_guess ? pl->partial.as<float2>() : nullptr;
+  a.D = f.want_align ? pl->Dspec.as<float2>() : nullptr; a.Ddc = f.want_align ? pl->Ddc.as<double>() : nullptr;
+  a.sigma = pl->sigma.as<double>(); a.Ssn = pl->Ssn.as<double>(); a.Sdn = pl->Sdn.as<double>();
+  a.tw8 = pl->tw8.as<cx<double>>();
+  a.s0 = s0; a.nchan = nchan; a.G = f.G; a.nparts = f.nparts;
+  a.dspec = nullptr; a.ddc = nullptr; a.nhalf = 0; a.kc_true = 0; a.njn = pl->njn.as<int>();
+  if (pl->anyn) {   // rows transformed by Bluestein into the spectrum scratch, then the same emit code
+    if (c == 0) {
+      CK(pl->any_spec.need(sizeof(double2) * (size_t)f.chunk * nchan * N));
+      CK(pl->any_dc.need(sizeof(double) * (size_t)f.chunk * nchan));
+    }
+    if (launch_fwd_any(pl, dchunk + (size_t)s0 * f.sub_bytes, f.i16, f.i16 ? f.dscl + (size_t)s0 * nchan : nullptr,
+                       f.i16 ? f.doffs + (size_t)s0 * nchan : nullptr, (long)ns * nchan, pl->any_spec.as<cx<double>>(),
+                       pl->any_dc.as<double>())) return -2;
+    a.dspec = pl->any_spec.as<cx<double>>(); a.ddc = pl->any_dc.as<double>();
+    a.nhalf = pl->L; a.kc_true = (3 * (pl->L + 1)) / 4;
+    DISPATCH_N(N, (k_spectra<NN, SpecPlan<NN>, false, true><<<dim3(f.gx, ns), SpecPlan<NN>::kThreads, 0, pl->stream>>>(a)));
+  } else if (N == 1024) {
+    launch_spectra16(f.i16, f.want_guess, f.want_align, dim3(f.gx, ns), pl->stream, a);
+  } else {
+    DISPATCH_N(N, launch_spectra<NN>(f.i16, dim3(f.gx, ns), pl->stream, a));
+  }
+  pl->stats.launches++;
+  return 0;
+}
 
-  // queue the device-to-host copies of chunk c's results on the copy stream
-  auto enqueue_results = [&](int c) -> int {
-    const int s0 = cstart[c], ns = cstart[c + 1] - s0;
-    CK(cudaStreamWaitEvent(pl->copy_stream, pl->ev_chunk[c], 0));
-    cudaStream_t cs = pl->copy_stream;
-    const size_t o1 = (size_t)s0, n1 = (size_t)ns, oc = (size_t)s0 * nchan, ncn = (size_t)ns * nchan;
-    if (copy_out_at(cs, out->params, pl->o_params.as<double>(), o1 * 5, n1 * 5)) return -2;
-    if (copy_out_at(cs, out->param_errs, pl->o_perrs.as<double>(), o1 * 5, n1 * 5)) return -2;
-    if (copy_out_at(cs, out->nu_out, pl->o_nuout.as<double>(), o1 * 3, n1 * 3)) return -2;
-    if (copy_out_at(cs, out->cov, pl->o_cov.as<double>(), o1 * 25, n1 * 25)) return -2;
-    if (copy_out_at(cs, out->chi2, pl->o_chi2.as<double>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->red_chi2, pl->o_rchi2.as<double>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->snr, pl->o_snr.as<double>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->nfeval, pl->o_nfev.as<int>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->return_code, pl->o_rc.as<int>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->scales, pl->o_scales.as<double>(), oc, ncn)) return -2;
-    if (copy_out_at(cs, out->scale_errs, pl->o_serrs.as<double>(), oc, ncn)) return -2;
-    if (copy_out_at(cs, out->channel_snrs, pl->o_csnr.as<double>(), oc, ncn)) return -2;
-    if (copy_out_at(cs, out->noise, pl->sigma.as<double>(), oc, ncn)) return -2;
-    if (copy_out_at(cs, out->lag_index, pl->o_lag.as<int>(), o1, n1)) return -2;
-    if (want_guess && copy_out_at(cs, out->phi_guess, pl->o_phig.as<double>(), o1, n1)) return -2;
-    if (copy_out_at(cs, out->chan_sums, pl->csum.as<double>(), oc * kNCsum, ncn * kNCsum)) return -2;
-    return 0;
-  };
-  int pending_out = -1;        // chunk whose result copies still have to be queued
-  bool expect_third = false;   // the previous chunk still had unfinished subints after two passes
+static int fit_guess(pp_plan* pl, const FitCall& f, int c) {
+  if (!f.want_guess) return 0;
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, N = pl->N;
+  SpanGuard g(pl, SP_GUESS);
+  GuessArgs ga;
+  memset(&ga, 0, sizeof ga);
+  ga.partial = pl->partial.as<float2>(); ga.mconj = pl->mmean.as<float2>(); ga.nparts = f.nparts; ga.nmodel = 1;
+  if (f.dmask) {   // the guess template is the mean model over the subint's usable channels (pptoas.py:446, 454)
+    CK(pl->mmean_sub.need(sizeof(float2) * (size_t)f.chunk * N));
+    k_model_mean_masked<<<dim3((N + 127) / 128, ns), 128, 0, pl->stream>>>(
+        pl->mconj64.as<cx<double>>(), f.dmask, pl->mmean.as<float2>(), pl->mmean_sub.as<float2>(), s0, pl->nchan, N);
+    pl->stats.launches++;
+    ga.mconj = pl->mmean_sub.as<float2>();
+    ga.nmodel = ns;  // one template per subint of the chunk
+  }
+  ga.N = N; ga.Ns = f.Ns; ga.wsum = pl->wsum.as<double>(); ga.noise = nullptr; ga.table = f.table; ga.s0 = s0;
+  ga.nhalf = pl->anyn ? pl->L : 0;
+  ga.nused = pl->kmax_used;   // the mean model has no power beyond the largest channel cut-off
+  ga.phase = pl->o_phig.as<double>(); ga.lag = pl->o_lag.as<int>();
+  ga.x = f.st.x; ga.DMg = f.ddmg; ga.P = f.dP; ga.nu_mean = pl->nu_mean.as<double>(); ga.nu_fit = pl->nu_fit.as<double>();
+  ga.polish_tol = 1e-6;   // a start value (the last step is still applied): the Newton solver refines it
+  ga.init = nullptr; ga.scat = f.dscat; ga.log10_tau = f.args->log10_tau; ga.fit_scat = f.args->fit_flags[3] ? 1 : 0;
+  k_guess<<<ns, 256, sizeof(double2) * N, pl->stream>>>(ga);
+  k_reset_state<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, s0, ns);
+  pl->stats.launches += 2;
+  if (f.box.on) { k_clamp_state<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, f.box, s0, ns); pl->stats.launches++; }
+  return 0;
+}
 
-  mark("before chunk loop");
-  for (int c = 0; c < nchunks; ++c) {
-    const int s0 = cstart[c], ns = cstart[c + 1] - s0;
-    if (trace) { char b[64]; snprintf(b, sizeof b, "chunk %d (%d subints)", c, ns); mark(b); }
-    const char* dchunk;
-    if (data_on_device && f64) {   // round the chunk to float32 next to the kernels that read it
-      convert_f64(data_bytes + (size_t)s0 * src_bytes, pl->data_stage[c & 1].p, ns, pl->stream);
-      dchunk = pl->data_stage[c & 1].as<char>() - (size_t)s0 * sub_bytes;
-    } else if (data_on_device) dchunk = data_bytes;
-    else {
-      if (c + 1 < nchunks) CK(issue_copy(c + 1));
-      CK(cudaStreamWaitEvent(pl->stream, pl->ev_copy[c & 1], 0));
-      // kernels index data with the global subint number: bias the base pointer
-      dchunk = pl->data_stage[c & 1].as<char>() - (size_t)s0 * sub_bytes;
-    }
-    {
-      SpanGuard g(pl, SP_SPECTRA);
-      SpectraArgs a;
-      a.data = dchunk; a.dat_scl = dscl; a.dat_offs = doffs;
-      a.mconj64 = pl->mconj64.as<cx<double>>(); a.mconj32 = pl->mconj32.as<cx<float>>();
-      a.pn = pl->pn.as<double>(); a.nu2 = pl->nu2.as<double>();
-      a.errs = derrs; a.mask = dmask; a.weights = dw; a.P = dP; a.DMg = ddmg; a.nu_mean = pl->nu_mean.as<double>();
-      a.X = pl->X.as<float2>(); a.Xlo = pl->Xlo.as<float2>(); a.partial = want_guess ? pl->partial.as<float2>() : nullptr;
-      a.D = want_align ? pl->Dspec.as<float2>() : nullptr; a.Ddc = want_align ? pl->Ddc.as<double>() : nullptr;
-      a.sigma = pl->sigma.as<double>(); a.Ssn = pl->Ssn.as<double>(); a.Sdn = pl->Sdn.as<double>();
-      a.tw8 = pl->tw8.as<cx<double>>();
-      a.s0 = s0; a.nchan = nchan; a.G = G; a.nparts = nparts;
-      a.dspec = nullptr; a.ddc = nullptr; a.nhalf = 0; a.kc_true = 0; a.njn = pl->njn.as<int>();
-      if (pl->anyn) {   // rows transformed by Bluestein into the spectrum scratch, then the same emit code
-        if (c == 0) {
-          CK(pl->any_spec.need(sizeof(double2) * (size_t)chunk * nchan * N));
-          CK(pl->any_dc.need(sizeof(double) * (size_t)chunk * nchan));
-        }
-        if (launch_fwd_any(pl, dchunk + (size_t)s0 * sub_bytes, i16, i16 ? dscl + (size_t)s0 * nchan : nullptr,
-                           i16 ? doffs + (size_t)s0 * nchan : nullptr, (long)ns * nchan, pl->any_spec.as<cx<double>>(),
-                           pl->any_dc.as<double>())) return -2;
-        a.dspec = pl->any_spec.as<cx<double>>(); a.ddc = pl->any_dc.as<double>();
-        a.nhalf = pl->L; a.kc_true = (3 * (pl->L + 1)) / 4;
-        DISPATCH_N(N, (k_spectra<NN, SpecPlan<NN>, false, true><<<dim3(gx, ns), SpecPlan<NN>::kThreads, 0, pl->stream>>>(a)));
-      } else if (N == 1024) {
-        launch_spectra16(i16, want_guess, want_align, dim3(gx, ns), pl->stream, a);
-      } else {
-        DISPATCH_N(N, launch_spectra<NN>(i16, dim3(gx, ns), pl->stream, a));
-      }
-      pl->stats.launches++;
-    }
-    if (!data_on_device) CK(cudaEventRecord(pl->ev_free[c & 1], pl->stream));
-    if (want_guess) {
-      SpanGuard g(pl, SP_GUESS);
-      GuessArgs ga;
-      memset(&ga, 0, sizeof ga);
-      ga.partial = pl->partial.as<float2>(); ga.mconj = pl->mmean.as<float2>(); ga.nparts = nparts; ga.nmodel = 1;
-      if (dmask) {   // the guess template is the mean model over the subint's usable channels (pptoas.py:446, 454)
-        CK(pl->mmean_sub.need(sizeof(float2) * (size_t)chunk * N));
-        k_model_mean_masked<<<dim3((N + 127) / 128, ns), 128, 0, pl->stream>>>(
-            pl->mconj64.as<cx<double>>(), dmask, pl->mmean.as<float2>(), pl->mmean_sub.as<float2>(), s0, nchan, N);
-        pl->stats.launches++;
-        ga.mconj = pl->mmean_sub.as<float2>();
-        ga.nmodel = ns;  // one template per subint of the chunk
-      }
-      ga.N = N; ga.Ns = Ns; ga.wsum = pl->wsum.as<double>(); ga.noise = nullptr; ga.table = table; ga.s0 = s0;
-      ga.nhalf = pl->anyn ? pl->L : 0;
-      ga.nused = pl->kmax_used;   // the mean model has no power beyond the largest channel cut-off
-      ga.phase = pl->o_phig.as<double>(); ga.lag = pl->o_lag.as<int>();
-      ga.x = st.x; ga.DMg = ddmg; ga.P = dP; ga.nu_mean = pl->nu_mean.as<double>(); ga.nu_fit = pl->nu_fit.as<double>();
-      ga.polish_tol = 1e-6;   // a start value (the last step is still applied): the Newton solver refines it
-      ga.init = nullptr; ga.scat = dscat; ga.log10_tau = args->log10_tau; ga.fit_scat = ff[3] ? 1 : 0;
-      k_guess<<<ns, 256, sizeof(double2) * N, pl->stream>>>(ga);
-      k_reset_state<<<(ns + 127) / 128, 128, 0, pl->stream>>>(st, s0, ns);
-      pl->stats.launches += 2;
-      if (box.on) { k_clamp_state<<<(ns + 127) / 128, 128, 0, pl->stream>>>(st, box, s0, ns); pl->stats.launches++; }
-    }
-    PassArgs pa;
-    pa.X = pl->X.as<float2>(); pa.Xlo = pl->Xlo.as<float2>(); pa.nu2 = pl->nu2.as<double>(); pa.P = dP; pa.nu_fit = pl->nu_fit.as<double>();
-    pa.Ssn = pl->Ssn.as<double>(); pa.sigma = pl->sigma.as<double>(); pa.csum = pl->csum.as<double>(); pa.st = st;
-    pa.s0 = s0; pa.nchan = nchan; pa.N = N; pa.nhalf = pl->anyn ? pl->L : 0; pa.njn = pl->njn.as<int>();
-    UpdateArgs ua;
-    memset(&ua, 0, sizeof ua);
-    ua.csum = pl->csum.as<double>(); ua.Ssn = pl->Ssn.as<double>(); ua.Sdn = pl->Sdn.as<double>(); ua.nu2 = pl->nu2.as<double>();
-    ua.freqs = pl->freqs.as<double>(); ua.P = dP; ua.nu_fit = pl->nu_fit.as<double>(); ua.nu_outs = dnuouts;
-    ua.nok = pl->nok.as<int>(); ua.st = st;
-    ua.params = pl->o_params.as<double>(); ua.param_errs = pl->o_perrs.as<double>(); ua.nu_out = pl->o_nuout.as<double>();
-    ua.cov = pl->o_cov.as<double>(); ua.chi2 = pl->o_chi2.as<double>(); ua.red_chi2 = pl->o_rchi2.as<double>();
-    ua.snr = pl->o_snr.as<double>(); ua.nfeval = pl->o_nfev.as<int>(); ua.rc = pl->o_rc.as<int>();
-    ua.scales = pl->o_scales.as<double>(); ua.scale_errs = pl->o_serrs.as<double>(); ua.channel_snrs = pl->o_csnr.as<double>();
-    ua.s0 = s0; ua.nchan = nchan; ua.nbin = pl->nbin; ua.max_iter = max_iter; ua.semantics = args->semantics;
-    ua.fit_phi = ff[0] ? 1 : 0; ua.fit_dm = ff[1] ? 1 : 0; ua.is_toa = args->is_toa; ua.tol = tol; ua.box = box;
-    ua.model_steps = pl->model_steps; ua.tol_model = (args->tol > 0 && args->tol < 1e-4) ? args->tol : 1e-4;
-    Pass5Args p5;
-    Update5Args u5;
-    if (general) {
-      p5.X = pl->X.as<float2>(); p5.Xlo = pl->Xlo.as<float2>(); p5.mpow = pl->mpow.as<double>(); p5.nu2 = pl->nu2.as<double>(); p5.lgf = pl->lgf.as<double>();
-      p5.freqs = pl->freqs.as<double>(); p5.P = dP; p5.nu_fit = pl->nu_fit.as<double>(); p5.Ssn = pl->Ssn.as<double>();
-      p5.sigma = pl->sigma.as<double>(); p5.csum = pl->csum.as<double>(); p5.st = st; p5.s0 = s0; p5.nchan = nchan;
-      p5.log10_tau = args->log10_tau; p5.nhalf = pl->anyn ? pl->L : 0; p5.nj = N / 16; p5.cstride = 1; p5.njn = pl->njn.as<int>();
-      memset(&u5, 0, sizeof u5);
-      u5.csum = pl->csum.as<double>(); u5.Sdn = pl->Sdn.as<double>(); u5.nu2 = pl->nu2.as<double>(); u5.lgf = pl->lgf.as<double>();
-      u5.freqs = pl->freqs.as<double>(); u5.P = dP; u5.nu_fit = pl->nu_fit.as<double>(); u5.nu_outs = dnuouts;
-      u5.nok = pl->nok.as<int>(); u5.st = st;
-      u5.params = ua.params; u5.param_errs = ua.param_errs; u5.nu_out = ua.nu_out; u5.cov = ua.cov; u5.chi2 = ua.chi2;
-      u5.red_chi2 = ua.red_chi2; u5.snr = ua.snr; u5.nfeval = ua.nfeval; u5.rc = ua.rc; u5.scales = ua.scales;
-      u5.scale_errs = ua.scale_errs; u5.channel_snrs = ua.channel_snrs;
-      u5.s0 = s0; u5.nchan = nchan; u5.nbin = pl->nbin; u5.max_iter = max_iter; u5.log10_tau = args->log10_tau;
-      u5.option = args->option; u5.is_toa = args->is_toa; u5.tol = tol; u5.box = box;
-      u5.taylor_finish = pl->model_steps != 1;
-      for (int i = 0; i < 5; ++i) u5.flags[i] = ff[i] ? 1 : 0;
-      u5.coarse = 0; u5.ctol = 0.0; u5.cstride = 1;
-    }
-    auto launch_update5 = [&]() {   // many channels: more threads per subint for the per-channel chain rule
-      if (nchan >= 1024) k_update5<256><<<ns, 256, 0, pl->stream>>>(u5);
-      else k_update5<128><<<ns, 128, 0, pl->stream>>>(u5);
-    };
-    // Coarse stage of the general solver: Newton iterations on the objective of the low harmonics only (those
-    // that hold coarse_frac of the model's phase information: a fraction of a pass each) carry the start values
-    // to within a fraction of a sigma of the optimum; the full-resolution iterations below then need two passes.
-    int coarse_nj = 0;
-    if (general && max_iter > 0 && pl->coarse_frac > 0.0 && pl->model_steps != 1 && N >= 128) {
-      // where the information sits, with the scattering of the chunk's first subint at its start values
-      const bool scat = ff[3] || ff[4] || dscat || dinit;
-      CK(pl->minfo.need(sizeof(double) * (N / 16)));
-      pl->model_info.assign(N / 16, 0.0);
-      k_model_info<<<N / 16, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->lgf.as<double>(), scat ? st.x + (size_t)s0 * 5 : nullptr,
-                                                   pl->nu_fit.as<double>() + (size_t)s0 * 3, args->log10_tau,
-                                                   pl->minfo.as<double>(), nchan, N);
-      pl->stats.launches++;
-      CK(cudaMemcpyAsync(pl->model_info.data(), pl->minfo.p, sizeof(double) * (N / 16), cudaMemcpyDeviceToHost, pl->stream));
-      CK(cudaStreamSynchronize(pl->stream));
-      coarse_nj = choose_coarse(pl->model_info, pl->coarse_frac, N);
-    }
-    if (coarse_nj > 0) {
-      // Two levels: most of the iterations run on a cheaper objective still -- the harmonics that hold coarse_frac0
-      // of the information (when that is clearly fewer) of every cstride-th channel -- the second level then needs
-      // one or two.  A level is left once its Newton step is below ctol sigma (the step is still taken): the next
-      // level, or the full-resolution iterations, start next to that level's optimum either way.
-      struct { int nj, cstride; double ctol; } levels[2];
-      int nlev = 0;
+static void launch_update5(pp_plan* pl, const FitCall& f, int ns) {   // many channels: more threads per subint for the per-channel chain rule
+  if (pl->nchan >= 1024) k_update5<256><<<ns, 256, 0, pl->stream>>>(f.u5);
+  else k_update5<128><<<ns, 128, 0, pl->stream>>>(f.u5);
+}
+
+// the count of the chunk's subints that `count` finds still running, read back on the host
+static int poll_running(pp_plan* pl, void (*count)(SolverState, int, int, int*), const FitCall& f, int s0, int ns,
+                        int* running) {
+  count<<<1, 256, 0, pl->stream>>>(f.st, s0, ns, pl->running.as<int>());
+  pl->stats.launches++;
+  *running = 0;
+  CK(cudaMemcpyAsync(running, pl->running.p, sizeof(int), cudaMemcpyDeviceToHost, pl->stream));
+  CK(cudaStreamSynchronize(pl->stream));
+  return 0;
+}
+
+// Coarse stage of the general solver: Newton iterations on the objective of the low harmonics only (those
+// that hold coarse_frac of the model's phase information: a fraction of a pass each) carry the start values
+// to within a fraction of a sigma of the optimum; the full-resolution iterations then need two passes.
+static int fit_coarse(pp_plan* pl, FitCall& f, int c) {
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan, N = pl->N;
+  const pp_fit_args_t* args = f.args;
+  f.coarse_nj = 0;
+  if (!(f.general && f.max_iter > 0 && pl->coarse_frac > 0.0 && pl->model_steps != 1 && N >= 128)) return 0;
+  // where the information sits, with the scattering of the chunk's first subint at its start values
+  const uint8_t* ff = args->fit_flags;
+  const bool scat = ff[3] || ff[4] || f.dscat || f.dinit;
+  CK(pl->minfo.need(sizeof(double) * (N / 16)));
+  pl->model_info.assign(N / 16, 0.0);
+  k_model_info<<<N / 16, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->lgf.as<double>(), scat ? f.st.x + (size_t)s0 * 5 : nullptr,
+                                               pl->nu_fit.as<double>() + (size_t)s0 * 3, args->log10_tau,
+                                               pl->minfo.as<double>(), nchan, N);
+  pl->stats.launches++;
+  CK(cudaMemcpyAsync(pl->model_info.data(), pl->minfo.p, sizeof(double) * (N / 16), cudaMemcpyDeviceToHost, pl->stream));
+  CK(cudaStreamSynchronize(pl->stream));
+  const int coarse_nj = f.coarse_nj = choose_coarse(pl->model_info, pl->coarse_frac, N);
+  if (coarse_nj == 0) return 0;
+  // Two levels: most of the iterations run on a cheaper objective still -- the harmonics that hold coarse_frac0
+  // of the information (when that is clearly fewer) of every cstride-th channel -- the second level then needs
+  // one or two.  A level is left once its Newton step is below ctol sigma (the step is still taken): the next
+  // level, or the full-resolution iterations, start next to that level's optimum either way.
+  struct { int nj, cstride; double ctol; } levels[2];
+  int nlev = 0;
+  {
+    int nj0 = choose_coarse(pl->model_info, std::min(0.65, pl->coarse_frac), N);
+    if (!(nj0 > 0 && 3 * nj0 <= 2 * coarse_nj)) nj0 = coarse_nj;
+    const int cst = nchan >= 2048 ? 8 : (nchan >= 512 ? 4 : (nchan >= 128 ? 2 : 1));
+    if (nj0 < coarse_nj || cst > 1) levels[nlev++] = {nj0, cst, 2.0};
+    levels[nlev++] = {coarse_nj, 1, 1.0};
+  }
+  Pass5Args& p5 = f.p5;
+  Update5Args& u5 = f.u5;
+  u5.coarse = 1;
+  for (int lv = 0; lv < nlev; ++lv) {
+    const int max_coarse = std::min(f.max_iter, 12);
+    p5.nj = levels[lv].nj; p5.cstride = u5.cstride = levels[lv].cstride; u5.ctol = levels[lv].ctol;
+    const int gx5 = ((nchan + p5.cstride - 1) / p5.cstride + 31) / 32;
+    mark(f, "coarse level: %d of %d harmonic groups, every %d-th channel", p5.nj, N / 16, p5.cstride);
+    for (int it = 0; it < max_coarse; ++it) {
       {
-        int nj0 = choose_coarse(pl->model_info, std::min(0.65, pl->coarse_frac), N);
-        if (!(nj0 > 0 && 3 * nj0 <= 2 * coarse_nj)) nj0 = coarse_nj;
-        const int cst = nchan >= 2048 ? 8 : (nchan >= 512 ? 4 : (nchan >= 128 ? 2 : 1));
-        if (nj0 < coarse_nj || cst > 1) levels[nlev++] = {nj0, cst, 2.0};
-        levels[nlev++] = {coarse_nj, 1, 1.0};
-      }
-      u5.coarse = 1;
-      for (int lv = 0; lv < nlev; ++lv) {
-        const int max_coarse = std::min(max_iter, 12);
-        p5.nj = levels[lv].nj; p5.cstride = u5.cstride = levels[lv].cstride; u5.ctol = levels[lv].ctol;
-        const int gx5 = ((nchan + p5.cstride - 1) / p5.cstride + 31) / 32;
-        if (trace) { char b[96]; snprintf(b, sizeof b, "coarse level: %d of %d harmonic groups, every %d-th channel", p5.nj, N / 16, p5.cstride); mark(b); }
-        for (int it = 0; it < max_coarse; ++it) {
-          {
-            SpanGuard g(pl, SP_COARSE);
-            DISPATCH_N(N, k_pass5<NN><<<dim3(gx5, ns), 256, Pass5Ring<NN>::kBytes, pl->stream>>>(p5));
-            launch_update5();
-          }
-          pl->stats.launches += 2;
-          pl->stats.coarse_launches++;
-          // the first level starts far from its optimum (three iterations before asking), the second next to it
-          if (it >= (lv == 0 ? 2 : 0) && it + 1 < max_coarse) {
-            k_count_coarse<<<1, 256, 0, pl->stream>>>(st, s0, ns, pl->running.as<int>());
-            pl->stats.launches++;
-            int running = 0;
-            CK(cudaMemcpyAsync(&running, pl->running.p, sizeof(int), cudaMemcpyDeviceToHost, pl->stream));
-            CK(cudaStreamSynchronize(pl->stream));
-            if (running == 0) break;
-          }
-        }
-        k_coarse_end<<<(ns + 127) / 128, 128, 0, pl->stream>>>(st, s0, ns);
-        pl->stats.launches++;
-      }
-      p5.nj = N / 16; p5.cstride = u5.cstride = 1; u5.coarse = 0;
-    }
-    for (int it = 0; it < n_launch_iter; ++it) {
-      {
-        SpanGuard g(pl, SP_PASS);
-        if (general) { DISPATCH_N(N, k_pass5<NN><<<dim3((nchan + 31) / 32, ns), 256, Pass5Ring<NN>::kBytes, pl->stream>>>(p5)); }
-        else { DISPATCH_N(N, k_pass2<NN><<<dim3((nchan + 31) / 32, ns), 256, Pass2Ring<NN>::kBytes, pl->stream>>>(pa)); }
-      }
-      {
-        SpanGuard g(pl, SP_UPDATE);
-        if (general) launch_update5();
-        else k_update2<<<ns, 128, 0, pl->stream>>>(ua);
+        SpanGuard g(pl, SP_COARSE);
+        DISPATCH_N(N, k_pass5<NN><<<dim3(gx5, ns), 256, Pass5Ring<NN>::kBytes, pl->stream>>>(p5));
+        launch_update5(pl, f, ns);
       }
       pl->stats.launches += 2;
-      pl->stats.pass_launches++;
-      // data-dependent number of passes: poll the count of unfinished subints (an empty
-      // launch of the full grid costs ~80 us, the poll ~20 us)
-      // (when the previous chunk needed a third pass this one most likely does too: launch it
-      // without asking first)
-      const bool poll = general ? (it >= (coarse_nj > 0 ? 1 : 3)) : (it >= 2 || (it == 1 && !expect_third));
-      if (it == 1 && pending_out >= 0) {   // this chunk's first passes are queued: now the old copies
-        if (enqueue_results(pending_out)) return -2;
-        pending_out = -1;
-      }
-      if (poll && it + 1 < n_launch_iter) {
-        k_count_running<<<1, 256, 0, pl->stream>>>(st, s0, ns, pl->running.as<int>());
-        pl->stats.launches++;
-        int running = 0;
-        CK(cudaMemcpyAsync(&running, pl->running.p, sizeof(int), cudaMemcpyDeviceToHost, pl->stream));
-        CK(cudaStreamSynchronize(pl->stream));
-        if (!general && it == 1) expect_third = running > 0;
-        if (!general && it == 2 && running == 0) expect_third = true;   // needed exactly three
+      pl->stats.coarse_launches++;
+      // the first level starts far from its optimum (three iterations before asking), the second next to it
+      if (it >= (lv == 0 ? 2 : 0) && it + 1 < max_coarse) {
+        int running;
+        if (poll_running(pl, k_count_coarse, f, s0, ns, &running)) return -2;
         if (running == 0) break;
       }
     }
-    if (pending_out >= 0) {   // (single-pass calls never reach it == 1)
-      if (enqueue_results(pending_out)) return -2;
-      pending_out = -1;
+    k_coarse_end<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, s0, ns);
+    pl->stats.launches++;
+  }
+  // (k_update5 reads ctol only in the coarse stage)
+  p5.nj = N / 16; p5.cstride = u5.cstride = 1; u5.coarse = 0; u5.ctol = 0.0;
+  return 0;
+}
+
+// queue the device-to-host copies of the results of chunk f.pending_out (if any) on the copy stream
+static int enqueue_results(pp_plan* pl, FitCall& f) {
+  const int c = f.pending_out;
+  if (c < 0) return 0;
+  f.pending_out = -1;
+  const pp_fit_out_t* out = f.out;
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan;
+  CK(cudaStreamWaitEvent(pl->copy_stream, pl->ev_chunk[c], 0));
+  cudaStream_t cs = pl->copy_stream;
+  const size_t o1 = (size_t)s0, n1 = (size_t)ns, oc = (size_t)s0 * nchan, ncn = (size_t)ns * nchan;
+  if (copy_out_at(cs, out->params, pl->o_params.as<double>(), o1 * 5, n1 * 5)) return -2;
+  if (copy_out_at(cs, out->param_errs, pl->o_perrs.as<double>(), o1 * 5, n1 * 5)) return -2;
+  if (copy_out_at(cs, out->nu_out, pl->o_nuout.as<double>(), o1 * 3, n1 * 3)) return -2;
+  if (copy_out_at(cs, out->cov, pl->o_cov.as<double>(), o1 * 25, n1 * 25)) return -2;
+  if (copy_out_at(cs, out->chi2, pl->o_chi2.as<double>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->red_chi2, pl->o_rchi2.as<double>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->snr, pl->o_snr.as<double>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->nfeval, pl->o_nfev.as<int>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->return_code, pl->o_rc.as<int>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->scales, pl->o_scales.as<double>(), oc, ncn)) return -2;
+  if (copy_out_at(cs, out->scale_errs, pl->o_serrs.as<double>(), oc, ncn)) return -2;
+  if (copy_out_at(cs, out->channel_snrs, pl->o_csnr.as<double>(), oc, ncn)) return -2;
+  if (copy_out_at(cs, out->noise, pl->sigma.as<double>(), oc, ncn)) return -2;
+  if (copy_out_at(cs, out->lag_index, pl->o_lag.as<int>(), o1, n1)) return -2;
+  if (f.want_guess && copy_out_at(cs, out->phi_guess, pl->o_phig.as<double>(), o1, n1)) return -2;
+  if (copy_out_at(cs, out->chan_sums, pl->csum.as<double>(), oc * kNCsum, ncn * kNCsum)) return -2;
+  return 0;
+}
+
+// the full-resolution passes of chunk c, launched while some subint is still running (polled)
+static int fit_passes(pp_plan* pl, FitCall& f, int c) {
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan, N = pl->N;
+  for (int it = 0; it < f.n_launch_iter; ++it) {
+    {
+      SpanGuard g(pl, SP_PASS);
+      if (f.general) { DISPATCH_N(N, k_pass5<NN><<<dim3((nchan + 31) / 32, ns), 256, Pass5Ring<NN>::kBytes, pl->stream>>>(f.p5)); }
+      else { DISPATCH_N(N, k_pass2<NN><<<dim3((nchan + 31) / 32, ns), 256, Pass2Ring<NN>::kBytes, pl->stream>>>(f.pa)); }
     }
-    if (want_align) {   // sum_s w_sn rotate(d_sn) with the fitted phi, DM of this chunk (ppalign.py:197-208)
-      AlignSpecArgs aa;
-      aa.D = pl->Dspec.as<float2>(); aa.Ddc = pl->Ddc.as<double>(); aa.params = pl->o_params.as<double>();
-      aa.nu_out = pl->o_nuout.as<double>(); aa.P = dP; aa.scales = pl->o_scales.as<double>(); aa.sigma = pl->sigma.as<double>();
-      aa.rc = pl->o_rc.as<int>(); aa.nu2 = pl->nu2.as<double>(); aa.acc = pl->al_acc.as<double2>();
-      aa.wsum = pl->al_wparts.as<double>(); aa.s0 = s0; aa.ns = ns; aa.nchan = nchan;
-      DISPATCH_N(N, k_align_spec<NN><<<dim3(nchan, align_nsplit), NN / 8, 0, pl->stream>>>(aa));
-      pl->stats.launches++;
+    {
+      SpanGuard g(pl, SP_UPDATE);
+      if (f.general) launch_update5(pl, f, ns);
+      else k_update2<<<ns, 128, 0, pl->stream>>>(f.ua);
     }
+    pl->stats.launches += 2;
+    pl->stats.pass_launches++;
+    // data-dependent number of passes: poll the count of unfinished subints (an empty
+    // launch of the full grid costs ~80 us, the poll ~20 us)
+    // (when the previous chunk needed a third pass this one most likely does too: launch it
+    // without asking first)
+    const bool poll = f.general ? (it >= (f.coarse_nj > 0 ? 1 : 3)) : (it >= 2 || (it == 1 && !f.expect_third));
+    // this chunk's first passes are queued: now the previous chunk's copies
+    if (it == 1 && enqueue_results(pl, f)) return -2;
+    if (poll && it + 1 < f.n_launch_iter) {
+      int running;
+      if (poll_running(pl, k_count_running, f, s0, ns, &running)) return -2;
+      if (!f.general && it == 1) f.expect_third = running > 0;
+      if (!f.general && it == 2 && running == 0) f.expect_third = true;   // needed exactly three
+      if (running == 0) break;
+    }
+  }
+  return enqueue_results(pl, f);   // (single-pass calls never reach it == 1)
+}
+
+// sum_s w_sn rotate(d_sn) with the fitted phi, DM of chunk c (ppalign.py:197-208)
+static int fit_align_chunk(pp_plan* pl, const FitCall& f, int c) {
+  if (!f.want_align) return 0;
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan;
+  AlignSpecArgs aa;
+  aa.D = pl->Dspec.as<float2>(); aa.Ddc = pl->Ddc.as<double>(); aa.params = pl->o_params.as<double>();
+  aa.nu_out = pl->o_nuout.as<double>(); aa.P = f.dP; aa.scales = pl->o_scales.as<double>(); aa.sigma = pl->sigma.as<double>();
+  aa.rc = pl->o_rc.as<int>(); aa.nu2 = pl->nu2.as<double>(); aa.acc = pl->al_acc.as<double2>();
+  aa.wsum = pl->al_wparts.as<double>(); aa.s0 = s0; aa.ns = ns; aa.nchan = nchan;
+  DISPATCH_N(pl->N, k_align_spec<NN><<<dim3(nchan, f.align_nsplit), NN / 8, 0, pl->stream>>>(aa));
+  pl->stats.launches++;
+  return 0;
+}
+
+// the aligned portrait from the chunks' partial sums, and its copies to the caller
+static int fit_align_finish(pp_plan* pl, const FitCall& f) {
+  if (!f.want_align) return 0;
+  const int nchan = pl->nchan, N = pl->N;
+  AlignFinishArgs fa;
+  fa.acc = pl->al_acc.as<double2>(); fa.wsum_parts = pl->al_wparts.as<double>(); fa.aligned = pl->al_out.as<double>();
+  fa.wsum = pl->al_wsum.as<double>(); fa.twN = pl->twN64.p; fa.tw2N = pl->tw2N64.p;
+  fa.nchan = nchan; fa.nsplit = f.align_nsplit;
+  if (pl->anyn) {
+    CK(pl->any_spec2.need(sizeof(double2) * (size_t)nchan * N));
+    CK(pl->any_dc2.need(sizeof(double) * (size_t)nchan));
+    k_align_reduce_any<<<nchan, 256, 0, pl->stream>>>(fa.acc, fa.wsum_parts, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(),
+                                                      fa.wsum, nchan, N, f.align_nsplit);
+    if (launch_inv_any(pl, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), fa.aligned, nchan, true)) return -2;
+  } else {
+    DISPATCH_N(N, (k_align_finish<NN><<<row_ctas<NN>(nchan), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(fa)));
+  }
+  pl->stats.launches++;
+  if (copy_out_at(pl->stream, f.out->align_sum, pl->al_out.as<double>(), 0, (size_t)nchan * pl->nbin)) return -2;
+  if (copy_out_at(pl->stream, f.out->align_wsum, pl->al_wsum.as<double>(), 0, (size_t)nchan)) return -2;
+  return 0;
+}
+
+extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_fit_out_t* out) {
+  if (!pl || !args || !out) return fail(-1, "NULL argument");
+  if (!pl->model_set) return fail(-1, "pp_set_model must be called before pp_fit_batch");
+  if (!args->data || !args->P) return fail(-1, "data and P are required");
+  const bool i16 = args->data_type == PP_DATA_I16, f64 = args->data_type == PP_DATA_F64;
+  if (args->data_type != PP_DATA_F32 && !i16 && !f64) return fail(-1, "unknown data_type %d", args->data_type);
+  if (i16 && (!args->dat_scl || !args->dat_offs)) return fail(-1, "int16 data need dat_scl and dat_offs");
+  if (args->nsub < 1) return fail(-1, "nsub must be >= 1");
+  const uint8_t* ff = args->fit_flags;
+  if (!ff[0] && !ff[1] && !ff[2] && !ff[3] && !ff[4]) return fail(-1, "nothing to fit");
+  // The (phi, DM) kernels apply when GM, tau, alpha are neither fit nor non-zero.
+  bool general = ff[2] || ff[3] || ff[4] || args->log10_tau;
+  if (!general && args->init) {
+    if (is_device_ptr(args->init)) general = true;   // cannot inspect cheaply: take the general path
+    else
+      for (int i = 0; i < args->nsub && !general; ++i)
+        if (args->init[(size_t)i * 5 + 2] != 0.0 || args->init[(size_t)i * 5 + 3] != 0.0) general = true;
+  }
+  if (!general && args->scat_guess) general = true;
+  if (general && args->semantics == PP_SEM_FIT_PORTRAIT)
+    return fail(-1, "PP_SEM_FIT_PORTRAIT is defined for the (phi, DM) fit only");
+  CK(cudaSetDevice(pl->device));
+  stats_begin(pl);
+  FitCall f;
+  f.tr0 = std::chrono::steady_clock::now();
+  f.args = args; f.out = out; f.general = general; f.i16 = i16; f.f64 = f64; f.nsub = args->nsub;
+  f.Ns = args->Ns > 0 ? args->Ns : 100;
+  if (f.Ns < 2) return fail(-1, "Ns must be >= 2");
+  // passes are launched only while some subint is still running (polled), so a generous limit costs
+  // nothing for batches started from the FFTFIT guess (1-2 passes) and lets caller-supplied start
+  // values far from the optimum converge (10-14 passes from 0.05-0.08 turn away, tools/far_start_probe.py)
+  const int dflt_iter = 40;
+  f.max_iter = args->max_iter > 0 ? args->max_iter : (args->max_iter < 0 ? -1 : dflt_iter);
+  f.n_launch_iter = f.max_iter < 0 ? 1 : (general ? f.max_iter + 1 : f.max_iter);
+  // (phi, DM): the epilogue applies the last Newton step through a second-order Taylor update of
+  // the per-channel sums, so stopping at 1e-2 sigma leaves < 2e-5 sigma (measured, tools/gpu_tol.py);
+  // the general solver re-evaluates at the final point instead and keeps 1e-3.
+  f.tol = args->tol > 0 ? args->tol : (general ? 1e-3 : 1e-2);
+
+  if (int rc = fit_stage_inputs(pl, f)) return rc;
+  if (int rc = fit_workspace(pl, f)) return rc;
+  fit_kernel_args(pl, f);
+  cudaEvent_t ev_t0 = nullptr;
+  if (pl->timing) { ev_t0 = get_event(pl); CK(cudaEventRecord(ev_t0, pl->stream)); }
+  if (int rc = fit_prep(pl, f)) return rc;
+  if (!f.data_on_device) {   // host data: the first chunk's copy starts right away
+    // the staging buffers are free at the start
+    CK(cudaEventRecord(pl->ev_free[0], pl->stream));
+    CK(cudaEventRecord(pl->ev_free[1], pl->stream));
+    CK(issue_copy(pl, f, 0));
+  }
+
+  mark(f, "before chunk loop");
+  const int nchunks = (int)f.cstart.size() - 1;
+  for (int c = 0; c < nchunks; ++c) {
+    mark(f, "chunk %d (%d subints)", c, f.cstart[c + 1] - f.cstart[c]);
+    if (int rc = fit_spectra(pl, f, c)) return rc;
+    if (!f.data_on_device) CK(cudaEventRecord(pl->ev_free[c & 1], pl->stream));
+    if (int rc = fit_guess(pl, f, c)) return rc;
+    f.pa.s0 = f.ua.s0 = f.p5.s0 = f.u5.s0 = f.cstart[c];
+    if (int rc = fit_coarse(pl, f, c)) return rc;
+    if (int rc = fit_passes(pl, f, c)) return rc;
+    if (int rc = fit_align_chunk(pl, f, c)) return rc;
     // the chunk is done at this point of the stream; its results go back on the copy stream
     // while the next chunk computes.  The (host-side) enqueue of those copies is deferred until
     // the next chunk's first kernels are in the queue, so that the device does not idle over it.
@@ -1335,49 +1374,27 @@ extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_f
       pl->ev_chunk.push_back(e);
     }
     CK(cudaEventRecord(pl->ev_chunk[c], pl->stream));
-    pending_out = c;
+    f.pending_out = c;
   }
-  if (pending_out >= 0 && enqueue_results(pending_out)) return -2;
-  mark("all chunks queued");
+  if (enqueue_results(pl, f)) return -2;
+  mark(f, "all chunks queued");
   CK(cudaGetLastError());
-  cudaEvent_t ev_t1 = nullptr;
   if (pl->timing) {
-    ev_t1 = get_event(pl);
+    cudaEvent_t ev_t1 = get_event(pl);
     CK(cudaEventRecord(ev_t1, pl->stream));
     pl->spans.push_back({SP_TOTAL, ev_t0, ev_t1});
   }
-
-  if (want_align) {
-    AlignFinishArgs fa;
-    fa.acc = pl->al_acc.as<double2>(); fa.wsum_parts = pl->al_wparts.as<double>(); fa.aligned = pl->al_out.as<double>();
-    fa.wsum = pl->al_wsum.as<double>(); fa.twN = pl->twN64.p; fa.tw2N = pl->tw2N64.p;
-    fa.nchan = nchan; fa.nsplit = align_nsplit;
-    if (pl->anyn) {
-      CK(pl->any_spec2.need(sizeof(double2) * (size_t)nchan * N));
-      CK(pl->any_dc2.need(sizeof(double) * (size_t)nchan));
-      k_align_reduce_any<<<nchan, 256, 0, pl->stream>>>(fa.acc, fa.wsum_parts, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(),
-                                                        fa.wsum, nchan, N, align_nsplit);
-      if (launch_inv_any(pl, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), fa.aligned, nchan, true)) return -2;
-    } else {
-      DISPATCH_N(N, {
-        const int rows = RowGeom<NN>::kRows;
-        k_align_finish<NN><<<(nchan + rows - 1) / rows, 256, fft_smem_bytes<NN, double>(), pl->stream>>>(fa);
-      });
-    }
-    pl->stats.launches++;
-    if (copy_out(pl, out->align_sum, pl->al_out.as<double>(), (size_t)nchan * pl->nbin)) return -2;
-    if (copy_out(pl, out->align_wsum, pl->al_wsum.as<double>(), (size_t)nchan)) return -2;
-  }
+  if (int rc = fit_align_finish(pl, f)) return rc;
   // ---- results (per-chunk copies were queued on the copy stream) -------------------------
-  if (!want_guess && out->phi_guess && dinit) {
+  if (!f.want_guess && out->phi_guess && f.dinit) {
     // phi_guess = init[:,0]
-    CK(cudaMemcpy2DAsync(out->phi_guess, sizeof(double), dinit, 5 * sizeof(double), sizeof(double), nsub,
+    CK(cudaMemcpy2DAsync(out->phi_guess, sizeof(double), f.dinit, 5 * sizeof(double), sizeof(double), f.nsub,
                          is_device_ptr(out->phi_guess) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, pl->stream));
   }
   CK(cudaStreamSynchronize(pl->copy_stream));
-  mark("copy stream drained");
+  mark(f, "copy stream drained");
   CK(cudaStreamSynchronize(pl->stream));
-  mark("done");
+  mark(f, "done");
   CK(cudaGetLastError());
   stats_end(pl);
   return 0;
@@ -1408,36 +1425,13 @@ static int launch_rfft_rows(pp_plan* pl, const float* in, int nrows, float2* spe
   a.spec64 = spec64; a.dc64 = dc64;
   if (bits == 64) {
     a.twN = tw1<double>(pl); a.tw2N = tw2<double>(pl);
-    DISPATCH_N(N, {
-      const int rows = RowGeom<NN>::kRows;
-      k_rfft_rows<NN, double><<<(nrows + rows - 1) / rows, 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a);
-    });
+    DISPATCH_N(N, (k_rfft_rows<NN, double><<<row_ctas<NN>(nrows), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a)));
   } else {
     a.twN = tw1<float>(pl); a.tw2N = tw2<float>(pl);
-    DISPATCH_N(N, {
-      const int rows = RowGeom<NN>::kRows;
-      k_rfft_rows<NN, float><<<(nrows + rows - 1) / rows, 256, fft_smem_bytes<NN, float>(), pl->stream>>>(a);
-    });
+    DISPATCH_N(N, (k_rfft_rows<NN, float><<<row_ctas<NN>(nrows), 256, fft_smem_bytes<NN, float>(), pl->stream>>>(a)));
   }
   pl->stats.launches++;
   return 0;
-}
-
-static int pshift_impl(pp_plan_t* pl, const float* profiles, int32_t n, const float* models, int32_t nmodel,
-                       const double* noise, int32_t Ns, bool general, double phi_lo, double phi_hi,
-                       const pp_pshift_out_t* out);
-
-extern "C" int pp_fit_phase_shift_batch(pp_plan_t* pl, const float* profiles, int32_t n, const float* models, int32_t nmodel,
-                                        const double* noise, int32_t Ns, const pp_pshift_out_t* out) {
-  return pshift_impl(pl, profiles, n, models, nmodel, noise, Ns, false, -0.5, 0.5, out);
-}
-
-extern "C" int pp_fit_phase_shift_batch_bounds(pp_plan_t* pl, const float* profiles, int32_t n, const float* models,
-                                               int32_t nmodel, const double* noise, int32_t Ns, double phi_lo,
-                                               double phi_hi, const pp_pshift_out_t* out) {
-  if (!(phi_hi > phi_lo)) return fail(-1, "bounds: need phi_lo < phi_hi");
-  const bool dflt = phi_lo == -0.5 && phi_hi == 0.5;
-  return pshift_impl(pl, profiles, n, models, nmodel, noise, Ns, !dflt, phi_lo, phi_hi, out);
 }
 
 static int pshift_impl(pp_plan_t* pl, const float* profiles, int32_t n, const float* models, int32_t nmodel,
@@ -1480,13 +1474,52 @@ static int pshift_impl(pp_plan_t* pl, const float* profiles, int32_t n, const fl
   k_guess<<<n, 256, sizeof(double2) * N, pl->stream>>>(ga);
   pl->stats.launches++;
   CK(cudaGetLastError());
-  if (copy_out(pl, out->phase, pl->ps_phase.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->phase_err, pl->ps_perr.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->scale, pl->ps_scale.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->scale_err, pl->ps_serr.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->snr, pl->ps_snr.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->red_chi2, pl->ps_rchi2.as<double>(), (size_t)n)) return -2;
-  if (copy_out(pl, out->lag_index, pl->ps_lag.as<int>(), (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->phase, pl->ps_phase.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->phase_err, pl->ps_perr.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->scale, pl->ps_scale.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->scale_err, pl->ps_serr.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->snr, pl->ps_snr.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->red_chi2, pl->ps_rchi2.as<double>(), 0, (size_t)n)) return -2;
+  if (copy_out_at(pl->stream, out->lag_index, pl->ps_lag.as<int>(), 0, (size_t)n)) return -2;
+  CK(cudaStreamSynchronize(pl->stream));
+  return 0;
+}
+
+extern "C" int pp_fit_phase_shift_batch(pp_plan_t* pl, const float* profiles, int32_t n, const float* models, int32_t nmodel,
+                                        const double* noise, int32_t Ns, const pp_pshift_out_t* out) {
+  return pshift_impl(pl, profiles, n, models, nmodel, noise, Ns, false, -0.5, 0.5, out);
+}
+
+extern "C" int pp_fit_phase_shift_batch_bounds(pp_plan_t* pl, const float* profiles, int32_t n, const float* models,
+                                               int32_t nmodel, const double* noise, int32_t Ns, double phi_lo,
+                                               double phi_hi, const pp_pshift_out_t* out) {
+  if (!(phi_hi > phi_lo)) return fail(-1, "bounds: need phi_lo < phi_hi");
+  const bool dflt = phi_lo == -0.5 && phi_hi == 0.5;
+  return pshift_impl(pl, profiles, n, models, nmodel, noise, Ns, !dflt, phi_lo, phi_hi, out);
+}
+
+// where an entry point writes its n results: the caller's array when it is device memory, else `stage`;
+// finish_out copies staged results back to the caller
+template <typename T> static int stage_out(DBuf& stage, T* dst, size_t n, T** dev) {
+  *dev = dst;
+  if (is_device_ptr(dst)) return 0;
+  CK(stage.need(sizeof(T) * n));
+  *dev = stage.as<T>();
+  return 0;
+}
+template <typename T> static int finish_out(pp_plan* pl, T* dst, const T* dev, size_t n) {
+  if (dev != dst) CK(cudaMemcpyAsync(dst, dev, sizeof(T) * n, cudaMemcpyDeviceToHost, pl->stream));
+  return 0;
+}
+
+// device scalars 0.0 (gm_zero) and 1.0 (gm_one): phase, DM and P, nu_ref of a rotation by nothing
+static int unit_scalars(pp_plan* pl) {
+  if (pl->gm_zero.p) return 0;
+  const double z = 0.0, o = 1.0;
+  CK(pl->gm_zero.need(sizeof(double)));
+  CK(pl->gm_one.need(sizeof(double)));
+  CK(cudaMemcpyAsync(pl->gm_zero.p, &z, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
+  CK(cudaMemcpyAsync(pl->gm_one.p, &o, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1500,13 +1533,12 @@ extern "C" int pp_rotate_full_batch(pp_plan_t* pl, const float* in, float* outp,
   if (!pl->freqs_set) return fail(-1, "pp_set_model or pp_set_freqs must be called before pp_rotate_batch");
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
-  const int N = pl->N, nchan = pl->nchan;
+  const int nchan = pl->nchan;
   const size_t tot = (size_t)nsub * nchan * pl->nbin;
   const float* din;
   if (stage_in(pl, pl->rot_in, in, tot, &din)) return -2;
-  float* dout = outp;
-  const bool out_dev = is_device_ptr(outp);
-  if (!out_dev) { CK(pl->rot_out.need(sizeof(float) * tot)); dout = pl->rot_out.as<float>(); }
+  float* dout;
+  if (stage_out(pl->rot_out, outp, tot, &dout)) return -2;
   const double *dph, *ddm, *dP, *dnr, *dgm, *dng;
   if (stage_in(pl, pl->rot_phase, phase, (size_t)nsub, &dph)) return -2;
   if (stage_in(pl, pl->rot_dm, DM, (size_t)nsub, &ddm)) return -2;
@@ -1517,10 +1549,9 @@ extern "C" int pp_rotate_full_batch(pp_plan_t* pl, const float* in, float* outp,
   RotateArgs a;
   a.in = din; a.out = dout; a.phase = dph; a.DM = ddm; a.P = dP; a.nu_ref = dnr; a.GM = dgm; a.nu_GM = dng;
   a.nu2 = pl->nu2.as<double>(); a.taus = nullptr; a.resp = nullptr; a.nsub = nsub; a.nchan = nchan;
-  (void)N;
   if (rotate_rows(pl, a, pl->fft_precision == 64)) return -2;
   CK(cudaGetLastError());
-  if (!out_dev) CK(cudaMemcpyAsync(outp, dout, sizeof(float) * tot, cudaMemcpyDeviceToHost, pl->stream));
+  if (finish_out(pl, outp, dout, tot)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1535,23 +1566,15 @@ extern "C" int pp_apply_response_batch(pp_plan_t* pl, const float* in, float* ou
   if (nsub < 1) return fail(-1, "nsub must be >= 1");
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
-  const int N = pl->N, nchan = pl->nchan;
+  const int nchan = pl->nchan;
   const size_t tot = (size_t)nsub * nchan * pl->nbin;
   const float* din;
   if (stage_in(pl, pl->rot_in, in, tot, &din)) return -2;
-  float* dout = outp;
-  const bool out_dev = is_device_ptr(outp);
-  if (!out_dev) { CK(pl->rot_out.need(sizeof(float) * tot)); dout = pl->rot_out.as<float>(); }
+  float* dout;
+  if (stage_out(pl->rot_out, outp, tot, &dout)) return -2;
   const double* dresp;
   if (stage_in(pl, pl->resp, resp, (size_t)nchan * (pl->nbin / 2 + 1), &dresp)) return -2;
-  if (!pl->gm_zero.p) {
-    const double z = 0.0, o = 1.0;
-    CK(pl->gm_zero.need(sizeof(double)));
-    CK(pl->gm_one.need(sizeof(double)));
-    CK(cudaMemcpyAsync(pl->gm_zero.p, &z, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
-    CK(cudaMemcpyAsync(pl->gm_one.p, &o, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
-    CK(cudaStreamSynchronize(pl->stream));
-  }
+  if (unit_scalars(pl)) return -2;
   // zero rotation for every subint: phase, DM from a zero-filled array
   CK(pl->rot_phase.need(sizeof(double) * nsub));
   CK(pl->rot_P.need(sizeof(double) * nsub));
@@ -1566,10 +1589,9 @@ extern "C" int pp_apply_response_batch(pp_plan_t* pl, const float* in, float* ou
   a.P = pl->rot_P.as<double>(); a.nu_ref = pl->rot_P.as<double>(); a.GM = nullptr; a.nu_GM = nullptr;
   a.nu2 = pl->nu2.as<double>(); a.taus = nullptr; a.resp = dresp; a.nsub = nsub; a.nchan = nchan;
   if (!pl->nu2.p) { CK(pl->nu2.need(sizeof(double) * nchan)); CK(cudaMemsetAsync(pl->nu2.p, 0, sizeof(double) * nchan, pl->stream)); a.nu2 = pl->nu2.as<double>(); }
-  (void)N;
   if (rotate_rows(pl, a, true)) return -2;
   CK(cudaGetLastError());
-  if (!out_dev) CK(cudaMemcpyAsync(outp, dout, sizeof(float) * tot, cudaMemcpyDeviceToHost, pl->stream));
+  if (finish_out(pl, outp, dout, tot)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1607,25 +1629,18 @@ extern "C" int pp_align_accumulate(pp_plan_t* pl, const float* data, int32_t nsu
                                                  pl->al_wsum.as<double>(), ns, nchan, pl->nbin, s0 == 0);
       pl->stats.launches++;
     }
-    CK(cudaGetLastError());
-    if (copy_out(pl, aligned, pl->al_out.as<double>(), (size_t)nchan * pl->nbin)) return -2;
-    if (copy_out(pl, wsum, pl->al_wsum.as<double>(), (size_t)nchan)) return -2;
-    CK(cudaStreamSynchronize(pl->stream));
-    return 0;
+  } else {
+    AlignArgs a;
+    a.r.in = din; a.r.out = nullptr; a.r.phase = dph; a.r.DM = ddm; a.r.P = dP; a.r.nu_ref = dnr; a.r.GM = nullptr;
+    a.r.nu_GM = nullptr; a.r.taus = nullptr; a.r.resp = nullptr; a.r.nu2 = pl->nu2.as<double>(); a.r.twN = pl->twN64.p; a.r.tw2N = pl->tw2N64.p;
+    a.r.nsub = nsub; a.r.nchan = nchan;
+    a.weights = dw; a.aligned = pl->al_out.as<double>(); a.wsum = pl->al_wsum.as<double>();
+    DISPATCH_N(N, (k_align_accum<NN><<<row_ctas<NN>(nchan), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a)));
+    pl->stats.launches++;
   }
-  AlignArgs a;
-  a.r.in = din; a.r.out = nullptr; a.r.phase = dph; a.r.DM = ddm; a.r.P = dP; a.r.nu_ref = dnr; a.r.GM = nullptr;
-  a.r.nu_GM = nullptr; a.r.taus = nullptr; a.r.resp = nullptr; a.r.nu2 = pl->nu2.as<double>(); a.r.twN = pl->twN64.p; a.r.tw2N = pl->tw2N64.p;
-  a.r.nsub = nsub; a.r.nchan = nchan;
-  a.weights = dw; a.aligned = pl->al_out.as<double>(); a.wsum = pl->al_wsum.as<double>();
-  DISPATCH_N(N, {
-    const int rows = RowGeom<NN>::kRows;
-    k_align_accum<NN><<<(nchan + rows - 1) / rows, 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a);
-  });
-  pl->stats.launches++;
   CK(cudaGetLastError());
-  if (copy_out(pl, aligned, pl->al_out.as<double>(), (size_t)nchan * pl->nbin)) return -2;
-  if (copy_out(pl, wsum, pl->al_wsum.as<double>(), (size_t)nchan)) return -2;
+  if (copy_out_at(pl->stream, aligned, pl->al_out.as<double>(), 0, (size_t)nchan * pl->nbin)) return -2;
+  if (copy_out_at(pl->stream, wsum, pl->al_wsum.as<double>(), 0, (size_t)nchan)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1642,24 +1657,19 @@ static int gen_gaussian_impl(pp_plan* pl, const char* model_code, const double* 
   if (is_device_ptr(params)) return fail(-1, "params must be a host array");
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
-  const int N = pl->N, nchan = pl->nchan;
+  const int nchan = pl->nchan;
   const size_t np = 2 + 6 * (size_t)ngauss, tot = (size_t)nchan * pl->nbin;
   CK(pl->gm_params.need(sizeof(double) * np));
   CK(pl->gm_taus.need(sizeof(double) * nchan));
   CK(cudaMemcpyAsync(pl->gm_params.p, params, sizeof(double) * np, cudaMemcpyHostToDevice, pl->stream));
   const bool scat = params[1] != 0.0;          // the scattering multiply works on float32 rows
   const bool want64 = outp64 != nullptr;
-  const bool out_dev = is_device_ptr(want64 ? (const void*)outp64 : (const void*)outp);
   float* dout = nullptr;
   double* dout64 = nullptr;
   if (want64) {
-    dout64 = outp64;
-    if (!out_dev) { CK(pl->model_stage64.need(sizeof(double) * tot)); dout64 = pl->model_stage64.as<double>(); }
+    if (stage_out(pl->model_stage64, outp64, tot, &dout64)) return -2;
     if (scat) { CK(pl->rot_out.need(sizeof(float) * tot)); dout = pl->rot_out.as<float>(); }
-  } else {
-    dout = outp;
-    if (!out_dev) { CK(pl->rot_out.need(sizeof(float) * tot)); dout = pl->rot_out.as<float>(); }
-  }
+  } else if (stage_out(pl->rot_out, outp, tot, &dout)) return -2;
   GaussModelArgs g;
   g.params = pl->gm_params.as<double>(); g.freqs = pl->freqs.as<double>(); g.taus = pl->gm_taus.as<double>();
   g.out = dout; g.out64 = (want64 && !scat) ? dout64 : nullptr;
@@ -1668,19 +1678,11 @@ static int gen_gaussian_impl(pp_plan* pl, const char* model_code, const double* 
   k_gauss_model<<<nchan, 256, 0, pl->stream>>>(g);
   pl->stats.launches++;
   if (scat) {   // scattering: rfft, times 1/(1 + 2 pi i k tau_n), irfft (pplib.py:921-927), in place
-    if (!pl->gm_zero.p) {
-      const double z = 0.0, o = 1.0;
-      CK(pl->gm_zero.need(sizeof(double)));
-      CK(pl->gm_one.need(sizeof(double)));
-      CK(cudaMemcpyAsync(pl->gm_zero.p, &z, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
-      CK(cudaMemcpyAsync(pl->gm_one.p, &o, sizeof(double), cudaMemcpyHostToDevice, pl->stream));
-      CK(cudaStreamSynchronize(pl->stream));
-    }
+    if (unit_scalars(pl)) return -2;
     RotateArgs a;
     a.in = dout; a.out = dout; a.phase = pl->gm_zero.as<double>(); a.DM = pl->gm_zero.as<double>();
     a.P = pl->gm_one.as<double>(); a.nu_ref = pl->gm_one.as<double>(); a.GM = nullptr; a.nu_GM = nullptr;
     a.nu2 = pl->nu2.as<double>(); a.taus = pl->gm_taus.as<double>(); a.resp = nullptr; a.nsub = 1; a.nchan = nchan;
-    (void)N;
     if (rotate_rows(pl, a, true)) return -2;
     if (want64) {
       k_cvt_f32_f64<<<(unsigned)std::min<size_t>((tot + 255) / 256, 148 * 32), 256, 0, pl->stream>>>(dout, dout64, tot);
@@ -1688,10 +1690,7 @@ static int gen_gaussian_impl(pp_plan* pl, const char* model_code, const double* 
     }
   }
   CK(cudaGetLastError());
-  if (!out_dev) {
-    if (want64) CK(cudaMemcpyAsync(outp64, dout64, sizeof(double) * tot, cudaMemcpyDeviceToHost, pl->stream));
-    else CK(cudaMemcpyAsync(outp, dout, sizeof(float) * tot, cudaMemcpyDeviceToHost, pl->stream));
-  }
+  if (want64 ? finish_out(pl, outp64, dout64, tot) : finish_out(pl, outp, dout, tot)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1734,9 +1733,8 @@ extern "C" int pp_gen_spline_portrait(pp_plan_t* pl, const double* mean_prof, co
     CK(cudaMemcpyAsync(base + n_mean + n_eig + n_kn, coefs, sizeof(double) * n_co, cudaMemcpyHostToDevice, pl->stream));
   }
   const size_t tot = (size_t)nchan * nbin;
-  float* dout = outp;
-  const bool out_dev = is_device_ptr(outp);
-  if (!out_dev) { CK(pl->rot_out.need(sizeof(float) * tot)); dout = pl->rot_out.as<float>(); }
+  float* dout;
+  if (stage_out(pl->rot_out, outp, tot, &dout)) return -2;
   SplineModelArgs g;
   g.mean_prof = base; g.eigvec = base + n_mean; g.knots = base + n_mean + n_eig; g.coefs = base + n_mean + n_eig + n_kn;
   g.freqs = pl->freqs.as<double>(); g.out = dout; g.ncomp = ncomp; g.nknots = nknots; g.degree = degree;
@@ -1744,7 +1742,7 @@ extern "C" int pp_gen_spline_portrait(pp_plan_t* pl, const double* mean_prof, co
   k_spline_model<<<nchan, 256, 0, pl->stream>>>(g);
   pl->stats.launches++;
   CK(cudaGetLastError());
-  if (!out_dev) CK(cudaMemcpyAsync(outp, dout, sizeof(float) * tot, cudaMemcpyDeviceToHost, pl->stream));
+  if (finish_out(pl, outp, dout, tot)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1773,7 +1771,7 @@ extern "C" int pp_get_noise_fit_batch(pp_plan_t* pl, const float* data, int32_t 
                                                           N, L, pl->anyn ? L : 0, fact);
   pl->stats.launches++;
   CK(cudaGetLastError());
-  if (copy_out(pl, noise_out, pl->ps_noise.as<double>(), (size_t)nrows)) return -2;
+  if (copy_out_at(pl->stream, noise_out, pl->ps_noise.as<double>(), 0, (size_t)nrows)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
@@ -1813,16 +1811,14 @@ extern "C" int pp_get_noise_cut_batch(pp_plan_t* pl, const float* data, int32_t 
   if (kc > pl->nbin / 2) return fail(-1, "kc must be <= nbin/2 (got %d)", kc);
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
-  const int N = pl->N, nchan = pl->nchan;
-  const long nrows = (long)nsub * nchan;
+  const long nrows = (long)nsub * pl->nchan;
   const float* din;
   if (stage_in(pl, pl->rot_in, data, (size_t)nrows * pl->nbin, &din)) return -2;
-  (void)N;
   CK(pl->ps_noise.need(sizeof(double) * nrows));
   const int bits = pl->fft_precision ? pl->fft_precision : 64;
   if (launch_rfft_rows(pl, din, (int)nrows, nullptr, 0, pl->ps_noise.as<double>(), bits, kc)) return -2;
   CK(cudaGetLastError());
-  if (copy_out(pl, noise_out, pl->ps_noise.as<double>(), (size_t)nrows)) return -2;
+  if (copy_out_at(pl->stream, noise_out, pl->ps_noise.as<double>(), 0, (size_t)nrows)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }
