@@ -89,7 +89,8 @@ int pp_plan_set_coarse(pp_plan_t* plan, double frac);
  * keeps them all.  eps = 0 keeps every harmonic of every channel.  pp_stats_t.x_keep_frac reports the kept share. */
 int pp_plan_set_model_cutoff(pp_plan_t* plan, double eps);
 
-/* Channel frequencies [nchan] MHz only (enough for pp_rotate_batch). */
+/* Channel frequencies [nchan] MHz only (enough for pp_rotate_batch).  After pp_set_models these replace model 0's
+ * table. */
 int pp_set_freqs(pp_plan_t* plan, const double* freqs);
 
 /* Model portrait [nchan, nbin] float32 and channel frequencies [nchan] MHz.
@@ -102,6 +103,23 @@ int pp_set_model(pp_plan_t* plan, const float* model, const double* freqs);
  * above drop the harmonics an analytic template has no power in.  (Arbitrary nbin: rounded to float32 on the
  * device, as pp_set_model.) */
 int pp_set_model_f64(pp_plan_t* plan, const double* model, const double* freqs);
+
+/* nmodel model portraits [nmodel, nchan, nbin] and their frequency tables [nmodel, nchan] MHz (host or device).
+ * Model m is everything pp_set_model computes, for table m; pp_set_model is the nmodel = 1 case.  Replaces the
+ * per-subint read_model of pptoas.py:356-394: pp_fit_batch_models then fits each subint of one batch against its own
+ * model and table.  Every frequency of every table must be positive.
+ * Device memory per model, N = nbin/2 for power-of-two nbin (other nbin: N = the padded row length, the smallest
+ * power of two above nbin/2):  nchan * (32 N + 36) + 8 N + 12 bytes (conj(m) in float and double, |m|^2, p_n, the
+ * harmonic cut-off and three frequency tables per channel; the mean spectrum, the cut-off and the coarse levels per
+ * model); other nbin add 16 N bytes per channel of transform scratch.  A staging copy of the portraits themselves
+ * (nchan * nbin * 4 or 8 bytes per model) is kept when they come from host memory.  The plan keeps the largest model
+ * set it has held.
+ * pp_rotate_batch, pp_rotate_full_batch, pp_apply_response_batch, pp_align_accumulate, the noise entry points and
+ * the model generators use one table: model 0's, or that of the last pp_set_freqs call.
+ * pp_plan_set_model_cutoff recomputes the cut-offs of every model; pp_stats_t.x_keep_frac is the kept share over
+ * all models' channels. */
+int pp_set_models(pp_plan_t* plan, int32_t nmodel, const float* models, const double* freqs);
+int pp_set_models_f64(pp_plan_t* plan, int32_t nmodel, const double* models, const double* freqs);
 
 /* ---- batched wideband fit ------------------------------------------------
  * Replaces, per subint, the sequence of pptoas.GetTOAs.get_TOAs
@@ -206,6 +224,17 @@ typedef struct {
 
 int pp_fit_batch(pp_plan_t* plan, const pp_fit_args_t* args,
                  const pp_fit_out_t* out);
+
+/* pp_fit_batch with model_index [nsub] int32 in [0, nmodel) (host or device): subint s is fit against model
+ * model_index[s] on frequency table model_index[s] (pp_set_models).  pp_fit_batch(plan, a, o) is
+ * pp_fit_batch_models(plan, a, NULL, o); NULL is valid only when the plan holds one model.  The index is checked
+ * before any kernel reads it (a device index costs one small copy to the host): an entry out of range is an error.
+ * The FFTFIT guess uses each subint's own model (its mean spectrum and harmonic cut-off); the coarse levels of the
+ * general solver are chosen per model present in a chunk, from that model's first subint of the chunk.  Results of a
+ * subint are those of a pp_fit_batch call on its model's subints alone, bit for bit, when the batch is one chunk (the
+ * (phi, DM) fit: for any chunking).  align_sum needs one model (ppalign has one template and one table). */
+int pp_fit_batch_models(pp_plan_t* plan, const pp_fit_args_t* args, const int32_t* model_index,
+                        const pp_fit_out_t* out);
 
 /* ---- batched 1-D FFTFIT ---------------------------------------------------
  * Replaces pplib.fit_phase_shift (pplib.py:2054-2100) for n profiles.

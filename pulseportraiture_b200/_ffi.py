@@ -22,7 +22,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3",
 # symbols declared in include/ppb200.h (checked by the CPU test-suite)
 SYMBOLS = ["pp_plan_create", "pp_plan_destroy", "pp_plan_set_stream",
            "pp_plan_set_chunk", "pp_plan_set_fft_precision", "pp_plan_set_model_steps", "pp_plan_set_coarse", "pp_plan_set_model_cutoff", "pp_set_freqs", "pp_set_model_f64",
-           "pp_set_model", "pp_fit_batch",
+           "pp_set_model", "pp_set_models", "pp_set_models_f64", "pp_fit_batch", "pp_fit_batch_models",
            "pp_fit_phase_shift_batch", "pp_fit_phase_shift_batch_bounds", "pp_rotate_batch", "pp_rotate_full_batch", "pp_apply_response_batch",
            "pp_align_accumulate", "pp_gen_gaussian_portrait", "pp_gen_gaussian_portrait_f64", "pp_gen_spline_portrait",
            "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64",
@@ -154,6 +154,12 @@ def lib():
     L.pp_set_model_f64.restype = C.c_int
     L.pp_fit_batch.argtypes = [vp, C.POINTER(FitArgs), C.POINTER(FitOut)]
     L.pp_fit_batch.restype = C.c_int
+    L.pp_set_models.argtypes = [vp, i32, vp, vp]
+    L.pp_set_models.restype = C.c_int
+    L.pp_set_models_f64.argtypes = [vp, i32, vp, vp]
+    L.pp_set_models_f64.restype = C.c_int
+    L.pp_fit_batch_models.argtypes = [vp, C.POINTER(FitArgs), vp, C.POINTER(FitOut)]
+    L.pp_fit_batch_models.restype = C.c_int
     L.pp_fit_phase_shift_batch.argtypes = [vp, vp, i32, vp, i32, vp, i32,
                                            C.POINTER(PShiftOut)]
     L.pp_fit_phase_shift_batch.restype = C.c_int

@@ -91,6 +91,17 @@ __device__ __forceinline__ double wrap_phase(double phi) {
   return phi;
 }
 
+// Model-side arrays (conj(m), |m|^2, p_n, cut-offs, frequency tables) hold nmodel models one after the other:
+// [nmodel * nchan, ...] rows.  Subint s is fit against model index[s]; index null: model 0, the one model of
+// pp_set_model.  A kernel reads channel ch of subint s's model at row row0(s) + ch (row0 is taken once per subint;
+// the base pointers stay kernel parameters).
+struct ModelRows {
+  const int* index;   // [nsub] model of each subint (global subint index), or null
+  int nchan;
+  __device__ __forceinline__ int of(int s) const { return index ? __ldg(index + s) : 0; }
+  __device__ __forceinline__ int row0(int s) const { return of(s) * nchan; }
+};
+
 // ----------------------------------------------------------------------------
 // k_model: one CTA of 256 threads, RowGeom<N>::kRows channels at a time.
 // Always runs in double (once per model); stores conj(m) both as double and
@@ -179,10 +190,12 @@ __global__ void __launch_bounds__(256) k_model(ModelArgs a) {
   if (t_row == 0 && valid) a.pn[ch] = psum;
 }
 
-// mean over (all) channels of conj(m): one thread per slot, fixed order.
+// mean over (all) channels of conj(m): one thread per slot, fixed order; grid.y = model.
 __global__ void k_model_mean(const cx<double>* __restrict__ mconj, float2* __restrict__ mmean, int nchan, int N) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= N) return;
+  mconj += (size_t)blockIdx.y * nchan * N;
+  mmean += (size_t)blockIdx.y * N;
   double sx = 0.0, sy = 0.0;
   for (int n = 0; n < nchan; ++n) {
     const cx<double> v = mconj[(size_t)n * N + i];
@@ -192,13 +205,16 @@ __global__ void k_model_mean(const cx<double>* __restrict__ mconj, float2* __res
 }
 
 // mean of conj(m) over the USED channels of each subint (modelx.mean(axis=0) with
-// modelx = model[ok_ichans], pptoas.py:446, 454): grid (ceil(N/128), subints in chunk).
+// modelx = model[ok_ichans], pptoas.py:446, 454) of the subint's model: grid (ceil(N/128), subints in chunk).
 __global__ void k_model_mean_masked(const cx<double>* __restrict__ mconj, const uint8_t* __restrict__ mask,
                                     const float2* __restrict__ mmean_all, float2* __restrict__ out, int s0, int nchan,
-                                    int N) {
+                                    int N, ModelRows mr) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int sl = blockIdx.y;
   if (i >= N) return;
+  const int mi = mr.of(s0 + sl);
+  mconj += (size_t)mi * nchan * N;
+  mmean_all += (size_t)mi * N;
   const uint8_t* m = mask + (size_t)(s0 + sl) * nchan;
   double sx = 0.0, sy = 0.0;
   int cnt = 0;
@@ -251,17 +267,19 @@ struct PrepArgs {
   double* wsum;             // [nsub] out
   int* nok;                 // [nsub] out
   int nsub, nchan, nu_fit_mode;
+  ModelRows mr;             // freqs of the subint's model
 };
 
 __global__ void k_prep(PrepArgs a) {
   const int s = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (s >= a.nsub) return;
+  const int mb = a.mr.row0(s);
   double cnt = 0, ws = 0, fs = 0, fmin = 1e300, fmax = -1e300, num = 0, den = 0;
   for (int n = lane; n < a.nchan; n += 32) {
     const bool ok = a.mask ? (a.mask[(size_t)s * a.nchan + n] != 0) : true;
     if (!ok) continue;
-    const double f = a.freqs[n];
+    const double f = a.freqs[mb + n];
     cnt += 1.0;
     ws += a.weights ? a.weights[(size_t)s * a.nchan + n] : 1.0;
     fs += f;
@@ -278,7 +296,7 @@ __global__ void k_prep(PrepArgs a) {
   for (int n = lane; n < a.nchan; n += 32) {
     const bool ok = a.mask ? (a.mask[(size_t)s * a.nchan + n] != 0) : true;
     if (!ok) continue;
-    const double f = a.freqs[n];
+    const double f = a.freqs[mb + n];
     const double w = (a.snrs ? a.snrs[(size_t)s * a.nchan + n] : 1.0) / (f * f);
     num += (f - nu0) * w;
     den += w;
@@ -338,6 +356,7 @@ struct SpectraArgs {
   int nhalf, kc_true;        // true nbin/2; first harmonic of the noise estimate, int(0.75 (nhalf + 1))
   const int* njn;            // [nchan] groups of 16 harmonics where the model has power (k_model_cutoff): X is stored
                              // for those only, the pass kernels read no others (null: all)
+  ModelRows mr;              // mconj64, mconj32, pn, nu2, njn of the subint's model
 };
 
 template <int N, class PL = SpecPlan<N>, bool I16 = false, bool FROMSPEC = false>
@@ -363,6 +382,7 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
   float* stage = stage_all + (size_t)slot * NSTG * (2 * N);
 
   const int sl = blockIdx.y, s = a.s0 + sl;
+  const int mb = a.mr.row0(s);   // the subint's model
   const int ch_begin = blockIdx.x * a.G;
   const int ch_end = min(ch_begin + a.G, a.nchan);
   const int nsteps = (a.G + NS - 1) / NS;
@@ -440,9 +460,9 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
     const bool first = (t == 0);
     auto slot_of = [&](int i, int q) -> int { return PL::slot_of(t, i, q, first); };
     const bool doX = a.X != nullptr && inrange;
-    const int kcut = (a.njn && inrange) ? 16 * a.njn[ch] : N;
-    const cx<F>* mc = a.mconj64 + (size_t)(inrange ? ch : 0) * N;
-    const cx<float>* mcf = a.mconj32 + (size_t)(inrange ? ch : 0) * N;
+    const int kcut = (a.njn && inrange) ? 16 * a.njn[mb + ch] : N;
+    const cx<F>* mc = a.mconj64 + (size_t)(mb + (inrange ? ch : 0)) * N;
+    const cx<float>* mcf = a.mconj32 + (size_t)(mb + (inrange ? ch : 0)) * N;
     cx<F> mc64[kMix ? 1 : NACC];
     cx<float> mc32[kMix ? NACC : 1];
     auto load_mc = [&]() {
@@ -470,7 +490,7 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
     float2* const Xlorow = a.Xlo + ((size_t)sl * a.nchan + (inrange ? ch : 0)) * kLo;
     float2* const Drow = a.D + ((size_t)sl * a.nchan + (inrange ? ch : 0)) * N;
     const float wgt = (used && want_guess) ? (float)(a.weights ? a.weights[(size_t)s * a.nchan + ch] : 1.0) : 0.f;
-    const double shift = (Dfac != 0.0 && inrange) ? Dfac * (a.nu2[ch] - numean2) : 0.0;
+    const double shift = (Dfac != 0.0 && inrange) ? Dfac * (a.nu2[mb + ch] - numean2) : 0.0;
     if constexpr (FROMSPEC) {     // the rows arrive transformed: only the barrier discipline of the power-sum hand-off
       PL::sync(slot);
       latch(step - 1);
@@ -589,7 +609,7 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
       const bool ok = fused && (sF2 > 0.0) && (sF2 < 1e300);
       const size_t o = (size_t)s * a.nchan + fch;
       a.sigma[o] = ok ? sig : 0.0;
-      a.Ssn[o] = ok ? a.pn[fch] / sF2 : 0.0;
+      a.Ssn[o] = ok ? a.pn[mb + fch] / sF2 : 0.0;
       a.Sdn[o] = ok ? keep_all / sF2 : 0.0;
     }
   }
@@ -636,6 +656,11 @@ struct GuessArgs {
   const double* init;      // [nsub,5] or null: template for GM,tau,alpha start values
   const double* scat;      // [nsub,2] tau_guess [rot, linear] and alpha_guess, or null
   int log10_tau, fit_scat;
+  // fit batch with several models: subint s uses template model[s] when tmpl_by_model (else the i mod nmodel rule,
+  // which picks the per-subint masked templates) and the cut-off nused_of[model[s]]; model null: one model
+  const int* model;        // [nsub] or null
+  const int* nused_of;     // [nmodel]
+  int tmpl_by_model;
 };
 
 __global__ void __launch_bounds__(256) k_guess(GuessArgs a) {
@@ -650,7 +675,10 @@ __global__ void __launch_bounds__(256) k_guess(GuessArgs a) {
   const int NH = a.nhalf > 0 ? a.nhalf : N;          // true nbin/2: noise cut, normalisations, degrees of freedom
   const int kc = (3 * (NH + 1)) / 4;
   const double inv_w = a.wsum ? 1.0 / a.wsum[ig] : 1.0;
-  const float2* mc = a.mconj + (size_t)(a.nmodel > 1 ? il % a.nmodel : 0) * N;   // profile i uses model i mod nmodel
+  const int mi = a.model ? __ldg(a.model + ig) : 0;
+  // profile i uses model i mod nmodel, a subint of a batch with several models its own model's template
+  const float2* mc = a.mconj + (size_t)(a.tmpl_by_model ? mi : (a.nmodel > 1 ? il % a.nmodel : 0)) * N;
+  const int nused = a.model ? __ldg(a.nused_of + mi) : a.nused;
   double v[3] = {0.0, 0.0, 0.0};  // sum |d|^2, sum |m|^2, top-quarter power
   const double tau_g = (a.scat && a.fit_scat) ? a.scat[(size_t)ig * 2] : 0.0;
   for (int i = tid; i < N; i += 256) {
@@ -685,7 +713,7 @@ __global__ void __launch_bounds__(256) k_guess(GuessArgs a) {
   // (two independent FP64 recurrences, no table look-up or index arithmetic in the loop); Y_k is a
   // shared-memory broadcast.  Harmonic N sits in slot 0.
   const int M = a.Ns - 1;
-  const int NU = (a.nused > 0 && a.nused < N) ? (a.nused & ~1) : N;   // even
+  const int NU = (nused > 0 && nused < N) ? (nused & ~1) : N;   // even
   double bv = CUDART_INF;
   int bi = 0x7fffffff;
   for (int j0 = w * 32; j0 < a.Ns; j0 += 256) {
@@ -839,6 +867,7 @@ struct PassArgs {
   int s0, nchan, N;
   int nhalf;               // true nbin/2 of the noise normalisation (0: N; arbitrary nbin runs on N = Npad slots)
   const int* njn;          // [nchan] groups of 16 harmonics where the model has power (k_model_cutoff); N/16 = all
+  ModelRows mr;            // nu2, njn of the subint's model
 };
 
 // streaming 16-byte load: read-only path, do not keep in L1
@@ -884,16 +913,17 @@ __global__ void __launch_bounds__(256, Pass2Ring<N>::kMinBlocks) k_pass2(PassArg
   // along the Newton path without another pass over X
   double C = 0.0, C1 = 0.0, C2 = 0.0, C3 = 0.0, C4 = 0.0;
   if (used) {
+    const int mb = a.mr.row0(s);   // the subint's model
     const double phi = a.st.x[(size_t)s * 5 + 0], DM = a.st.x[(size_t)s * 5 + 1];
     const double nf = a.nu_fit[(size_t)s * 3 + 0];
-    const double g = kDconst * (a.nu2[ch] - 1.0 / (nf * nf)) / a.P[s];
+    const double g = kDconst * (a.nu2[mb + ch] - 1.0 / (nf * nf)) / a.P[s];
     double theta = phi + DM * g;               // pplib.py:1319-1320
     theta -= rint(theta);
     const float4* row = reinterpret_cast<const float4*>(a.X + ((size_t)sl * a.nchan + ch) * N);
     constexpr int NJ = N / 16;
     constexpr int KJ = LoK<N>::value / 16;                     // iterations that carry lo parts
     constexpr int D = Pass2Ring<N>::D;
-    const int nj = a.njn[ch];                                  // groups of 16 harmonics the model has power in (>= KJ)
+    const int nj = a.njn[mb + ch];                             // groups of 16 harmonics the model has power in (>= KJ)
     const float4* lorow = reinterpret_cast<const float4*>(a.Xlo + ((size_t)sl * a.nchan + ch) * LoK<N>::value);
     // the X row pieces arrive through a thread-private ring in shared memory (cp.async, D iterations in flight);
     // the first copies go out before the phasor set-up so that its latency is hidden
@@ -1019,6 +1049,7 @@ struct UpdateArgs {
   double tol;              // one step per pass: convergence when the step is below tol sigma
   double tol_model;        // model steps: step and estimated truncation shift below tol_model sigma
   Box box;
+  ModelRows mr;            // nu2, freqs of the subint's model
 };
 
 // C_n, dC_n/dtheta, d2C_n/dtheta2 at theta + t from the derivatives c[0..4] at theta
@@ -1035,6 +1066,7 @@ __device__ __forceinline__ Tay4 taylor4(const double* c, double t) {
 __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
   const int s = a.s0 + blockIdx.x;
   if (a.st.done[s]) return;
+  const int mb = a.mr.row0(s);   // the subint's model
   __shared__ double sh[8 * 4];
   const int tid = threadIdx.x;
   const int nchan = a.nchan;
@@ -1051,7 +1083,7 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
     const double S = Sv[n];
     if (!(S > 0.0)) continue;
     const double C = cs[n * kNCsum], C1 = cs[n * kNCsum + 1], C2 = cs[n * kNCsum + 2];
-    const double g = KP * (a.nu2[n] - nf2);
+    const double g = KP * (a.nu2[mb + n] - nf2);
     const double t = -2.0 * C * C1 / S;            // pplib.py:1348-1349
     const double W = (C1 * C1 + C * C2) / S;       // pplib.py:1385-1386
     v[0] -= C * C / S;
@@ -1106,7 +1138,7 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
         for (int n = tid; n < nchan; n += 128) {
           const double S = Sv[n];
           if (!(S > 0.0)) continue;
-          const double g = KP * (a.nu2[n] - nf2);
+          const double g = KP * (a.nu2[mb + n] - nf2);
           const Tay4 y = taylor4(cs + n * kNCsum, d0 + d1 * g);
           const double t = -2.0 * y.C * y.C1 / S;
           const double W = (y.C1 * y.C1 + y.C * y.C2) / S;
@@ -1161,7 +1193,7 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
         const double S = Sv[n];
         if (!(S > 0.0)) continue;
         const double* c = cs + n * kNCsum;
-        const double g = KP * (a.nu2[n] - nf2);
+        const double g = KP * (a.nu2[mb + n] - nf2);
         const double t = fabs(d0 + d1 * g);
         const double e = 2.0 * fabs(c[0]) * fabs(c[4]) * t * t * t / (6.0 * S);
         q[0] += fabs(c[2]); q[1] += fabs(c[4]); q[2] += e; q[3] += e * fabs(g); q[4] += e * t * 0.25;
@@ -1199,11 +1231,11 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
   for (int n = tid; n < nchan; n += 128) {
     const double S = Sv[n];
     if (!(S > 0.0)) continue;
-    const double g = KP * (a.nu2[n] - nf2);
+    const double g = KP * (a.nu2[mb + n] - nf2);
     const Tay4 y = taylor4(cs + n * kNCsum, d0 + d1 * g);
     const double W = (y.C1 * y.C1 + y.C * y.C2) / S;
     u[0] -= y.C * y.C / S;
-    u[1] += W; u[2] += W * a.nu2[n];
+    u[1] += W; u[2] += W * a.nu2[mb + n];
     u[3] += y.C * y.C / S;
   }
   block_sum<4, 128>(u, sh);
@@ -1219,10 +1251,10 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
   for (int n = tid; n < nchan; n += 128) {
     const double S = Sv[n];
     if (!(S > 0.0)) continue;
-    const double g = KP * (a.nu2[n] - nf2);
+    const double g = KP * (a.nu2[mb + n] - nf2);
     const Tay4 y = taylor4(cs + n * kNCsum, d0 + d1 * g);
     const double W = (y.C1 * y.C1 + y.C * y.C2) / S;
-    const double go = KP * (a.nu2[n] - no2);
+    const double go = KP * (a.nu2[mb + n] - no2);
     hh[0] -= 2.0 * W; hh[1] -= 2.0 * W * go; hh[2] -= 2.0 * W * go * go;
   }
   block_sum<3, 128>(hh, sh);
@@ -1244,7 +1276,7 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
     const size_t o = (size_t)s * nchan + n;
     double sc = 0.0, se = 0.0, csn = 0.0;
     if (S > 0.0) {
-      const double g = KP * (a.nu2[n] - nf2);
+      const double g = KP * (a.nu2[mb + n] - nf2);
       const Tay4 y = taylor4(cs + n * kNCsum, d0 + d1 * g);
       const double C = y.C, C1 = y.C1;
       sc = C / S;                                         // pptoaslib.py:688
@@ -1252,7 +1284,7 @@ __global__ void __launch_bounds__(128) k_update2(UpdateArgs a) {
       if (a.semantics == 1) se = 1.0 / sqrt(S);           // pplib.py:2197
       else {
         // diag(2 LR), LR = Cinv + Cinv V Xinv U Cinv (pptoaslib.py:713-724)
-        const double go = KP * (a.nu2[n] - no2);
+        const double go = KP * (a.nu2[mb + n] - no2);
         const double U0 = a.fit_phi ? -2.0 * C1 : 0.0, U1 = a.fit_dm ? -2.0 * C1 * go : 0.0;
         // Xinv = inv(H_out) = cov/2
         const double q = 0.5 * (U0 * U0 * c00 + 2.0 * U0 * U1 * c01 + U1 * U1 * c11);
@@ -1320,13 +1352,24 @@ __global__ void k_reset_state(SolverState st, int s0, int n) {
   st.fprev[s] = 0.0; st.lam[s] = 1.0; st.iter[s] = 0; st.iterc[s] = 0; st.done[s] = 0;
 }
 
+// Coarse level of the general fit with several models: a running subint whose model has no such level (nj[model]
+// = 0) waits in state kSitsOut, untouched by the level's kernels (on = 1), and runs again afterwards (on = 0).
+constexpr int kSitsOut = 4;
+__global__ void k_coarse_sitout(SolverState st, ModelRows mr, const int* nj, int s0, int n, int on) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int s = s0 + i;
+  if (on) { if (st.done[s] == 0 && nj[mr.of(s)] == 0) st.done[s] = kSitsOut; }
+  else if (st.done[s] == kSitsOut) st.done[s] = 0;
+}
+
 // end of the coarse stage of the general fit: every unfinished subint starts the full-resolution Newton
 // iterations from where the coarse ones left it (the objective changes: no comparison with the old value)
 __global__ void k_coarse_end(SolverState st, int s0, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const int s = s0 + i;
-  if (st.done[s] == 1) return;
+  if (st.done[s] == 1 || st.done[s] == kSitsOut) return;
   st.done[s] = 0;
   st.fprev[s] = CUDART_INF;
   st.lam[s] = 1.0;
@@ -1380,10 +1423,19 @@ __global__ void __launch_bounds__(256) k_model_cutoff(const double* mpow, int* n
 //   info[j] = sum_n sum_{16 j <= k < 16 (j+1)} k^2 |m_nk|^2 |B_nk|^2,  |B_nk|^2 = 1 / (1 + (2 pi k tau_n)^2)
 // with tau_n from the start values of subint s (x = null: no scattering).  The host accumulates the groups and
 // takes the leading ones that hold coarse_frac of the total as the coarse objective of the general solver
-// (the Nyquist term is left out).
+// (the Nyquist term is left out).  grid.y: one model each, from its subint first[y] (global index: x, nu_fit and
+// info [gridDim.y, N/16] then start at subint 0); first null: one model, x and nu_fit at subint s.
 __global__ void k_model_info(const double* mpow, const double* lgf, const double* x, const double* nu_fit, int log10_tau,
-                             double* info, int nchan, int N) {
+                             double* info, int nchan, int N, ModelRows mr, const int* first) {
   const int j = blockIdx.x;
+  if (first) {
+    const int s = first[blockIdx.y];
+    const size_t r = mr.row0(s);
+    mpow += r * N; lgf += r;
+    if (x) x += (size_t)s * 5;
+    nu_fit += (size_t)s * 3;
+    info += (size_t)blockIdx.y * (N / 16);
+  }
   double tau = 0.0, alpha = 0.0, lg2nT = 0.0;
   if (x) {
     tau = log10_tau ? exp2(x[3] * 3.3219280948873623479) : x[3];
@@ -1453,6 +1505,8 @@ struct Pass5Args {
                            // also leaves the Nyquist term out and skips subints already coarse-converged (done == 3)
   int cstride;             // coarse objective: every cstride-th channel only (1: all)
   const int* njn;          // [nchan] groups of 16 harmonics where the model has power (k_model_cutoff)
+  ModelRows mr;            // mpow, nu2, freqs, lgf, njn of the subint's model
+  const int* njm;          // [nmodel] coarse level with several models: its groups per model (then nj = 0), or null
 };
 
 // k_pass5 keeps D iterations of loads (X row piece + |m|^2 piece, 16 bytes each per thread) in flight through a
@@ -1474,8 +1528,10 @@ __global__ void __launch_bounds__(256, Pass5Ring<N>::kMinBlocks) k_pass5(Pass5Ar
   const bool coarse = a.nj < NJ;
   {
     const int dn = a.st.done[s];
-    if (dn == 1 || (coarse && dn == 3)) return;
+    if (dn == 1 || (coarse && dn >= 3)) return;
   }
+  const int m = a.mr.of(s), mb = m * a.nchan;   // the subint's model
+  const int lvnj = a.njm ? __ldg(a.njm + m) : a.nj;
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int sub = lane >> 3, l8 = lane & 7;
   const int ch = (blockIdx.x * 32 + w * 4 + sub) * a.cstride;
@@ -1492,9 +1548,9 @@ __global__ void __launch_bounds__(256, Pass5Ring<N>::kMinBlocks) k_pass5(Pass5Ar
     float4* rm = rv + D * 256;                                 // [D][256] |m|^2 pieces (double2)
     float4* rl = rm + D * 256;                                 // [KJ][256] float32 residuals of the low harmonics
     const float4* row = reinterpret_cast<const float4*>(a.X + ((size_t)sl * a.nchan + ch) * N) + l8;
-    const float4* mrow = reinterpret_cast<const float4*>(a.mpow + (size_t)ch * N) + l8;
+    const float4* mrow = reinterpret_cast<const float4*>(a.mpow + (size_t)(mb + ch) * N) + l8;
     const float4* lorow = reinterpret_cast<const float4*>(a.Xlo + ((size_t)sl * a.nchan + ch) * LoK<N>::value) + l8;
-    const int nj = min(a.nj, a.njn[ch]);   // harmonics the model has power in (>= KJ groups), fewer on a coarse level
+    const int nj = min(lvnj, a.njn[mb + ch]);   // harmonics the model has power in (>= KJ groups), fewer on a coarse level
     auto issue = [&](int j) {            // one commit group per iteration, empty past the end
       if (j < nj) {
         cp_async16(rv + (j % D) * 256, row + j * 8);
@@ -1511,14 +1567,14 @@ __global__ void __launch_bounds__(256, Pass5Ring<N>::kMinBlocks) k_pass5(Pass5Ar
     const double* x = a.st.x + (size_t)s * 5;
     const double P = a.P[s];
     const double nD = a.nu_fit[(size_t)s * 3 + 0], nG = a.nu_fit[(size_t)s * 3 + 1], nT = a.nu_fit[(size_t)s * 3 + 2];
-    const double n2 = a.nu2[ch];
+    const double n2 = a.nu2[mb + ch];
     const double gD = kDconst * (n2 - 1.0 / (nD * nD)) / P;                       // pptoaslib.py:206
     const double gG = kDconst * kDconst * (n2 * n2 - 1.0 / (nG * nG * nG * nG)) / P;  // :207
     double theta = x[0] + x[1] * gD + x[2] * gG;
     theta -= rint(theta);
     // tau_n = tau (nu_n/nu_tau)^alpha (pplib.py:4049-4053) as one exp2: log2(nu_n) is tabulated
     {
-      const double lr = x[4] * (a.lgf[ch] - log2(nT));
+      const double lr = x[4] * (a.lgf[mb + ch] - log2(nT));
       taun = a.log10_tau ? exp2(fma(x[3], 3.3219280948873623479, lr)) : x[3] * exp2(lr);
     }
     // phasors for k = 2 l8, 2 l8 + 1 and the step 16 from one sincospi by repeated squaring (as k_pass2)
@@ -1598,7 +1654,7 @@ __global__ void __launch_bounds__(256, Pass5Ring<N>::kMinBlocks) k_pass5(Pass5Ar
     if (l8 == 0 && nj == NJ) {  // Nyquist harmonic k = N stored in slot 0
       const float2 xh = __ldg(reinterpret_cast<const float2*>(row));
       const float2 xl = __ldg(reinterpret_cast<const float2*>(lorow));
-      const double mn = __ldg(a.mpow + (size_t)ch * N);
+      const double mn = __ldg(a.mpow + (size_t)(mb + ch) * N);
       cx<double> en = e16;          // e^{2 pi i N theta} = (e^{2 pi i 16 theta})^(N/16)
 #pragma unroll
       for (int q = 16; q < N; q *= 2) en = csqr(en);
@@ -1772,6 +1828,7 @@ struct Update5Args {
                        // <= ctol sigma waits in state done == 3
   double tol, ctol;
   Box box;
+  ModelRows mr;        // nu2, freqs, lgf of the subint's model
 };
 
 // the per-channel sums c[0..8] = C, C_th, C_thth, C_t, C_tt, C_tht, S, S_t, S_tt carried from (theta_n, tau_n) to
@@ -1874,7 +1931,8 @@ template <int NT>
 __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
   const int s = a.s0 + blockIdx.x;
   const int state = a.st.done[s];
-  if (state == 1 || state == 3) return;
+  if (state == 1 || state >= 3) return;   // finished, coarse-converged, or sitting a coarse level out
+  const int mb = a.mr.row0(s);   // the subint's model
   __shared__ double sh[24 * (NT / 32)];
   __shared__ double bc[48];
   const int tid = threadIdx.x, nchan = a.nchan;
@@ -1913,15 +1971,15 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
       const double S = c[6];
       if (!(S > 0.0)) continue;
       if (!scat_on) { c[3] = c[4] = c[5] = c[7] = c[8] = 0.0; }
-      const ChanJ j = chan_jac(a.lgf[n] - lg2nT, a.nu2[n], P, nD, nG, tau_lin, alpha, a.log10_tau);
+      const ChanJ j = chan_jac(a.lgf[mb + n] - lg2nT, a.nu2[mb + n], P, nD, nG, tau_lin, alpha, a.log10_tau);
       const ChanK k = chan_k(c);
       v[0] += k.f;
       v[1] += k.G1; v[2] = fma(k.G1, j.Jth[1], v[2]); v[3] = fma(k.G1, j.Jth[2], v[3]);   // :572
       v[4] = fma(k.G2, j.Jt[0], v[4]); v[5] = fma(k.G2, j.Jt[1], v[5]);
       chan_hess(k, j, v + 6);
       v[21] += a.Sdn[(size_t)s * nchan + n];
-      gmax1 = fmax(gmax1, a.nu2[n]);      // range of nu^-2 over the used channels (step limit below)
-      gmax2 = fmax(gmax2, -a.nu2[n]);
+      gmax1 = fmax(gmax1, a.nu2[mb + n]);      // range of nu^-2 over the used channels (step limit below)
+      gmax2 = fmax(gmax2, -a.nu2[mb + n]);
     }
     for (int i = 0; i < 5; ++i) v[1 + i] *= fl[i];
     {
@@ -2074,12 +2132,12 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
     if (!(c[6] > 0.0)) return;
     if (!scat_on) { c[3] = c[4] = c[5] = c[7] = c[8] = 0.0; }
     if (shifted) {
-      const double n2 = a.nu2[n];
+      const double n2 = a.nu2[mb + n];
       const double dth = dx[0] + dx[1] * (kDconst * (n2 - 1.0 / (nD * nD)) / P) +
                          dx[2] * (kDconst * kDconst * (n2 * n2 - 1.0 / (nG * nG * nG * nG)) / P);
       double dta = 0.0;
       if (scat_on) {
-        const double lg2r = a.lgf[n] - lg2nT;
+        const double lg2r = a.lgf[mb + n] - lg2nT;
         const double dl = (a.log10_tau ? 2.302585092994045684 * dx[3] : log1p(dx[3] / tau_lin)) + dx[4] * lg2r * 0.69314718055994530942;
         dta = tau_lin * exp2(alpha * lg2r) * expm1(dl);
       }
@@ -2108,9 +2166,9 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
     const double S = c[6];
     if (!(S > 0.0)) continue;
     if (!scat_on) { c[3] = c[4] = c[5] = c[7] = c[8] = 0.0; }
-    const ChanJ j = chan_jac(a.lgf[n] - lg2nT, a.nu2[n], P, nD, nG, tau_e, alpha_e, a.log10_tau);
+    const ChanJ j = chan_jac(a.lgf[mb + n] - lg2nT, a.nu2[mb + n], P, nD, nG, tau_e, alpha_e, a.log10_tau);
     const ChanK k = chan_k(c);
-    const double n2 = a.nu2[n], lnnu = a.lgf[n] * 0.69314718055994530942;
+    const double n2 = a.nu2[mb + n], lnnu = a.lgf[mb + n] * 0.69314718055994530942;
     for (int p = 0; p < 5; ++p) {
       // Hessian row w.r.t. theta_n (= Hn[DM,p]/gDM_n etc.): d2C[theta,p], no S-dependence on theta
       const double h = (p < 3 ? k.A * j.Jth[p] : k.M * j.Jt[p - 3]) * zfl[p];
@@ -2127,7 +2185,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
     u[22] += a.Sdn[(size_t)s * nchan + n];
     u[23] -= k.f;
     chan_hess(k, j, hv);
-    fmean += a.freqs[n];
+    fmean += a.freqs[mb + n];
   }
   {
     int q = 0;
@@ -2228,7 +2286,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
     const double S = c[6];
     if (!(S > 0.0)) continue;
     if (!scat_on) { c[3] = c[4] = c[5] = c[7] = c[8] = 0.0; }
-    const ChanJ j = chan_jac(a.lgf[n] - lg2noT, a.nu2[n], P, noD, noG, tau_out_lin, alpha_e, a.log10_tau);
+    const ChanJ j = chan_jac(a.lgf[mb + n] - lg2noT, a.nu2[mb + n], P, noD, noG, tau_out_lin, alpha_e, a.log10_tau);
     chan_hess(chan_k(c), j, ho);
   }
   {
@@ -2257,7 +2315,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) k_update5(Update5Args a) {
     double sc = 0.0, se = 0.0, csn = 0.0;
     if (S > 0.0) {
       if (!scat_on) { c[3] = c[4] = c[5] = c[7] = c[8] = 0.0; }
-      const ChanJ j = chan_jac(a.lgf[n] - lg2noT, a.nu2[n], P, noD, noG, tau_out_lin, alpha_e, a.log10_tau);
+      const ChanJ j = chan_jac(a.lgf[mb + n] - lg2noT, a.nu2[mb + n], P, noD, noG, tau_out_lin, alpha_e, a.log10_tau);
       double dC[5], dS[5];
       chan_first(c, j, dC, dS);
       sc = c[0] / S;                                               // :688

@@ -99,12 +99,14 @@ struct pp_plan {
   int chunk_req = 0;
   int l2_bytes = 0, sm_count = 0;
   bool model_set = false;
+  int nmodel = 0;   // models set (pp_set_models): the model-side buffers hold nmodel * nchan rows (kernels.cuh ModelRows)
   // tables + model
   DBuf tw8, twN32, tw2N32, twN64, tw2N64, freqs, nu2, lgf, gm_params, gm_taus, gm_zero, gm_one, mconj32, mconj64, mpow, pn, mmean, mmean_sub, model_stage, model_stage64;
   int fft_precision = 0;   // 0 auto, 32, 64
   int model_steps = 8;     // (phi, DM) solver: Newton steps on the local fourth-order model per pass
   double cutoff_eps2 = 1e-20;  // harmonics outside which the model holds less than this share of its k^2-weighted power are skipped
-  int kmax_used = 0;           // 16 x the largest per-channel cut-off (0: not set)
+  std::vector<int> kmax_used;  // per model: 16 x the largest per-channel cut-off
+  DBuf kmax_dev;               // ... on the device (the FFTFIT guess of a batch with several models)
   double x_keep = 1.0;         // ... which leaves this share of the cross-spectrum to compute, store and stream
   double coarse_frac = 0.99;   // general solver: share of the model's phase information the coarse objective keeps
   std::vector<double> model_info;   // per group of 16 harmonics (scratch of the per-chunk choice)
@@ -113,7 +115,7 @@ struct pp_plan {
   std::vector<std::pair<int, DBuf>> grid_tables;
   DBuf grid_general;   // table of the last grid with bounds other than [-0.5, 0.5]
   // per-batch staging of small inputs and per-subint / per-channel workspace
-  DBuf running, minfo, njn, in_scat, in_scl, in_offs, in_P, in_errs, in_mask, in_w, in_init, in_dmg, in_snrs, in_nufits, in_nuouts, in_noise, in_models;
+  DBuf running, minfo, njn, coarse_first, coarse_njm, in_scat, in_scl, in_offs, in_P, in_errs, in_mask, in_w, in_init, in_dmg, in_snrs, in_nufits, in_nuouts, in_noise, in_models;
   DBuf nu_fit, nu_mean, wsum, nok, sigma, Ssn, Sdn, csum;
   DBuf st_x, st_xprev, st_step, st_fprev, st_lam, st_iter, st_iterc, st_done;
   DBuf o_params, o_perrs, o_nuout, o_cov, o_chi2, o_rchi2, o_snr, o_nfev, o_rc, o_scales, o_serrs, o_csnr, o_lag, o_phig;
@@ -558,13 +560,17 @@ static int rotate_rows(pp_plan* pl, RotateArgs a, bool fp64) {
   return 0;
 }
 
-static int set_freqs_impl(pp_plan* pl, const double* freqs) {
-  const int nchan = pl->nchan;
+// the frequency tables of models 0 .. ntab - 1 ([ntab, nchan]; pp_set_freqs: model 0's)
+static int set_freqs_impl(pp_plan* pl, const double* freqs, int ntab = 1) {
+  const int nchan = pl->nchan * ntab;   // rows
   std::vector<double> hf(nchan), hn2(nchan), hlg(nchan);
   if (is_device_ptr(freqs)) CK(cudaMemcpy(hf.data(), freqs, sizeof(double) * nchan, cudaMemcpyDeviceToHost));
   else memcpy(hf.data(), freqs, sizeof(double) * nchan);
   for (int n = 0; n < nchan; ++n) {
-    if (!(hf[n] > 0.0)) return fail(-1, "freqs[%d] = %g is not positive", n, hf[n]);
+    if (!(hf[n] > 0.0)) {
+      if (ntab == 1) return fail(-1, "freqs[%d] = %g is not positive", n, hf[n]);
+      return fail(-1, "freqs[%d, %d] = %g is not positive", n / pl->nchan, n % pl->nchan, hf[n]);
+    }
     hn2[n] = 1.0 / (hf[n] * hf[n]);
     hlg[n] = log2(hf[n]);
   }
@@ -594,11 +600,11 @@ extern "C" int pp_plan_set_model_steps(pp_plan_t* pl, int32_t steps) {
 
 // The coarse objective of the general solver: the leading groups of 16 harmonics that hold `frac` of the
 // (scattered) model's phase information; 0 = no coarse stage (it would not be at most half of the harmonics).
-static int choose_coarse(const std::vector<double>& info, double frac, int N) {
+static int choose_coarse(const double* info, double frac, int N) {
   const int NJ = N / 16;
-  if (!(frac > 0.0) || info.size() != (size_t)NJ || NJ < 8) return 0;
+  if (!(frac > 0.0) || NJ < 8) return 0;
   double tot = 0.0;
-  for (double v : info) tot += v;
+  for (int j = 0; j < NJ; ++j) tot += info[j];
   if (!(tot > 0.0) || !(tot < INFINITY)) return 0;
   double cum = 0.0;
   int nj = NJ;
@@ -607,19 +613,27 @@ static int choose_coarse(const std::vector<double>& info, double frac, int N) {
   return 2 * nj <= NJ ? nj : 0;
 }
 
+// the cut-offs of every channel of every model; x_keep over all of them, kmax_used per model
 static int model_cutoffs(pp_plan* pl) {
   const int N = pl->N, nchan = pl->nchan, NJ = N / 16, KJ = (N < 64 ? N : 64) / 16;
-  CK(pl->njn.need(sizeof(int) * nchan));
-  k_model_cutoff<<<nchan, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->njn.as<int>(), N, KJ, pl->cutoff_eps2);
+  const int nrows = pl->nmodel * nchan;
+  CK(pl->njn.need(sizeof(int) * nrows));
+  k_model_cutoff<<<nrows, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->njn.as<int>(), N, KJ, pl->cutoff_eps2);
   pl->stats.launches++;
-  std::vector<int> h(nchan);
-  CK(cudaMemcpyAsync(h.data(), pl->njn.p, sizeof(int) * nchan, cudaMemcpyDeviceToHost, pl->stream));
+  std::vector<int> h(nrows);
+  CK(cudaMemcpyAsync(h.data(), pl->njn.p, sizeof(int) * nrows, cudaMemcpyDeviceToHost, pl->stream));
   CK(cudaStreamSynchronize(pl->stream));
   double keep = 0.0;
-  int vmax = 0;
-  for (int v : h) { keep += v; vmax = std::max(vmax, v); }
-  pl->x_keep = keep / ((double)nchan * NJ);
-  pl->kmax_used = 16 * vmax;
+  pl->kmax_used.assign(pl->nmodel, 0);
+  for (int r = 0; r < nrows; ++r) {
+    keep += h[r];
+    int& vmax = pl->kmax_used[r / nchan];
+    vmax = std::max(vmax, 16 * h[r]);
+  }
+  pl->x_keep = keep / ((double)nrows * NJ);
+  // (a pageable source: the copy has read it when the call returns)
+  CK(pl->kmax_dev.need(sizeof(int) * pl->nmodel));
+  CK(cudaMemcpyAsync(pl->kmax_dev.p, pl->kmax_used.data(), sizeof(int) * pl->nmodel, cudaMemcpyHostToDevice, pl->stream));
   return 0;
 }
 
@@ -652,10 +666,11 @@ static void cvt_f64_f32(const void* src, void* dst, size_t n2, cudaStream_t st) 
       static_cast<const double2*>(src), static_cast<float2*>(dst), n2);
 }
 
-static int set_model_impl(pp_plan* pl, const float* model, const double* model64, const double* freqs) {
+static int set_model_impl(pp_plan* pl, int nmodel, const float* model, const double* model64, const double* freqs) {
+  if (nmodel < 1) return fail(-1, "nmodel must be >= 1 (got %d)", nmodel);
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
-  const int N = pl->N, nchan = pl->nchan;
+  const int N = pl->N, nchan = nmodel * pl->nchan;   // the model rows of all models: one transform
   const float* dmodel = nullptr;
   const double* dmodel64 = nullptr;
   const size_t nsamp = (size_t)nchan * pl->nbin;
@@ -668,12 +683,14 @@ static int set_model_impl(pp_plan* pl, const float* model, const double* model64
       dmodel64 = nullptr;
     }
   } else if (stage_in(pl, pl->model_stage, model, nsamp, &dmodel)) return -2;
-  if (set_freqs_impl(pl, freqs)) return -2;
+  if (set_freqs_impl(pl, freqs, nmodel)) return -2;
+  pl->model_set = false;
+  pl->nmodel = nmodel;
   CK(pl->mconj32.need(sizeof(float2) * (size_t)nchan * N));
   CK(pl->mconj64.need(sizeof(double2) * (size_t)nchan * N));
   CK(pl->mpow.need(sizeof(double) * (size_t)nchan * N));
   CK(pl->pn.need(sizeof(double) * nchan));
-  CK(pl->mmean.need(sizeof(float2) * N));
+  CK(pl->mmean.need(sizeof(float2) * (size_t)nmodel * N));
   ModelArgs a;
   a.model = dmodel; a.model64 = dmodel64; a.mconj32 = pl->mconj32.as<cx<float>>(); a.mconj64 = pl->mconj64.as<cx<double>>();
   a.mpow = pl->mpow.as<double>(); a.pn = pl->pn.as<double>();
@@ -685,7 +702,8 @@ static int set_model_impl(pp_plan* pl, const float* model, const double* model64
   } else {
     DISPATCH_N(N, (k_model<NN><<<row_ctas<NN>(nchan), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a)));
   }
-  k_model_mean<<<(N + 127) / 128, 128, 0, pl->stream>>>(pl->mconj64.as<cx<double>>(), pl->mmean.as<float2>(), nchan, N);
+  k_model_mean<<<dim3((N + 127) / 128, nmodel), 128, 0, pl->stream>>>(pl->mconj64.as<cx<double>>(), pl->mmean.as<float2>(),
+                                                                      pl->nchan, N);
   pl->stats.launches += 2;
   CK(cudaGetLastError());
   if (model_cutoffs(pl)) return -2;
@@ -693,14 +711,22 @@ static int set_model_impl(pp_plan* pl, const float* model, const double* model64
   return 0;
 }
 
+extern "C" int pp_set_models(pp_plan_t* pl, int32_t nmodel, const float* models, const double* freqs) {
+  if (!pl || !models || !freqs) return fail(-1, "NULL argument");
+  return set_model_impl(pl, nmodel, models, nullptr, freqs);
+}
+
+extern "C" int pp_set_models_f64(pp_plan_t* pl, int32_t nmodel, const double* models, const double* freqs) {
+  if (!pl || !models || !freqs) return fail(-1, "NULL argument");
+  return set_model_impl(pl, nmodel, nullptr, models, freqs);
+}
+
 extern "C" int pp_set_model(pp_plan_t* pl, const float* model, const double* freqs) {
-  if (!pl || !model || !freqs) return fail(-1, "NULL argument");
-  return set_model_impl(pl, model, nullptr, freqs);
+  return pp_set_models(pl, 1, model, freqs);
 }
 
 extern "C" int pp_set_model_f64(pp_plan_t* pl, const double* model, const double* freqs) {
-  if (!pl || !model || !freqs) return fail(-1, "NULL argument");
-  return set_model_impl(pl, nullptr, model, freqs);
+  return pp_set_models_f64(pl, 1, model, freqs);
 }
 
 // ----------------------------------------------------------------------------
@@ -816,6 +842,9 @@ struct FitCall {
   const uint8_t* dmask;
   const float *dscl = nullptr, *doffs = nullptr;
   const double2* table = nullptr;   // FFTFIT grid
+  const int* dmidx = nullptr;       // the model of each subint on the device (null: the plan's one model)
+  std::vector<int> hmidx;           // ... and on the host
+  std::vector<int> cfirst, cnjm;    // coarse stage with several models: the models' first subints, their levels' groups
   const char* data;                 // the caller's rows
   size_t sub_bytes, src_bytes;      // one subint as the kernels read it, and as the caller stores it
   int chunk, G, gx, nparts, align_nsplit = 1;
@@ -974,6 +1003,8 @@ static void fit_kernel_args(pp_plan* pl, FitCall& f) {
   pa.X = pl->X.as<float2>(); pa.Xlo = pl->Xlo.as<float2>(); pa.nu2 = pl->nu2.as<double>(); pa.P = f.dP; pa.nu_fit = pl->nu_fit.as<double>();
   pa.Ssn = pl->Ssn.as<double>(); pa.sigma = pl->sigma.as<double>(); pa.csum = pl->csum.as<double>(); pa.st = st;
   pa.s0 = 0; pa.nchan = nchan; pa.N = N; pa.nhalf = pl->anyn ? pl->L : 0; pa.njn = pl->njn.as<int>();
+  const ModelRows mr{f.dmidx, nchan};
+  pa.mr = mr;
   UpdateArgs& ua = f.ua;
   memset(&ua, 0, sizeof ua);
   ua.csum = pl->csum.as<double>(); ua.Ssn = pl->Ssn.as<double>(); ua.Sdn = pl->Sdn.as<double>(); ua.nu2 = pl->nu2.as<double>();
@@ -986,12 +1017,14 @@ static void fit_kernel_args(pp_plan* pl, FitCall& f) {
   ua.s0 = 0; ua.nchan = nchan; ua.nbin = pl->nbin; ua.max_iter = f.max_iter; ua.semantics = args->semantics;
   ua.fit_phi = ff[0] ? 1 : 0; ua.fit_dm = ff[1] ? 1 : 0; ua.is_toa = args->is_toa; ua.tol = f.tol; ua.box = f.box;
   ua.model_steps = pl->model_steps; ua.tol_model = (args->tol > 0 && args->tol < 1e-4) ? args->tol : 1e-4;
+  ua.mr = mr;
   if (!f.general) return;
   Pass5Args& p5 = f.p5;
   p5.X = pl->X.as<float2>(); p5.Xlo = pl->Xlo.as<float2>(); p5.mpow = pl->mpow.as<double>(); p5.nu2 = pl->nu2.as<double>(); p5.lgf = pl->lgf.as<double>();
   p5.freqs = pl->freqs.as<double>(); p5.P = f.dP; p5.nu_fit = pl->nu_fit.as<double>(); p5.Ssn = pl->Ssn.as<double>();
   p5.sigma = pl->sigma.as<double>(); p5.csum = pl->csum.as<double>(); p5.st = st; p5.s0 = 0; p5.nchan = nchan;
   p5.log10_tau = args->log10_tau; p5.nhalf = pl->anyn ? pl->L : 0; p5.nj = N / 16; p5.cstride = 1; p5.njn = pl->njn.as<int>();
+  p5.mr = mr; p5.njm = nullptr;
   Update5Args& u5 = f.u5;
   memset(&u5, 0, sizeof u5);
   u5.csum = pl->csum.as<double>(); u5.Sdn = pl->Sdn.as<double>(); u5.nu2 = pl->nu2.as<double>(); u5.lgf = pl->lgf.as<double>();
@@ -1005,6 +1038,7 @@ static void fit_kernel_args(pp_plan* pl, FitCall& f) {
   u5.taylor_finish = pl->model_steps != 1;
   for (int i = 0; i < 5; ++i) u5.flags[i] = ff[i] ? 1 : 0;
   u5.coarse = 0; u5.ctol = 0.0; u5.cstride = 1;
+  u5.mr = mr;
 }
 
 // per-subint scalars, the start state of fits from caller-supplied values, the FFTFIT grid
@@ -1014,6 +1048,7 @@ static int fit_prep(pp_plan* pl, FitCall& f) {
   p.freqs = pl->freqs.as<double>(); p.mask = f.dmask; p.weights = f.dw; p.snrs = f.dsnrs; p.nu_fits_in = f.dnufits;
   p.nu_fit = pl->nu_fit.as<double>(); p.nu_mean = pl->nu_mean.as<double>(); p.wsum = pl->wsum.as<double>();
   p.nok = pl->nok.as<int>(); p.nsub = nsub; p.nchan = pl->nchan; p.nu_fit_mode = f.args->nu_fit_mode;
+  p.mr = ModelRows{f.dmidx, pl->nchan};
   k_prep<<<(nsub + 3) / 4, 128, 0, pl->stream>>>(p);
   pl->stats.launches++;
   if (!f.want_guess) {
@@ -1072,6 +1107,7 @@ static int fit_spectra(pp_plan* pl, const FitCall& f, int c) {
   a.tw8 = pl->tw8.as<cx<double>>();
   a.s0 = s0; a.nchan = nchan; a.G = f.G; a.nparts = f.nparts;
   a.dspec = nullptr; a.ddc = nullptr; a.nhalf = 0; a.kc_true = 0; a.njn = pl->njn.as<int>();
+  a.mr = ModelRows{f.dmidx, nchan};
   if (pl->anyn) {   // rows transformed by Bluestein into the spectrum scratch, then the same emit code
     if (c == 0) {
       CK(pl->any_spec.need(sizeof(double2) * (size_t)f.chunk * nchan * N));
@@ -1099,17 +1135,22 @@ static int fit_guess(pp_plan* pl, const FitCall& f, int c) {
   GuessArgs ga;
   memset(&ga, 0, sizeof ga);
   ga.partial = pl->partial.as<float2>(); ga.mconj = pl->mmean.as<float2>(); ga.nparts = f.nparts; ga.nmodel = 1;
+  if (f.dmidx) {   // each subint's own model: its mean spectrum and its cut-off
+    ga.model = f.dmidx; ga.nused_of = pl->kmax_dev.as<int>(); ga.tmpl_by_model = 1;
+  }
   if (f.dmask) {   // the guess template is the mean model over the subint's usable channels (pptoas.py:446, 454)
     CK(pl->mmean_sub.need(sizeof(float2) * (size_t)f.chunk * N));
     k_model_mean_masked<<<dim3((N + 127) / 128, ns), 128, 0, pl->stream>>>(
-        pl->mconj64.as<cx<double>>(), f.dmask, pl->mmean.as<float2>(), pl->mmean_sub.as<float2>(), s0, pl->nchan, N);
+        pl->mconj64.as<cx<double>>(), f.dmask, pl->mmean.as<float2>(), pl->mmean_sub.as<float2>(), s0, pl->nchan, N,
+        ModelRows{f.dmidx, pl->nchan});
     pl->stats.launches++;
     ga.mconj = pl->mmean_sub.as<float2>();
     ga.nmodel = ns;  // one template per subint of the chunk
+    ga.tmpl_by_model = 0;
   }
   ga.N = N; ga.Ns = f.Ns; ga.wsum = pl->wsum.as<double>(); ga.noise = nullptr; ga.table = f.table; ga.s0 = s0;
   ga.nhalf = pl->anyn ? pl->L : 0;
-  ga.nused = pl->kmax_used;   // the mean model has no power beyond the largest channel cut-off
+  ga.nused = pl->kmax_used[0];   // the mean model has no power beyond the largest channel cut-off
   ga.phase = pl->o_phig.as<double>(); ga.lag = pl->o_lag.as<int>();
   ga.x = f.st.x; ga.DMg = f.ddmg; ga.P = f.dP; ga.nu_mean = pl->nu_mean.as<double>(); ga.nu_fit = pl->nu_fit.as<double>();
   ga.polish_tol = 1e-6;   // a start value (the last step is still applied): the Newton solver refines it
@@ -1140,45 +1181,88 @@ static int poll_running(pp_plan* pl, void (*count)(SolverState, int, int, int*),
 // Coarse stage of the general solver: Newton iterations on the objective of the low harmonics only (those
 // that hold coarse_frac of the model's phase information: a fraction of a pass each) carry the start values
 // to within a fraction of a sigma of the optimum; the full-resolution iterations then need two passes.
+// With several models the levels are chosen per model present in the chunk, from that model's first subint of
+// the chunk: a subint gets the levels a call with its model alone would give it, and sits out the others.
 static int fit_coarse(pp_plan* pl, FitCall& f, int c) {
-  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan, N = pl->N;
+  const int s0 = f.cstart[c], ns = f.cstart[c + 1] - s0, nchan = pl->nchan, N = pl->N, NJ = N / 16;
   const pp_fit_args_t* args = f.args;
   f.coarse_nj = 0;
   if (!(f.general && f.max_iter > 0 && pl->coarse_frac > 0.0 && pl->model_steps != 1 && N >= 128)) return 0;
-  // where the information sits, with the scattering of the chunk's first subint at its start values
+  // where the information sits, with the scattering of the (model's) first subint at its start values
   const uint8_t* ff = args->fit_flags;
   const bool scat = ff[3] || ff[4] || f.dscat || f.dinit;
-  CK(pl->minfo.need(sizeof(double) * (N / 16)));
-  pl->model_info.assign(N / 16, 0.0);
-  k_model_info<<<N / 16, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->lgf.as<double>(), scat ? f.st.x + (size_t)s0 * 5 : nullptr,
-                                               pl->nu_fit.as<double>() + (size_t)s0 * 3, args->log10_tau,
-                                               pl->minfo.as<double>(), nchan, N);
+  std::vector<int> models;   // the chunk's models, in order of first appearance (f.cfirst: their first subints)
+  f.cfirst.clear();
+  if (f.dmidx) {
+    std::vector<char> seen(pl->nmodel, 0);
+    for (int s = s0; s < s0 + ns; ++s) {
+      const int m = f.hmidx[s];
+      if (!seen[m]) { seen[m] = 1; models.push_back(m); f.cfirst.push_back(s); }
+    }
+  }
+  const int nm = f.dmidx ? (int)models.size() : 1;
+  CK(pl->minfo.need(sizeof(double) * NJ * nm));
+  pl->model_info.assign((size_t)NJ * nm, 0.0);
+  if (f.dmidx) {
+    CK(pl->coarse_first.need(sizeof(int) * nm));
+    CK(cudaMemcpyAsync(pl->coarse_first.p, f.cfirst.data(), sizeof(int) * nm, cudaMemcpyHostToDevice, pl->stream));
+    k_model_info<<<dim3(NJ, nm), 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->lgf.as<double>(), scat ? f.st.x : nullptr,
+                                                        pl->nu_fit.as<double>(), args->log10_tau, pl->minfo.as<double>(),
+                                                        nchan, N, ModelRows{f.dmidx, nchan}, pl->coarse_first.as<int>());
+  } else {
+    k_model_info<<<NJ, 256, 0, pl->stream>>>(pl->mpow.as<double>(), pl->lgf.as<double>(), scat ? f.st.x + (size_t)s0 * 5 : nullptr,
+                                             pl->nu_fit.as<double>() + (size_t)s0 * 3, args->log10_tau,
+                                             pl->minfo.as<double>(), nchan, N, ModelRows{nullptr, nchan}, nullptr);
+  }
   pl->stats.launches++;
-  CK(cudaMemcpyAsync(pl->model_info.data(), pl->minfo.p, sizeof(double) * (N / 16), cudaMemcpyDeviceToHost, pl->stream));
+  CK(cudaMemcpyAsync(pl->model_info.data(), pl->minfo.p, sizeof(double) * NJ * nm, cudaMemcpyDeviceToHost, pl->stream));
   CK(cudaStreamSynchronize(pl->stream));
-  const int coarse_nj = f.coarse_nj = choose_coarse(pl->model_info, pl->coarse_frac, N);
-  if (coarse_nj == 0) return 0;
   // Two levels: most of the iterations run on a cheaper objective still -- the harmonics that hold coarse_frac0
   // of the information (when that is clearly fewer) of every cstride-th channel -- the second level then needs
   // one or two.  A level is left once its Newton step is below ctol sigma (the step is still taken): the next
   // level, or the full-resolution iterations, start next to that level's optimum either way.
-  struct { int nj, cstride; double ctol; } levels[2];
-  int nlev = 0;
-  {
-    int nj0 = choose_coarse(pl->model_info, std::min(0.65, pl->coarse_frac), N);
+  // Per model: the groups of level A (0: no such level) and of level B (0: no coarse stage).
+  const int cst = nchan >= 2048 ? 8 : (nchan >= 512 ? 4 : (nchan >= 128 ? 2 : 1));
+  std::vector<int> njA(nm, 0), njB(nm, 0);
+  bool anyA = false;
+  for (int i = 0; i < nm; ++i) {
+    const double* info = pl->model_info.data() + (size_t)i * NJ;
+    const int coarse_nj = choose_coarse(info, pl->coarse_frac, N);
+    if (coarse_nj == 0) continue;
+    f.coarse_nj = std::max(f.coarse_nj, coarse_nj);
+    int nj0 = choose_coarse(info, std::min(0.65, pl->coarse_frac), N);
     if (!(nj0 > 0 && 3 * nj0 <= 2 * coarse_nj)) nj0 = coarse_nj;
-    const int cst = nchan >= 2048 ? 8 : (nchan >= 512 ? 4 : (nchan >= 128 ? 2 : 1));
-    if (nj0 < coarse_nj || cst > 1) levels[nlev++] = {nj0, cst, 2.0};
-    levels[nlev++] = {coarse_nj, 1, 1.0};
+    if (nj0 < coarse_nj || cst > 1) { njA[i] = nj0; anyA = true; }
+    njB[i] = coarse_nj;
+  }
+  if (f.coarse_nj == 0) return 0;
+  struct { int cstride; double ctol; const std::vector<int>* nj; } levels[2];
+  int nlev = 0;
+  if (anyA) levels[nlev++] = {cst, 2.0, &njA};
+  levels[nlev++] = {1, 1.0, &njB};
+  if (f.dmidx) {   // the levels' groups by model number, read by k_pass5 through the subint's model
+    f.cnjm.assign((size_t)2 * pl->nmodel, 0);
+    for (int lv = 0; lv < nlev; ++lv)
+      for (int i = 0; i < nm; ++i) f.cnjm[(size_t)lv * pl->nmodel + models[i]] = (*levels[lv].nj)[i];
+    CK(pl->coarse_njm.need(sizeof(int) * 2 * pl->nmodel));
+    CK(cudaMemcpyAsync(pl->coarse_njm.p, f.cnjm.data(), sizeof(int) * 2 * pl->nmodel, cudaMemcpyHostToDevice, pl->stream));
   }
   Pass5Args& p5 = f.p5;
   Update5Args& u5 = f.u5;
   u5.coarse = 1;
   for (int lv = 0; lv < nlev; ++lv) {
     const int max_coarse = std::min(f.max_iter, 12);
-    p5.nj = levels[lv].nj; p5.cstride = u5.cstride = levels[lv].cstride; u5.ctol = levels[lv].ctol;
+    const std::vector<int>& nj = *levels[lv].nj;
+    const bool sitout = std::find(nj.begin(), nj.end(), 0) != nj.end();   // some model has no such level
+    if (f.dmidx) { p5.nj = 0; p5.njm = pl->coarse_njm.as<int>() + (size_t)lv * pl->nmodel; }
+    else p5.nj = nj[0];
+    p5.cstride = u5.cstride = levels[lv].cstride; u5.ctol = levels[lv].ctol;
     const int gx5 = ((nchan + p5.cstride - 1) / p5.cstride + 31) / 32;
-    mark(f, "coarse level: %d of %d harmonic groups, every %d-th channel", p5.nj, N / 16, p5.cstride);
+    if (sitout) {
+      k_coarse_sitout<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, p5.mr, p5.njm, s0, ns, 1);
+      pl->stats.launches++;
+    }
+    mark(f, "coarse level: %d of %d harmonic groups, every %d-th channel", *std::max_element(nj.begin(), nj.end()), NJ, p5.cstride);
     for (int it = 0; it < max_coarse; ++it) {
       {
         SpanGuard g(pl, SP_COARSE);
@@ -1196,9 +1280,13 @@ static int fit_coarse(pp_plan* pl, FitCall& f, int c) {
     }
     k_coarse_end<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, s0, ns);
     pl->stats.launches++;
+    if (sitout) {
+      k_coarse_sitout<<<(ns + 127) / 128, 128, 0, pl->stream>>>(f.st, p5.mr, p5.njm, s0, ns, 0);
+      pl->stats.launches++;
+    }
   }
   // (k_update5 reads ctol only in the coarse stage)
-  p5.nj = N / 16; p5.cstride = u5.cstride = 1; u5.coarse = 0; u5.ctol = 0.0;
+  p5.nj = NJ; p5.njm = nullptr; p5.cstride = u5.cstride = 1; u5.coarse = 0; u5.ctol = 0.0;
   return 0;
 }
 
@@ -1302,7 +1390,39 @@ static int fit_align_finish(pp_plan* pl, const FitCall& f) {
   return 0;
 }
 
+// the model of each subint, checked on the host before any kernel reads it (a device index costs one small copy)
+static int fit_model_index(pp_plan* pl, FitCall& f, const int32_t* model_index) {
+  if (!model_index) {
+    if (pl->nmodel > 1) return fail(-1, "model_index is required: the plan holds %d models", pl->nmodel);
+    return 0;
+  }
+  const int nsub = f.nsub;
+  f.hmidx.resize(nsub);
+  const bool dev = is_device_ptr(model_index);
+  if (dev) {
+    CK(cudaMemcpyAsync(f.hmidx.data(), model_index, sizeof(int) * nsub, cudaMemcpyDeviceToHost, pl->stream));
+    CK(cudaStreamSynchronize(pl->stream));
+  } else {
+    memcpy(f.hmidx.data(), model_index, sizeof(int) * nsub);
+  }
+  for (int s = 0; s < nsub; ++s)
+    if (f.hmidx[s] < 0 || f.hmidx[s] >= pl->nmodel)
+      return fail(-1, "model_index[%d] = %d is outside [0, %d)", s, f.hmidx[s], pl->nmodel);
+  if (dev) f.dmidx = model_index;
+  else {
+    CK(pl->in_models.need(sizeof(int) * nsub));
+    CK(cudaMemcpyAsync(pl->in_models.p, f.hmidx.data(), sizeof(int) * nsub, cudaMemcpyHostToDevice, pl->stream));
+    f.dmidx = pl->in_models.as<int>();
+  }
+  return 0;
+}
+
 extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_fit_out_t* out) {
+  return pp_fit_batch_models(pl, args, nullptr, out);
+}
+
+extern "C" int pp_fit_batch_models(pp_plan_t* pl, const pp_fit_args_t* args, const int32_t* model_index,
+                                   const pp_fit_out_t* out) {
   if (!pl || !args || !out) return fail(-1, "NULL argument");
   if (!pl->model_set) return fail(-1, "pp_set_model must be called before pp_fit_batch");
   if (!args->data || !args->P) return fail(-1, "data and P are required");
@@ -1330,6 +1450,8 @@ extern "C" int pp_fit_batch(pp_plan_t* pl, const pp_fit_args_t* args, const pp_f
   f.args = args; f.out = out; f.general = general; f.i16 = i16; f.f64 = f64; f.nsub = args->nsub;
   f.Ns = args->Ns > 0 ? args->Ns : 100;
   if (f.Ns < 2) return fail(-1, "Ns must be >= 2");
+  if (out->align_sum && pl->nmodel > 1) return fail(-1, "align_sum needs one model (the plan holds %d)", pl->nmodel);
+  if (int rc = fit_model_index(pl, f, model_index)) return rc;
   // passes are launched only while some subint is still running (polled), so a generous limit costs
   // nothing for batches started from the FFTFIT guess (1-2 passes) and lets caller-supplied start
   // values far from the optimum converge (10-14 passes from 0.05-0.08 turn away, tools/far_start_probe.py)

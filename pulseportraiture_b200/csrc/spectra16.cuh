@@ -51,6 +51,7 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
   __syncthreads();
 
   const int sl = blockIdx.y, s = a.s0 + sl;
+  const int mb = KEEPD ? 0 : a.mr.row0(s);   // the subint's model (the fused ppalign sum takes one model)
   const int ch_begin = blockIdx.x * a.G;
   const int ch_end = min(ch_begin + a.G, a.nchan);
   const int nsteps = ch_end - ch_begin;
@@ -81,7 +82,7 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
   auto fetch_model = [&](int ch) {   // ... and the float conj(model) row of channel ch
     if (t == 0) {
       mbar_expect_tx(&mbar[1], N * (unsigned)sizeof(cx<float>));
-      bulk_g2s(mstage, a.mconj32 + (size_t)ch * N, N * (unsigned)sizeof(cx<float>), &mbar[1]);
+      bulk_g2s(mstage, a.mconj32 + (size_t)(mb + ch) * N, N * (unsigned)sizeof(cx<float>), &mbar[1]);
     }
   };
   fetch(0);
@@ -134,7 +135,7 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
     __syncthreads();   // staged row consumed; the previous row's split reads of buf and of the model row are done
     fetch(step + 1);
     const bool doX = a.X != nullptr;
-    const int kcut = a.njn ? 16 * a.njn[ch] : N;
+    const int kcut = a.njn ? 16 * a.njn[mb + ch] : N;
     if (doX) fetch_model(ch);
     dft16(v);
     {
@@ -162,12 +163,12 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
     // (p = t + 64 i; the special unit of thread 0 uses p = 0 / 128).
     cx<F> mc64 = mk<F>(0.5, 0.25);
     const int po0 = first ? 128 : t;           // the odd outputs of unit 0
-    if (doX) mc64 = a.mconj64[(size_t)ch * N + t];   // the one double-precision factor (lo slot t)
+    if (doX) mc64 = a.mconj64[(size_t)(mb + ch) * N + t];   // the one double-precision factor (lo slot t)
     float wgt = 0.f;
     double shift = 0.0;
     if constexpr (GUESS) {
       wgt = (float)(a.weights ? a.weights[(size_t)s * a.nchan + ch] : 1.0);
-      shift = Dfac != 0.0 ? Dfac * (a.nu2[ch] - numean2) : 0.0;
+      shift = Dfac != 0.0 ? Dfac * (a.nu2[mb + ch] - numean2) : 0.0;
     }
     twiddle16(v, tw[kk]);
     dft16(v);
@@ -280,7 +281,7 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
     const bool ok = fused && (sF2 > 0.0) && (sF2 < 1e300);
     const size_t o = (size_t)s * a.nchan + fch;
     a.sigma[o] = ok ? sig : 0.0;
-    a.Ssn[o] = ok ? a.pn[fch] / sF2 : 0.0;
+    a.Ssn[o] = ok ? a.pn[mb + fch] / sF2 : 0.0;
     a.Sdn[o] = ok ? keep_all / sF2 : 0.0;
   }
   if constexpr (GUESS) {

@@ -90,6 +90,21 @@ def bounds_array(bounds):
     return None if np.all(np.isnan(out)) else out
 
 
+def model_bytes(nchan, nbin):
+    """Device memory one model of pp_set_models costs on a [nchan, nbin] plan (include/ppb200.h): nchan * (32 N + 36)
+    + 8 N + 12 bytes, N = nbin/2 slots per spectrum row (other than power-of-two nbin: the smallest power of two above
+    nbin/2, plus 16 N bytes per channel of transform scratch).  The portraits' staging copy is not counted."""
+    nchan, nbin = int(nchan), int(nbin)
+    pow2 = nbin & (nbin - 1) == 0
+    N = nbin // 2
+    if not pow2:
+        N = 1
+        while N < nbin // 2 + 1:
+            N *= 2
+    per_chan = 32 * N + 36 + (0 if pow2 else 16 * N)
+    return nchan * per_chan + 8 * N + 12
+
+
 class WidebandPlan(object):
     """Device plan for portraits of shape [nchan, nbin] (C ABI pp_plan_*)."""
 
@@ -100,6 +115,7 @@ class WidebandPlan(object):
                                             C.byref(self._h)), "pp_plan_create")
         self.nchan, self.nbin, self.device = int(nchan), int(nbin), int(device)
         self.freqs = None
+        self.nmodel = 0
         self._pool = PinnedPool(self._lib)
         if stream is not None:
             self.set_stream(stream)
@@ -179,17 +195,30 @@ class WidebandPlan(object):
         """Model portrait [nchan, nbin] (numpy array or torch tensor, host or CUDA).  float64 models go to the
         device as they are (pp_set_model_f64: no float32 rounding floor in the model spectrum, which the
         harmonic cut-off needs to be effective); anything else is taken as float32."""
+        self._set_models(1, model, freqs, (self.nchan, self.nbin), (self.nchan,))
+
+    def set_models(self, models, freqs):
+        """nmodel model portraits [nmodel, nchan, nbin] and their frequency tables [nmodel, nchan] MHz
+        (pp_set_models; dtypes as set_model).  fit_batch(..., model_index) then fits subint s against model
+        model_index[s].  Each model costs model_bytes(nchan, nbin) of device memory."""
+        nmodel = int(models.shape[0])
+        self._set_models(nmodel, models, freqs, (nmodel, self.nchan, self.nbin), (nmodel, self.nchan))
+
+    def _set_models(self, nmodel, models, freqs, mshape, fshape):
         keep = []
-        fp = _ptr(np.asarray(freqs, dtype=np.float64), np.float64, keep, "freqs",
-                  (self.nchan,))
-        is64 = (str(model.dtype).endswith("float64")) if hasattr(model, "dtype") else False
+        fp = _ptr(freqs if _is_torch(freqs) else np.asarray(freqs, dtype=np.float64), np.float64, keep, "freqs",
+                  fshape)
+        is64 = (str(models.dtype).endswith("float64")) if hasattr(models, "dtype") else False
         if is64:
-            mp = _ptr(model, np.float64, keep, "model", (self.nchan, self.nbin))
-            _ffi.check(self._lib.pp_set_model_f64(self._h, mp, fp), "pp_set_model_f64")
+            mp = _ptr(models, np.float64, keep, "model", mshape)
+            _ffi.check(self._lib.pp_set_models_f64(self._h, nmodel, mp, fp), "pp_set_model_f64")
         else:
-            mp = _ptr(model, np.float32, keep, "model", (self.nchan, self.nbin))
-            _ffi.check(self._lib.pp_set_model(self._h, mp, fp), "pp_set_model")
-        self.freqs = np.array(freqs, dtype=np.float64)
+            mp = _ptr(models, np.float32, keep, "model", mshape)
+            _ffi.check(self._lib.pp_set_models(self._h, nmodel, mp, fp), "pp_set_model")
+        f = freqs.detach().cpu().numpy() if _is_torch(freqs) else freqs
+        # the table of the rotation, alignment and model-generation calls: model 0's
+        self.freqs = np.array(f, dtype=np.float64).reshape(-1, self.nchan)[0]
+        self.nmodel = nmodel
 
     # ---- batched wideband fit ---------------------------------------------------
     def fit_batch(self, data, P, errs=None, chan_mask=None, weights=None,
@@ -198,9 +227,12 @@ class WidebandPlan(object):
                   log10_tau=False, option=0, is_toa=True, Ns=100, max_iter=0,
                   tol=0.0, semantics="full", want_chan_sums=False, nsub=None,
                   pinned_results=False, scat_guess=None, align=False, dat_scl=None, dat_offs=None,
-                  bounds=None):
+                  bounds=None, model_index=None):
         """Fit every subint of data[nsub, nchan, nbin] (float32, host numpy or
         CUDA torch tensor).  Returns a dict of numpy arrays.
+
+        model_index: [nsub] int32 (numpy or torch, host or CUDA) after set_models: subint s is fit against
+        model model_index[s] and its frequency table.  None: the plan's one model.
 
         bounds: up to five (lower, upper) pairs for phi, DM, GM, tau (log10 tau with
         log10_tau) and alpha as scipy's TNC takes them (None = unbounded).
@@ -257,6 +289,7 @@ class WidebandPlan(object):
         a.tol = float(tol)
         a.scat_guess = _ptr(scat_guess, np.float64, keep, "scat_guess", (nsub, 2))
         a.bounds = _ptr(bounds_array(bounds), np.float64, keep, "bounds", (5, 2))
+        mi = _ptr(model_index, np.int32, keep, "model_index", (nsub,))
 
         spec = {
             "params": ((nsub, 5), np.float64), "param_errs": ((nsub, 5), np.float64),
@@ -280,7 +313,7 @@ class WidebandPlan(object):
         o = _ffi.FitOut()
         for k, v in res.items():
             setattr(o, k, v.ctypes.data)
-        _ffi.check(self._lib.pp_fit_batch(self._h, C.byref(a), C.byref(o)),
+        _ffi.check(self._lib.pp_fit_batch_models(self._h, C.byref(a), mi, C.byref(o)),
                    "pp_fit_batch")
         del keep
         return res

@@ -160,13 +160,18 @@ class MultiGPUFitter(object):
         for p in self.plans:
             p.set_model(model, freqs)
 
+    def set_models(self, models, freqs):
+        """Every plan holds every model (WidebandPlan.set_models); model_index is sliced with the subints."""
+        for p in self.plans:
+            p.set_models(models, freqs)
+
     def close(self):
         for p in self.plans:
             p.close()
 
     # keyword arguments of WidebandPlan.fit_batch that carry one row per subint
     PER_SUBINT = ("errs", "chan_mask", "weights", "init", "DM_guess", "snrs", "nu_fits", "nu_outs",
-                  "scat_guess", "dat_scl", "dat_offs")
+                  "scat_guess", "dat_scl", "dat_offs", "model_index")
     # results that are sums over the subints of a shard (the fused ppalign accumulation)
     SUMMED = ("align_sum", "align_wsum")
 

@@ -16,6 +16,11 @@ import numpy as np
 from . import pplib
 from .pplib import DataBunch, read_model, gen_gaussian_portrait, scattering_alpha  # noqa: F401
 from .pplib import get_plan, _f32, _dev, _mdl
+from .engine import model_bytes
+
+# device memory GetTOAs.get_TOAs lets one archive's models take at once (pp_set_models); more models are set and
+# fit in several rounds
+_MODEL_BUDGET_BYTES = 4 << 30
 
 max_nfile = 999                                  # pptoas.py:18-23
 rm_baseline = bool(pplib.F0_fact)                # pptoas.py:25-29
@@ -427,7 +432,10 @@ class GetTOAs:
 
             # subints with a single usable channel are fit for phase only
             # (pptoas.py:475-478); two channels drop GM (479-483)
-            groups = {}
+            # Every model of the archive goes to the plan in one pp_set_models call (several when they exceed
+            # _MODEL_BUDGET_BYTES of device memory) and every flags group is one fit_batch: each subint is fit
+            # against its own model (pp_fit_batch_models), as the reference's per-subint loop does.
+            flags_by_sub = {}
             for isub in ok_isubs:
                 if nok[isub] == 1:
                     flags = (1, 0, 0, 0, 0)
@@ -435,15 +443,33 @@ class GetTOAs:
                     flags = tuple(self.fit_flags[:2] + [0] + self.fit_flags[3:])
                 else:
                     flags = tuple(self.fit_flags)
-                groups.setdefault((int(table_of[isub]), flags), []).append(isub)
+                flags_by_sub[isub] = flags
+            model_ids = sorted(models)
+            per_call = max(1, int(_MODEL_BUDGET_BYTES // model_bytes(nchan, nbin)))
+            work = []                                  # (model ids set at once, flags, subints)
+            for m0 in range(0, len(model_ids), per_call):
+                mset = model_ids[m0:m0 + per_call]
+                inset = set(mset)
+                groups = {}
+                for isub in ok_isubs:
+                    if int(table_of[isub]) in inset:
+                        groups.setdefault(flags_by_sub[isub], []).append(isub)
+                for flags, isubs in sorted(groups.items()):
+                    work.append((mset, flags, isubs))
             res, flags_of = {}, {}
             fit_start = time.time()
-            table_set = None
-            for (t, flags), isubs in sorted(groups.items()):
-                if t != table_set:
-                    pl.set_model(_mdl(models[t]), tables[t])
-                    table_set = t
+            mset_on = None
+            for mset, flags, isubs in work:
+                if mset is not mset_on:
+                    ms = [_mdl(models[t]) for t in mset]
+                    dt = np.float32 if all(m.dtype == np.float32 for m in ms) else np.float64
+                    pl.set_models(np.stack([np.asarray(m, dtype=dt) for m in ms]),
+                                  np.stack([tables[t] for t in mset]))
+                    local = {t: i for i, t in enumerate(mset)}
+                    mset_on = mset
                 idx = np.asarray(isubs, dtype=int)
+                model_index = None if len(mset) == 1 else \
+                    np.array([local[int(table_of[i])] for i in isubs], dtype=np.int32)
                 if len(idx) > 1 and np.all(np.diff(idx) == 1):
                     idx = slice(int(idx[0]), int(idx[-1]) + 1)      # a contiguous range: views, no gather copy
                 nidx = len(isubs)
@@ -461,7 +487,7 @@ class GetTOAs:
                     nu_fit_mode=mode, nu_outs=None if nu_outs_in is None else nu_outs_in[idx],
                     fit_flags=flags, log10_tau=self.log10_tau, option=0, is_toa=True,
                     Ns=100, semantics="full", bounds=fit_bounds,
-                    scat_guess=None if scat_in is None else scat_in[idx])
+                    scat_guess=None if scat_in is None else scat_in[idx], model_index=model_index)
                 for k, v in r.items():                     # results of all groups, by subint
                     if isinstance(v, np.ndarray) and len(v) == nidx:
                         if k not in res:
