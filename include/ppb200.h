@@ -163,7 +163,11 @@ typedef struct {
   int32_t is_toa;           /* pptoaslib.py:1048-1050                          */
   int32_t Ns;               /* FFTFIT grid size (pplib.py:2054), default 100   */
   int32_t max_iter;         /* Newton passes per subint (0 = default 40; passes run
-                               only while some subint has not converged)       */
+                               only while some subint has not converged).
+                               < 0: evaluate only: one pass at init (or at the
+                               FFTFIT guess), the epilogue (chi2, scales, snr,
+                               errors, nu_out, chan_sums) at that point, no
+                               step; return code 0 (pplib.get_scales)         */
   double tol;               /* convergence: |step| < tol * 1-sigma (0 = default:
                                1e-3; the (phi, DM) solver's model-based steps
                                stop at min(tol, 1e-4), see
@@ -213,7 +217,11 @@ typedef struct {
   double* chan_sums;    /* [nsub,nchan,9] per-channel C,Cth,Cthth,Ct,Ctt,Ctht,
                            S,St,Stt at the last evaluated point (for host
                            epilogues); for the (phi, DM) solver slots 3, 4 hold
-                           the third and fourth theta-derivatives of C instead */
+                           the third and fourth theta-derivatives of C instead
+                           and slots 5-8 are 0.  The (phi, DM) solver runs when
+                           GM, tau and alpha are not fit, GM and tau are 0 in a
+                           host init, log10_tau is off and scat_guess is NULL
+                           (a device init takes the general solver)           */
   double* align_sum;    /* [nchan,nbin] ppalign (ppalign.py:197-213), fused: the
                            sum over the batch of w_sn * rotate(data_sn, phi_s,
                            DM_s about nu_out_s) with the FITTED phi_s, DM_s and

@@ -914,6 +914,8 @@ static int fit_workspace(pp_plan* pl, FitCall& f) {
   CK(pl->Ssn.need(sizeof(double) * nsc));
   CK(pl->Sdn.need(sizeof(double) * nsc));
   CK(pl->csum.need(sizeof(double) * nsc * kNCsum));
+  // k_pass2 writes slots 0-4 only: the (phi, DM) layout returns slots 5-8 as 0, not what an earlier call left there
+  if (!f.general && f.out->chan_sums) CK(cudaMemsetAsync(pl->csum.p, 0, sizeof(double) * nsc * kNCsum, pl->stream));
   CK(pl->st_x.need(sizeof(double) * nsub * 5));
   CK(pl->st_xprev.need(sizeof(double) * nsub * 5));
   CK(pl->st_step.need(sizeof(double) * nsub * 5));
