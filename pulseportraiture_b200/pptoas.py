@@ -89,6 +89,14 @@ _DB_FIELDS = ["backend", "backend_delay", "bw", "doppler_factors", "DM", "dmc",
               "flux_prof", "prof", "prof_noise", "prof_SNR"]
 
 
+def _chan_mask(nsub, nchan, ok_ichans, isubs):
+    """uint8 [nsub, nchan]: 1 at the usable channels ok_ichans[i] of every subint i in isubs, 0 elsewhere."""
+    m = np.zeros((nsub, nchan), dtype=np.uint8)
+    for i in isubs:
+        m[i, np.asarray(ok_ichans[i], dtype=int)] = 1
+    return m
+
+
 def save_databunch(path, data):
     """Write the load_data field contract (pplib.py:2803-2813) to ``.npz``."""
     out = {}
@@ -100,10 +108,7 @@ def save_databunch(path, data):
             out["epochs_day"] = np.array([e.intday() for e in v])
             out["epochs_frac"] = np.array([e.fracday() for e in v])
         elif k == "ok_ichans":
-            m = np.zeros((data["nsub"], data["nchan"]), dtype=np.uint8)
-            for i, idx in enumerate(v):
-                m[i, np.asarray(idx, dtype=int)] = 1
-            out["ok_mask"] = m
+            out["ok_mask"] = _chan_mask(data["nsub"], data["nchan"], v, range(len(v)))
         else:
             out[k] = np.asarray(v)
     for k in _RAW_FIELDS:
@@ -212,6 +217,37 @@ def tscrunch_databunch(d):
     return out
 
 
+# the result lists of GetTOAs (pptoas.py:102-143): the TOA methods append one entry per archive fitted, except
+# TOA_list (one per TOA) and ok_idatafiles (one per archive loaded)
+_RESULT_LISTS = ("obs", "doppler_fs", "nu0s", "nu_fits", "nu_refs", "ok_idatafiles",
+                 "ok_isubs", "epochs", "MJDs", "Ps", "phis", "phi_errs", "TOAs",
+                 "TOA_errs", "DM0s", "DMs", "DM_errs", "DeltaDM_means", "DeltaDM_errs",
+                 "GMs", "GM_errs", "taus", "tau_errs", "alphas", "alpha_errs", "scales",
+                 "scale_errs", "snrs", "channel_snrs", "profile_fluxes",
+                 "profile_flux_errs", "fluxes", "flux_errs", "flux_freqs", "red_chi2s",
+                 "channel_red_chi2s", "covariances", "nfevals", "rcs", "fit_durations",
+                 "order", "TOA_list", "zap_channels")
+
+
+def _archive_entries(d):
+    """The result-list entries that describe the archive itself, the same for both TOA methods."""
+    return dict(order=d.filename, obs=DataBunch(telescope=d.telescope, backend=d.backend, frontend=d.frontend),
+                doppler_fs=d.doppler_factors, ok_isubs=np.asarray(d.ok_isubs, dtype=int), epochs=d.epochs,
+                MJDs=np.array([e.in_days() for e in d.epochs], dtype=np.double),
+                Ps=np.asarray(d.Ps, dtype=np.float64))
+
+
+def _nu_fit_guesses(d, mask):
+    """[nsub, 3] nu_fits: guess_fit_freq (pptoas.py:402) of every subint in ok_isubs over its usable channels (mask),
+    0 for the other subints."""
+    ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+    out = np.zeros((int(d.nsub), 3))
+    out[ok_isubs, :] = pplib.guess_fit_freq_batch(np.asarray(d.freqs, dtype=np.float64)[ok_isubs],
+                                                  np.asarray(d.SNRs, dtype=np.float64)[ok_isubs, 0],
+                                                  mask[ok_isubs])[:, None]
+    return out
+
+
 class GetTOAs:
     """Measure TOAs and DMs from wideband data (pptoas.py:75-743)."""
 
@@ -228,17 +264,42 @@ class GetTOAs:
             sys.exit()
         self.is_FITS_model = False
         self.modelfile = modelfile
-        for name in ("obs", "doppler_fs", "nu0s", "nu_fits", "nu_refs", "ok_idatafiles",
-                     "ok_isubs", "epochs", "MJDs", "Ps", "phis", "phi_errs", "TOAs",
-                     "TOA_errs", "DM0s", "DMs", "DM_errs", "DeltaDM_means", "DeltaDM_errs",
-                     "GMs", "GM_errs", "taus", "tau_errs", "alphas", "alpha_errs", "scales",
-                     "scale_errs", "snrs", "channel_snrs", "profile_fluxes",
-                     "profile_flux_errs", "fluxes", "flux_errs", "flux_freqs", "red_chi2s",
-                     "channel_red_chi2s", "covariances", "nfevals", "rcs", "fit_durations",
-                     "order", "TOA_list", "zap_channels"):
-            setattr(self, name, [])                         # pptoas.py:102-143
+        for name in _RESULT_LISTS:
+            setattr(self, name, [])
+        # by index into datafiles: the archive as fitted, and (table_of, models) of get_TOAs, for get_channels_to_zap
+        self._archives, self._model_tables = {}, {}
         self.instrumental_response_dict = self.ird = {'DM': 0.0, 'wids': [], 'irf_types': []}
         self.quiet = quiet
+
+    def _append_archive(self, entries):
+        """Append one archive's results, {result-list name: entry}, to the lists _RESULT_LISTS names."""
+        for name, value in entries.items():
+            getattr(self, name).append(value)
+
+    def _archives_to_fit(self, datafile, tscrunch, quiet):
+        """(iarch, DataBunch) of every archive that loads and has subints to fit, listed in ok_idatafiles and kept in
+        _archives (pptoas.py:247-265)."""
+        datafiles = self.datafiles if datafile is None else [datafile]
+        for iarch, datafile in enumerate(datafiles):
+            try:
+                d = datafile if isinstance(datafile, dict) else load_data(datafile)
+            except (RuntimeError, IOError, OSError):
+                if not quiet:
+                    print("Cannot load_data(%s).  Skipping it." % datafile)
+                continue
+            if d.get("dmc"):                                # pptoas.py:256-265
+                if not quiet:
+                    print("%s is dedispersed (dmc = 1).  Restoring the dispersion." % d.filename)
+                d = restore_dispersion(d)
+            if tscrunch:                                    # load_data(..., tscrunch=True), pptoas.py:253
+                d = tscrunch_databunch(d)
+            if not len(d.ok_isubs):
+                if not quiet:
+                    print("No subints to fit for %s.  Skipping it." % d.filename)
+                continue
+            self.ok_idatafiles.append(iarch)
+            self._archives[iarch] = d
+            yield iarch, d
 
     def _model_depends_on_P(self, fit_scat, add_instrumental_response):
         """True when the model portrait differs from subint to subint through the period: a .gmodel
@@ -279,6 +340,37 @@ class GetTOAs:
         return pplib.gen_gaussian_portrait_device(self.model_code, unscat_params, 0.0, phases,
                                                   freqs_row, self.model_nu_ref)
 
+    def _model_tables_of(self, d, fit_scat, add_instrumental_response, by_period):
+        """(tables, table_of, models): an archive's frequency tables, each subint's index into them (-1: not fit) and
+        the model of every index an ok subint uses.  The reference builds a model per subint (freqs = data.freqs[isub],
+        pptoas.py:346, 356-379); here subints share one when they share a table, or with by_period a (table, period)."""
+        freqs = np.asarray(d.freqs, dtype=np.float64)
+        Ps = np.asarray(d.Ps, dtype=np.float64)
+        ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+        tables, table_of = _freq_tables(freqs)
+        if not by_period:
+            models = {t: self._model_for(d.phases, tables[t], Ps[ok_isubs[table_of[ok_isubs] == t][0]],
+                                         fit_scat, add_instrumental_response)
+                      for t in np.unique(table_of[ok_isubs])}
+            return tables, table_of, models
+
+        # (the smearing width uses the spacing of the subint's first two usable channels: the
+        # reference evaluates instrumental_response_port_FT on freqsx, pptoas.py:390-392)
+        def cbw(i):
+            okc_ = np.asarray(d.ok_ichans[i], dtype=int)
+            if not (add_instrumental_response and self.ird['DM']) or len(okc_) < 2:
+                return 0.0
+            return float(abs(freqs[i, okc_[1]] - freqs[i, okc_[0]]))
+        ok = set(ok_isubs)
+        keys = [(int(table_of[i]), float(Ps[i]), cbw(i) if i in ok else 0.0) for i in range(int(d.nsub))]
+        uniq = sorted(set(keys[i] for i in ok_isubs))
+        table_of = np.array([uniq.index(k) if k in uniq else -1 for k in keys])
+        tables = np.array([tables[k[0]] for k in uniq])
+        models = {t: self._model_for(d.phases, tables[t], uniq[t][1], fit_scat, add_instrumental_response,
+                                     chan_bw=uniq[t][2] or None)
+                  for t in range(len(uniq))}
+        return tables, table_of, models
+
     def get_TOAs(self, datafile=None, tscrunch=False, nu_refs=None, DM0=None,
                  bary=True, fit_DM=True, fit_GM=False, fit_scat=False,
                  log10_tau=True, scat_guess=None, fix_alpha=False,
@@ -309,164 +401,124 @@ class GetTOAs:
             log10_tau = False                               # pptoas.py:229-230
         self.log10_tau = log10_tau
         self.scat_guess, self.DM0, self.bary = scat_guess, DM0, bary
-        nu_ref_tuple, nu_fit_tuple = nu_refs, nu_fits
         start = time.time()
-        datafiles = self.datafiles if datafile is None else [datafile]
-        for iarch, datafile in enumerate(datafiles):
-            try:
-                data = datafile if isinstance(datafile, dict) else load_data(datafile)
-            except (RuntimeError, IOError, OSError):
-                if not quiet:
-                    print("Cannot load_data(%s).  Skipping it." % datafile)
-                continue
-            if data.get("dmc"):                             # pptoas.py:256-265
-                if not quiet:
-                    print("%s is dedispersed (dmc = 1).  Restoring the dispersion." % data.filename)
-                data = restore_dispersion(data)
-            if tscrunch:                                    # load_data(..., tscrunch=True), pptoas.py:253
-                data = tscrunch_databunch(data)
-            if not len(data.ok_isubs):
-                if not quiet:
-                    print("No subints to fit for %s.  Skipping it." % data.filename)
-                continue
-            self.ok_idatafiles.append(iarch)
-            self._archives = getattr(self, "_archives", {})
-            self._archives[iarch] = data
-            d = data
-            nsub, nchan, nbin = int(d.nsub), int(d.nchan), int(d.nbin)
-            ok_isubs = np.asarray(d.ok_isubs, dtype=int)
-            source = d.source if d.source is not None else "noname"  # noqa: F841
-            obs = DataBunch(telescope=d.telescope, backend=d.backend, frontend=d.frontend)
-            freqs = np.asarray(d.freqs, dtype=np.float64)
-            Ps = np.asarray(d.Ps, dtype=np.float64)
-            DM_stored = float(d.DM)
-            DM0_arch = DM_stored if self.DM0 is None else self.DM0
-            MJDs = np.array([e.in_days() for e in d.epochs], dtype=np.double)
-            # Per-subint frequency tables (freqs = data.freqs[isub], pptoas.py:346): the reference
-            # rebuilds the model for every subint (pptoas.py:356-379); here subints that share a
-            # table share one model and one batch.
-            tables, table_of = _freq_tables(freqs)
-            if self._model_depends_on_P(fit_scat, add_instrumental_response):
-                # one model per (frequency table, period): subints with their own period get their own
-                # model and batch, as in the reference's per-subint loop
-                # (the smearing width uses the spacing of the subint's first two usable channels: the
-                # reference evaluates instrumental_response_port_FT on freqsx, pptoas.py:390-392)
-                def cbw(i):
-                    okc_ = np.asarray(d.ok_ichans[i], dtype=int)
-                    if not (add_instrumental_response and self.ird['DM']) or len(okc_) < 2:
-                        return 0.0
-                    return float(abs(freqs[i, okc_[1]] - freqs[i, okc_[0]]))
-                keys = [(int(table_of[i]), float(Ps[i]), cbw(i) if i in set(ok_isubs) else 0.0) for i in range(nsub)]
-                uniq = sorted(set(keys[i] for i in ok_isubs))
-                table_of = np.array([uniq.index(k) if k in uniq else -1 for k in keys])
-                tables = np.array([tables[k[0]] for k in uniq])
-                models = {t: self._model_for(d.phases, tables[t], uniq[t][1], fit_scat, add_instrumental_response,
-                                             chan_bw=uniq[t][2] or None)
-                          for t in range(len(uniq))}
-            else:
-                models = {t: self._model_for(d.phases, tables[t], Ps[ok_isubs[table_of[ok_isubs] == t][0]],
-                                             fit_scat, add_instrumental_response)
-                          for t in np.unique(table_of[ok_isubs])}
-            model = models[table_of[ok_isubs[0]]]
+        for iarch, d in self._archives_to_fit(datafile, tscrunch, quiet):
+            by_period = self._model_depends_on_P(fit_scat, add_instrumental_response)
+            tables, table_of, models = self._model_tables_of(d, fit_scat, add_instrumental_response, by_period)
+            mask = _chan_mask(int(d.nsub), int(d.nchan), d.ok_ichans, d.ok_isubs)
+            if method == 'TNC' and bounds is None:          # pptoas.py:461-469
+                # bounds is rebound: the later archives keep this box, its tau floor from this archive's nbin
+                tau_bounds = (np.log10((10 * int(d.nbin)) ** -1), None) if self.log10_tau else (0.0, None)
+                bounds = [(None, None), (None, None), (None, None), tau_bounds, (-10.0, 10.0)]
+            nu_fits_in, mode, nu_outs_in, scat_in, fit_bounds = self._fit_inputs(d, mask, nu_refs, nu_fits,
+                                                                                 fit_scat, method, bounds)
+            self._model_tables[iarch] = (table_of, {t: np.asarray(m, dtype=np.float64) for t, m in models.items()})
+            res, flags_of, fit_duration = self._fit_archive(d, tables, table_of, models, mask, nu_fits_in, mode,
+                                                            nu_outs_in, scat_in, fit_bounds)
+            out = _archive_entries(d)
+            out.update(nu0s=d.nu0, fit_durations=fit_duration)
+            out.update(self._subint_toas(d, models, table_of, mask, res, flags_of, nu_fits_in, nu_refs,
+                                         print_phase, print_flux, print_parangle, addtnl_toa_flags))
+            out.update(self._archive_arrays(d, res, out["DMs"], out["DM_errs"], method))
+            self._append_archive(out)
+            if not quiet:
+                ok_isubs = out["ok_isubs"]
+                print("--------------------------")
+                print(d.filename)
+                print("~%.4f sec/TOA" % (fit_duration / len(ok_isubs)))
+                print("Med. TOA error is %.3f us" % (np.median(out["phi_errs"][ok_isubs]) * out["Ps"].mean() * 1e6))
+        tot_duration = time.time() - start
+        if not quiet and len(self.ok_isubs):
+            print("--------------------------")
+            print("Total time: %.2f sec, ~%.4f sec/TOA" % (
+                tot_duration, tot_duration / (np.array(list(map(len, self.ok_isubs))).sum())))
 
-            mask = np.zeros((nsub, nchan), dtype=np.uint8)
+    def _fit_inputs(self, d, mask, nu_ref_tuple, nu_fit_tuple, fit_scat, method, bounds):
+        """Start values and bounds of an archive's fit (pptoas.py:400-469): nu_fits [nsub, 3] and nu_fit_mode
+        (None and 1: the device guesses nu_fit), nu_outs [nsub, 3] or None, the scattering start values
+        [nsub, 2] or None, and the bounds as fit_batch takes them."""
+        nsub = int(d.nsub)
+        ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+        freqs = np.asarray(d.freqs, dtype=np.float64)
+        Ps = np.asarray(d.Ps, dtype=np.float64)
+        if nu_fit_tuple is None and fit_scat:
+            # the scattering start value needs nu_fit_tau on the host (pptoas.py:402, 431-441)
+            nu_fits_in = _nu_fit_guesses(d, mask)
+            empty = nu_fits_in[:, 0] == 0
+            nu_fits_in[empty] = freqs[empty].mean(axis=1)[:, None]
+            mode = 0
+        elif nu_fit_tuple is None:
+            nu_fits_in, mode = None, 1                     # guess_fit_freq, pptoas.py:402
+        else:
+            nu_fits_in = np.tile([nu_fit_tuple[0], nu_fit_tuple[0], nu_fit_tuple[-1]],
+                                 (nsub, 1)).astype(np.float64)
+            mode = 0
+        nu_outs_in = None
+        if nu_ref_tuple is not None:
+            nu_outs_in = np.full((nsub, 3), np.nan)
+            if nu_ref_tuple[0]:
+                nu_outs_in[:, 0] = nu_outs_in[:, 1] = nu_ref_tuple[0]
+            if nu_ref_tuple[-1]:
+                nu_outs_in[:, 2] = nu_ref_tuple[-1]
+                if self.bary:
+                    nu_outs_in[:, 2] /= np.asarray(d.doppler_factors)
+        scat_in = None
+        if fit_scat:                                        # pptoas.py:427-441
+            scat_in = np.zeros((nsub, 2))
             for isub in ok_isubs:
-                mask[isub, np.asarray(d.ok_ichans[isub], dtype=int)] = 1
-            nok = mask.sum(axis=1)
-            subints = _dev(np.asarray(d.subints)[:, 0])      # float64 goes to the device as it is
-            errs = np.ascontiguousarray(np.asarray(d.noise_stds)[:, 0], dtype=np.float64)
-            snrs = np.ascontiguousarray(np.asarray(d.SNRs)[:, 0], dtype=np.float64)
-            weights = np.ascontiguousarray(d.weights, dtype=np.float64)
-            if nu_fit_tuple is None and fit_scat:
-                # the scattering start value needs nu_fit_tau on the host (pptoas.py:402, 431-441)
-                nu_fits_in = np.zeros((nsub, 3))
-                nu_fits_in[ok_isubs, :] = pplib.guess_fit_freq_batch(freqs[ok_isubs], snrs[ok_isubs],
-                                                                    mask[ok_isubs])[:, None]
-                empty = nu_fits_in[:, 0] == 0
-                nu_fits_in[empty] = freqs[empty].mean(axis=1)[:, None]
-                mode = 0
-            elif nu_fit_tuple is None:
-                nu_fits_in, mode = None, 1                 # guess_fit_freq, pptoas.py:402
-            else:
-                nu_fits_in = np.tile([nu_fit_tuple[0], nu_fit_tuple[0], nu_fit_tuple[-1]],
-                                     (nsub, 1)).astype(np.float64)
-                mode = 0
-            nu_outs_in = None
-            if nu_ref_tuple is not None:
-                nu_outs_in = np.full((nsub, 3), np.nan)
-                if nu_ref_tuple[0]:
-                    nu_outs_in[:, 0] = nu_outs_in[:, 1] = nu_ref_tuple[0]
-                if nu_ref_tuple[-1]:
-                    nu_outs_in[:, 2] = nu_ref_tuple[-1]
-                    if bary:
-                        nu_outs_in[:, 2] /= np.asarray(d.doppler_factors)
-            scat_in = None
-            if fit_scat:                                    # pptoas.py:427-441
-                scat_in = np.zeros((nsub, 2))
-                for isub in ok_isubs:
-                    if self.scat_guess is not None:
-                        tau_guess_s, tau_guess_ref, alpha_guess = self.scat_guess
-                        tau_guess = (tau_guess_s / Ps[isub]) * \
-                            (nu_fits_in[isub, 2] / tau_guess_ref) ** alpha_guess
-                    else:
-                        alpha_guess = getattr(self, "alpha", scattering_alpha)
-                        if hasattr(self, "gparams"):
-                            tau_guess = (self.gparams[1] / Ps[isub]) * \
-                                (nu_fits_in[isub, 2] / self.model_nu_ref) ** alpha_guess
-                        else:
-                            tau_guess = 0.0
-                    scat_in[isub] = [tau_guess, alpha_guess]
-            if method == 'TNC':                             # bounds act with TNC only (pptoaslib.py:1008)
-                if bounds is None:                          # pptoas.py:461-469
-                    tau_bounds = (np.log10((10 * nbin) ** -1), None) if self.log10_tau else (0.0, None)
-                    bounds = [(None, None), (None, None), (None, None), tau_bounds, (-10.0, 10.0)]
-                fit_bounds = pplib._check_bounds(bounds, 5)
-            else:
-                fit_bounds = None
-            pl = get_plan(nchan, nbin)
-            self._models = getattr(self, "_models", {})
-            self._models[iarch] = np.asarray(model, dtype=np.float64)
-            self._model_tables = getattr(self, "_model_tables", {})
-            self._model_tables[iarch] = (table_of, {t: np.asarray(m, dtype=np.float64)
-                                                    for t, m in models.items()})
-
-            # subints with a single usable channel are fit for phase only
-            # (pptoas.py:475-478); two channels drop GM (479-483)
-            # Every model of the archive goes to the plan in one pp_set_models call (several when they exceed
-            # _MODEL_BUDGET_BYTES of device memory) and every flags group is one fit_batch: each subint is fit
-            # against its own model (pp_fit_batch_models), as the reference's per-subint loop does.
-            flags_by_sub = {}
-            for isub in ok_isubs:
-                if nok[isub] == 1:
-                    flags = (1, 0, 0, 0, 0)
-                elif nok[isub] == 2 and self.fit_DM and self.fit_GM:
-                    flags = tuple(self.fit_flags[:2] + [0] + self.fit_flags[3:])
+                if self.scat_guess is not None:
+                    tau_guess_s, tau_guess_ref, alpha_guess = self.scat_guess
+                    tau_guess = (tau_guess_s / Ps[isub]) * \
+                        (nu_fits_in[isub, 2] / tau_guess_ref) ** alpha_guess
                 else:
-                    flags = tuple(self.fit_flags)
-                flags_by_sub[isub] = flags
-            model_ids = sorted(models)
-            per_call = max(1, int(_MODEL_BUDGET_BYTES // model_bytes(nchan, nbin)))
-            work = []                                  # (model ids set at once, flags, subints)
-            for m0 in range(0, len(model_ids), per_call):
-                mset = model_ids[m0:m0 + per_call]
-                inset = set(mset)
-                groups = {}
-                for isub in ok_isubs:
-                    if int(table_of[isub]) in inset:
-                        groups.setdefault(flags_by_sub[isub], []).append(isub)
-                for flags, isubs in sorted(groups.items()):
-                    work.append((mset, flags, isubs))
-            res, flags_of = {}, {}
-            fit_start = time.time()
-            mset_on = None
-            for mset, flags, isubs in work:
-                if mset is not mset_on:
-                    ms = [_mdl(models[t]) for t in mset]
-                    dt = np.float32 if all(m.dtype == np.float32 for m in ms) else np.float64
-                    pl.set_models(np.stack([np.asarray(m, dtype=dt) for m in ms]),
-                                  np.stack([tables[t] for t in mset]))
-                    local = {t: i for i, t in enumerate(mset)}
-                    mset_on = mset
+                    alpha_guess = getattr(self, "alpha", scattering_alpha)
+                    if hasattr(self, "gparams"):
+                        tau_guess = (self.gparams[1] / Ps[isub]) * \
+                            (nu_fits_in[isub, 2] / self.model_nu_ref) ** alpha_guess
+                    else:
+                        tau_guess = 0.0
+                scat_in[isub] = [tau_guess, alpha_guess]
+        # bounds act with TNC only (pptoaslib.py:1008)
+        fit_bounds = pplib._check_bounds(bounds, 5) if method == 'TNC' else None
+        return nu_fits_in, mode, nu_outs_in, scat_in, fit_bounds
+
+    def _fit_archive(self, d, tables, table_of, models, mask, nu_fits_in, mode, nu_outs_in, scat_in, fit_bounds):
+        """Fit every subint in ok_isubs against its own model: ([nsub, ...] fit_batch results, fit_flags by subint,
+        wall time of the fits).  Subints with a single usable channel are fit for phase only (pptoas.py:475-478); two
+        channels drop GM (479-483).  Every model goes to the plan in one pp_set_models call (several when they exceed
+        _MODEL_BUDGET_BYTES of device memory) and every flags group is one fit_batch (pp_fit_batch_models)."""
+        nsub, nchan, nbin = int(d.nsub), int(d.nchan), int(d.nbin)
+        ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+        Ps = np.asarray(d.Ps, dtype=np.float64)
+        nok = mask.sum(axis=1)
+        subints = _dev(np.asarray(d.subints)[:, 0])          # float64 goes to the device as it is
+        errs = np.ascontiguousarray(np.asarray(d.noise_stds)[:, 0], dtype=np.float64)
+        snrs = np.ascontiguousarray(np.asarray(d.SNRs)[:, 0], dtype=np.float64)
+        weights = np.ascontiguousarray(d.weights, dtype=np.float64)
+        pl = get_plan(nchan, nbin)
+        flags_of = {}
+        for isub in ok_isubs:
+            if nok[isub] == 1:
+                flags_of[isub] = (1, 0, 0, 0, 0)
+            elif nok[isub] == 2 and self.fit_DM and self.fit_GM:
+                flags_of[isub] = tuple(self.fit_flags[:2] + [0] + self.fit_flags[3:])
+            else:
+                flags_of[isub] = tuple(self.fit_flags)
+        model_ids = sorted(models)
+        per_call = max(1, int(_MODEL_BUDGET_BYTES // model_bytes(nchan, nbin)))
+        res = {}
+        fit_start = time.time()
+        for m0 in range(0, len(model_ids), per_call):      # every round holds the model of some ok subint
+            mset = model_ids[m0:m0 + per_call]
+            ms = [_mdl(models[t]) for t in mset]
+            dt = np.float32 if all(m.dtype == np.float32 for m in ms) else np.float64
+            pl.set_models(np.stack([np.asarray(m, dtype=dt) for m in ms]), np.stack([tables[t] for t in mset]))
+            local = {t: i for i, t in enumerate(mset)}
+            groups = {}
+            for isub in ok_isubs:
+                if int(table_of[isub]) in local:
+                    groups.setdefault(flags_of[isub], []).append(isub)
+            for flags, isubs in sorted(groups.items()):
                 idx = np.asarray(isubs, dtype=int)
                 model_index = None if len(mset) == 1 else \
                     np.array([local[int(table_of[i])] for i in isubs], dtype=np.int32)
@@ -482,7 +534,7 @@ class GetTOAs:
                     batch = np.ascontiguousarray(subints[idx])
                 r = pl.fit_batch(
                     batch, Ps[idx], errs=errs[idx], **raw_kw,
-                    chan_mask=mask[idx], weights=weights[idx], DM_guess=np.full(nidx, DM_stored),
+                    chan_mask=mask[idx], weights=weights[idx], DM_guess=np.full(nidx, float(d.DM)),
                     snrs=snrs[idx], nu_fits=None if nu_fits_in is None else nu_fits_in[idx],
                     nu_fit_mode=mode, nu_outs=None if nu_outs_in is None else nu_outs_in[idx],
                     fit_flags=flags, log10_tau=self.log10_tau, option=0, is_toa=True,
@@ -493,190 +545,159 @@ class GetTOAs:
                         if k not in res:
                             res[k] = np.zeros((nsub,) + v.shape[1:], dtype=v.dtype)
                         res[k][idx] = v
-                for isub in isubs:
-                    flags_of[isub] = flags
-            fit_duration = time.time() - fit_start
+        return res, flags_of, time.time() - fit_start
 
-            phis = np.zeros(nsub); phi_errs = np.zeros(nsub)
-            TOAs = np.zeros(nsub, dtype="object"); TOA_errs = np.zeros(nsub, dtype="object")
-            DMs = np.zeros(nsub); DM_errs = np.zeros(nsub)
-            GMs = np.zeros(nsub); GM_errs = np.zeros(nsub)
-            taus = np.zeros(nsub); tau_errs = np.zeros(nsub)
-            alphas = np.zeros(nsub); alpha_errs = np.zeros(nsub)
-            scales = np.zeros([nsub, nchan]); scale_errs = np.zeros([nsub, nchan])
-            snrs_out = np.zeros(nsub); channel_snrs = np.zeros([nsub, nchan])
-            profile_fluxes = np.zeros([nsub, nchan]); profile_flux_errs = np.zeros([nsub, nchan])
-            fluxes = np.zeros(nsub); flux_errs = np.zeros(nsub); flux_freqs = np.zeros(nsub)
-            red_chi2s = np.zeros(nsub)
-            covariances = np.zeros([nsub, self.nfit, self.nfit])
-            nfevals = np.zeros(nsub, dtype="int"); rcs = np.zeros(nsub, dtype="int")
-            nu_fits_arr = list(np.zeros([nsub, 3])); nu_refs_arr = list(np.zeros([nsub, 3]))
-            # everything that is the same arithmetic for every subint, for all of them at once
-            okm = mask.astype(bool)
-            okm[np.setdiff1d(np.arange(nsub), ok_isubs)] = False
-            if res:
-                scales[okm] = res["scales"][okm]
-                scale_errs[okm] = res["scale_errs"][okm]
-                channel_snrs[okm] = res["channel_snrs"][okm]
-            fmax = np.where(okm, freqs, -np.inf).max(axis=1)
-            fmin = np.where(okm, freqs, np.inf).min(axis=1)
-            if nu_fits_in is None:                          # pptoas.py:400-407
-                nu_fit_vals = np.zeros(nsub)
-                nu_fit_vals[ok_isubs] = pplib.guess_fit_freq_batch(freqs[ok_isubs], snrs[ok_isubs], mask[ok_isubs])
-            doppler = np.asarray(d.doppler_factors, dtype=np.float64)
-            subtimes = np.asarray(d.subtimes)
-            parangles = np.asarray(d.parallactic_angles) if print_parangle else None
-            tmplt = self.modelfile if isinstance(self.modelfile, str) else "array"
-            fe_be = d.frontend + "_" + d.backend
-            chbw = abs(d.bw) / nchan
-            ifit_of = {}
-            for isub in ok_isubs:
-                flags = flags_of[isub]
-                par, perr = res["params"][isub], res["param_errs"][isub]
-                nu_out = res["nu_out"][isub]
-                P = Ps[isub]
-                phi, phi_err = par[0], perr[0]
-                DM, DM_err = par[1], perr[1]
-                GM, GM_err = par[2], perr[2]
-                # TOA (pptoas.py:528-531)
-                TOA_mjd = d.epochs[isub] + MJD(0, ((phi * P) + d.backend_delay) / (3600 * 24.))
-                TOA_err = phi_err * P * 1e6
-                # Doppler correction (pptoas.py:539-549)
-                if self.bary:
-                    df = doppler[isub]
-                    if flags[1]:
-                        DM *= df
-                    if flags[2]:
-                        GM *= df ** 3
-                else:
-                    df = 1.0
-                if print_flux:                              # pptoas.py:554-577
-                    okc = np.nonzero(okm[isub])[0]
-                    means = np.asarray(models[table_of[isub]])[okc].mean(axis=1)
-                    profile_fluxes[isub, okc] = means * scales[isub, okc]
-                    profile_flux_errs[isub, okc] = abs(means) * scale_errs[isub, okc]
-                    fluxes[isub], flux_errs[isub] = weighted_mean(profile_fluxes[isub, okc],
-                                                                 profile_flux_errs[isub, okc])
-                    flux_freqs[isub], _ = weighted_mean(freqs[isub, okc], profile_flux_errs[isub, okc])
-                nu_refs_arr[isub] = list(nu_out)
-                if nu_fits_in is not None:                  # pptoas.py:400-407
-                    nu_fits_arr[isub] = list(nu_fits_in[isub])
-                else:
-                    nu_fits_arr[isub] = [nu_fit_vals[isub]] * 3
-                phis[isub], phi_errs[isub] = phi, phi_err
-                TOAs[isub], TOA_errs[isub] = TOA_mjd, TOA_err
-                DMs[isub], DM_errs[isub] = DM, DM_err
-                GMs[isub], GM_errs[isub] = GM, GM_err
-                if flags not in ifit_of:
-                    ifit_of[flags] = np.where(flags)[0]
-                ifit = ifit_of[flags]
-                cm = res["cov"][isub][np.ix_(ifit, ifit)]
-                if cm.shape == covariances[isub].shape:
-                    covariances[isub] = cm
-                else:                                       # pptoas.py:596-600
-                    for ii, a_ in enumerate(ifit):
-                        for jj, b_ in enumerate(ifit):
-                            if a_ < self.nfit and b_ < self.nfit:
-                                covariances[isub][a_, b_] = cm[ii, jj]
-                snr, gof = res["snr"][isub], res["red_chi2"][isub]
-                toa_flags = {}                              # pptoas.py:604-651
-                DM_out, DM_err_out = (DM, DM_err) if flags[1] else (None, None)
+    def _subint_toas(self, d, models, table_of, mask, res, flags_of, nu_fits_in, nu_ref_tuple,
+                     print_phase, print_flux, print_parangle, addtnl_toa_flags):
+        """Append a TOA with its flags per fitted subint to TOA_list (pptoas.py:528-651); the per-subint results."""
+        nsub, nchan, nbin = int(d.nsub), int(d.nchan), int(d.nbin)
+        ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+        freqs = np.asarray(d.freqs, dtype=np.float64)
+        Ps = np.asarray(d.Ps, dtype=np.float64)
+        nok = mask.sum(axis=1)
+        phis = np.zeros(nsub); phi_errs = np.zeros(nsub)
+        TOAs = np.zeros(nsub, dtype="object"); TOA_errs = np.zeros(nsub, dtype="object")
+        DMs = np.zeros(nsub); DM_errs = np.zeros(nsub)
+        GMs = np.zeros(nsub); GM_errs = np.zeros(nsub)
+        scales = np.zeros([nsub, nchan]); scale_errs = np.zeros([nsub, nchan])
+        channel_snrs = np.zeros([nsub, nchan])
+        profile_fluxes = np.zeros([nsub, nchan]); profile_flux_errs = np.zeros([nsub, nchan])
+        fluxes = np.zeros(nsub); flux_errs = np.zeros(nsub); flux_freqs = np.zeros(nsub)
+        covariances = np.zeros([nsub, self.nfit, self.nfit])
+        nu_fits_arr = list(np.zeros([nsub, 3])); nu_refs_arr = list(np.zeros([nsub, 3]))
+        # everything that is the same arithmetic for every subint, for all of them at once
+        okm = mask.astype(bool)
+        okm[np.setdiff1d(np.arange(nsub), ok_isubs)] = False
+        scales[okm] = res["scales"][okm]
+        scale_errs[okm] = res["scale_errs"][okm]
+        channel_snrs[okm] = res["channel_snrs"][okm]
+        fmax = np.where(okm, freqs, -np.inf).max(axis=1)
+        fmin = np.where(okm, freqs, np.inf).min(axis=1)
+        nu_fits_rows = _nu_fit_guesses(d, mask) if nu_fits_in is None else nu_fits_in   # pptoas.py:400-407
+        doppler = np.asarray(d.doppler_factors, dtype=np.float64)
+        subtimes = np.asarray(d.subtimes)
+        parangles = np.asarray(d.parallactic_angles) if print_parangle else None
+        tmplt = self.modelfile if isinstance(self.modelfile, str) else "array"
+        fe_be = d.frontend + "_" + d.backend
+        chbw = abs(d.bw) / nchan
+        ifit_of = {}
+        for isub in ok_isubs:
+            flags = flags_of[isub]
+            par, perr = res["params"][isub], res["param_errs"][isub]
+            nu_out = res["nu_out"][isub]
+            P = Ps[isub]
+            phi, phi_err = par[0], perr[0]
+            DM, DM_err = par[1], perr[1]
+            GM, GM_err = par[2], perr[2]
+            # TOA (pptoas.py:528-531)
+            TOA_mjd = d.epochs[isub] + MJD(0, ((phi * P) + d.backend_delay) / (3600 * 24.))
+            TOA_err = phi_err * P * 1e6
+            # Doppler correction (pptoas.py:539-549)
+            if self.bary:
+                df = doppler[isub]
+                if flags[1]:
+                    DM *= df
                 if flags[2]:
-                    toa_flags['gm'], toa_flags['gm_err'] = GM, GM_err
-                if flags[3]:                                # pptoas.py:611-624
-                    tau_r, tau_e = par[3], perr[3]
-                    if self.log10_tau:
-                        toa_flags['scat_time'] = 10 ** tau_r * P / df * 1e6
-                        toa_flags['log10_scat_time'] = tau_r + np.log10(P / df)
-                        toa_flags['log10_scat_time_err'] = tau_e
-                    else:
-                        toa_flags['scat_time'] = tau_r * P / df * 1e6
-                        toa_flags['scat_time_err'] = tau_e * P / df * 1e6
-                    toa_flags['scat_ref_freq'] = nu_out[2] * df
-                    toa_flags['scat_ind'] = par[4]
-                if flags[4]:
-                    toa_flags['scat_ind_err'] = perr[4]
-                toa_flags['be'] = d.backend
-                toa_flags['fe'] = d.frontend
-                toa_flags['f'] = fe_be
-                toa_flags['nbin'] = nbin
-                toa_flags['nch'] = nchan
-                toa_flags['nchx'] = int(nok[isub])
-                toa_flags['bw'] = fmax[isub] - fmin[isub]
-                toa_flags['chbw'] = chbw
-                toa_flags['subint'] = int(isub)
-                toa_flags['tobs'] = subtimes[isub]
-                toa_flags['fratio'] = fmax[isub] / fmin[isub]
-                toa_flags['tmplt'] = tmplt
-                toa_flags['snr'] = snr
-                if nu_ref_tuple is not None and nu_ref_tuple[0] is not None and np.all(flags[:2]):
-                    toa_flags['phi_DM_cov'] = cm[0, 1]
-                toa_flags['gof'] = gof
-                if print_phase:
-                    toa_flags['phs'], toa_flags['phs_err'] = phi, phi_err
-                if print_flux:
-                    toa_flags['flux'] = fluxes[isub]
-                    toa_flags['flux_err'] = flux_errs[isub]
-                    toa_flags['flux_ref_freq'] = flux_freqs[isub]
-                if print_parangle:
-                    toa_flags['par_angle'] = parangles[isub]
-                for k, v in addtnl_toa_flags.items():
-                    toa_flags[k] = v
-                self.TOA_list.append(TOA(d.filename, nu_out[0], TOA_mjd, TOA_err,
-                                         d.telescope, d.telescope_code, DM_out, DM_err_out,
-                                         toa_flags))
-            oks = np.asarray(ok_isubs if res else [], dtype=int)
-            taus[oks], tau_errs[oks] = res["params"][oks, 3], res["param_errs"][oks, 3]
-            alphas[oks], alpha_errs[oks] = res["params"][oks, 4], res["param_errs"][oks, 4]
-            nfevals[oks] = res["nfeval"][oks]
-            rcs[oks] = [pplib.scipy_return_code(c, method) for c in res["return_code"][oks]]   # pptoaslib.py:1017
-            snrs_out[oks] = res["snr"][oks]
-            red_chi2s[oks] = res["red_chi2"][oks]
-            # per-archive Delta-DM mean (pptoas.py:665-682)
-            DeltaDMs = DMs - DM0_arch
-            if np.all(DM_errs[ok_isubs]):
-                DM_weights = DM_errs[ok_isubs] ** -2
+                    GM *= df ** 3
             else:
-                DM_weights = np.ones(len(ok_isubs))
-            DeltaDM_mean, DeltaDM_var = np.average(DeltaDMs[ok_isubs], weights=DM_weights,
-                                                   returned=True)
-            DeltaDM_var = DeltaDM_var ** -1
-            if len(ok_isubs) > 1:
-                DeltaDM_var *= np.sum(((DeltaDMs[ok_isubs] - DeltaDM_mean) ** 2) * DM_weights) / \
-                    (len(ok_isubs) - 1)
-            DeltaDM_err = DeltaDM_var ** 0.5
-            self.order.append(d.filename); self.obs.append(obs)
-            self.doppler_fs.append(d.doppler_factors); self.nu0s.append(d.nu0)
-            self.nu_fits.append(nu_fits_arr); self.nu_refs.append(nu_refs_arr)
-            self.ok_isubs.append(ok_isubs); self.epochs.append(d.epochs)
-            self.MJDs.append(MJDs); self.Ps.append(Ps)
-            self.phis.append(phis); self.phi_errs.append(phi_errs)
-            self.TOAs.append(TOAs); self.TOA_errs.append(TOA_errs)
-            self.DM0s.append(DM0_arch); self.DMs.append(DMs); self.DM_errs.append(DM_errs)
-            self.DeltaDM_means.append(DeltaDM_mean); self.DeltaDM_errs.append(DeltaDM_err)
-            self.GMs.append(GMs); self.GM_errs.append(GM_errs)
-            self.taus.append(taus); self.tau_errs.append(tau_errs)
-            self.alphas.append(alphas); self.alpha_errs.append(alpha_errs)
-            self.scales.append(scales); self.scale_errs.append(scale_errs)
-            self.snrs.append(snrs_out); self.channel_snrs.append(channel_snrs)
-            self.profile_fluxes.append(profile_fluxes)
-            self.profile_flux_errs.append(profile_flux_errs)
-            self.fluxes.append(fluxes); self.flux_errs.append(flux_errs)
-            self.flux_freqs.append(flux_freqs)
-            self.covariances.append(covariances); self.red_chi2s.append(red_chi2s)
-            self.nfevals.append(nfevals); self.rcs.append(rcs)
-            self.fit_durations.append(fit_duration)
-            if not quiet:
-                print("--------------------------")
-                print(d.filename)
-                print("~%.4f sec/TOA" % (fit_duration / len(ok_isubs)))
-                print("Med. TOA error is %.3f us" % (np.median(phi_errs[ok_isubs]) * Ps.mean() * 1e6))
-        self._models = getattr(self, "_models", {})
-        tot_duration = time.time() - start
-        if not quiet and len(self.ok_isubs):
-            print("--------------------------")
-            print("Total time: %.2f sec, ~%.4f sec/TOA" % (
-                tot_duration, tot_duration / (np.array(list(map(len, self.ok_isubs))).sum())))
+                df = 1.0
+            if print_flux:                                  # pptoas.py:554-577
+                okc = np.nonzero(okm[isub])[0]
+                means = np.asarray(models[table_of[isub]])[okc].mean(axis=1)
+                profile_fluxes[isub, okc] = means * scales[isub, okc]
+                profile_flux_errs[isub, okc] = abs(means) * scale_errs[isub, okc]
+                fluxes[isub], flux_errs[isub] = weighted_mean(profile_fluxes[isub, okc],
+                                                             profile_flux_errs[isub, okc])
+                flux_freqs[isub], _ = weighted_mean(freqs[isub, okc], profile_flux_errs[isub, okc])
+            nu_refs_arr[isub] = list(nu_out)
+            nu_fits_arr[isub] = list(nu_fits_rows[isub])
+            phis[isub], phi_errs[isub] = phi, phi_err
+            TOAs[isub], TOA_errs[isub] = TOA_mjd, TOA_err
+            DMs[isub], DM_errs[isub] = DM, DM_err
+            GMs[isub], GM_errs[isub] = GM, GM_err
+            if flags not in ifit_of:
+                ifit_of[flags] = np.where(flags)[0]
+            ifit = ifit_of[flags]
+            cm = res["cov"][isub][np.ix_(ifit, ifit)]
+            if cm.shape == covariances[isub].shape:
+                covariances[isub] = cm
+            else:                                           # pptoas.py:596-600
+                for ii, a_ in enumerate(ifit):
+                    for jj, b_ in enumerate(ifit):
+                        if a_ < self.nfit and b_ < self.nfit:
+                            covariances[isub][a_, b_] = cm[ii, jj]
+            snr, gof = res["snr"][isub], res["red_chi2"][isub]
+            toa_flags = {}                                  # pptoas.py:604-651
+            DM_out, DM_err_out = (DM, DM_err) if flags[1] else (None, None)
+            if flags[2]:
+                toa_flags['gm'], toa_flags['gm_err'] = GM, GM_err
+            if flags[3]:                                    # pptoas.py:611-624
+                tau_r, tau_e = par[3], perr[3]
+                if self.log10_tau:
+                    toa_flags['scat_time'] = 10 ** tau_r * P / df * 1e6
+                    toa_flags['log10_scat_time'] = tau_r + np.log10(P / df)
+                    toa_flags['log10_scat_time_err'] = tau_e
+                else:
+                    toa_flags['scat_time'] = tau_r * P / df * 1e6
+                    toa_flags['scat_time_err'] = tau_e * P / df * 1e6
+                toa_flags['scat_ref_freq'] = nu_out[2] * df
+                toa_flags['scat_ind'] = par[4]
+            if flags[4]:
+                toa_flags['scat_ind_err'] = perr[4]
+            toa_flags.update(be=d.backend, fe=d.frontend, f=fe_be, nbin=nbin, nch=nchan, nchx=int(nok[isub]),
+                             bw=fmax[isub] - fmin[isub], chbw=chbw, subint=int(isub), tobs=subtimes[isub],
+                             fratio=fmax[isub] / fmin[isub], tmplt=tmplt, snr=snr)
+            if nu_ref_tuple is not None and nu_ref_tuple[0] is not None and np.all(flags[:2]):
+                toa_flags['phi_DM_cov'] = cm[0, 1]
+            toa_flags['gof'] = gof
+            if print_phase:
+                toa_flags['phs'], toa_flags['phs_err'] = phi, phi_err
+            if print_flux:
+                toa_flags['flux'] = fluxes[isub]
+                toa_flags['flux_err'] = flux_errs[isub]
+                toa_flags['flux_ref_freq'] = flux_freqs[isub]
+            if print_parangle:
+                toa_flags['par_angle'] = parangles[isub]
+            toa_flags.update(addtnl_toa_flags)
+            self.TOA_list.append(TOA(d.filename, nu_out[0], TOA_mjd, TOA_err,
+                                     d.telescope, d.telescope_code, DM_out, DM_err_out,
+                                     toa_flags))
+        return dict(phis=phis, phi_errs=phi_errs, TOAs=TOAs, TOA_errs=TOA_errs, DMs=DMs, DM_errs=DM_errs,
+                    GMs=GMs, GM_errs=GM_errs, scales=scales, scale_errs=scale_errs, channel_snrs=channel_snrs,
+                    profile_fluxes=profile_fluxes, profile_flux_errs=profile_flux_errs, fluxes=fluxes,
+                    flux_errs=flux_errs, flux_freqs=flux_freqs, covariances=covariances, nu_fits=nu_fits_arr,
+                    nu_refs=nu_refs_arr)
+
+    def _archive_arrays(self, d, res, DMs, DM_errs, method):
+        """The per-archive result arrays taken from the fit as they are, and the Delta-DM mean (pptoas.py:665-682)."""
+        nsub = int(d.nsub)
+        ok_isubs = np.asarray(d.ok_isubs, dtype=int)
+        taus = np.zeros(nsub); tau_errs = np.zeros(nsub)
+        alphas = np.zeros(nsub); alpha_errs = np.zeros(nsub)
+        nfevals = np.zeros(nsub, dtype="int"); rcs = np.zeros(nsub, dtype="int")
+        snrs = np.zeros(nsub); red_chi2s = np.zeros(nsub)
+        taus[ok_isubs], tau_errs[ok_isubs] = res["params"][ok_isubs, 3], res["param_errs"][ok_isubs, 3]
+        alphas[ok_isubs], alpha_errs[ok_isubs] = res["params"][ok_isubs, 4], res["param_errs"][ok_isubs, 4]
+        nfevals[ok_isubs] = res["nfeval"][ok_isubs]
+        # pptoaslib.py:1017
+        rcs[ok_isubs] = [pplib.scipy_return_code(c, method) for c in res["return_code"][ok_isubs]]
+        snrs[ok_isubs] = res["snr"][ok_isubs]
+        red_chi2s[ok_isubs] = res["red_chi2"][ok_isubs]
+        DM0 = float(d.DM) if self.DM0 is None else self.DM0
+        DeltaDMs = DMs - DM0
+        if np.all(DM_errs[ok_isubs]):
+            DM_weights = DM_errs[ok_isubs] ** -2
+        else:
+            DM_weights = np.ones(len(ok_isubs))
+        DeltaDM_mean, DeltaDM_var = np.average(DeltaDMs[ok_isubs], weights=DM_weights,
+                                               returned=True)
+        DeltaDM_var = DeltaDM_var ** -1
+        if len(ok_isubs) > 1:
+            DeltaDM_var *= np.sum(((DeltaDMs[ok_isubs] - DeltaDM_mean) ** 2) * DM_weights) / \
+                (len(ok_isubs) - 1)
+        return dict(taus=taus, tau_errs=tau_errs, alphas=alphas, alpha_errs=alpha_errs, nfevals=nfevals, rcs=rcs,
+                    snrs=snrs, red_chi2s=red_chi2s, DM0s=DM0, DeltaDM_means=DeltaDM_mean,
+                    DeltaDM_errs=DeltaDM_var ** 0.5)
 
     def get_narrowband_TOAs(self, datafile=None, tscrunch=False, fit_scat=False, log10_tau=True,
                             scat_guess=None, print_phase=False, print_flux=False,
@@ -694,38 +715,18 @@ class GetTOAs:
         self.fit_flags = [1, 0]
         self.log10_tau = False
         start = time.time()
-        datafiles = self.datafiles if datafile is None else [datafile]
-        for iarch, datafile in enumerate(datafiles):
-            try:
-                d = datafile if isinstance(datafile, dict) else load_data(datafile)
-            except (RuntimeError, IOError, OSError):
-                if not quiet:
-                    print("Cannot load_data(%s).  Skipping it." % datafile)
-                continue
-            if d.get("dmc"):                                # pptoas.py:817-826
-                d = restore_dispersion(d)
-            if tscrunch:
-                d = tscrunch_databunch(d)
-            if not len(d.ok_isubs):
-                continue
-            self.ok_idatafiles.append(iarch)
+        for _, d in self._archives_to_fit(datafile, tscrunch, quiet):
             nsub, nchan, nbin = int(d.nsub), int(d.nchan), int(d.nbin)
             ok_isubs = np.asarray(d.ok_isubs, dtype=int)
             freqs = np.asarray(d.freqs, dtype=np.float64)
             Ps = np.asarray(d.Ps, dtype=np.float64)
-            tables, table_of = _freq_tables(freqs)          # freqs = data.freqs[isub], pptoas.py:927
-            models = {t: self._model_for(d.phases, tables[t], Ps[ok_isubs[table_of[ok_isubs] == t][0]], False,
-                                         add_instrumental_response)
-                      for t in np.unique(table_of[ok_isubs])}
+            _, table_of, models = self._model_tables_of(d, False, add_instrumental_response, by_period=False)
             model_of = [models[t] for t in table_of]
             pl = get_plan(nchan, nbin)
             fit_start = time.time()
             profs = _f32(np.asarray(d.subints)[ok_isubs, 0]).reshape(len(ok_isubs) * nchan, nbin)
             noise = np.ascontiguousarray(np.asarray(d.noise_stds)[ok_isubs, 0], dtype=np.float64)
-            okmask = np.zeros((len(ok_isubs), nchan), dtype=bool)
-            for i, isub in enumerate(ok_isubs):
-                okmask[i, np.asarray(d.ok_ichans[isub], dtype=int)] = True
-            okmask &= noise > 0
+            okmask = _chan_mask(nsub, nchan, d.ok_ichans, ok_isubs)[ok_isubs].astype(bool) & (noise > 0)
             if len(models) == 1:
                 mstack = _f32(model_of[ok_isubs[0]])
             else:                                           # one model row per profile
@@ -740,8 +741,6 @@ class GetTOAs:
             scales, scale_errs = np.zeros(shape), np.zeros(shape)
             channel_snrs, channel_red_chi2s = np.zeros(shape), np.zeros(shape)
             profile_fluxes, profile_flux_errs = np.zeros(shape), np.zeros(shape)
-            MJDs = np.array([e.in_days() for e in d.epochs], dtype=np.double)
-            obs = DataBunch(telescope=d.telescope, backend=d.backend, frontend=d.frontend)
             get = lambda k: r[k].reshape(len(ok_isubs), nchan)  # noqa: E731
             for i, isub in enumerate(ok_isubs):
                 P = Ps[isub]
@@ -774,16 +773,12 @@ class GetTOAs:
                     toa_flags.update(addtnl_toa_flags)
                     self.TOA_list.append(TOA(d.filename, freqs[isub, ichan], toa, toa_err, d.telescope,
                                              d.telescope_code, None, None, toa_flags))
-            for name, val in (("order", d.filename), ("obs", obs), ("doppler_fs", d.doppler_factors),
-                              ("ok_isubs", ok_isubs), ("epochs", d.epochs), ("MJDs", MJDs), ("Ps", Ps),
-                              ("phis", phis), ("phi_errs", phi_errs), ("TOAs", TOAs), ("TOA_errs", TOA_errs),
-                              ("taus", taus), ("tau_errs", tau_errs), ("scales", scales),
-                              ("scale_errs", scale_errs), ("channel_snrs", channel_snrs),
-                              ("profile_fluxes", profile_fluxes), ("profile_flux_errs", profile_flux_errs),
-                              ("channel_red_chi2s", channel_red_chi2s), ("fit_durations", fit_duration)):
-                if not hasattr(self, name):
-                    setattr(self, name, [])
-                getattr(self, name).append(val)
+            out = _archive_entries(d)
+            out.update(phis=phis, phi_errs=phi_errs, TOAs=TOAs, TOA_errs=TOA_errs, taus=taus, tau_errs=tau_errs,
+                       scales=scales, scale_errs=scale_errs, channel_snrs=channel_snrs, profile_fluxes=profile_fluxes,
+                       profile_flux_errs=profile_flux_errs, channel_red_chi2s=channel_red_chi2s,
+                       fit_durations=fit_duration)
+            self._append_archive(out)
             if not quiet:
                 print("--------------------------")
                 print(d.filename)
