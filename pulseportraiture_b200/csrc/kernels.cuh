@@ -504,6 +504,9 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
     // ---- split + power sums; X and the guess accumulators need no sigma ------------
     double s_all = 0.0, s_top = 0.0;
     float wrow = wgt;
+    // rows that arrive transformed: thread 0's first output is slot 0, which holds no harmonic of the row, so
+    // the test below cannot see a non-finite row there; the row's DC term can
+    if (FROMSPEC && used && !isfinite(a.ddc[(size_t)sl * a.nchan + ch])) wrow = 0.f;
 #pragma unroll
     for (int i = 0; i < NUNIT; ++i) {
       cx<F> d[NOUT];
@@ -568,7 +571,10 @@ __global__ void __launch_bounds__(PL::kThreads, PL::kMinBlocks) k_spectra(Spectr
         for (int q = 0; q < NOUT; ++q) {
           const int sk = slot_of(i, q);
           const float2 r = rot2pi(vx[q], vy[q], (double)(sk == 0 ? N : sk) * shift);
-          vx[q] = r.x; vy[q] = r.y;
+          // the Nyquist term (slot 0; harmonic nbin/2 in slot nhalf of rows that arrive transformed) keeps its
+          // real part only, as the irfft of rotate_data does
+          const bool nyquist = FROMSPEC ? (sk == a.nhalf) : (sk == 0);
+          vx[q] = r.x; vy[q] = nyquist ? 0.f : r.y;
         }
       }
       if (wrow != 0.f) {   // uniform: 0 when no guess is wanted, the row is unused or not finite
@@ -693,7 +699,8 @@ __global__ void __launch_bounds__(256) k_guess(GuessArgs a) {
     if (tau_g != 0.0) {   // scattered mean model (pptoas.py:444-447): conj(m B) = conj(m) conj(B)
       const double b = kTwoPi * (double)k * tau_g, q = 1.0 / (1.0 + b * b);
       const double tx = mx * q - my * (b * q);
-      my = mx * (b * q) + my * q; mx = tx;
+      // the irfft there keeps the real part of the Nyquist term: Re(B m) at k = nbin/2
+      my = (k == NH) ? 0.0 : mx * (b * q) + my * q; mx = tx;
     }
     Y[i] = make_double2(dx * mx - dy * my, dx * my + dy * mx);
     const double pw = dx * dx + dy * dy;

@@ -252,7 +252,7 @@ __global__ void __launch_bounds__(64, SpecPlan16::kMinBlocks) k_spectra16(Spectr
           for (int q = 0; q < 8; ++q) {
             const int sk = (q & 1) ? N - po - 256 * (q >> 1) : p + 256 * (q >> 1);
             const float2 r = rot2pi(vx[q], vy[q], (double)(sk == 0 ? N : sk) * shift);
-            vx[q] = r.x; vy[q] = r.y;
+            vx[q] = r.x; vy[q] = sk == 0 ? 0.f : r.y;   // the Nyquist term keeps its real part (irfft of rotate_data)
           }
         }
         if (wrow != 0.f) {   // uniform: 0 when the row is not finite
