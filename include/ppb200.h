@@ -360,6 +360,52 @@ int pp_get_noise_batch(pp_plan_t* plan, const float* data, int32_t nsub,
 int pp_get_noise_cut_batch(pp_plan_t* plan, const float* data, int32_t nsub, int32_t kc,
                            double* noise_out);
 
+/* ---- evolving-Gaussian model fit (ppgauss) ----------------------------------------
+ * Replaces the numerical core of pplib.fit_gaussian_portrait (pplib.py:1924-2052): a weighted least-squares
+ * fit of the evolving-Gaussian portrait of gen_gaussian_portrait (pplib.py:853-930), scattered when tau or
+ * alpha is free or tau != 0, to nport portraits at once.  P = 3 + 6*ngauss parameters per portrait:
+ *   [DC, tau [bin at nu_ref], (loc, m_loc, wid, m_wid, amp, m_amp) x ngauss, alpha]
+ * chi^2 = sum_n sum_t (d_nt - m_nt)^2 / sigma_n^2, the DC harmonic included, evaluated in the Fourier domain
+ * (Parseval) in FP64 with analytic derivatives.  Levenberg-Marquardt on the Marquardt-scaled normal
+ * equations; bounds as an active set (starts are moved into the box, a parameter on a bound whose gradient
+ * points outwards is held, steps are clipped to the box).  Stops when every free parameter's Gauss-Newton
+ * step is below tol x its sigma.  Frequencies from pp_set_freqs; nbin a power of two (64..4096).  Results of
+ * a portrait do not depend on the batch or chunk it is fit in (pp_plan_set_chunk: portraits per chunk). */
+typedef struct {
+  int32_t nport;
+  const double* data;       /* [nport,nchan,nbin] float64, host or device         */
+  const double* errs;       /* [nport,nchan] sigma_n > 0, host or device         */
+  const char* model_code;   /* three characters '0' (power law) / '1' (linear)
+                               for loc, wid, amp                                 */
+  int32_t ngauss;           /* 1..16                                             */
+  double nu_ref;            /* reference frequency of the parameters [MHz] > 0   */
+  const double* init;       /* [nport,P] start values, host or device            */
+  const uint8_t* fit_flags; /* HOST [P] nonzero = free; alpha's flag last        */
+  const double* bounds;     /* HOST [P,2] (lower, upper); NaN = unbounded; NULL =
+                               no bounds                                         */
+  int32_t max_iter;         /* objective evaluations per portrait (0 = default
+                               200); < 0: evaluate only: chi2, jtr, jtj at the
+                               (boxed) start point, no step, return code 0       */
+  double tol;               /* 0 = default 1e-4                                  */
+} pp_gfit_args_t;
+
+typedef struct {
+  double* params;       /* [nport,P]                                              */
+  double* param_errs;   /* [nport,P] sqrt(diag(cov)); 0 for fixed parameters      */
+  double* cov;          /* [nport,P,P] (J^T J)^-1 red_chi2 over the free parameters
+                           (lmfit's scale_covar); 0 rows / columns for fixed ones */
+  double* chi2;         /* [nport]                                                */
+  double* red_chi2;     /* [nport] chi2 / (nchan nbin - n_free)                   */
+  int32_t* nfeval;      /* [nport] model + Jacobian evaluations                   */
+  int32_t* return_code; /* [nport] 0 converged, 1 max_iter, 3 non-finite          */
+  double* jtr;          /* [nport,P] J^T (d - m) / sigma^2 at params (free only)  */
+  double* jtj;          /* [nport,P,P] J^T J / sigma^2 at params (free only)      */
+  double* model;        /* [nport,nchan,nbin] float64 model portrait at params    */
+} pp_gfit_out_t;        /* any member may be NULL; host or device pointers        */
+
+int pp_fit_gaussian_portraits(pp_plan_t* plan, const pp_gfit_args_t* args,
+                              const pp_gfit_out_t* out);
+
 /* ---- diagnostics ------------------------------------------------------------ */
 typedef struct {
   int64_t launches;        /* kernels launched by the last pp_* call            */

@@ -25,7 +25,7 @@ SYMBOLS = ["pp_plan_create", "pp_plan_destroy", "pp_plan_set_stream",
            "pp_set_model", "pp_set_models", "pp_set_models_f64", "pp_fit_batch", "pp_fit_batch_models",
            "pp_fit_phase_shift_batch", "pp_fit_phase_shift_batch_bounds", "pp_rotate_batch", "pp_rotate_full_batch", "pp_apply_response_batch",
            "pp_align_accumulate", "pp_gen_gaussian_portrait", "pp_gen_gaussian_portrait_f64", "pp_gen_spline_portrait",
-           "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64",
+           "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64", "pp_fit_gaussian_portraits",
            "pp_plan_enable_timing", "pp_get_stats", "pp_host_alloc",
            "pp_host_free", "pp_last_error",
            "pp_abi_version"]
@@ -103,6 +103,28 @@ class PShiftOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in (
         "phase", "phase_err", "scale", "scale_err", "snr", "red_chi2",
         "lag_index")]
+
+
+class GfitArgs(C.Structure):
+    _fields_ = [
+        ("nport", C.c_int32),
+        ("data", C.c_void_p),
+        ("errs", C.c_void_p),
+        ("model_code", C.c_char_p),
+        ("ngauss", C.c_int32),
+        ("nu_ref", C.c_double),
+        ("init", C.c_void_p),
+        ("fit_flags", C.c_void_p),
+        ("bounds", C.c_void_p),
+        ("max_iter", C.c_int32),
+        ("tol", C.c_double),
+    ]
+
+
+class GfitOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in (
+        "params", "param_errs", "cov", "chi2", "red_chi2", "nfeval", "return_code",
+        "jtr", "jtj", "model")]
 
 
 class Stats(C.Structure):
@@ -188,6 +210,8 @@ def lib():
     L.pp_get_noise_fit_batch.restype = C.c_int
     L.pp_measure_fp64.argtypes = [vp, C.POINTER(C.c_double)]
     L.pp_measure_fp64.restype = C.c_int
+    L.pp_fit_gaussian_portraits.argtypes = [vp, C.POINTER(GfitArgs), C.POINTER(GfitOut)]
+    L.pp_fit_gaussian_portraits.restype = C.c_int
     L.pp_plan_enable_timing.argtypes = [vp, i32]
     L.pp_plan_enable_timing.restype = C.c_int
     L.pp_get_stats.argtypes = [vp, C.POINTER(Stats)]

@@ -2476,44 +2476,68 @@ __device__ __forceinline__ double evolve_param(double f, double nu_ref, double p
 
 constexpr int kMaxGauss = 64;
 
+// bin centres: np.linspace(lo + d/(2 nbin), hi - d/(2 nbin), nbin) (pplib.py:671-684)
+struct BinCentres {
+  double lo, hi, dx;
+  int nbin;
+  __device__ explicit BinCentres(int n)
+      : lo(1.0 / (2.0 * n)), hi(1.0 - 1.0 / (2.0 * n)), dx(n > 1 ? (hi - lo) / (double)(n - 1) : 0.0), nbin(n) {}
+  __device__ double operator()(int i) const { return i == nbin - 1 ? hi : lo + (double)i * dx; }
+};
+
+// phases wrapped once around the component's centre (pplib.py:805-808)
+__device__ __forceinline__ double gauss_wrapx(double x, double mean) {
+  if (mean < 0.5) return x > mean + 0.5 ? x - 1.0 : x;
+  return x < mean - 0.5 ? x + 1.0 : x;
+}
+
+// One component of gaussian_profile(norm=False) in one channel: value at bin centre x is
+// scale * exp(-z^2/2) with z = gauss_z(x), where |z| < 20 (pplib.py:770-825).  renorm = scale / amp is
+// the reference's peak renormalisation: 1 while loc lies in [0, 1), ~0 for a component centred outside.
+// An invalid component (wid <= 0, or no bin within |z| < 20) has scale = renorm = 0.
+struct GaussComp {
+  double mean, isig, scale, renorm;
+  __device__ double z(double x) const { return (gauss_wrapx(x, mean) - mean) * isig; }
+};
+
+__device__ __forceinline__ GaussComp gauss_comp(double loc, double wid, double amp, const BinCentres& xbin) {
+  GaussComp c{0.0, 0.0, 0.0, 0.0};
+  if (wid > 0.0) {
+    const int nbin = xbin.nbin;
+    const double sigma = wid / (2.0 * sqrt(2.0 * log(2.0)));
+    c.mean = loc - floor(loc);                      // loc % 1
+    c.isig = 1.0 / sigma;
+    // the peak bin (argmax of the profile = smallest |z|, first index on ties) fixes the
+    // amplitude: value exp(-0.5 ((x[ipk] - loc)/sigma)^2) at the peak bin (pplib.py:820-823)
+    int i0 = (int)floor(c.mean * nbin);
+    double best = CUDART_INF; int ipk = -1;
+    for (int d = -1; d <= 1; ++d) {
+      const int i = ((i0 + d) % nbin + nbin) % nbin;
+      const double z = fabs((gauss_wrapx(xbin(i), c.mean) - c.mean) * c.isig);
+      if (z < best || (z == best && i < ipk)) { best = z; ipk = i; }
+    }
+    if (best < 20.0) {
+      const double xp = gauss_wrapx(xbin(ipk), c.mean);
+      const double zl = (xp - loc) * c.isig;
+      const double el = exp(-0.5 * zl * zl), eb = exp(-0.5 * best * best);
+      c.scale = amp * el / eb;
+      c.renorm = el / eb;
+    }
+  }
+  return c;
+}
+
 __global__ void __launch_bounds__(256) k_gauss_model(GaussModelArgs a) {
-  __shared__ double g_mean[kMaxGauss], g_isig[kMaxGauss], g_amp[kMaxGauss];
+  __shared__ GaussComp comp[kMaxGauss];
   const int ch = blockIdx.x, tid = threadIdx.x, nbin = a.nbin;
   const double f = a.freqs[ch];
-  // bin centres: np.linspace(lo + d/(2 nbin), hi - d/(2 nbin), nbin) (pplib.py:671-684)
-  const double x_lo = 1.0 / (2.0 * nbin), x_hi = 1.0 - 1.0 / (2.0 * nbin);
-  const double dx = nbin > 1 ? (x_hi - x_lo) / (double)(nbin - 1) : 0.0;
-  auto xbin = [&](int i) { return i == nbin - 1 ? x_hi : x_lo + (double)i * dx; };
-  auto wrapx = [&](double x, double mean) {   // pplib.py:805-808
-    if (mean < 0.5) return x > mean + 0.5 ? x - 1.0 : x;
-    return x < mean - 0.5 ? x + 1.0 : x;
-  };
+  const BinCentres xbin(nbin);
   for (int g = tid; g < a.ngauss; g += 256) {
     const double* q = a.params + 2 + 6 * g;
     const double loc = evolve_param(f, a.nu_ref, q[0], q[1], a.code_loc);
     const double wid = evolve_param(f, a.nu_ref, q[2], q[3], a.code_wid);
     const double amp = evolve_param(f, a.nu_ref, q[4], q[5], a.code_amp);
-    double mean = 0.0, isig = 0.0, scale = 0.0;
-    if (wid > 0.0) {
-      const double sigma = wid / (2.0 * sqrt(2.0 * log(2.0)));
-      mean = loc - floor(loc);                      // loc % 1
-      isig = 1.0 / sigma;
-      // the peak bin (argmax of the profile = smallest |z|, first index on ties) fixes the
-      // amplitude: value exp(-0.5 ((x[ipk] - loc)/sigma)^2) at the peak bin (pplib.py:820-823)
-      int i0 = (int)floor(mean * nbin);
-      double best = CUDART_INF; int ipk = -1;
-      for (int d = -1; d <= 1; ++d) {
-        const int i = ((i0 + d) % nbin + nbin) % nbin;
-        const double z = fabs((wrapx(xbin(i), mean) - mean) * isig);
-        if (z < best || (z == best && i < ipk)) { best = z; ipk = i; }
-      }
-      if (best < 20.0) {
-        const double xp = wrapx(xbin(ipk), mean);
-        const double zl = (xp - loc) * isig;
-        scale = amp * exp(-0.5 * zl * zl) / exp(-0.5 * best * best);
-      }
-    }
-    g_mean[g] = mean; g_isig[g] = isig; g_amp[g] = scale;
+    comp[g] = gauss_comp(loc, wid, amp, xbin);
   }
   if (tid == 0) a.taus[ch] = (a.params[1] / (double)nbin) * pow(f / a.nu_ref, a.alpha);   // pplib.py:4049-4053
   __syncthreads();
@@ -2522,9 +2546,10 @@ __global__ void __launch_bounds__(256) k_gauss_model(GaussModelArgs a) {
     const double x = xbin(i);
     double v = dc;
     for (int g = 0; g < a.ngauss; ++g) {
-      if (g_amp[g] == 0.0) continue;
-      const double z = (wrapx(x, g_mean[g]) - g_mean[g]) * g_isig[g];
-      if (fabs(z) < 20.0) v += g_amp[g] * exp(-0.5 * z * z);
+      const GaussComp& c = comp[g];
+      if (c.scale == 0.0) continue;
+      const double z = c.z(x);
+      if (fabs(z) < 20.0) v += c.scale * exp(-0.5 * z * z);
     }
     if (a.out64) a.out64[(size_t)ch * nbin + i] = v;
     else a.out[(size_t)ch * nbin + i] = (float)v;

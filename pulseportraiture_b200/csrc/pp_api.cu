@@ -17,6 +17,7 @@
 
 #include "../../include/ppb200.h"
 #include "kernels.cuh"
+#include "gaussfit.cuh"
 #include "tw_host.h"
 
 using namespace ppb;
@@ -123,6 +124,8 @@ struct pp_plan {
       rot_phase, rot_dm, rot_P, rot_nuref;
   // chunk-sized
   DBuf X, Xlo, partial, data_stage[2], data_stage64[2], Dspec, Ddc, al_acc, al_wparts;
+  // evolving-Gaussian portrait fit (pp_fit_gaussian_portraits): per-chunk state and outputs, per-CTA slabs
+  DBuf gf_data, gf_errs, gf_rec, gf_slab, gf_state, gf_out, gf_model, gf_par;
   // timing
   bool timing = false;
   std::vector<cudaEvent_t> ev_chunk;   // "chunk finished" events for the overlapped result copies
@@ -1944,5 +1947,200 @@ extern "C" int pp_get_noise_cut_batch(pp_plan_t* pl, const float* data, int32_t 
   CK(cudaGetLastError());
   if (copy_out_at(pl->stream, noise_out, pl->ps_noise.as<double>(), 0, (size_t)nrows)) return -2;
   CK(cudaStreamSynchronize(pl->stream));
+  return 0;
+}
+
+// ----------------------------------------------------------------------------
+// evolving-Gaussian portrait fit (gaussfit.cuh)
+// ----------------------------------------------------------------------------
+// Device scratch of one call: the per-CTA slabs, nslab x (L + 1) x (nbin/2 + 1) x 16 bytes with nslab =
+// (resident CTAs of k_gfit_pass), and per chunk of portraits the channel records (nchan x S doubles),
+// the staged data, the state and the outputs (~ 3 P^2 + nchan nbin doubles) of each portrait.  The
+// chunk is sized so that this per-chunk part stays under kGfitChunkBytes (at least one portrait, at most
+// 65535), or is pp_plan_set_chunk's count: the scratch does not grow with nport.
+static const size_t kGfitChunkBytes = 256u << 20;
+
+template <int N> static int gfit_slabs(pp_plan* pl, int* nslab) {
+  const size_t smem = fft_smem_bytes<N, double>();
+  CK(cudaFuncSetAttribute(k_gfit_pass<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int per_sm = 0;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_gfit_pass<N>, 256, smem));
+  *nslab = std::max(1, per_sm) * pl->sm_count;
+  return 0;
+}
+
+template <int N> static int gfit_pass(pp_plan* pl, const GfitArgs& a, int nslab) {
+  const long units = (long)a.nc * a.nchan;
+  const unsigned grid = (unsigned)std::min<long>(units, nslab);
+  k_gfit_pass<N><<<grid, 256, fft_smem_bytes<N, double>(), pl->stream>>>(a);
+  pl->stats.launches++;
+  pl->stats.pass_launches++;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* args, const pp_gfit_out_t* out) {
+  if (!pl || !args || !out) return fail(-1, "NULL argument");
+  const pp_gfit_args_t& A = *args;
+  if (A.nport < 1) return fail(-1, "nport must be >= 1");
+  if (!A.data || !A.errs || !A.init || !A.model_code || !A.fit_flags) return fail(-1, "NULL input array");
+  if (A.ngauss < 1 || A.ngauss > kGfitMaxGauss) return fail(-1, "ngauss must be in [1, %d] (got %d)", kGfitMaxGauss, A.ngauss);
+  if (strlen(A.model_code) < 3) return fail(-1, "model_code needs three characters (loc, wid, amp)");
+  for (int i = 0; i < 3; ++i)
+    if (A.model_code[i] != '0' && A.model_code[i] != '1') return fail(-1, "model_code digit %d must be '0' or '1'", i);
+  if (!(A.nu_ref > 0.0)) return fail(-1, "nu_ref must be positive");
+  if (pl->anyn) return fail(-1, "the Gaussian portrait fit needs nbin a power of two in [64, 4096] (got %d)", pl->nbin);
+  if (!pl->freqs_set) return fail(-1, "pp_set_freqs must be called before pp_fit_gaussian_portraits");
+  if (is_device_ptr(A.fit_flags) || (A.bounds && is_device_ptr(A.bounds))) return fail(-1, "fit_flags and bounds must be host arrays");
+  CK(cudaSetDevice(pl->device));
+  stats_begin(pl);
+  const int N = pl->N, nbin = pl->nbin, nchan = pl->nchan, ng = A.ngauss;
+  const int P = 3 + 6 * ng, L = 2 + 3 * ng, S = (L + 1) * (L + 2) / 2 + P;
+  const int nport = A.nport;
+  // host checks of sigma (a device array is read back once)
+  {
+    std::vector<double> e((size_t)nport * nchan);
+    CK(cudaMemcpy(e.data(), A.errs, sizeof(double) * e.size(), cudaMemcpyDefault));
+    for (size_t i = 0; i < e.size(); ++i)
+      if (!(e[i] > 0.0) || !std::isfinite(e[i]))
+        return fail(-1, "errs must be positive and finite (portrait %d, channel %d: %g)", (int)(i / nchan), (int)(i % nchan), e[i]);
+  }
+  std::vector<uint8_t> fr(P);
+  std::vector<double> lo(P, -INFINITY), hi(P, INFINITY);
+  int nfree = 0;
+  for (int i = 0; i < P; ++i) { fr[i] = A.fit_flags[i] ? 1 : 0; nfree += fr[i]; }
+  if (A.bounds)
+    for (int i = 0; i < P; ++i) {
+      if (!std::isnan(A.bounds[2 * i])) lo[i] = A.bounds[2 * i];
+      if (!std::isnan(A.bounds[2 * i + 1])) hi[i] = A.bounds[2 * i + 1];
+      if (lo[i] > hi[i]) return fail(-1, "bounds of parameter %d: lower > upper", i);
+    }
+  const int max_iter = A.max_iter == 0 ? 200 : A.max_iter;
+  const double tol = A.tol > 0.0 ? A.tol : 1e-4;
+  // chunk of portraits
+  const size_t per_port = sizeof(double) * ((size_t)nchan * S + (size_t)nchan * nbin * (out->model ? 2 : 1) + 4 * (size_t)P * P + 8 * P + 16);
+  size_t want = pl->chunk_req > 0 ? (size_t)pl->chunk_req : std::max<size_t>(1, kGfitChunkBytes / per_port);
+  // the chunk's portraits are gridDim.y of k_gfit_reduce (<= 65535)
+  const int chunk = (int)std::min<size_t>(std::min<size_t>(want, 65535), (size_t)nport);
+  int nslab = 0;
+  DISPATCH_N(N, if (gfit_slabs<NN>(pl, &nslab)) return -2);
+  nslab = (int)std::min<long>(nslab, (long)chunk * nchan);
+  CK(pl->gf_slab.need(sizeof(double2) * (size_t)nslab * (L + 1) * (N + 1)));
+  CK(pl->gf_rec.need(sizeof(double) * (size_t)chunk * nchan * S));
+  CK(pl->gf_data.need(sizeof(double) * (size_t)chunk * nchan * nbin));
+  CK(pl->gf_errs.need(sizeof(double) * (size_t)chunk * nchan));
+  if (out->model) CK(pl->gf_model.need(sizeof(double) * (size_t)chunk * nchan * nbin));
+  // parameter tables: free flags (as bytes after lo, hi)
+  CK(pl->gf_par.need(sizeof(double) * 2 * P + P));
+  {
+    std::vector<unsigned char> h(sizeof(double) * 2 * P + P);
+    memcpy(h.data(), lo.data(), sizeof(double) * P);
+    memcpy(h.data() + sizeof(double) * P, hi.data(), sizeof(double) * P);
+    memcpy(h.data() + sizeof(double) * 2 * P, fr.data(), P);
+    CK(cudaMemcpyAsync(pl->gf_par.p, h.data(), h.size(), cudaMemcpyHostToDevice, pl->stream));
+    CK(cudaStreamSynchronize(pl->stream));
+  }
+  const double* d_lo = pl->gf_par.as<double>();
+  const double* d_hi = d_lo + P;
+  const uint8_t* d_free = reinterpret_cast<const uint8_t*>(d_lo + 2 * P);
+  // chunk state
+  const size_t PP = (size_t)P * P;
+  const size_t n_state = (size_t)chunk * (4 * P + 2 * PP + 3);
+  CK(pl->gf_state.need(sizeof(double) * n_state + sizeof(int) * (2 * (size_t)chunk + 1)));
+  GfitState st;
+  {
+    double* b = pl->gf_state.as<double>();
+    st.x = b; b += (size_t)chunk * P;
+    st.xt = b; b += (size_t)chunk * P;
+    st.jtj_t = b; b += chunk * PP;
+    st.jtj = b; b += chunk * PP;
+    st.jtr_t = b; b += (size_t)chunk * P;
+    st.jtr = b; b += (size_t)chunk * P;
+    st.chi2_t = b; b += chunk;
+    st.chi2 = b; b += chunk;
+    st.lam = b; b += chunk;
+    int* ib = reinterpret_cast<int*>(b);
+    st.nfev = ib; ib += chunk;
+    st.done = ib; ib += chunk;
+  }
+  int* d_running = reinterpret_cast<int*>(st.done + chunk);
+  // chunk outputs: params, errs, cov, chi2, red_chi2, jtr, jtj (doubles), nfeval, rc (ints)
+  const size_t n_out = (size_t)chunk * (2 * P + 2 * PP + 2 + P);
+  CK(pl->gf_out.need(sizeof(double) * n_out + sizeof(int) * 2 * (size_t)chunk));
+  GfitUpdateArgs u;
+  {
+    double* b = pl->gf_out.as<double>();
+    u.params = b; b += (size_t)chunk * P;
+    u.errs = b; b += (size_t)chunk * P;
+    u.cov = b; b += chunk * PP;
+    u.jtj = b; b += chunk * PP;
+    u.jtr = b; b += (size_t)chunk * P;
+    u.chi2 = b; b += chunk;
+    u.red_chi2 = b; b += chunk;
+    u.nfeval = reinterpret_cast<int*>(b);
+    u.rc = u.nfeval + chunk;
+  }
+  u.free_ = d_free; u.lo = d_lo; u.hi = d_hi; u.P = P; u.max_iter = max_iter; u.tol = tol;
+  u.ndata = (double)nchan * (double)nbin; u.running = d_running;
+  const size_t usmem = sizeof(double) * 2 * PP;
+  CK(cudaFuncSetAttribute(k_gfit_update, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)usmem));
+  GfitArgs g;
+  g.freqs = pl->freqs.as<double>(); g.rec = pl->gf_rec.as<double>(); g.slab = pl->gf_slab.as<double2>();
+  g.twN = pl->twN64.p; g.tw2N = pl->tw2N64.p; g.nu_ref = A.nu_ref; g.nchan = nchan; g.ngauss = ng;
+  g.P = P; g.L = L; g.S = S;
+  for (int i = 0; i < 3; ++i) g.code[i] = A.model_code[i] - '0';
+  const int npair_all = P * (P + 1) / 2 + P + 1;
+  std::vector<double> x0((size_t)chunk * P);
+  for (int s0 = 0; s0 < nport; s0 += chunk) {
+    const int nc = std::min(chunk, nport - s0);
+    const size_t rows = (size_t)nc * nchan;
+    CK(cudaMemcpyAsync(pl->gf_data.p, A.data + (size_t)s0 * nchan * nbin, sizeof(double) * rows * nbin,
+                       cudaMemcpyDefault, pl->stream));
+    CK(cudaMemcpyAsync(pl->gf_errs.p, A.errs + (size_t)s0 * nchan, sizeof(double) * rows, cudaMemcpyDefault, pl->stream));
+    // start values moved into the box
+    CK(cudaMemcpyAsync(x0.data(), A.init + (size_t)s0 * P, sizeof(double) * nc * P, cudaMemcpyDefault, pl->stream));
+    CK(cudaStreamSynchronize(pl->stream));
+    for (int s = 0; s < nc; ++s)
+      for (int i = 0; i < P; ++i) x0[(size_t)s * P + i] = std::min(std::max(x0[(size_t)s * P + i], lo[i]), hi[i]);
+    CK(cudaMemcpyAsync(st.xt, x0.data(), sizeof(double) * nc * P, cudaMemcpyHostToDevice, pl->stream));
+    {
+      std::vector<double> lam(nc, kGfitLam0);
+      CK(cudaMemcpyAsync(st.lam, lam.data(), sizeof(double) * nc, cudaMemcpyHostToDevice, pl->stream));
+      CK(cudaMemsetAsync(st.nfev, 0, sizeof(int) * 2 * chunk, pl->stream));   // nfev and done
+      CK(cudaStreamSynchronize(pl->stream));
+    }
+    g.data = pl->gf_data.as<double>(); g.errs = pl->gf_errs.as<double>(); g.nc = nc;
+    // passes are launched while some portrait of the chunk is still running
+    for (;;) {
+      g.xt = st.xt; g.done = st.done; g.model = nullptr;
+      DISPATCH_N(N, if (gfit_pass<NN>(pl, g, nslab)) return -2);
+      k_gfit_reduce<<<dim3((npair_all + 255) / 256, nc), 256, 0, pl->stream>>>(g, st, d_free);
+      CK(cudaMemsetAsync(d_running, 0, sizeof(int), pl->stream));
+      k_gfit_update<<<nc, 256, usmem, pl->stream>>>(st, u);
+      pl->stats.launches += 2;
+      CK(cudaGetLastError());
+      int running = 0;
+      CK(cudaMemcpyAsync(&running, d_running, sizeof(int), cudaMemcpyDeviceToHost, pl->stream));
+      CK(cudaStreamSynchronize(pl->stream));
+      if (running == 0) break;
+    }
+    if (out->model) {   // the fitted portraits, evaluated at the final point of each
+      g.xt = st.x; g.done = nullptr; g.model = pl->gf_model.as<double>();
+      DISPATCH_N(N, if (gfit_pass<NN>(pl, g, nslab)) return -2);
+      if (copy_out_at(pl->stream, out->model + (size_t)s0 * nchan * nbin, pl->gf_model.as<double>(), 0, rows * nbin)) return -2;
+    }
+    const cudaStream_t sm = pl->stream;
+    if (copy_out_at(sm, out->params + (out->params ? (size_t)s0 * P : 0), u.params, 0, (size_t)nc * P)) return -2;
+    if (copy_out_at(sm, out->param_errs + (out->param_errs ? (size_t)s0 * P : 0), u.errs, 0, (size_t)nc * P)) return -2;
+    if (copy_out_at(sm, out->cov + (out->cov ? (size_t)s0 * PP : 0), u.cov, 0, (size_t)nc * PP)) return -2;
+    if (copy_out_at(sm, out->jtj + (out->jtj ? (size_t)s0 * PP : 0), u.jtj, 0, (size_t)nc * PP)) return -2;
+    if (copy_out_at(sm, out->jtr + (out->jtr ? (size_t)s0 * P : 0), u.jtr, 0, (size_t)nc * P)) return -2;
+    if (copy_out_at(sm, out->chi2 + (out->chi2 ? s0 : 0), u.chi2, 0, (size_t)nc)) return -2;
+    if (copy_out_at(sm, out->red_chi2 + (out->red_chi2 ? s0 : 0), u.red_chi2, 0, (size_t)nc)) return -2;
+    if (copy_out_at(sm, out->nfeval + (out->nfeval ? s0 : 0), u.nfeval, 0, (size_t)nc)) return -2;
+    if (copy_out_at(sm, out->return_code + (out->return_code ? s0 : 0), u.rc, 0, (size_t)nc)) return -2;
+    CK(cudaStreamSynchronize(pl->stream));
+  }
+  CK(cudaGetLastError());
   return 0;
 }

@@ -318,6 +318,60 @@ class WidebandPlan(object):
         del keep
         return res
 
+    # ---- evolving-Gaussian model fit ----------------------------------------------------
+    def fit_gaussian_portraits(self, data, errs, model_code, init, fit_flags, nu_ref, bounds=None,
+                               max_iter=0, tol=0, want_model=False, want_sums=False):
+        """Fit evolving-Gaussian portraits (pplib.py:1924-2052) to ``data`` [nport, nchan, nbin] float64
+        with per-channel sigma ``errs`` [nport, nchan], on the plan's frequencies (set_freqs first).
+        ``init`` [nport, P] and ``fit_flags`` [P] use the layout [DC, tau [bin], (loc, m_loc, wid, m_wid,
+        amp, m_amp) * ngauss, alpha], P = 3 + 6 ngauss; ``bounds`` [P, 2] with NaN (or None) for open
+        ends.  ``max_iter`` < 0 evaluates chi2, J^T r and J^T J at the start point only (0: default 200);
+        ``tol`` 0 = 1e-4.  numpy arrays or CUDA tensors.  Returns a dict of numpy arrays: params,
+        param_errs, cov, chi2, red_chi2, dof, nfeval, return_code, and with ``want_model`` the model
+        portraits [nport, nchan, nbin], with ``want_sums`` jtr [nport, P] and jtj [nport, P, P]."""
+        fit_flags = np.ascontiguousarray(np.asarray(fit_flags) != 0, dtype=np.uint8).ravel()
+        P = fit_flags.size
+        if P < 9 or (P - 3) % 6:
+            raise ValueError("fit_flags must have 3 + 6*ngauss entries")
+        ngauss = (P - 3) // 6
+        nport = int(data.shape[0])
+        nchan, nbin = self.nchan, self.nbin
+        keep = []
+        a = _ffi.GfitArgs()
+        a.nport = nport
+        a.data = _ptr(data, np.float64, keep, "data", (nport, nchan, nbin))
+        a.errs = _ptr(errs, np.float64, keep, "errs", (nport, nchan))
+        a.model_code = str(model_code).encode("ascii")
+        a.ngauss = ngauss
+        a.nu_ref = float(nu_ref)
+        a.init = _ptr(init, np.float64, keep, "init", (nport, P))
+        a.fit_flags = fit_flags.ctypes.data
+        if bounds is not None:
+            b = np.array([[np.nan if v is None else v for v in pair] for pair in bounds], dtype=np.float64)
+            if b.shape != (P, 2):
+                raise ValueError("bounds must be [P, 2]")
+            a.bounds = _ptr(b, np.float64, keep, "bounds")
+        a.max_iter = int(max_iter)
+        a.tol = float(tol)
+        spec = {"params": ((nport, P), np.float64), "param_errs": ((nport, P), np.float64),
+                "cov": ((nport, P, P), np.float64), "chi2": ((nport,), np.float64),
+                "red_chi2": ((nport,), np.float64), "nfeval": ((nport,), np.int32),
+                "return_code": ((nport,), np.int32)}
+        if want_model:
+            spec["model"] = ((nport, nchan, nbin), np.float64)
+        if want_sums:
+            spec["jtr"] = ((nport, P), np.float64)
+            spec["jtj"] = ((nport, P, P), np.float64)
+        res = {k: np.empty(sh, dtype=dt) for k, (sh, dt) in spec.items()}
+        o = _ffi.GfitOut()
+        for k, v in res.items():
+            setattr(o, k, v.ctypes.data)
+        _ffi.check(self._lib.pp_fit_gaussian_portraits(self._h, C.byref(a), C.byref(o)),
+                   "pp_fit_gaussian_portraits")
+        del keep
+        res["dof"] = np.full(nport, nchan * nbin - int(fit_flags.sum()), dtype=np.int64)
+        return res
+
     # ---- batched 1-D FFTFIT --------------------------------------------------------
     def fit_phase_shift_batch(self, profiles, models, noise=None, Ns=100, bounds=(-0.5, 0.5)):
         """Batched pplib.fit_phase_shift; ``bounds`` = ends of the brute-force grid (pplib.py:2085)."""

@@ -557,6 +557,108 @@ def read_model(modelfile, phases=None, freqs=None, P=None, quiet=False, device=F
     return (modelname, ngauss, model)
 
 
+# ---- ppgauss: fitting and writing evolving-Gaussian models --------------------------------------
+# lower edge of the facade's 0 < wid box: far below one bin of the largest nbin (1/4096 ~ 2.4e-4 rot)
+_gauss_wid_min = 1e-6
+
+
+def _gauss_default_bounds(model_code, ngauss):
+    """[P, 2] bounds (NaN = open) in the layout [DC, tau, comps..., alpha]: tau >= 0,
+    _gauss_wid_min <= wid <= wid_max, amp >= 0, and loc >= 0 where the loc code is a power law (its
+    logarithm is taken)."""
+    P = 3 + 6 * ngauss
+    b = np.full((P, 2), np.nan)
+    b[1, 0] = 0.0
+    for ig in range(ngauss):
+        o = 2 + 6 * ig
+        if model_code[0] == "0":
+            b[o, 0] = 0.0
+        b[o + 2] = (_gauss_wid_min, wid_max)
+        b[o + 4, 0] = 0.0
+    return b
+
+
+def fit_gaussian_portrait(model_code, data, init_params, scattering_index, errs, fit_flags,
+                          fit_scattering_index, phases, freqs, nu_ref, join_params=[], P=None,
+                          quiet=True):
+    """Fit an evolving-Gaussian model portrait to ``data`` [nchan, nbin] (pplib.py:1924-2052), on the GPU.
+
+    init_params = [DC, tau [bin], (loc, m_loc, wid, m_wid, amp, m_amp) * ngauss] as gen_gaussian_portrait
+    takes them, scattering_index the start value of alpha, errs [nchan] the per-channel sigma, fit_flags
+    one flag per entry of init_params and fit_scattering_index alpha's flag.  ``phases`` must be
+    get_bin_centers(nbin); nbin a power of two in [64, 4096].  The objective is the reference's
+    chi^2 = sum (data - model)^2 / errs^2 with the model of gen_gaussian_portrait (scattered when tau != 0
+    or tau / alpha are free), minimised by a Levenberg-Marquardt solver with analytic derivatives
+    (WidebandPlan.fit_gaussian_portraits).
+
+    Bounds, the policy of this facade: tau >= 0, 0 < wid <= wid_max (wid_max = 0.25 in this module's
+    settings; the lower edge is wid = 1e-6 rot, far below one bin), amp >= 0, and loc >= 0 when its
+    evolution code is a power law.  A free parameter that cannot move the model at the fitted point (alpha
+    while tau = 0, for example) gets fit_err 0 and a zero covariance row, MINPACK's convention.  Join
+    parameters (multi-receiver offsets) are not supported.
+
+    Returns a DataBunch with fitted_params (layout of init_params, tau in bins), fit_errs,
+    scattering_index, scattering_index_err, chi2, dof, red_chi2, nfeval, return_code (0 converged,
+    1 iteration limit, 3 non-finite), duration, and the extras covariance ([P, P] in the layout
+    [params..., alpha], scaled by red_chi2 as lmfit's scale_covar) and model (the fitted portrait,
+    float64).  The reference's lm_results (the lmfit object) cannot be provided."""
+    if len(join_params):
+        raise NotImplementedError("join parameters are a ppgauss feature")
+    start = time.time()
+    data = np.asarray(data, dtype=np.float64)
+    nchan, nbin = data.shape
+    if len(phases) != nbin or not np.allclose(phases, get_bin_centers(nbin), rtol=0, atol=1e-12):
+        raise ValueError("the device fit works on get_bin_centers(nbin)")
+    init_params = np.asarray(init_params, dtype=np.float64)
+    if init_params.ndim != 1 or (init_params.size - 2) % 6 or init_params.size < 8:
+        raise ValueError("init_params must have 2 + 6*ngauss entries")
+    ngauss = (init_params.size - 2) // 6
+    x0 = np.append(init_params, float(scattering_index))
+    flags = np.append(np.asarray(fit_flags, dtype=bool), bool(fit_scattering_index))
+    pl = get_plan(nchan, nbin)
+    pl.set_freqs(np.asarray(freqs, dtype=np.float64))
+    r = pl.fit_gaussian_portraits(data[None], np.asarray(errs, dtype=np.float64).reshape(1, nchan), model_code,
+                                  x0[None], flags, nu_ref, bounds=_gauss_default_bounds(model_code, ngauss),
+                                  want_model=True)
+    params, perrs = r["params"][0], r["param_errs"][0]
+    rc = int(r["return_code"][0])
+    if not quiet:
+        print("Fit %d-component model: chi2 %.3f, red_chi2 %.5f, %d evaluations (%s)"
+              % (ngauss, r["chi2"][0], r["red_chi2"][0], r["nfeval"][0], DEVICE_RCSTRINGS.get(str(rc), rc)))
+    return DataBunch(fitted_params=params[:-1].copy(), fit_errs=perrs[:-1].copy(),
+                     scattering_index=params[-1], scattering_index_err=perrs[-1],
+                     chi2=r["chi2"][0], dof=int(r["dof"][0]), red_chi2=r["red_chi2"][0],
+                     nfeval=int(r["nfeval"][0]), return_code=rc, duration=time.time() - start,
+                     covariance=r["cov"][0], model=r["model"][0])
+
+
+def write_model(filenm, name, model_code, nu_ref, model_params, fit_flags, alpha, fit_alpha,
+                append=False, quiet=False):
+    """Write a .gmodel file that read_model parses (pplib.py:2830-2865), in the layout of ppgauss's
+    output: MODEL, CODE, FREQ, DC, TAU, ALPHA and one COMPnn line per component.
+
+    model_params = [DC, TAU, (loc, m_loc, wid, m_wid, amp, m_amp) * ngauss] with TAU in seconds, the
+    file's unit: a tau fitted in bins (fit_gaussian_portrait) is written as tau_bin * P / nbin for a
+    period P [s].  Values are printed with 12 decimals (FREQ with 10)."""
+    model_params = np.asarray(model_params, dtype=np.float64)
+    fit_flags = np.asarray(fit_flags).astype(int)
+    ngauss = (len(model_params) - 2) // 6
+    lines = ["MODEL   %s" % name,
+             "CODE    %s" % model_code,
+             "FREQ    %.10f" % nu_ref,
+             "DC     % .12f %d" % (model_params[0], fit_flags[0]),
+             "TAU    % .12f %d" % (model_params[1], fit_flags[1]),
+             "ALPHA  % .12f %d" % (alpha, int(fit_alpha))]
+    for ig in range(ngauss):
+        o = 2 + 6 * ig
+        fields = "".join("  % .12f %d" % (model_params[o + k], fit_flags[o + k]) for k in range(6))
+        lines.append("COMP%02d%s" % (ig + 1, fields))
+    with open(filenm, "a" if append else "w") as fh:
+        fh.write("\n".join(lines) + "\n")
+    if not quiet:
+        print("%s written." % filenm)
+
+
 # ---- TOA output (host text formatting; pplib.py:3380-3503) ----------------------------------
 def filter_TOAs(TOAs, flag, cutoff, criterion=">=", pass_unflagged=False, return_culled=False):
     """Keep the TOAs whose attribute ``flag`` satisfies ``<criterion> cutoff`` (pplib.py:3380-3407)."""
