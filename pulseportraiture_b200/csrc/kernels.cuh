@@ -3070,22 +3070,32 @@ __global__ void __launch_bounds__(256) k_rot_mul(RotateArgs a, cx<double>* spec,
   if (threadIdx.x == 0 && resp) dc[row] *= resp[0];
 }
 
-// aligned[n] += sum_s w[s,n] rot[s,n,:] in double (the accumulation of ppalign.py:202-208 on rotated rows)
-__global__ void __launch_bounds__(256) k_wsum_rows(const float* __restrict__ rot, const double* __restrict__ w, double* aligned,
-                                                    double* wsum, int nsub, int nchan, int nbin, int first_call) {
+// acc[n] += sum_s w[s,n] spec[s,n] over the rotated spectrum rows (slot layout) and dc[n] likewise, in double,
+// subints in order: the accumulation of ppalign.py:202-208 for any nbin (one inverse transform of acc follows)
+__global__ void __launch_bounds__(256) k_wsum_spec(const cx<double>* __restrict__ spec, const double* __restrict__ dc,
+                                                    const double* __restrict__ w, cx<double>* acc, double* acc_dc, double* wsum,
+                                                    int nsub, int nchan, int Npad, int first_call) {
   const int ch = blockIdx.x;
-  for (int j = threadIdx.x; j < nbin; j += 256) {
-    double acc = first_call ? 0.0 : aligned[(size_t)ch * nbin + j];
+  for (int k = threadIdx.x; k < Npad; k += 256) {
+    cx<double> v = first_call ? mk<double>(0.0, 0.0) : acc[(size_t)ch * Npad + k];
     for (int s = 0; s < nsub; ++s) {
       const double ws = w[(size_t)s * nchan + ch];
-      if (ws != 0.0 && fabs(ws) < 1e300) acc = fma(ws, (double)rot[((size_t)s * nchan + ch) * nbin + j], acc);
+      if (ws != 0.0 && fabs(ws) < 1e300) {
+        const cx<double> d = spec[((size_t)s * nchan + ch) * Npad + k];
+        v.x = fma(ws, d.x, v.x);
+        v.y = fma(ws, d.y, v.y);
+      }
     }
-    aligned[(size_t)ch * nbin + j] = acc;
+    acc[(size_t)ch * Npad + k] = v;
   }
   if (threadIdx.x == 0) {
-    double t = first_call ? 0.0 : wsum[ch];
-    for (int s = 0; s < nsub; ++s) { const double ws = w[(size_t)s * nchan + ch]; if (ws != 0.0 && fabs(ws) < 1e300) t += ws; }
+    double t = first_call ? 0.0 : wsum[ch], d0 = first_call ? 0.0 : acc_dc[ch];
+    for (int s = 0; s < nsub; ++s) {
+      const double ws = w[(size_t)s * nchan + ch];
+      if (ws != 0.0 && fabs(ws) < 1e300) { t += ws; d0 = fma(ws, dc[(size_t)s * nchan + ch], d0); }
+    }
     wsum[ch] = t;
+    acc_dc[ch] = d0;
   }
 }
 

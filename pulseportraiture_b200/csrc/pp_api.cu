@@ -123,7 +123,7 @@ struct pp_plan {
   DBuf resp, rot_gm, rot_nugm, al_w, al_out, al_wsum, ps_phase, ps_perr, ps_scale, ps_serr, ps_snr, ps_rchi2, ps_lag, ps_spec, ps_mspec, ps_noise, rot_in, rot_out,
       rot_phase, rot_dm, rot_P, rot_nuref;
   // chunk-sized
-  DBuf X, Xlo, partial, data_stage[2], data_stage64[2], Dspec, Ddc, al_acc, al_wparts;
+  DBuf X, Xlo, partial, data_stage[2], data_stage64[2], Dspec, Ddc, al_acc, al_wparts, al_dc;
   // evolving-Gaussian portrait fit (pp_fit_gaussian_portraits): per-chunk state and outputs, per-CTA slabs
   DBuf gf_data, gf_errs, gf_rec, gf_slab, gf_state, gf_out, gf_model, gf_par;
   // timing
@@ -539,17 +539,25 @@ static int launch_inv_any(pp_plan* pl, const cx<double>* spec, const double* dc,
   pl->stats.launches++;
   return 0;
 }
+// (nbin not a power of two) the rotated / multiplied spectra of the a.nsub * a.nchan rows into any_spec2 / any_dc2
+static int rotate_spectra_any(pp_plan* pl, const RotateArgs& a) {
+  const int N = pl->N;
+  const long nrows = (long)a.nsub * a.nchan;
+  CK(pl->any_spec2.need(sizeof(double2) * (size_t)nrows * N));
+  CK(pl->any_dc2.need(sizeof(double) * (size_t)nrows));
+  if (launch_fwd_any(pl, a.in, false, nullptr, nullptr, nrows, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>())) return -2;
+  k_rot_mul<<<(unsigned)nrows, 256, 0, pl->stream>>>(a, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), N, pl->L);
+  pl->stats.launches++;
+  return 0;
+}
+
 // rfft -> multiply (rotation / scattering kernel / response) -> irfft of nrows = a.nsub * a.nchan rows: one
 // fused kernel for nbin = 2^m, transform / multiply / transform through the spectrum scratch otherwise
 static int rotate_rows(pp_plan* pl, RotateArgs a, bool fp64) {
   const int N = pl->N;
   const long nrows = (long)a.nsub * a.nchan;
   if (pl->anyn) {
-    CK(pl->any_spec2.need(sizeof(double2) * (size_t)nrows * N));
-    CK(pl->any_dc2.need(sizeof(double) * (size_t)nrows));
-    if (launch_fwd_any(pl, a.in, false, nullptr, nullptr, nrows, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>())) return -2;
-    k_rot_mul<<<(unsigned)nrows, 256, 0, pl->stream>>>(a, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), N, pl->L);
-    pl->stats.launches++;
+    if (rotate_spectra_any(pl, a)) return -2;
     return launch_inv_any(pl, pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), a.out, nrows, false);
   }
   if (fp64) {
@@ -1742,20 +1750,23 @@ extern "C" int pp_align_accumulate(pp_plan_t* pl, const float* data, int32_t nsu
   if (stage_in(pl, pl->al_w, weights, (size_t)nsub * nchan, &dw)) return -2;
   CK(pl->al_out.need(sizeof(double) * (size_t)nchan * pl->nbin));
   CK(pl->al_wsum.need(sizeof(double) * nchan));
-  if (pl->anyn) {   // rotate blocks of subints through the Bluestein transforms, add them up in double
+  if (pl->anyn) {   // rotate blocks of subints in the Fourier domain, add their spectra up in double, transform once
     const int blk = 64;
-    CK(pl->rot_out.need(sizeof(float) * (size_t)std::min(blk, nsub) * nchan * pl->nbin));
+    CK(pl->al_acc.need(sizeof(double2) * (size_t)nchan * N));
+    CK(pl->al_dc.need(sizeof(double) * nchan));
     for (int s0 = 0; s0 < nsub; s0 += blk) {
       const int ns = std::min(blk, nsub - s0);
       RotateArgs r;
-      r.in = din + (size_t)s0 * nchan * pl->nbin; r.out = pl->rot_out.as<float>(); r.phase = dph + s0; r.DM = ddm + s0;
+      r.in = din + (size_t)s0 * nchan * pl->nbin; r.out = nullptr; r.phase = dph + s0; r.DM = ddm + s0;
       r.P = dP + s0; r.nu_ref = dnr + s0; r.GM = nullptr; r.nu_GM = nullptr; r.nu2 = pl->nu2.as<double>(); r.taus = nullptr;
       r.resp = nullptr; r.nsub = ns; r.nchan = nchan;
-      if (rotate_rows(pl, r, true)) return -2;
-      k_wsum_rows<<<nchan, 256, 0, pl->stream>>>(pl->rot_out.as<float>(), dw + (size_t)s0 * nchan, pl->al_out.as<double>(),
-                                                 pl->al_wsum.as<double>(), ns, nchan, pl->nbin, s0 == 0);
+      if (rotate_spectra_any(pl, r)) return -2;
+      k_wsum_spec<<<nchan, 256, 0, pl->stream>>>(pl->any_spec2.as<cx<double>>(), pl->any_dc2.as<double>(), dw + (size_t)s0 * nchan,
+                                                 pl->al_acc.as<cx<double>>(), pl->al_dc.as<double>(), pl->al_wsum.as<double>(),
+                                                 ns, nchan, N, s0 == 0);
       pl->stats.launches++;
     }
+    if (launch_inv_any(pl, pl->al_acc.as<cx<double>>(), pl->al_dc.as<double>(), pl->al_out.as<double>(), nchan, true)) return -2;
   } else {
     AlignArgs a;
     a.r.in = din; a.r.out = nullptr; a.r.phase = dph; a.r.DM = ddm; a.r.P = dP; a.r.nu_ref = dnr; a.r.GM = nullptr;
