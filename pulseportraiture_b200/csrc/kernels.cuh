@@ -3123,8 +3123,19 @@ __global__ void __launch_bounds__(256) k_align_reduce_any(const double2* __restr
 // of chi2(a, b, dc) = sum_k (log10 pows_k - b e^{-a k} - dc)^2 over a in [1/nharm, 1], b in
 // [0, max - min], dc in [min, max] of log10 pows; the first k with e^{-a k} < 0.005.  One CTA per row:
 // the table e^{-a k} of one a at a time in shared memory, the 400 (b, dc) points of that slice spread over
-// the threads; flat argmin in scipy's C order (a slowest), lowest index on ties.
+// the threads.  The grid values are np.mgrid's, i * step + start rounded twice, and the model term is
+// b e^{-a k} + dc rounded twice, as numpy evaluates them.  The flat argmin in scipy's C order (a slowest)
+// follows np.argmin (noise_argmin_before).
 // ----------------------------------------------------------------------------
+// np.argmin's order over the flat grid: a NaN chi2 wins, the first one; otherwise the lowest chi2, the lowest
+// index on ties.  A row with an exactly zero harmonic has log10 pows = -inf, which makes every chi2 NaN: then
+// grid point 0 (a = 1/nharm) is the minimiser, as in the reference.
+__device__ __forceinline__ bool noise_argmin_before(double c, int i, double best, int besti) {
+  if (isnan(c)) return !isnan(best) || i < besti;
+  if (isnan(best)) return false;
+  return c < best || (c == best && i < besti);
+}
+
 __global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ spec, const double* __restrict__ dc, double* noise,
                                                     int nslot, int L, int nyq_slot, double fact) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -3155,33 +3166,35 @@ __global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ s
   __syncthreads();
   const double ymin = lim[0], ymax = lim[1];
   const double a_lo = 1.0 / (double)nh, a_st = (1.0 - a_lo) / 19.0, b_st = (ymax - ymin) / 19.0, d_st = (ymax - ymin) / 19.0;
+  auto mgrid = [](int i, double st, double lo) { return __dadd_rn(__dmul_rn((double)i, st), lo); };
+  // every thread evaluates at least one point (400 per a, 256 threads), so besti is a grid index after the loop
   double best = CUDART_INF;
   int besti = 0x7fffffff;
   for (int ia = 0; ia < 20; ++ia) {
-    const double av = (ia == 19) ? 1.0 : a_lo + ia * a_st;          // np.mgrid endpoints
+    const double av = mgrid(ia, a_st, a_lo);
     __syncthreads();
     for (int k = tid; k < nh; k += 256) ek[k] = exp(-av * (double)k);
     __syncthreads();
     for (int q = tid; q < 400; q += 256) {
       const int ib = q / 20, id = q % 20;
-      const double bv = (ib == 19) ? (ymax - ymin) : ib * b_st, dv = (id == 19) ? ymax : ymin + id * d_st;
+      const double bv = mgrid(ib, b_st, 0.0), dv = mgrid(id, d_st, ymin);
       double c2 = 0.0;
-      for (int k = 0; k < nh; ++k) { const double r = y[k] - (bv * ek[k] + dv); c2 = fma(r, r, c2); }
+      for (int k = 0; k < nh; ++k) { const double r = y[k] - __dadd_rn(__dmul_rn(bv, ek[k]), dv); c2 = fma(r, r, c2); }
       const int flat = ia * 400 + q;
-      if (c2 < best || (c2 == best && flat < besti)) { best = c2; besti = flat; }
+      if (noise_argmin_before(c2, flat, best, besti)) { best = c2; besti = flat; }
     }
   }
   for (int o = 16; o > 0; o >>= 1) {
     const double ov = __shfl_xor_sync(0xffffffffu, best, o);
     const int oi = __shfl_xor_sync(0xffffffffu, besti, o);
-    if (ov < best || (ov == best && oi < besti)) { best = ov; besti = oi; }
+    if (noise_argmin_before(ov, oi, best, besti)) { best = ov; besti = oi; }
   }
   if ((tid & 31) == 0) { shv[tid >> 5] = best; shi[tid >> 5] = besti; }
   __syncthreads();
   if (tid == 0) {
-    for (int w = 1; w < 8; ++w) if (shv[w] < best || (shv[w] == best && shi[w] < besti)) { best = shv[w]; besti = shi[w]; }
+    for (int w = 1; w < 8; ++w) if (noise_argmin_before(shv[w], shi[w], best, besti)) { best = shv[w]; besti = shi[w]; }
     const int ia = besti / 400;
-    const double av = (ia == 19) ? 1.0 : a_lo + ia * a_st;
+    const double av = mgrid(ia, a_st, a_lo);
     int kcrit = nh - 1;
     for (int k = 0; k < nh; ++k) if (exp(-av * (double)k) < 0.005) { kcrit = k; break; }
     double kf = fact * (double)kcrit;

@@ -221,29 +221,65 @@ def get_noise(data, method=default_noise_method, **kwargs):
     return 0
 
 
+def _power_spectrum(data):
+    """|rfft(data.ravel())|^2 / n in float64, on the facade's device.  The whole-portrait estimate is one
+    row of nchan * nbin samples, longer than any row plan takes, so it is transformed as one float64 rfft."""
+    import torch
+    x = torch.as_tensor(np.ascontiguousarray(np.ravel(data), dtype=np.float64), device=torch.device("cuda", _device))
+    X = torch.fft.rfft(x)
+    return (X.real * X.real + X.imag * X.imag) / x.numel()
+
+
+def _find_kc(pows):
+    """find_kc (pplib.py:1465-1495) of a power spectrum on the device: chi2 of b exp(-a k) + dc against
+    log10 pows at every point of scipy.optimize.brute's 20 x 20 x 20 np.mgrid, in chunks of grid points (C
+    order, a slowest); np.argmin's order picks the point (a NaN chi2 wins, the first one; otherwise the
+    lowest chi2, the lowest index on ties); the first k with exp(-a k) < 0.005, or nharm - 1."""
+    import torch
+    y = torch.log10(pows)
+    nh = y.numel()
+    lo, hi = float(y.min()), float(y.max())
+    with np.errstate(invalid="ignore"):    # an exactly zero harmonic: lo = -inf, the grid is NaN
+        grid = np.mgrid[nh ** -1.0:1.0:20j, 0:hi - lo:20j, lo:hi:20j].reshape(3, -1)
+    g = torch.as_tensor(grid, device=pows.device)
+    k = torch.arange(nh, dtype=torch.float64, device=pows.device)
+    c2 = torch.empty(g.shape[1], dtype=torch.float64, device=pows.device)
+    step = max(1, (1 << 24) // nh)          # grid points per chunk: at most 2^24 terms
+    for i0 in range(0, g.shape[1], step):
+        a, b, dc = g[:, i0:i0 + step, None]
+        c2[i0:i0 + step] = ((y - (b * torch.exp(-a * k) + dc)) ** 2).sum(-1)
+    nan = torch.isnan(c2)
+    i = int(torch.nonzero(nan)[0, 0]) if bool(nan.any()) else int(torch.argmin(c2))
+    hit = np.nonzero(np.exp(-grid[0, i] * np.arange(nh)) < 0.005)[0]
+    return int(hit[0]) if len(hit) else nh - 1
+
+
 def get_noise_fit(data, fact=1.1, chans=False):
     """Noise from the harmonics above fact * the cutoff a fit of b exp(-a k) + dc to the log power
-    spectrum finds (pplib.py:2255-2284, find_kc 1465-1495)."""
+    spectrum finds (pplib.py:2255-2284, find_kc 1465-1495).  chans=False: the whole of data as one row of
+    any length (_power_spectrum, _find_kc)."""
     data = np.asarray(data)
     if chans:
         nchan, nbin = data.shape
         return get_plan(nchan, nbin).get_noise_fit_batch(_f32(data)[None], fact)[0]
-    rav = data.ravel()
-    n = rav.size
-    return get_plan(1, n).get_noise_fit_batch(_f32(rav).reshape(1, 1, n), fact)[0, 0]
+    pows = _power_spectrum(data)
+    k_crit = fact * _find_kc(pows)
+    if k_crit >= pows.numel():
+        k_crit = min(int(0.99 * pows.numel()), k_crit)
+    return np.float64(pows[int(k_crit):].mean().sqrt().item())
 
 
 def get_noise_PS(data, frac=4, chans=False):
-    """Mean of the highest 1/frac of the power spectrum (pplib.py:2227-2253)."""
+    """Mean of the highest 1/frac of the power spectrum (pplib.py:2227-2253).  chans=False: the whole of
+    data as one row of any length (_power_spectrum)."""
     data = np.asarray(data)
     if chans:
         nchan, nbin = data.shape
         kc = int((1 - frac ** -1) * (nbin // 2 + 1))         # pplib.py:2244
         return get_plan(nchan, nbin).get_noise_batch(_f32(data)[None], kc=kc)[0]
-    rav = data.ravel()
-    n = rav.size
-    kc = int((1 - frac ** -1) * (n // 2 + 1))
-    return get_plan(1, n).get_noise_batch(_f32(rav).reshape(1, 1, n), kc=kc)[0, 0]
+    pows = _power_spectrum(data)
+    kc = int((1 - frac ** -1) * pows.numel())
+    return np.float64(pows[kc:].mean().sqrt().item())
 
 
 # ---- A10: rotation ----------------------------------------------------------------------
