@@ -406,6 +406,58 @@ typedef struct {
 int pp_fit_gaussian_portraits(pp_plan_t* plan, const pp_gfit_args_t* args,
                               const pp_gfit_out_t* out);
 
+/* ---- simulated archives ---------------------------------------------------------
+ * Replaces the data generation of pplib.make_fake_pulsar (pplib.py:3183-3378) for a batch of subints, without the
+ * PSRFITS writing.  Row (s, n), m = model_index[s]:
+ *   Y_k = S_sn M_mnk e^{-2 pi i k theta_sn} B_snk  (k = 0..nbin/2),   out = irfft(Y) + sigma_sn z(seed, s_global, n, b)
+ *   theta_sn = phase_s + Dconst DM_s (nu_n^-2 - nu_DM_s^-2)/P_s + Dconst^2 GM_s (nu_n^-4 - nu_GM_s^-4)/P_s
+ *   B_snk = 1/(1 + 2 pi i k tau_sn),  tau_sn = tau_s (nu_n/nu_tau_s)^alpha_s [rot]
+ * with M = rfft(models) in double (the DC and Nyquist terms included; irfft keeps the real part of the Nyquist
+ * term).  The parameters are the injected ones: pp_fit_batch on the output recovers phase, DM, GM, tau and alpha
+ * (a row is rotate_data(model, -phase, -DM), scattered).  The inverse transform is FP64.
+ * Noise z: Philox4x32-10 with key (seed low, seed high) and counter (b/4, n, s_global low, s_global high),
+ * s_global = first_subint + s, four uint32 per quad of bins 4q..4q+3, each mapped to u = f32((x >> 8) 2^-24 + 2^-25)
+ * and pairs through Box-Muller in float32 (accurate logf, sqrtf, sincospif): (z0, z1) = sqrt(-2 ln u0) (cos 2 pi u1,
+ * sin 2 pi u1); |z| <= 5.89.  A subint's samples depend only on (seed, s_global, its model and its parameters): not
+ * on the batch, the chunk (pp_plan_set_chunk) or the device, so a study can be split over calls and GPUs.
+ * Outputs: float32 rows and / or int16 rows with DAT_SCL / DAT_OFFS that are pptoas.quantize_subints of the float32
+ * rows bit for bit (offs = f32((hi + lo)/2), scl = f32((hi - lo)/65000) or 1, raw = clip(rint((x - offs)/scl)) in
+ * double).  Each array is taken for what it is, host or device, independently of the others: device outputs are
+ * written in place, host outputs go through the plan's page-locked staging chunk by chunk, and host per-subint inputs
+ * are staged chunk by chunk, so that device scratch is bounded independently of nsub.  The fit's model set and
+ * frequency tables are not touched.
+ * Errors (nothing is launched): nmodel < 1, a model index out of range, P <= 0, a frequency <= 0 (freqs, nu_DM,
+ * nu_GM, nu_tau), a negative sigma, no output.  nsub = 0 does nothing. */
+typedef struct {
+  const double* models;       /* [nmodel,nchan,nbin] float64 model portraits (host or device)       */
+  const double* freqs;        /* [nmodel,nchan] MHz                                                  */
+  int32_t nmodel;
+  const int32_t* model_index; /* [nsub] in [0, nmodel) or NULL (model 0)                             */
+  int32_t nsub;
+  int64_t first_subint;       /* global index of subint 0: the noise counter                         */
+  uint64_t seed;
+  const double* phase;        /* [nsub] rot                                                          */
+  const double* DM;           /* [nsub]                                                              */
+  const double* P;            /* [nsub] s, > 0                                                       */
+  const double* nu_DM;        /* [nsub] MHz (inf allowed)                                            */
+  const double* GM;           /* [nsub] or NULL, with nu_GM                                          */
+  const double* nu_GM;
+  const double* tau;          /* [nsub] rot at nu_tau, or NULL (unscattered), with alpha and nu_tau  */
+  const double* alpha;
+  const double* nu_tau;
+  const double* scales;       /* [nsub,nchan] or NULL (= 1)                                          */
+  const double* noise_std;    /* [nsub,nchan] time-domain sigma >= 0, or NULL (= 0)                  */
+} pp_sim_args_t;
+
+typedef struct {
+  float* data;                /* [nsub,nchan,nbin] float32 or NULL                                   */
+  int16_t* raw;               /* [nsub,nchan,nbin] int16 or NULL; dat_scl and dat_offs with it        */
+  float* dat_scl;             /* [nsub,nchan]                                                        */
+  float* dat_offs;            /* [nsub,nchan]                                                        */
+} pp_sim_out_t;               /* host or device pointers; data or raw must be given                  */
+
+int pp_simulate_batch(pp_plan_t* plan, const pp_sim_args_t* args, const pp_sim_out_t* out);
+
 /* ---- diagnostics ------------------------------------------------------------ */
 typedef struct {
   int64_t launches;        /* kernels launched by the last pp_* call            */

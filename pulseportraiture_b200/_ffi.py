@@ -26,6 +26,7 @@ SYMBOLS = ["pp_plan_create", "pp_plan_destroy", "pp_plan_set_stream",
            "pp_fit_phase_shift_batch", "pp_fit_phase_shift_batch_bounds", "pp_rotate_batch", "pp_rotate_full_batch", "pp_apply_response_batch",
            "pp_align_accumulate", "pp_gen_gaussian_portrait", "pp_gen_gaussian_portrait_f64", "pp_gen_spline_portrait",
            "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64", "pp_fit_gaussian_portraits",
+           "pp_simulate_batch",
            "pp_plan_enable_timing", "pp_get_stats", "pp_host_alloc",
            "pp_host_free", "pp_last_error",
            "pp_abi_version"]
@@ -127,6 +128,23 @@ class GfitOut(C.Structure):
         "jtr", "jtj", "model")]
 
 
+class SimArgs(C.Structure):
+    _fields_ = [
+        ("models", C.c_void_p),
+        ("freqs", C.c_void_p),
+        ("nmodel", C.c_int32),
+        ("model_index", C.c_void_p),
+        ("nsub", C.c_int32),
+        ("first_subint", C.c_int64),
+        ("seed", C.c_uint64),
+    ] + [(n, C.c_void_p) for n in ("phase", "DM", "P", "nu_DM", "GM", "nu_GM", "tau", "alpha", "nu_tau",
+                                   "scales", "noise_std")]
+
+
+class SimOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("data", "raw", "dat_scl", "dat_offs")]
+
+
 class Stats(C.Structure):
     _fields_ = [("launches", C.c_int64), ("pass_launches", C.c_int64),
                 ("pass_rows", C.c_int64), ("ms_spectra", C.c_double),
@@ -212,6 +230,8 @@ def lib():
     L.pp_measure_fp64.restype = C.c_int
     L.pp_fit_gaussian_portraits.argtypes = [vp, C.POINTER(GfitArgs), C.POINTER(GfitOut)]
     L.pp_fit_gaussian_portraits.restype = C.c_int
+    L.pp_simulate_batch.argtypes = [vp, C.POINTER(SimArgs), C.POINTER(SimOut)]
+    L.pp_simulate_batch.restype = C.c_int
     L.pp_plan_enable_timing.argtypes = [vp, i32]
     L.pp_plan_enable_timing.restype = C.c_int
     L.pp_get_stats.argtypes = [vp, C.POINTER(Stats)]

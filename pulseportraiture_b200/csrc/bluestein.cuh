@@ -141,6 +141,7 @@ struct FwdAnyArgs {
   const void* in;          // [nrows, 2L] float32 (or int16: I16) real rows
   const float* dat_scl;    // [nrows] int16 only
   const float* dat_offs;
+  const double* in64;      // [nrows, 2L] float64 rows read instead of `in` when non-null (not with I16)
   cx<double>* spec;        // [nrows, Npad] out: slot k = harmonic k (1 <= k <= L), the rest zero
   double* dc;              // [nrows] out: harmonic 0, or null
   AnyPlan p;
@@ -162,6 +163,9 @@ __global__ void __launch_bounds__(256) k_fwd_any(FwdAnyArgs a) {
         const short2 v = src[j];
         bufA[j] = mk<double>((double)__fadd_rn(__fmul_rn((float)v.x, scl), offs), (double)__fadd_rn(__fmul_rn((float)v.y, scl), offs));
       }
+    } else if (a.in64) {
+      const double2* src = reinterpret_cast<const double2*>(a.in64) + (size_t)row * L;
+      for (int j = tid; j < L; j += 256) { const double2 v = src[j]; bufA[j] = mk<double>(v.x, v.y); }
     } else {
       const float2* src = static_cast<const float2*>(a.in) + (size_t)row * L;
       for (int j = tid; j < L; j += 256) { const float2 v = src[j]; bufA[j] = mk<double>((double)v.x, (double)v.y); }

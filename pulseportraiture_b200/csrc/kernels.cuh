@@ -116,6 +116,8 @@ struct ModelArgs {
   double* pn;           // [nchan]
   const cx<double>* twN;
   const cx<double>* tw2N;
+  cx<double>* spec;     // [nchan, N + 1] or null: harmonic k at slot k, 0..N, and nothing else is written
+                        // (the model spectra of pp_simulate_batch; the fit's model set is left alone)
   int nchan;
 };
 
@@ -156,6 +158,10 @@ __global__ void __launch_bounds__(256) k_model(ModelArgs a) {
   double psum = 0.0;
   const size_t ro = (size_t)(valid ? ch : 0) * N;
   auto put = [&](int slot, cx<T> d) {
+    if (a.spec) {
+      if (valid) a.spec[(size_t)ch * (N + 1) + (slot == 0 ? N : slot)] = d;
+      return;
+    }
     const double pw = d.x * d.x + d.y * d.y;
     psum += pw;
     if (valid) {
@@ -175,6 +181,10 @@ __global__ void __launch_bounds__(256) k_model(ModelArgs a) {
     }
   }
   if (t_row == 0) put(0, mk<T>(Z[0].x - Z[0].y, 0.0));  // harmonic N (real)
+  if (a.spec) {   // (uniform over the grid) harmonic 0: the row sum
+    if (t_row == 0 && valid) a.spec[(size_t)ch * (N + 1)] = mk<T>(Z[0].x + Z[0].y, 0.0);
+    return;
+  }
   // reduce psum over the row-slot
 #pragma unroll
   for (int o = (G::kTRow < 32 ? G::kTRow : 32) / 2; o > 0; o >>= 1) psum += __shfl_xor_sync(0xffffffffu, psum, o);
@@ -3204,6 +3214,258 @@ __global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ s
     for (int k = k0; k < nh; ++k) sum += pw[k];
     noise[row] = sqrt(sum / (double)(nh - k0));
   }
+}
+
+// ----------------------------------------------------------------------------
+// Simulated archives (pp_simulate_batch): row (s, n) is
+//   Y_k = S_sn M_mnk e^{-2 pi i k theta_sn} B_snk,  out = irfft(Y) + sigma_sn z(seed, s_global, n, b)
+// with m = model_index[s], theta_sn = rot_theta (the injected phi, DM, GM: pp_fit_batch recovers them) and
+// B_snk = 1/(1 + 2 pi i k tau_sn), tau_sn = tau_s (nu_n/nu_tau_s)^alpha_s [rot].  The model spectra M are float64
+// rows computed once per call; the inverse transform is FP64.
+//
+// Noise: Philox4x32-10 (Salmon et al. 2011, the Random123 constants) with key (seed lo, seed hi) and counter
+// (q, n, s_global lo, s_global hi) gives four uint32 for bins 4q .. 4q+3 of channel n of subint s_global; each is
+// mapped to u = f32((x >> 8) 2^-24 + 2^-25) in (0, 1] (exact below 1/2, rounded to nearest even above) and pairs
+// go through Box-Muller in float32 with the accurate logf / sqrtf / sincospif:
+//   (z0, z1) = sqrt(-2 ln u0) (cos 2 pi u1, sin 2 pi u1), (z2, z3) likewise from (u2, u3);  |z| <= 5.89.
+// A subint's samples depend on (seed, its global index, its model and parameters) only, not on the batch, the
+// chunk or the device.
+// ----------------------------------------------------------------------------
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    if (i) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+  }
+  return c;
+}
+
+__device__ __forceinline__ float sim_uniform(unsigned x) {
+  return __fadd_rn((float)(x >> 8) * 5.9604644775390625e-8f, 2.98023223876953125e-8f);   // 2^-24, 2^-25
+}
+
+__device__ __forceinline__ void box_muller(unsigned a, unsigned b, float& z0, float& z1) {
+  const float r = sqrtf(-2.0f * logf(sim_uniform(a)));
+  float sn, cs;
+  sincospif(2.0f * sim_uniform(b), &sn, &cs);
+  z0 = r * cs;
+  z1 = r * sn;
+}
+
+struct SimArgs {
+  RotateArgs r;               // phase, DM, P, nu_ref (= nu_DM), GM, nu_GM of the chunk's subints; nu2 [nmodel * nchan]
+  const cx<double>* mspec;    // [nmodel * nchan, sstride] model spectra: slot k = harmonic k, 1..nbin/2; slot 0 = the DC
+                              // term (power-of-two nbin) or unused (mdc)
+  const double* mdc;          // [nmodel * nchan] DC terms (other nbin) or null
+  const double* freqs;        // [nmodel * nchan]
+  const int* index;           // [nsub] model of each subint or null (model 0)
+  const double* tau;          // [nsub] or null (unscattered); alpha, nu_tau with it
+  const double* alpha;
+  const double* nu_tau;
+  const double* scales;       // [nsub, nchan] or null (1)
+  const double* sigma;        // [nsub, nchan] or null (0)
+  float* out;                 // [nsub, nchan, nbin] float32 or null
+  int16_t* raw;               // [nsub, nchan, nbin] or null; dat_scl, dat_offs [nsub, nchan] with it
+  float* dat_scl;
+  float* dat_offs;
+  long long s_first;          // global index of subint 0 of the chunk (first_subint + chunk start)
+  unsigned key0, key1;
+  int nchan, nbin, sstride;
+};
+
+// row geometry shared by the simulate kernels: the model row, theta, the scattering and the scale of row (s, ch)
+struct SimRow {
+  const cx<double>* M;
+  double theta, wtau, S, sigma;
+  int mrow;
+};
+__device__ __forceinline__ SimRow sim_row(const SimArgs& a, int s, int ch) {
+  SimRow w;
+  const int m = a.index ? __ldg(a.index + s) : 0;
+  w.mrow = m * a.nchan + ch;
+  w.M = a.mspec + (size_t)w.mrow * a.sstride;
+  w.theta = rot_theta(a.r, s, w.mrow);
+  w.wtau = a.tau ? kTwoPi * a.tau[s] * pow(a.freqs[w.mrow] / a.nu_tau[s], a.alpha[s]) : 0.0;
+  const size_t sc = (size_t)s * a.nchan + ch;
+  w.S = a.scales ? a.scales[sc] : 1.0;
+  w.sigma = a.sigma ? a.sigma[sc] : 0.0;
+  return w;
+}
+
+// S e^{-2 pi i k theta} / (1 + 2 pi i k tau) times M_k
+__device__ __forceinline__ cx<double> sim_harmonic(const SimRow& w, int k) {
+  double c, sn;
+  cis2pi((double)k * w.theta, c, sn);
+  sn = -sn;
+  if (w.wtau != 0.0) scatter_factor(c, sn, w.wtau * (double)k);
+  return cmul(w.M[k], mk<double>(w.S * c, w.S * sn));
+}
+
+// samples 4q .. 4q+3 (the first n of them) of row (s, ch): clean values y plus sigma z, rounded to float32
+__device__ __forceinline__ void sim_noise(const SimArgs& a, const SimRow& w, int q, int ch, int s, const double (&y)[4],
+                                          float (&v)[4]) {
+  float z[4] = {0.f, 0.f, 0.f, 0.f};
+  if (w.sigma != 0.0) {
+    const unsigned long long sg = (unsigned long long)(a.s_first + s);
+    const uint4 x = philox4x32_10(make_uint4((unsigned)q, (unsigned)ch, (unsigned)sg, (unsigned)(sg >> 32)),
+                                  make_uint2(a.key0, a.key1));
+    box_muller(x.x, x.y, z[0], z[1]);
+    box_muller(x.z, x.w, z[2], z[3]);
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) v[i] = (float)fma(w.sigma, (double)z[i], y[i]);
+}
+
+// pptoas.quantize_subints of one row, given its float32 min / max: raw = clip(rint((x - offs) / scl)) in double,
+// offs = f32((hi + lo) / 2), scl = f32((hi - lo) / 65000) (1 for a constant row)
+struct SimQuant {
+  double offs, scl;
+  __device__ __forceinline__ SimQuant(float lo, float hi) {
+    offs = (double)(float)(0.5 * ((double)hi + (double)lo));
+    scl = hi > lo ? (double)(float)(((double)hi - (double)lo) / 65000.0) : 1.0;
+  }
+  __device__ __forceinline__ int16_t operator()(float x) const {
+    const double r = rint(((double)x - offs) / scl);
+    return (int16_t)fmin(fmax(r, -32768.0), 32767.0);
+  }
+};
+
+// Power-of-two nbin: one row slot per output row: the spectrum row (L2-resident) times the phasor and scattering
+// factor, packed for the inverse, one FP64 inverse transform, then noise and the store (float32 and / or int16 after
+// a row-slot min / max).  Half of k_rotate's transforms, and no input portrait.
+template <int N>
+__global__ void __launch_bounds__(256) k_simulate(SimArgs a, int nsub) {
+  using G = RowGeom<N>;
+  using T = double;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  cx<T>* twN = reinterpret_cast<cx<T>*>(smem_raw);
+  cx<T>* tw2N = twN + N;
+  cx<T>* bufs = tw2N + (N / 2 + 2);
+  __shared__ float red[2][8];
+  const int tid = threadIdx.x, r = tid / G::kTRow, t_row = tid % G::kTRow;
+  {
+    const cx<T>* g1 = reinterpret_cast<const cx<T>*>(a.r.twN);
+    const cx<T>* g2 = reinterpret_cast<const cx<T>*>(a.r.tw2N);
+    for (int i = tid; i < N; i += 256) twN[i] = g1[i];
+    for (int i = tid; i <= N / 2; i += 256) tw2N[i] = g2[i];
+  }
+  __syncthreads();   // the packing below reads tw2N[p], stored by other warps (no input load barrier here)
+  cx<T>* bufA = bufs + (size_t)r * 2 * N;
+  cx<T>* bufB = bufA + N;
+  const long nrows = (long)nsub * a.nchan;
+  const long row = (long)blockIdx.x * G::kRows + r;
+  const bool valid = row < nrows;
+  const long rowc = valid ? row : 0;
+  const int s = (int)(rowc / a.nchan), ch = (int)(rowc % a.nchan);
+  const SimRow w = sim_row(a, s, ch);
+#pragma unroll
+  for (int i = 0; i < G::kPairs; ++i) {
+    const int p = t_row + 1 + i * G::kTRow;
+    if (p <= N / 2) {
+      const cx<T> dp = sim_harmonic(w, p);
+      const cx<T> dq = p < N / 2 ? sim_harmonic(w, N - p) : dp;
+      cx<T> zp, zq;
+      pack_pair<T>(dp, dq, tw2N[p], zp, zq);
+      bufA[p] = cconj(zp);           // conj for the inverse transform
+      if (p < N / 2) bufA[N - p] = cconj(zq);
+    }
+  }
+  if (t_row == 0) {
+    const T d0 = w.S * w.M[0].x;
+    const T dN = sim_harmonic(w, N).x;   // irfft keeps the real part of the Nyquist term
+    bufA[0] = mk<T>(T(0.5) * (d0 + dN), -T(0.5) * (d0 - dN));
+  }
+  __syncthreads();
+  const cx<T>* Y = fft_forward<N, G::kTRow, T>(bufA, bufB, twN, t_row);
+  const T sc = T(1) / T(N);
+  float v[G::kLoads][4];
+  float lo = CUDART_INF_F, hi = -CUDART_INF_F;
+#pragma unroll
+  for (int m = 0; m < G::kLoads; ++m) {
+    const int q = t_row + m * G::kTRow;
+    const cx<T> y0 = Y[2 * q], y1 = Y[2 * q + 1];
+    const double y[4] = {y0.x * sc, -y0.y * sc, y1.x * sc, -y1.y * sc};
+    sim_noise(a, w, q, ch, s, y, v[m]);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { lo = fminf(lo, v[m][i]); hi = fmaxf(hi, v[m][i]); }
+    if (a.out && valid)
+      reinterpret_cast<float4*>(a.out + (size_t)row * 2 * N)[q] = make_float4(v[m][0], v[m][1], v[m][2], v[m][3]);
+  }
+  if (!a.raw) return;   // (uniform over the grid)
+#pragma unroll
+  for (int o = (G::kTRow < 32 ? G::kTRow : 32) / 2; o > 0; o >>= 1) {
+    lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+  }
+  if (G::kTRow > 32) {
+    if ((tid & 31) == 0) { red[0][tid >> 5] = lo; red[1][tid >> 5] = hi; }
+    __syncthreads();
+#pragma unroll
+    for (int ww = 0; ww < G::kTRow / 32; ++ww) {
+      lo = fminf(lo, red[0][r * (G::kTRow / 32) + ww]);
+      hi = fmaxf(hi, red[1][r * (G::kTRow / 32) + ww]);
+    }
+  }
+  if (!valid) return;
+  const SimQuant qz(lo, hi);
+#pragma unroll
+  for (int m = 0; m < G::kLoads; ++m) {
+    const int q = t_row + m * G::kTRow;
+    short4 o4;
+    o4.x = qz(v[m][0]); o4.y = qz(v[m][1]); o4.z = qz(v[m][2]); o4.w = qz(v[m][3]);
+    reinterpret_cast<short4*>(a.raw + (size_t)row * 2 * N)[q] = o4;
+  }
+  if (t_row == 0) { a.dat_scl[row] = (float)qz.scl; a.dat_offs[row] = (float)qz.offs; }
+}
+
+// Other even nbin, step 1: the spectrum rows Y of a chunk into the any-nbin scratch (slot k = harmonic k, 1..L;
+// dc = harmonic 0), for k_inv_any.  One CTA per row.
+__global__ void __launch_bounds__(256) k_sim_mul(SimArgs a, cx<double>* spec, double* dc, int Npad, int L) {
+  const long row = blockIdx.x;
+  const int s = (int)(row / a.nchan), ch = (int)(row % a.nchan);
+  const SimRow w = sim_row(a, s, ch);
+  for (int k = threadIdx.x + 1; k <= L; k += 256) {
+    const cx<double> d = sim_harmonic(w, k);
+    spec[(size_t)row * Npad + k] = (k < L) ? d : mk<double>(d.x, 0.0);   // irfft keeps the real part of the Nyquist term
+  }
+  if (threadIdx.x == 0) dc[row] = w.S * a.mdc[w.mrow];
+}
+
+// Other even nbin, step 2: the noise and store epilogue of k_simulate on the float64 rows of k_inv_any.  One CTA per
+// row; the row's float32 values wait in shared memory for the int16 pass.
+__global__ void __launch_bounds__(256) k_sim_store(SimArgs a, const double* __restrict__ y) {
+  __shared__ float vrow[4096];
+  __shared__ float red[2][8];
+  const long row = blockIdx.x;
+  const int s = (int)(row / a.nchan), ch = (int)(row % a.nchan), tid = threadIdx.x, nbin = a.nbin;
+  const SimRow w = sim_row(a, s, ch);
+  const double* yr = y + (size_t)row * nbin;
+  float lo = CUDART_INF_F, hi = -CUDART_INF_F;
+  for (int q = tid; 4 * q < nbin; q += 256) {
+    const int n = min(4, nbin - 4 * q);   // the last quad is partial when 4 does not divide nbin
+    double yq[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int i = 0; i < n; ++i) yq[i] = yr[4 * q + i];
+    float v[4];
+    sim_noise(a, w, q, ch, s, yq, v);
+    for (int i = 0; i < n; ++i) {
+      vrow[4 * q + i] = v[i];
+      lo = fminf(lo, v[i]); hi = fmaxf(hi, v[i]);
+      if (a.out) a.out[(size_t)row * nbin + 4 * q + i] = v[i];
+    }
+  }
+  if (!a.raw) return;
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+  }
+  if ((tid & 31) == 0) { red[0][tid >> 5] = lo; red[1][tid >> 5] = hi; }
+  __syncthreads();
+  for (int ww = 0; ww < 8; ++ww) { lo = fminf(lo, red[0][ww]); hi = fmaxf(hi, red[1][ww]); }
+  const SimQuant qz(lo, hi);
+  for (int j = tid; j < nbin; j += 256) a.raw[(size_t)row * nbin + j] = qz(vrow[j]);
+  if (tid == 0) { a.dat_scl[row] = (float)qz.scl; a.dat_offs[row] = (float)qz.offs; }
 }
 
 }  // namespace ppb

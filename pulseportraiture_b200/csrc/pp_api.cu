@@ -126,6 +126,9 @@ struct pp_plan {
   DBuf X, Xlo, partial, data_stage[2], data_stage64[2], Dspec, Ddc, al_acc, al_wparts, al_dc;
   // evolving-Gaussian portrait fit (pp_fit_gaussian_portraits): per-chunk state and outputs, per-CTA slabs
   DBuf gf_data, gf_errs, gf_rec, gf_slab, gf_state, gf_out, gf_model, gf_par;
+  // simulated archives (pp_simulate_batch): the call's models, spectra and tables, staged inputs, chunk scratch
+  DBuf sim_models, sim_freqs, sim_nu2, sim_mspec, sim_mdc, sim_index, sim_par[9], sim_scales, sim_sigma, sim_spec, sim_dc,
+      sim_rows, sim_out, sim_raw, sim_scl, sim_offs;
   // timing
   bool timing = false;
   std::vector<cudaEvent_t> ev_chunk;   // "chunk finished" events for the overlapped result copies
@@ -319,6 +322,7 @@ template <int N> static cudaError_t setup_attrs() {
   SET_((k_align_finish<N>), b64)
   SET_((k_rotate<N, float>), b32)
   SET_((k_rotate<N, double>), b64)
+  SET_((k_simulate<N>), b64)
 #undef SET_
   return cudaFuncSetAttribute(k_guess, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double2) * 2048));
 }
@@ -518,9 +522,9 @@ static AnyPlan any_dev(pp_plan* pl) {
   return p;
 }
 static int launch_fwd_any(pp_plan* pl, const void* in, bool i16, const float* scl, const float* offs, long nrows,
-                          cx<double>* spec, double* dc) {
+                          cx<double>* spec, double* dc, const double* in64 = nullptr) {
   FwdAnyArgs a;
-  a.in = in; a.dat_scl = scl; a.dat_offs = offs; a.spec = spec; a.dc = dc; a.p = any_dev(pl); a.nrows = nrows;
+  a.in = in; a.in64 = in64; a.dat_scl = scl; a.dat_offs = offs; a.spec = spec; a.dc = dc; a.p = any_dev(pl); a.nrows = nrows;
   const unsigned grid = (unsigned)std::min<long>(nrows, 148L * 64);
   // (the direct mixed-radix transform works on 2 L points, the Bluestein convolution on 2 M)
   const size_t sm = 2 * sizeof(cx<double>) * (pl->any_rad.empty() ? (size_t)pl->M : (size_t)pl->L);
@@ -705,7 +709,7 @@ static int set_model_impl(pp_plan* pl, int nmodel, const float* model, const dou
   ModelArgs a;
   a.model = dmodel; a.model64 = dmodel64; a.mconj32 = pl->mconj32.as<cx<float>>(); a.mconj64 = pl->mconj64.as<cx<double>>();
   a.mpow = pl->mpow.as<double>(); a.pn = pl->pn.as<double>();
-  a.twN = pl->twN64.as<cx<double>>(); a.tw2N = pl->tw2N64.as<cx<double>>(); a.nchan = nchan;
+  a.twN = pl->twN64.as<cx<double>>(); a.tw2N = pl->tw2N64.as<cx<double>>(); a.spec = nullptr; a.nchan = nchan;
   if (pl->anyn) {
     CK(pl->any_spec2.need(sizeof(double2) * (size_t)nchan * N));
     if (launch_fwd_any(pl, dmodel, false, nullptr, nullptr, nchan, pl->any_spec2.as<cx<double>>(), nullptr)) return -2;
@@ -2153,5 +2157,213 @@ extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* ar
     CK(cudaStreamSynchronize(pl->stream));
   }
   CK(cudaGetLastError());
+  return 0;
+}
+
+// ----------------------------------------------------------------------------
+// simulated archives (kernels.cuh k_simulate / k_sim_mul / k_sim_store)
+// ----------------------------------------------------------------------------
+// a page-locked piece of the plan's ring for a device -> host copy (the copy that last used it has finished)
+static int pin_piece(pp_plan* pl, void** buf) {
+  const int slot = (int)(pl->pin_count++ % pp_plan::kPinSlots);
+  if (!pl->pin_ring[slot]) {
+    CK(cudaHostAlloc(&pl->pin_ring[slot], pp_plan::kPinPiece, cudaHostAllocDefault));
+    CK(cudaEventCreateWithFlags(&pl->pin_ev[slot], cudaEventDisableTiming));
+  } else {
+    CK(cudaEventSynchronize(pl->pin_ev[slot]));
+  }
+  *buf = pl->pin_ring[slot];
+  return 0;
+}
+
+// index of the first of n values (host or device) for which bad(v) holds, or n; device values are read back
+// in pieces through the page-locked ring
+template <typename T, typename Bad> static int find_bad(pp_plan* pl, const T* p, size_t n, Bad bad, size_t* at) {
+  *at = n;
+  if (!is_device_ptr(p)) {
+    for (size_t i = 0; i < n; ++i) if (bad(p[i])) { *at = i; return 0; }
+    return 0;
+  }
+  const size_t per = pp_plan::kPinPiece / sizeof(T);
+  for (size_t off = 0; off < n; off += per) {
+    const size_t len = std::min(per, n - off);
+    void* buf;
+    if (pin_piece(pl, &buf)) return -2;
+    CK(cudaMemcpyAsync(buf, p + off, len * sizeof(T), cudaMemcpyDeviceToHost, pl->stream));
+    CK(cudaStreamSynchronize(pl->stream));
+    const T* h = static_cast<const T*>(buf);
+    for (size_t i = 0; i < len; ++i) if (bad(h[i])) { *at = off + i; return 0; }
+  }
+  return 0;
+}
+
+// device -> caller's host memory through the plan's page-locked ring (page-locked destinations directly)
+static int d2h_staged(pp_plan* pl, void* dst, const void* src, size_t bytes) {
+  if (mem_kind(dst) == kMemPinned) {
+    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, pl->stream));
+    return 0;
+  }
+  static const int nthreads = std::max(1, std::min(8, (int)std::thread::hardware_concurrency() / 2));
+  for (size_t off = 0; off < bytes; off += pp_plan::kPinPiece) {
+    const size_t len = std::min(pp_plan::kPinPiece, bytes - off);
+    void* buf;
+    if (pin_piece(pl, &buf)) return -2;
+    CK(cudaMemcpyAsync(buf, (const char*)src + off, len, cudaMemcpyDeviceToHost, pl->stream));
+    CK(cudaStreamSynchronize(pl->stream));
+    parallel_memcpy((char*)dst + off, buf, len, nthreads);
+  }
+  return 0;
+}
+
+// elements [off, off + n) of an input for one chunk: a device array in place, a host one copied into buf
+template <typename T> static int chunk_in(pp_plan* pl, DBuf& buf, const T* src, bool dev, size_t off, size_t n, const T** out) {
+  if (!src) { *out = nullptr; return 0; }
+  if (dev) { *out = src + off; return 0; }
+  CK(buf.need(sizeof(T) * n));
+  CK(cudaMemcpyAsync(buf.p, src + off, sizeof(T) * n, cudaMemcpyHostToDevice, pl->stream));
+  *out = buf.as<T>();
+  return 0;
+}
+
+static const size_t kSimChunkBytes = 256u << 20;   // device scratch of one chunk of a simulate call
+
+extern "C" int pp_simulate_batch(pp_plan_t* pl, const pp_sim_args_t* args, const pp_sim_out_t* out) {
+  if (!pl || !args || !out) return fail(-1, "NULL argument");
+  const pp_sim_args_t& A = *args;
+  if (A.nsub < 0) return fail(-1, "nsub must be >= 0 (got %d)", A.nsub);
+  if (A.nsub == 0) return 0;
+  if (A.nmodel < 1) return fail(-1, "nmodel must be >= 1 (got %d)", A.nmodel);
+  if (!A.models || !A.freqs || !A.phase || !A.DM || !A.P || !A.nu_DM) return fail(-1, "NULL input array");
+  if ((A.GM == nullptr) != (A.nu_GM == nullptr)) return fail(-1, "GM and nu_GM must be given together");
+  if (!((A.tau && A.alpha && A.nu_tau) || (!A.tau && !A.alpha && !A.nu_tau)))
+    return fail(-1, "tau, alpha and nu_tau must be given together");
+  if (!out->data && !out->raw) return fail(-1, "no output: data or raw must be given");
+  if (out->raw && (!out->dat_scl || !out->dat_offs)) return fail(-1, "raw output needs dat_scl and dat_offs");
+  CK(cudaSetDevice(pl->device));
+  const int nsub = A.nsub, nchan = pl->nchan, nbin = pl->nbin, nmodel = A.nmodel;
+  const size_t nsc = (size_t)nsub * nchan, nfreq = (size_t)nmodel * nchan;
+  // ---- validation (device inputs are read back in pieces): nothing runs before it passes
+  std::vector<double> hf(nfreq), hn2(nfreq);
+  if (is_device_ptr(A.freqs)) CK(cudaMemcpy(hf.data(), A.freqs, sizeof(double) * nfreq, cudaMemcpyDeviceToHost));
+  else memcpy(hf.data(), A.freqs, sizeof(double) * nfreq);
+  for (size_t i = 0; i < nfreq; ++i) {
+    if (!(hf[i] > 0.0)) return fail(-1, "freqs[%d, %d] = %g is not positive", (int)(i / nchan), (int)(i % nchan), hf[i]);
+    hn2[i] = 1.0 / (hf[i] * hf[i]);
+  }
+  size_t at;
+  if (A.model_index) {
+    if (find_bad(pl, A.model_index, (size_t)nsub, [nmodel](int32_t v) { return v < 0 || v >= nmodel; }, &at)) return -2;
+    if (at < (size_t)nsub) return fail(-1, "model_index[%d] is out of range [0, %d)", (int)at, nmodel);
+  }
+  struct PosCheck { const double* p; const char* name; };
+  for (const PosCheck& c : {PosCheck{A.P, "P"}, PosCheck{A.nu_DM, "nu_DM"}, PosCheck{A.nu_GM, "nu_GM"}, PosCheck{A.nu_tau, "nu_tau"}}) {
+    if (!c.p) continue;
+    if (find_bad(pl, c.p, (size_t)nsub, [](double v) { return !(v > 0.0); }, &at)) return -2;
+    if (at < (size_t)nsub) return fail(-1, "%s[%d] is not positive", c.name, (int)at);
+  }
+  if (A.noise_std) {
+    if (find_bad(pl, A.noise_std, nsc, [](double v) { return !(v >= 0.0); }, &at)) return -2;
+    if (at < nsc) return fail(-1, "noise_std[%d, %d] is negative", (int)(at / nchan), (int)(at % nchan));
+  }
+  stats_begin(pl);
+  // ---- the call's model spectra and frequency tables (own buffers: the fit's model set stays as it is)
+  const int N = pl->N, L = nbin / 2;
+  const int sstride = pl->anyn ? N : N + 1;
+  const double* dmodels;
+  if (stage_in(pl, pl->sim_models, A.models, nfreq * nbin, &dmodels)) return -2;
+  CK(pl->sim_freqs.need(sizeof(double) * nfreq));
+  CK(pl->sim_nu2.need(sizeof(double) * nfreq));
+  CK(cudaMemcpyAsync(pl->sim_freqs.p, hf.data(), sizeof(double) * nfreq, cudaMemcpyHostToDevice, pl->stream));
+  CK(cudaMemcpyAsync(pl->sim_nu2.p, hn2.data(), sizeof(double) * nfreq, cudaMemcpyHostToDevice, pl->stream));
+  CK(pl->sim_mspec.need(sizeof(double2) * nfreq * sstride));
+  if (pl->anyn) {
+    CK(pl->sim_mdc.need(sizeof(double) * nfreq));
+    if (launch_fwd_any(pl, nullptr, false, nullptr, nullptr, (long)nfreq, pl->sim_mspec.as<cx<double>>(),
+                       pl->sim_mdc.as<double>(), dmodels)) return -2;
+  } else {
+    ModelArgs m;
+    memset(&m, 0, sizeof m);
+    m.model64 = dmodels; m.spec = pl->sim_mspec.as<cx<double>>(); m.nchan = (int)nfreq;
+    m.twN = pl->twN64.as<cx<double>>(); m.tw2N = pl->tw2N64.as<cx<double>>();
+    DISPATCH_N(N, (k_model<NN><<<row_ctas<NN>((long)nfreq), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(m)));
+    pl->stats.launches++;
+  }
+  CK(cudaGetLastError());
+  // ---- per-subint inputs and outputs: device arrays are used in place, host ones go through chunk-sized buffers,
+  // so that the device scratch does not grow with nsub; each pointer is taken for what it is
+  const double* src[9] = {A.phase, A.DM, A.P, A.nu_DM, A.GM, A.nu_GM, A.tau, A.alpha, A.nu_tau};
+  bool src_dev[9];
+  for (int i = 0; i < 9; ++i) src_dev[i] = src[i] && is_device_ptr(src[i]);
+  const bool idx_dev = A.model_index && is_device_ptr(A.model_index);
+  const bool scales_dev = A.scales && is_device_ptr(A.scales), sigma_dev = A.noise_std && is_device_ptr(A.noise_std);
+  const bool data_dev = out->data && is_device_ptr(out->data), raw_dev = out->raw && is_device_ptr(out->raw);
+  const bool scl_dev = out->raw && is_device_ptr(out->dat_scl), offs_dev = out->raw && is_device_ptr(out->dat_offs);
+  size_t per_sub = sizeof(double) * 9 + sizeof(int);   // scratch bytes per subint (upper bound)
+  if (A.scales && !scales_dev) per_sub += (size_t)nchan * sizeof(double);
+  if (A.noise_std && !sigma_dev) per_sub += (size_t)nchan * sizeof(double);
+  if (out->data && !data_dev) per_sub += (size_t)nchan * nbin * sizeof(float);
+  if (out->raw && !raw_dev) per_sub += (size_t)nchan * nbin * sizeof(int16_t);
+  if (out->raw && !scl_dev) per_sub += (size_t)nchan * sizeof(float);
+  if (out->raw && !offs_dev) per_sub += (size_t)nchan * sizeof(float);
+  if (pl->anyn) per_sub += (size_t)nchan * (sizeof(double2) * N + sizeof(double) + sizeof(double) * nbin);
+  int chunk = pl->chunk_req > 0 ? std::min(pl->chunk_req, nsub)
+                                : (int)std::max<size_t>(1, std::min<size_t>((size_t)nsub, kSimChunkBytes / per_sub));
+  // (one CTA per row for the other-nbin kernels: gridDim.x <= 2^31 - 1 rows)
+  chunk = (int)std::min<long>(chunk, std::max(1L, 2000000000L / nchan));
+  if (out->data && !data_dev) CK(pl->sim_out.need((size_t)chunk * nchan * nbin * sizeof(float)));
+  if (out->raw && !raw_dev) CK(pl->sim_raw.need((size_t)chunk * nchan * nbin * sizeof(int16_t)));
+  if (out->raw && !scl_dev) CK(pl->sim_scl.need((size_t)chunk * nchan * sizeof(float)));
+  if (out->raw && !offs_dev) CK(pl->sim_offs.need((size_t)chunk * nchan * sizeof(float)));
+  if (pl->anyn) {
+    CK(pl->sim_spec.need(sizeof(double2) * (size_t)chunk * nchan * N));
+    CK(pl->sim_dc.need(sizeof(double) * (size_t)chunk * nchan));
+    CK(pl->sim_rows.need(sizeof(double) * (size_t)chunk * nchan * nbin));
+  }
+  SimArgs a;
+  memset(&a, 0, sizeof a);
+  a.r.nu2 = pl->sim_nu2.as<double>(); a.r.nchan = nchan;
+  a.r.twN = pl->twN64.p; a.r.tw2N = pl->tw2N64.p;
+  a.mspec = pl->sim_mspec.as<cx<double>>(); a.mdc = pl->anyn ? pl->sim_mdc.as<double>() : nullptr;
+  a.freqs = pl->sim_freqs.as<double>();
+  a.key0 = (unsigned)A.seed; a.key1 = (unsigned)(A.seed >> 32);
+  a.nchan = nchan; a.nbin = nbin; a.sstride = sstride;
+  {
+    SpanGuard sg(pl, SP_TOTAL);
+    for (int s0 = 0; s0 < nsub; s0 += chunk) {
+      const int ns = std::min(chunk, nsub - s0);
+      const size_t r0 = (size_t)s0 * nchan, rows = (size_t)ns * nchan;
+      const double* par[9];
+      for (int i = 0; i < 9; ++i)
+        if (chunk_in(pl, pl->sim_par[i], src[i], src_dev[i], (size_t)s0, (size_t)ns, &par[i])) return -2;
+      a.r.phase = par[0]; a.r.DM = par[1]; a.r.P = par[2]; a.r.nu_ref = par[3]; a.r.GM = par[4]; a.r.nu_GM = par[5];
+      a.tau = par[6]; a.alpha = par[7]; a.nu_tau = par[8];
+      const int32_t* idx;
+      if (chunk_in(pl, pl->sim_index, A.model_index, idx_dev, (size_t)s0, (size_t)ns, &idx)) return -2;
+      a.index = idx;
+      if (chunk_in(pl, pl->sim_scales, A.scales, scales_dev, r0, rows, &a.scales)) return -2;
+      if (chunk_in(pl, pl->sim_sigma, A.noise_std, sigma_dev, r0, rows, &a.sigma)) return -2;
+      a.s_first = (long long)A.first_subint + s0;
+      a.out = !out->data ? nullptr : data_dev ? out->data + r0 * nbin : pl->sim_out.as<float>();
+      a.raw = !out->raw ? nullptr : raw_dev ? out->raw + r0 * nbin : pl->sim_raw.as<int16_t>();
+      a.dat_scl = !out->raw ? nullptr : scl_dev ? out->dat_scl + r0 : pl->sim_scl.as<float>();
+      a.dat_offs = !out->raw ? nullptr : offs_dev ? out->dat_offs + r0 : pl->sim_offs.as<float>();
+      if (pl->anyn) {
+        k_sim_mul<<<(unsigned)rows, 256, 0, pl->stream>>>(a, pl->sim_spec.as<cx<double>>(), pl->sim_dc.as<double>(), N, L);
+        if (launch_inv_any(pl, pl->sim_spec.as<cx<double>>(), pl->sim_dc.as<double>(), pl->sim_rows.p, (long)rows, true)) return -2;
+        k_sim_store<<<(unsigned)rows, 256, 0, pl->stream>>>(a, pl->sim_rows.as<double>());
+        pl->stats.launches += 2;
+      } else {
+        DISPATCH_N(N, (k_simulate<NN><<<row_ctas<NN>((long)rows), 256, fft_smem_bytes<NN, double>(), pl->stream>>>(a, ns)));
+        pl->stats.launches++;
+      }
+      CK(cudaGetLastError());
+      if (out->data && !data_dev && d2h_staged(pl, out->data + r0 * nbin, a.out, rows * nbin * sizeof(float))) return -2;
+      if (out->raw && !raw_dev && d2h_staged(pl, out->raw + r0 * nbin, a.raw, rows * nbin * sizeof(int16_t))) return -2;
+      if (out->raw && !scl_dev && d2h_staged(pl, out->dat_scl + r0, a.dat_scl, rows * sizeof(float))) return -2;
+      if (out->raw && !offs_dev && d2h_staged(pl, out->dat_offs + r0, a.dat_offs, rows * sizeof(float))) return -2;
+    }
+  }
+  CK(cudaStreamSynchronize(pl->stream));
+  stats_end(pl);
   return 0;
 }

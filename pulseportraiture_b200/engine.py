@@ -536,6 +536,100 @@ class WidebandPlan(object):
             _ptr(bc(nu_GM), np.float64, keep, "nu_GM")), "pp_rotate_full_batch")
         return out
 
+    # ---- simulated archives -------------------------------------------------------------
+    def simulate_batch(self, models, freqs, phase, DM, P, nu_DM=np.inf, GM=None, nu_GM=None, tau=None,
+                       alpha=None, nu_tau=None, scales=None, noise_stds=None, seed=0, first_subint=0,
+                       model_index=None, quantize=False, out=None, device_out=False):
+        """Simulated subints (pp_simulate_batch): row (s, n) is the model portrait model_index[s] rotated by the
+        injected phase, DM (about nu_DM) and GM (about nu_GM, default inf), scattered by tau [rot at nu_tau] with
+        index alpha (default -4), times scales, plus noise_stds * N(0, 1) from the counter-based generator keyed by
+        ``seed`` (subint s draws as global subint first_subint + s, whatever the batch).  fit_batch recovers the
+        injected parameters.
+
+        models: float64 [nchan, nbin] or [nmodel, nchan, nbin] with freqs [nchan] or [nmodel, nchan] (numpy or
+        torch, host or CUDA).  phase, DM, P, nu_DM, GM, nu_GM, tau, alpha, nu_tau: scalars or [nsub]; scales,
+        noise_stds: scalars, [nchan] or [nsub, nchan] (None: 1 and 0).  nsub is the longest of these (1 when all
+        are scalars), or out's.
+
+        Returns float32 [nsub, nchan, nbin], or with ``quantize`` (raw int16 [nsub, nchan, nbin], dat_scl,
+        dat_offs float32 [nsub, nchan]) = pptoas.quantize_subints of the float32 rows: numpy arrays, or torch
+        CUDA tensors with ``device_out`` (which fit_batch takes as they are).  ``out`` (an array, or the
+        (raw, dat_scl, dat_offs) tuple) receives the result instead."""
+        nchan, nbin = self.nchan, self.nbin
+        keep = []
+        mshape = tuple(models.shape)
+        nmodel = 1 if len(mshape) == 2 else int(mshape[0])
+        if mshape[-2:] != (nchan, nbin) or len(mshape) not in (2, 3):
+            raise ValueError("models must be [nchan, nbin] or [nmodel, nchan, nbin] with (nchan, nbin) = (%d, %d)"
+                             % (nchan, nbin))
+        if GM is not None and nu_GM is None:
+            nu_GM = np.inf
+        if tau is not None:
+            if nu_tau is None:
+                raise ValueError("tau needs nu_tau, the frequency it refers to")
+            if alpha is None:
+                alpha = -4.0
+        elif alpha is not None or nu_tau is not None:
+            raise ValueError("alpha and nu_tau describe tau: give tau too")
+        per_sub = dict(phase=phase, DM=DM, P=P, nu_DM=nu_DM, GM=GM, nu_GM=nu_GM, tau=tau, alpha=alpha, nu_tau=nu_tau)
+        lens = [int(np.shape(v)[0]) for v in list(per_sub.values()) + [model_index] if v is not None and np.ndim(v) >= 1]
+        lens += [int(np.shape(v)[0]) for v in (scales, noise_stds) if v is not None and np.ndim(v) == 2]
+        if out is not None:
+            lens.append(int(np.shape(out[0] if quantize else out)[0]))
+        nsub = max(lens) if lens else 1
+
+        def sub(v, name):
+            if v is None:
+                return None
+            if _is_torch(v):
+                return _ptr(v, np.float64, keep, name, (nsub,))
+            return _ptr(np.broadcast_to(np.asarray(v, dtype=np.float64), (nsub,)), np.float64, keep, name)
+
+        def chan(v, name):
+            if v is None:
+                return None
+            if _is_torch(v):
+                return _ptr(v, np.float64, keep, name, (nsub, nchan))
+            return _ptr(np.broadcast_to(np.asarray(v, dtype=np.float64), (nsub, nchan)), np.float64, keep, name)
+
+        a = _ffi.SimArgs()
+        a.models = _ptr(models, np.float64, keep, "models", (nmodel, nchan, nbin))
+        a.freqs = _ptr(freqs if _is_torch(freqs) else np.asarray(freqs, dtype=np.float64), np.float64, keep,
+                       "freqs", (nmodel, nchan))
+        a.nmodel = nmodel
+        a.model_index = _ptr(model_index, np.int32, keep, "model_index", (nsub,))
+        a.nsub = nsub
+        a.first_subint = int(first_subint)
+        a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        for k, v in per_sub.items():
+            setattr(a, k, sub(v, k))
+        a.scales = chan(scales, "scales")
+        a.noise_std = chan(noise_stds, "noise_stds")
+        if out is None:
+            shapes = [((nsub, nchan, nbin), np.int16), ((nsub, nchan), np.float32), ((nsub, nchan), np.float32)] \
+                if quantize else [((nsub, nchan, nbin), np.float32)]
+            if device_out:
+                import torch
+                tdt = {np.int16: torch.int16, np.float32: torch.float32}
+                res = [torch.empty(sh, dtype=tdt[dt], device=torch.device("cuda", self.device)) for sh, dt in shapes]
+            else:
+                res = [np.empty(sh, dtype=dt) for sh, dt in shapes]
+        else:
+            res = list(out) if quantize else [out]
+        o = _ffi.SimOut()
+        if quantize:
+            o.raw = _ptr(res[0], np.int16, keep, "raw", (nsub, nchan, nbin))
+            o.dat_scl = _ptr(res[1], np.float32, keep, "dat_scl", (nsub, nchan))
+            o.dat_offs = _ptr(res[2], np.float32, keep, "dat_offs", (nsub, nchan))
+        else:
+            o.data = _ptr(res[0], np.float32, keep, "out", (nsub, nchan, nbin))
+        for r in res:
+            if isinstance(r, np.ndarray) and not (r.flags.c_contiguous and r.flags.writeable):
+                raise ValueError("outputs must be writeable C-contiguous arrays")
+        _ffi.check(self._lib.pp_simulate_batch(self._h, C.byref(a), C.byref(o)), "pp_simulate_batch")
+        del keep
+        return tuple(res) if quantize else res[0]
+
     def get_noise_batch(self, data, kc=-1):
         """Per-row noise level from the harmonics k >= kc (default int(0.75 nharm), pplib.py:2244)."""
         keep = []

@@ -695,6 +695,153 @@ def write_model(filenm, name, model_code, nu_ref, model_params, fit_flags, alpha
         print("%s written." % filenm)
 
 
+# ---- simulated archives (pplib.py:3183-3378) --------------------------------------------------
+def read_ephemeris(ephemeris):
+    """(F0 [Hz], F1 [Hz/s], PEPOCH [MJD], DM, source) from a .par file (F0, optional F1 and PEPOCH, DM, PSRJ / PSR)
+    or a spin period in seconds (F1 = 0, DM = 0)."""
+    if np.ndim(ephemeris) == 0 and not isinstance(ephemeris, str):
+        P = float(ephemeris)
+        if not P > 0.0:
+            raise ValueError("the period must be positive (got %g)" % P)
+        return 1.0 / P, 0.0, 0.0, 0.0, "fake"
+    vals, source = {}, "fake"
+    with open(ephemeris, "r") as fh:
+        for line in fh:
+            info = line.split()
+            if len(info) < 2:
+                continue
+            key = info[0].upper()
+            if key in ("PSRJ", "PSR", "PSRB"):
+                source = info[1]
+            elif key in ("F0", "F1", "PEPOCH", "DM"):
+                vals[key] = float(info[1].replace("D", "E").replace("d", "e"))
+    if not vals.get("F0", 0.0) > 0.0:
+        raise ValueError("%s: no positive F0" % ephemeris)
+    return vals["F0"], vals.get("F1", 0.0), vals.get("PEPOCH", 0.0), vals.get("DM", 0.0), source
+
+
+def _per_subint(v, nsub, name):
+    a = np.asarray(v, dtype=np.float64)
+    if a.ndim > 1 or (a.ndim == 1 and len(a) != nsub):
+        raise ValueError("%s must be a scalar or [nsub = %d]" % (name, nsub))
+    return np.broadcast_to(a, (nsub,)).copy()
+
+
+def _per_chan(v, nsub, nchan, name):
+    a = np.asarray(v, dtype=np.float64)
+    if a.shape not in ((), (nchan,), (nsub, nchan)):
+        raise ValueError("%s must be a scalar, [nchan = %d] or [nsub, nchan] = [%d, %d]" % (name, nchan, nsub, nchan))
+    return np.broadcast_to(a, (nsub, nchan)).copy()
+
+
+def make_fake_pulsar(modelfile, ephemeris, outfile=None, nsub=1, npol=1, nchan=512, nbin=2048, nu0=1500.0, bw=800.0,
+                     tsub=300.0, phase=0.0, dDM=0.0, start_MJD=None, weights=None, noise_stds=1.0, scales=1.0,
+                     dedispersed=False, t_scat=0.0, alpha=scattering_alpha, scint=False, nu_DM=np.inf,
+                     state="Intensity", obs="GBT", seed=0, quantize=False, quiet=False):
+    """A simulated archive (pplib.py:3183-3378), made on the device (WidebandPlan.simulate_batch) and returned as
+    the DataBunch that load_data gives, written with pptoas.save_databunch when ``outfile`` is given (so that
+    load_data, GetTOAs, align_archives and tscrunch_databunch take it).  PSRFITS writing is not provided.
+
+    modelfile: a .gmodel file (a TAU != 0 gives one model per distinct period), a spline model, or a [nchan, nbin]
+    array.  ephemeris: a .par file (F0, optional F1 and PEPOCH, DM) or a period [s]; subint s is folded with
+    P_s = 1/(F0 + F1 (t_s - PEPOCH)) at its mid-epoch t_s = start_MJD + (s + 1/2) tsub (start_MJD default 56000).
+    Channels: nchan centre frequencies across bw about nu0 [MHz].  phase [rot], dDM, t_scat [s at nu0] and alpha:
+    scalars or [nsub]; noise_stds and scales: scalars, [nchan] or [nsub, nchan].  The subints are dispersed by
+    DM_par + dDM about nu_DM, scattered by t_scat, scaled and given Gaussian noise of rms noise_stds drawn from
+    ``seed`` (subint s always draws the same numbers).  dedispersed=True stores them with DM_par removed about nu0
+    (dmc = 1) by a second device rotation of the simulated rows, which pptoas.restore_dispersion undoes in every
+    harmonic but the Nyquist one (a rotation keeps only the real part of that term).  quantize=True also stores them as the int16 samples with
+    DAT_SCL / DAT_OFFS a PSRFITS file holds (raw_subints, dat_scl, dat_offs) and ``subints`` holds the decoded
+    values.  A scintillation pattern can be given as [nsub, nchan] ``scales`` (scint=True, the reference's own
+    pattern, is not provided); npol > 1 is not provided.
+
+    noise_stds in the result are measured from the profiles on the device (get_noise, as load_data does).  SNRs
+    are the injected matched-filter S/N per channel, scale ||m_n - mean(m_n)|| / sigma_n; the reference measures
+    them from the profiles."""
+    from .pptoas import MJD, quantize_subints, save_databunch
+    if npol != 1:
+        raise ValueError("npol = %d: only total intensity (npol = 1) is simulated" % npol)
+    if scint:
+        raise NotImplementedError("scint: pass a scintillation pattern as [nsub, nchan] scales")
+    nsub, nchan, nbin = int(nsub), int(nchan), int(nbin)
+    if nsub < 1:
+        raise ValueError("nsub must be >= 1")
+    F0, F1, PEPOCH, DM_par, source = read_ephemeris(ephemeris)
+    freqs = np.linspace(nu0 - bw / 2.0 + bw / (2.0 * nchan), nu0 + bw / 2.0 - bw / (2.0 * nchan), nchan)
+    phases = get_bin_centers(nbin)
+    start = MJD(56000, 0.0) if start_MJD is None else (start_MJD if isinstance(start_MJD, MJD) else MJD(start_MJD))
+    epochs = [start + (s + 0.5) * tsub / 86400.0 for s in range(nsub)]
+    dt = np.array([((e.intday() - PEPOCH) + e.fracday()) * 86400.0 for e in epochs]) if F1 else np.zeros(nsub)
+    Ps = 1.0 / (F0 + F1 * dt)
+    if not np.all(Ps > 0.0):
+        raise ValueError("the ephemeris gives a non-positive period")
+    phase = _per_subint(phase, nsub, "phase")
+    DMs = DM_par + _per_subint(dDM, nsub, "dDM")
+    t_scat = _per_subint(t_scat, nsub, "t_scat")
+    alpha = _per_subint(alpha, nsub, "alpha")
+    noise = _per_chan(noise_stds, nsub, nchan, "noise_stds")
+    scl = _per_chan(scales, nsub, nchan, "scales")
+    w = np.ones((nsub, nchan)) if weights is None else _per_chan(weights, nsub, nchan, "weights")
+    if np.any(noise < 0):
+        raise ValueError("noise_stds must be >= 0")
+    # model portraits: one per distinct period when the .gmodel's TAU makes the model depend on it
+    if isinstance(modelfile, np.ndarray) or hasattr(modelfile, "shape"):
+        models, model_index = np.asarray(modelfile, dtype=np.float64)[None], None
+        if models.shape[1:] != (nchan, nbin):
+            raise ValueError("the model array must be [nchan, nbin] = [%d, %d]" % (nchan, nbin))
+    elif is_spline_model(modelfile):
+        m = read_spline_model(modelfile, freqs, nbin, quiet=True, device=True)[1]
+        models, model_index = np.asarray(m, dtype=np.float64)[None], None
+    else:
+        if read_model(modelfile, quiet=True)[4][1] != 0.0:
+            uP, model_index = np.unique(Ps, return_inverse=True)
+            models = np.stack([read_model(modelfile, phases, freqs, p, quiet=True, device=True)[2] for p in uP])
+            model_index = np.asarray(model_index, dtype=np.int32).reshape(-1)
+        else:
+            models, model_index = read_model(modelfile, phases, freqs, Ps[0], quiet=True, device=True)[2][None], None
+        models = np.ascontiguousarray(models, dtype=np.float64)
+    scat = t_scat != 0.0
+    pl = get_plan(nchan, nbin)
+    data = pl.simulate_batch(models, np.tile(freqs, (len(models), 1)), phase, DMs, Ps, nu_DM=nu_DM,
+                             tau=t_scat / Ps if scat.any() else None, alpha=alpha if scat.any() else None,
+                             nu_tau=nu0 if scat.any() else None, scales=scl, noise_stds=noise, seed=seed,
+                             model_index=model_index, device_out=dedispersed)
+    if dedispersed:
+        # The stored archive, as arch.dedisperse() writes it: the simulated rows rotated by DM_par about nu0, in place
+        # on the device.  This is a second pass over the rows rather than DM_par folded into the simulation's phase
+        # and DM: folded in, the noise would be drawn in the dedispersed frame, and restore_dispersion could not give
+        # back the dedispersed=False archive.  A plan of its own, so that the cached plan's frequency table and FFT
+        # precision stay as the caller left them.
+        with WidebandPlan(nchan, nbin, device=pl.device) as rp:
+            rp.set_freqs(freqs)
+            rp.set_fft_precision(64)
+            rp.rotate_batch(data, 0.0, DM_par, Ps, nu0, out=data)
+        data = data.cpu().numpy()
+    raw = dat_scl = dat_offs = None
+    if quantize:
+        raw, dat_scl, dat_offs, data = quantize_subints(data)
+    sig = pl.get_noise_batch(_f32(data))
+    mnorm = np.linalg.norm(models - models.mean(axis=-1, keepdims=True), axis=-1)     # [nmodel, nchan]
+    mnorm = mnorm[np.zeros(nsub, dtype=int) if model_index is None else model_index]
+    with np.errstate(divide="ignore"):
+        snrs = np.where(noise > 0, scl * mnorm / np.where(noise > 0, noise, 1.0), np.inf)
+    ok_ichans = [np.where(w[s] > 0)[0] for s in range(nsub)]
+    d = DataBunch(
+        arch=None, backend="fake", backend_delay=0.0, bw=float(bw), doppler_factors=np.ones(nsub),
+        DM=float(DM_par), dmc=int(bool(dedispersed)), epochs=epochs, filename=outfile or "fake_pulsar",
+        flux_prof=None, freqs=np.tile(freqs, (nsub, 1)), frontend="fake", integration_length=float(nsub * tsub),
+        masks=None, nbin=nbin, nchan=nchan, noise_stds=sig[:, None], npol=1, nsub=nsub, nu0=float(nu0),
+        ok_ichans=ok_ichans, ok_isubs=np.where((w > 0).any(axis=1))[0], parallactic_angles=np.zeros(nsub),
+        phases=phases, prof=None, prof_noise=None, prof_SNR=None, Ps=Ps, SNRs=snrs[:, None], source=source,
+        state=state, subints=np.asarray(data, dtype=np.float64)[:, None], subtimes=np.full(nsub, float(tsub)),
+        telescope=obs, telescope_code=obs, weights=w, raw_subints=raw, dat_scl=dat_scl, dat_offs=dat_offs)
+    if outfile is not None:
+        save_databunch(outfile, d)
+        if not quiet:
+            print("Wrote %s (%d subints, %d channels, %d bins)." % (outfile, nsub, nchan, nbin))
+    return d
+
+
 # ---- TOA output (host text formatting; pplib.py:3380-3503) ----------------------------------
 def filter_TOAs(TOAs, flag, cutoff, criterion=">=", pass_unflagged=False, return_culled=False):
     """Keep the TOAs whose attribute ``flag`` satisfies ``<criterion> cutoff`` (pplib.py:3380-3407)."""
