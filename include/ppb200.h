@@ -458,6 +458,27 @@ typedef struct {
 
 int pp_simulate_batch(pp_plan_t* plan, const pp_sim_args_t* args, const pp_sim_out_t* out);
 
+/* ---- PCA / B-spline model building ----------------------------------------------
+ * The device steps of pplib.make_spline_model (after ppspline.py make_spline_model), FP64, on the plan's
+ * [nchan, nbin] shape (any even nbin the plan takes).  With d_n = sqrt(w_n) (x_n - mu), W = sum_n w_n:
+ *   pp_pca_moments: mu = sum_n w_n x_n / W [nbin], and C = sum_n d_n d_n^T / W [nbin, nbin] (gram = 0) or
+ *     G = D D^T / W [nchan, nchan] (gram != 0), both triangles written and bit-symmetric.  Weights >= 0 (0 = excluded);
+ *     W must be positive.
+ *   pp_pca_project, back != 0: e_j = D^T u_j for the columns of vecs = U [nchan, m] (mean = mu, weights = w), each
+ *     normalised to unit norm with its entry of largest |value| positive: out = E [nbin, m].
+ *   pp_pca_project, back == 0: out = P [nchan, m], P_nj = sum_b (x_nb - mean_b) E_bj for vecs = E [nbin, m]
+ *     (unweighted; weights unused).
+ *   pp_lowpass_rows: per row of nbin samples: rfft, k_c = find_kc of the row's power spectrum (the rule of
+ *     pp_get_noise_fit_batch, fact = 1), harmonics above k_c set to zero (DC kept, the Nyquist term kept only when
+ *     k_c = nbin/2), irfft.  out [nrows, nbin], kc [nrows].
+ * No floating-point atomics and a fixed summation order: outputs are bit-identical run to run.  Inputs and outputs
+ * may be host or device pointers. */
+int pp_pca_moments(pp_plan_t* plan, const double* port, const double* weights, int32_t gram, double* mean_out,
+                   double* moment_out);
+int pp_pca_project(pp_plan_t* plan, const double* port, const double* weights, const double* mean,
+                   const double* vecs, int32_t m, int32_t back, double* out);
+int pp_lowpass_rows(pp_plan_t* plan, const double* rows, int32_t nrows, double* out, int32_t* kc);
+
 /* ---- diagnostics ------------------------------------------------------------ */
 typedef struct {
   int64_t launches;        /* kernels launched by the last pp_* call            */

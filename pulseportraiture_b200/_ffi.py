@@ -26,7 +26,7 @@ SYMBOLS = ["pp_plan_create", "pp_plan_destroy", "pp_plan_set_stream",
            "pp_fit_phase_shift_batch", "pp_fit_phase_shift_batch_bounds", "pp_rotate_batch", "pp_rotate_full_batch", "pp_apply_response_batch",
            "pp_align_accumulate", "pp_gen_gaussian_portrait", "pp_gen_gaussian_portrait_f64", "pp_gen_spline_portrait",
            "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64", "pp_fit_gaussian_portraits",
-           "pp_simulate_batch",
+           "pp_simulate_batch", "pp_pca_moments", "pp_pca_project", "pp_lowpass_rows",
            "pp_plan_enable_timing", "pp_get_stats", "pp_host_alloc",
            "pp_host_free", "pp_last_error",
            "pp_abi_version"]
@@ -232,6 +232,12 @@ def lib():
     L.pp_fit_gaussian_portraits.restype = C.c_int
     L.pp_simulate_batch.argtypes = [vp, C.POINTER(SimArgs), C.POINTER(SimOut)]
     L.pp_simulate_batch.restype = C.c_int
+    L.pp_pca_moments.argtypes = [vp, vp, vp, i32, vp, vp]
+    L.pp_pca_moments.restype = C.c_int
+    L.pp_pca_project.argtypes = [vp, vp, vp, vp, vp, i32, i32, vp]
+    L.pp_pca_project.restype = C.c_int
+    L.pp_lowpass_rows.argtypes = [vp, vp, i32, vp, vp]
+    L.pp_lowpass_rows.restype = C.c_int
     L.pp_plan_enable_timing.argtypes = [vp, i32]
     L.pp_plan_enable_timing.restype = C.c_int
     L.pp_get_stats.argtypes = [vp, C.POINTER(Stats)]

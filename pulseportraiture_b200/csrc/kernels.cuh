@@ -3146,27 +3146,16 @@ __device__ __forceinline__ bool noise_argmin_before(double c, int i, double best
   return c < best || (c == best && i < besti);
 }
 
-__global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ spec, const double* __restrict__ dc, double* noise,
-                                                    int nslot, int L, int nyq_slot, double fact) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  double* y = reinterpret_cast<double*>(smem_raw);     // [L + 1] log10 pows
-  double* pw = y + (L + 1);                            // [L + 1] pows
-  double* ek = pw + (L + 1);                           // [L + 1] e^{-a k}
+// find_kc of one row, called by all 256 threads of the CTA after y[0 .. nh) (the row's log10 powers, shared memory)
+// is written and synchronised; ek [nh] is shared scratch.  Returns k_crit, the first k with e^{-a k} < 0.005 at the
+// grid minimiser (nh - 1 if there is none), in every thread.  k_noise_fit and the low-pass of make_spline_model
+// (k_lowpass, k_lowpass_spec) both take their cut-off from here.
+__device__ int find_kc(const double* y, double* ek, int nh) {
   __shared__ double shv[8];
   __shared__ int shi[8];
   __shared__ double lim[2];
-  const long row = blockIdx.x;
-  const int tid = threadIdx.x, nh = L + 1;
-  const double inv_n = 1.0 / (double)(2 * L);
-  for (int k = tid; k < nh; k += 256) {
-    double p;
-    if (k == 0) p = dc[row] * dc[row];
-    else { const double2 d = spec[(size_t)row * nslot + (k == L ? nyq_slot : k)]; p = d.x * d.x + d.y * d.y; }
-    p *= inv_n;
-    pw[k] = p;
-    y[k] = log10(p);
-  }
-  __syncthreads();
+  __shared__ int kc_sh;
+  const int tid = threadIdx.x;
   if (tid < 32) {   // min / max of y
     double lo = CUDART_INF, hi = -CUDART_INF;
     for (int k = tid; k < nh; k += 32) { lo = fmin(lo, y[k]); hi = fmax(hi, y[k]); }
@@ -3207,6 +3196,32 @@ __global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ s
     const double av = mgrid(ia, a_st, a_lo);
     int kcrit = nh - 1;
     for (int k = 0; k < nh; ++k) if (exp(-av * (double)k) < 0.005) { kcrit = k; break; }
+    kc_sh = kcrit;
+  }
+  __syncthreads();
+  return kc_sh;
+}
+
+__global__ void __launch_bounds__(256) k_noise_fit(const double2* __restrict__ spec, const double* __restrict__ dc, double* noise,
+                                                    int nslot, int L, int nyq_slot, double fact) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* y = reinterpret_cast<double*>(smem_raw);     // [L + 1] log10 pows
+  double* pw = y + (L + 1);                            // [L + 1] pows
+  double* ek = pw + (L + 1);                           // [L + 1] e^{-a k}
+  const long row = blockIdx.x;
+  const int tid = threadIdx.x, nh = L + 1;
+  const double inv_n = 1.0 / (double)(2 * L);
+  for (int k = tid; k < nh; k += 256) {
+    double p;
+    if (k == 0) p = dc[row] * dc[row];
+    else { const double2 d = spec[(size_t)row * nslot + (k == L ? nyq_slot : k)]; p = d.x * d.x + d.y * d.y; }
+    p *= inv_n;
+    pw[k] = p;
+    y[k] = log10(p);
+  }
+  __syncthreads();
+  const int kcrit = find_kc(y, ek, nh);
+  if (tid == 0) {
     double kf = fact * (double)kcrit;
     if (kf >= (double)nh) kf = fmin((double)(int)(0.99 * nh), kf);
     const int k0 = (int)kf;

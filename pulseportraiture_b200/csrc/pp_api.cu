@@ -18,6 +18,7 @@
 #include "../../include/ppb200.h"
 #include "kernels.cuh"
 #include "gaussfit.cuh"
+#include "pca.cuh"
 #include "tw_host.h"
 
 using namespace ppb;
@@ -129,6 +130,8 @@ struct pp_plan {
   // simulated archives (pp_simulate_batch): the call's models, spectra and tables, staged inputs, chunk scratch
   DBuf sim_models, sim_freqs, sim_nu2, sim_mspec, sim_mdc, sim_index, sim_par[9], sim_scales, sim_sigma, sim_spec, sim_dc,
       sim_rows, sim_out, sim_raw, sim_scl, sim_offs;
+  // PCA model building (pp_pca_moments, pp_pca_project, pp_lowpass_rows)
+  DBuf pca_x, pca_w, pca_mu, pca_rw, pca_wsum, pca_vecs, pca_out, lp_in, lp_out, lp_kc;
   // timing
   bool timing = false;
   std::vector<cudaEvent_t> ev_chunk;   // "chunk finished" events for the overlapped result copies
@@ -2365,5 +2368,147 @@ extern "C" int pp_simulate_batch(pp_plan_t* pl, const pp_sim_args_t* args, const
   }
   CK(cudaStreamSynchronize(pl->stream));
   stats_end(pl);
+  return 0;
+}
+
+// ----------------------------------------------------------------------------
+// PCA / B-spline model building (pca.cuh)
+// ----------------------------------------------------------------------------
+static int pca_tile(pp_plan* pl, const PcaTileArgs& t) {
+  const dim3 grid((unsigned)((t.J + kPcaTile - 1) / kPcaTile), (unsigned)((t.I + kPcaTile - 1) / kPcaTile));
+  k_pca_tile<<<grid, 256, 0, pl->stream>>>(t);
+  pl->stats.launches++;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+static PcaOp pca_op(const double* p, const double* mean, const double* rw, int ld, int trans) {
+  PcaOp o;
+  o.p = p; o.mean = mean; o.rw = rw; o.ld = ld; o.trans = trans;
+  return o;
+}
+
+extern "C" int pp_pca_moments(pp_plan_t* pl, const double* port, const double* weights, int32_t gram, double* mean_out,
+                              double* moment_out) {
+  if (!pl || !port || !weights || !mean_out || !moment_out) return fail(-1, "NULL argument");
+  CK(cudaSetDevice(pl->device));
+  stats_begin(pl);
+  const int nchan = pl->nchan, nbin = pl->nbin;
+  const double *dx, *dw;
+  if (stage_in(pl, pl->pca_x, port, (size_t)nchan * nbin, &dx)) return -2;
+  if (stage_in(pl, pl->pca_w, weights, (size_t)nchan, &dw)) return -2;
+  CK(pl->pca_mu.need(sizeof(double) * nbin));
+  CK(pl->pca_rw.need(sizeof(double) * nchan));
+  CK(pl->pca_wsum.need(sizeof(double)));
+  const int dim = gram ? nchan : nbin;
+  CK(pl->pca_out.need(sizeof(double) * (size_t)dim * dim));
+  double* mu = pl->pca_mu.as<double>();
+  double* rw = pl->pca_rw.as<double>();
+  double* W = pl->pca_wsum.as<double>();
+  k_pca_mean<<<(unsigned)((std::max(nbin, nchan) + 255) / 256), 256, 0, pl->stream>>>(dx, dw, mu, rw, W, nchan, nbin);
+  pl->stats.launches++;
+  CK(cudaGetLastError());
+  double wsum = 0.0;
+  CK(cudaMemcpyAsync(&wsum, W, sizeof(double), cudaMemcpyDeviceToHost, pl->stream));
+  CK(cudaStreamSynchronize(pl->stream));
+  if (!(wsum > 0.0) || !std::isfinite(wsum)) return fail(-1, "the weights must sum to a positive finite value (got %g)", wsum);
+  PcaTileArgs t;
+  const PcaOp D = pca_op(dx, mu, rw, nbin, 0);
+  t.a = D; t.b = D;
+  t.a.trans = gram ? 0 : 1;   // covariance: a(i, k) = d_k[i]; Gram: a(i, k) = d_i[k]
+  t.b.trans = gram ? 1 : 0;
+  t.out = pl->pca_out.as<double>(); t.div = W;
+  t.I = t.J = dim; t.K = gram ? nbin : nchan; t.sym = 1;
+  if (pca_tile(pl, t)) return -2;
+  if (copy_out_at(pl->stream, mean_out, mu, 0, (size_t)nbin)) return -2;
+  if (copy_out_at(pl->stream, moment_out, t.out, 0, (size_t)dim * dim)) return -2;
+  CK(cudaStreamSynchronize(pl->stream));
+  return 0;
+}
+
+extern "C" int pp_pca_project(pp_plan_t* pl, const double* port, const double* weights, const double* mean,
+                              const double* vecs, int32_t m, int32_t back, double* out) {
+  if (!pl || !port || !mean || !vecs || !out || (back && !weights)) return fail(-1, "NULL argument");
+  const int nchan = pl->nchan, nbin = pl->nbin;
+  const int rows_in = back ? nchan : nbin;   // rows of vecs
+  if (m < 1 || m > rows_in) return fail(-1, "m must be in [1, %d] (got %d)", rows_in, m);
+  CK(cudaSetDevice(pl->device));
+  stats_begin(pl);
+  const double *dx, *dmu, *dv, *dw = nullptr;
+  if (stage_in(pl, pl->pca_x, port, (size_t)nchan * nbin, &dx)) return -2;
+  if (stage_in(pl, pl->pca_mu, mean, (size_t)nbin, &dmu)) return -2;
+  if (stage_in(pl, pl->pca_vecs, vecs, (size_t)rows_in * m, &dv)) return -2;
+  const int rows_out = back ? nbin : nchan;
+  CK(pl->pca_out.need(sizeof(double) * (size_t)rows_out * m));
+  PcaTileArgs t;
+  if (back) {
+    if (stage_in(pl, pl->pca_w, weights, (size_t)nchan, &dw)) return -2;
+    CK(pl->pca_rw.need(sizeof(double) * nchan));
+    k_pca_mean<<<(unsigned)((nchan + 255) / 256), 256, 0, pl->stream>>>(dx, dw, nullptr, pl->pca_rw.as<double>(), nullptr,
+                                                                        nchan, nbin);   // rw only
+    pl->stats.launches++;
+    CK(cudaGetLastError());
+    t.a = pca_op(dx, dmu, pl->pca_rw.as<double>(), nbin, 1);   // a(b, n) = d_n[b]
+  } else {
+    t.a = pca_op(dx, dmu, nullptr, nbin, 0);                   // a(n, b) = x_n[b] - mean[b]
+  }
+  t.b = pca_op(dv, nullptr, nullptr, m, 0);
+  t.out = pl->pca_out.as<double>(); t.div = nullptr;
+  t.I = rows_out; t.J = m; t.K = rows_in; t.sym = 0;
+  if (pca_tile(pl, t)) return -2;
+  if (back) {
+    k_pca_unit<<<(unsigned)m, 256, 0, pl->stream>>>(t.out, nbin, m);
+    pl->stats.launches++;
+    CK(cudaGetLastError());
+  }
+  if (copy_out_at(pl->stream, out, t.out, 0, (size_t)rows_out * m)) return -2;
+  CK(cudaStreamSynchronize(pl->stream));
+  return 0;
+}
+
+template <int N> static cudaError_t launch_lowpass(pp_plan* pl, const LowpassArgs& a, int nrows) {
+  const cudaError_t e = cudaFuncSetAttribute(k_lowpass<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)lowpass_smem_bytes<N>());
+  if (e != cudaSuccess) return e;
+  k_lowpass<N><<<(unsigned)nrows, 256, lowpass_smem_bytes<N>(), pl->stream>>>(a);
+  return cudaGetLastError();
+}
+
+extern "C" int pp_lowpass_rows(pp_plan_t* pl, const double* rows, int32_t nrows, double* out, int32_t* kc_out) {
+  if (!pl || !rows || !out || !kc_out) return fail(-1, "NULL argument");
+  if (nrows < 1) return fail(-1, "nrows must be >= 1");
+  CK(cudaSetDevice(pl->device));
+  stats_begin(pl);
+  const int nbin = pl->nbin;
+  const double* din;
+  if (stage_in(pl, pl->lp_in, rows, (size_t)nrows * nbin, &din)) return -2;
+  CK(pl->lp_out.need(sizeof(double) * (size_t)nrows * nbin));
+  CK(pl->lp_kc.need(sizeof(int) * (size_t)nrows));
+  double* dout = pl->lp_out.as<double>();
+  int* dkc = pl->lp_kc.as<int>();
+  if (pl->anyn) {
+    const int N = pl->N, L = pl->L;
+    CK(pl->any_spec2.need(sizeof(double2) * (size_t)nrows * N));
+    CK(pl->any_dc2.need(sizeof(double) * (size_t)nrows));
+    cx<double>* spec = pl->any_spec2.as<cx<double>>();
+    double* dc = pl->any_dc2.as<double>();
+    if (launch_fwd_any(pl, nullptr, false, nullptr, nullptr, nrows, spec, dc, din)) return -2;
+    const size_t smem = sizeof(double) * 2 * (size_t)(L + 1);
+    CK(cudaFuncSetAttribute(k_lowpass_spec, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_lowpass_spec<<<(unsigned)nrows, 256, smem, pl->stream>>>(spec, dc, dkc, N, L);
+    pl->stats.launches++;
+    CK(cudaGetLastError());
+    if (launch_inv_any(pl, spec, dc, dout, nrows, true)) return -2;
+  } else {
+    LowpassArgs a;
+    a.in = din; a.out = dout; a.kc = dkc; a.twN = pl->twN64.p; a.tw2N = pl->tw2N64.p;
+    cudaError_t e = cudaSuccess;
+    DISPATCH_N(pl->N, e = launch_lowpass<NN>(pl, a, nrows));
+    CK(e);
+    pl->stats.launches++;
+  }
+  CK(cudaGetLastError());
+  if (copy_out_at(pl->stream, out, dout, 0, (size_t)nrows * nbin)) return -2;
+  if (copy_out_at(pl->stream, kc_out, (int32_t*)dkc, 0, (size_t)nrows)) return -2;
+  CK(cudaStreamSynchronize(pl->stream));
   return 0;
 }

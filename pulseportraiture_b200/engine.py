@@ -476,6 +476,60 @@ class WidebandPlan(object):
             degree, op), "pp_gen_spline_portrait")
         return out
 
+    def pca_moments(self, port, weights, gram=False):
+        """Weighted mean profile mu [nbin] and second-moment matrix of d_n = sqrt(w_n) (x_n - mu), normalised by
+        sum(w): the covariance [nbin, nbin], or with ``gram`` the Gram matrix [nchan, nchan] (pp_pca_moments).
+        ``port`` [nchan, nbin] and ``weights`` [nchan] (>= 0, 0 = excluded) are float64 numpy arrays or CUDA
+        tensors."""
+        keep = []
+        if not _is_torch(weights) and np.any(np.asarray(weights, dtype=np.float64) < 0):
+            raise ValueError("weights must be >= 0")
+        dim = self.nchan if gram else self.nbin
+        mean = np.empty(self.nbin)
+        mat = np.empty((dim, dim))
+        _ffi.check(self._lib.pp_pca_moments(
+            self._h, _ptr(port, np.float64, keep, "port", (self.nchan, self.nbin)),
+            _ptr(weights, np.float64, keep, "weights", (self.nchan,)), int(bool(gram)),
+            mean.ctypes.data, mat.ctypes.data), "pp_pca_moments")
+        return mean, mat
+
+    def pca_backproject(self, port, weights, mean, U):
+        """Unit basis vectors e_j = D^T u_j / ||D^T u_j|| [nbin, m] from Gram eigenvectors U [nchan, m], with
+        d_n = sqrt(w_n) (x_n - mean); each with its entry of largest |value| positive (pp_pca_project)."""
+        keep = []
+        m = int(U.shape[1])
+        out = np.empty((self.nbin, m))
+        _ffi.check(self._lib.pp_pca_project(
+            self._h, _ptr(port, np.float64, keep, "port", (self.nchan, self.nbin)),
+            _ptr(weights, np.float64, keep, "weights", (self.nchan,)),
+            _ptr(mean, np.float64, keep, "mean", (self.nbin,)), _ptr(U, np.float64, keep, "U", (self.nchan, m)),
+            m, 1, out.ctypes.data), "pp_pca_project")
+        return out
+
+    def pca_project(self, port, mean, E):
+        """Projections P [nchan, m] of x_n - mean onto the columns of E [nbin, m] (pp_pca_project)."""
+        keep = []
+        m = int(E.shape[1])
+        out = np.empty((self.nchan, m))
+        _ffi.check(self._lib.pp_pca_project(
+            self._h, _ptr(port, np.float64, keep, "port", (self.nchan, self.nbin)), None,
+            _ptr(mean, np.float64, keep, "mean", (self.nbin,)), _ptr(E, np.float64, keep, "E", (self.nbin, m)),
+            m, 0, out.ctypes.data), "pp_pca_project")
+        return out
+
+    def lowpass_rows(self, rows):
+        """Low-pass float64 rows [nrows, nbin]: rfft, k_c from find_kc (get_noise_fit's rule, fact = 1), harmonics
+        above k_c zeroed (DC kept, Nyquist only when k_c reaches it), irfft (pp_lowpass_rows).  Returns (smoothed
+        rows [nrows, nbin], kc [nrows] int32)."""
+        keep = []
+        nrows = int(rows.shape[0])
+        out = np.empty((nrows, self.nbin))
+        kc = np.empty(nrows, dtype=np.int32)
+        _ffi.check(self._lib.pp_lowpass_rows(
+            self._h, _ptr(rows, np.float64, keep, "rows", (nrows, self.nbin)), nrows, out.ctypes.data,
+            kc.ctypes.data), "pp_lowpass_rows")
+        return out, kc
+
     def rotate_batch(self, data, phase, DM, P, nu_ref, out=None, GM=None, nu_GM=None):
         if GM is not None:
             return self._rotate_full(data, phase, DM, GM, P, nu_ref, nu_GM, out)

@@ -695,6 +695,146 @@ def write_model(filenm, name, model_code, nu_ref, model_params, fit_flags, alpha
         print("%s written." % filenm)
 
 
+# ---- ppspline: PCA / B-spline models -------------------------------------------------------------
+def _sign_convention(vecs):
+    """Columns of vecs [nbin, m] with their entry of largest |value| (the first such) made positive."""
+    vecs = np.array(vecs, dtype=np.float64)
+    if vecs.shape[1]:
+        ipk = np.argmax(np.abs(vecs), axis=0)
+        vecs *= np.where(vecs[ipk, np.arange(vecs.shape[1])] < 0.0, -1.0, 1.0)
+    return vecs
+
+
+def make_spline_model(port, freqs, weights=None, noise_stds=None, max_ncomp=10, smooth=True, snr_cutoff=150.0, k=3,
+                      sfac=1.0, max_nbreak=None, norm="prof", model_name=None, source=None, datafile=None, quiet=True):
+    """Build a PCA + B-spline model portrait (ppspline.py make_spline_model, pplib pca / find_significant_eigvec)
+    from an aligned portrait port [nchan, nbin] at frequencies freqs [nchan] (MHz), on the device.
+
+    1. Usable channels: weight > 0 and a row not all zero, sorted by frequency (duplicate frequencies raise
+       ValueError).  With ``norm`` they are normalised by ppalign.normalize_portrait(norm) and noise_stds scaled by
+       the same factors; the default noise_stds are get_noise ("PS") per channel, measured on the device.
+    2. PCA: the weighted mean profile mu and the second-moment matrix of sqrt(w_n) (x_n - mu) on the device, on the
+       smaller side (the covariance when the usable channels outnumber the bins, else the Gram matrix, whose
+       eigenvectors are back-projected); the top max_ncomp eigenpairs on the host, eigenvalues descending.
+    3. Significance: with ``smooth`` mu and each eigenvector e_j are low-passed (rfft, harmonics above find_kc's k_c
+       zeroed, irfft: WidebandPlan.lowpass_rows); snr_j = ||e~_j|| / sigma(e_j) with sigma the get_noise "PS" noise
+       of the unsmoothed e_j, and the e_j with snr_j >= snr_cutoff are kept in eigenvalue order (ieig).  The
+       reference smooths with wavelets (pywt), which is not used here, so the S/N of an eigenvector and therefore
+       the number kept for a given cutoff can differ from the reference's.
+    4. Basis: the kept smoothed vectors orthonormalised (QR, then each with its entry of largest |value| positive),
+       eigvec [nbin, ncomp]; the projections proj_port [n_ok, ncomp] of x_n - mu~ on the device.
+    5. Spline: scipy.interpolate.splprep(proj_port.T, u=freqs, w=1/noise_stds, k=k, s=sfac ncomp n_ok,
+       nest=None or max_nbreak + 2k): s is the expected chi^2 of pure noise under FITPACK's weighted condition.
+       ncomp = 0 gives the smoothed mean alone, tck = (zeros(2k + 2), [], k).
+
+    Returns a DataBunch: model_name, source, datafile, mean_prof, eigvec, tck, ncomp, ieig, eigval, snrs, kc (of
+    [mean, e_0, ...]; None without smoothing), proj_port, freqs, weights, noise_stds and channel_red_chi2s (all of the
+    usable channels in frequency order), fp, ier, msg (splprep's), model (gen_spline_portrait(..., device=True) at the
+    input freqs) and duration.  channel_red_chi2s = sum_b ((x_nb - model_nb) / noise_std_n)^2 / nbin of the normalised
+    data.  write_spline_model writes the model for read_spline_model / GetTOAs."""
+    import scipy.interpolate as si
+    import scipy.linalg as sl
+    start = time.time()
+    port = np.asarray(port, dtype=np.float64)
+    if port.ndim != 2:
+        raise ValueError("port must be [nchan, nbin]")
+    nchan, nbin = port.shape
+    freqs = np.asarray(freqs, dtype=np.float64).reshape(-1)
+    if len(freqs) != nchan:
+        raise ValueError("freqs has %d entries for %d channels" % (len(freqs), nchan))
+    weights = np.ones(nchan) if weights is None else np.asarray(weights, dtype=np.float64).reshape(-1)
+    if len(weights) != nchan or np.any(weights < 0) or not np.all(np.isfinite(weights)):
+        raise ValueError("weights must be [nchan] finite values >= 0")
+    k = int(k)
+    if not 1 <= k <= 5:
+        raise ValueError("the spline degree k must be in [1, 5] (got %d)" % k)
+    if int(max_ncomp) < 0:
+        raise ValueError("max_ncomp must be >= 0")
+    iok = np.nonzero((weights > 0) & port.any(axis=1))[0]
+    order = iok[np.argsort(freqs[iok], kind="stable")]
+    fok = freqs[order]
+    if np.any(np.diff(fok) == 0):
+        raise ValueError("duplicate frequencies among the usable channels")
+    n_ok = len(order)
+    if n_ok <= k:
+        raise ValueError("%d usable channels: the spline of degree %d needs more than %d" % (n_ok, k, k))
+    X, w = port[order], weights[order]
+    norms = np.ones(n_ok)
+    if norm is not None:
+        from .ppalign import normalize_portrait
+        r = normalize_portrait(X, norm, weights=w, return_norms=True)
+        if r is None:
+            raise ValueError("unknown norm %r" % (norm,))
+        X, norms = r
+    pl = get_plan(n_ok, nbin)
+    if noise_stds is None:
+        sig = get_noise_PS(X, chans=True)
+    else:
+        sig = np.asarray(noise_stds, dtype=np.float64).reshape(-1)
+        if len(sig) != nchan:
+            raise ValueError("noise_stds has %d entries for %d channels" % (len(sig), nchan))
+        sig = sig[order] / norms
+    if not np.all(sig > 0):
+        raise ValueError("the noise of every usable channel must be positive")
+
+    # PCA.  The eigen decomposition runs on the host (LAPACK's syevr through scipy.linalg.eigh, the top max_ncomp
+    # pairs only): the matrix has at most min(n_ok, nbin)^2 entries and the decomposition is a small, latency-bound
+    # part of the whole, which a device eigensolver would not shorten enough to be worth writing and pinning.
+    gram = n_ok <= nbin
+    mu, M = pl.pca_moments(X, w, gram=gram)
+    dim = M.shape[0]
+    m = min(int(max_ncomp), dim)
+    if m:
+        eigval, U = sl.eigh(M, subset_by_index=[dim - m, dim - 1])
+        eigval, U = eigval[::-1].copy(), np.ascontiguousarray(U[:, ::-1])
+        E = pl.pca_backproject(X, w, mu, U) if gram else _sign_convention(U)
+    else:
+        eigval, E = np.zeros(0), np.zeros((nbin, 0))
+
+    # significance
+    rows = np.ascontiguousarray(np.vstack([mu[None], E.T]))
+    if smooth:
+        srows, kc = get_plan(len(rows), nbin).lowpass_rows(rows)
+    else:
+        srows, kc = rows, None
+    mean_prof = srows[0].copy()
+    if m:
+        snrs = np.linalg.norm(srows[1:], axis=1) / get_noise_PS(E.T, chans=True)
+    else:
+        snrs = np.zeros(0)
+    ieig = np.nonzero(snrs >= snr_cutoff)[0]
+    ncomp = len(ieig)
+    if ncomp:
+        eigvec = _sign_convention(np.linalg.qr(srows[1:][ieig].T)[0])
+        proj = pl.pca_project(X, mean_prof, eigvec)
+        nest = None if max_nbreak is None else int(max_nbreak) + 2 * k
+        (tck, _), fp, ier, msg = si.splprep(proj.T, u=fok, w=1.0 / sig, k=k, s=float(sfac) * ncomp * n_ok, nest=nest,
+                                            full_output=1, quiet=1)
+        tck = (np.asarray(tck[0]), [np.asarray(c) for c in tck[1]], int(tck[2]))
+    else:
+        eigvec, proj = np.zeros((nbin, 0)), np.zeros((n_ok, 0))
+        tck, fp, ier, msg = (np.zeros(2 * k + 2), [], k), 0.0, 0, "no significant eigenvector: the model is the mean"
+    model = gen_spline_portrait(mean_prof, freqs, eigvec, tck, device=True)
+    red_chi2s = (((X - model[order]) / sig[:, None]) ** 2).sum(axis=1) / nbin
+    if not quiet:
+        print("%d of %d eigenvectors significant (S/N >= %g); splprep: fp = %.4g, ier = %s"
+              % (ncomp, m, snr_cutoff, fp, ier))
+    return DataBunch(model_name=model_name, source=source, datafile=datafile, mean_prof=mean_prof, eigvec=eigvec,
+                     tck=tck, ncomp=ncomp, ieig=ieig, eigval=eigval, snrs=snrs, kc=kc, proj_port=proj, freqs=fok,
+                     weights=w, noise_stds=sig, fp=fp, ier=ier, msg=msg, model=model, channel_red_chi2s=red_chi2s,
+                     duration=time.time() - start)
+
+
+def write_spline_model(outfile, model_name, source, datafile, mean_prof, eigvec, tck, quiet=False):
+    """Pickle a PCA / B-spline model as the list [model_name, source, datafile, mean_prof, eigvec, tck] (protocol 2),
+    the layout of ppspline.py's write_model that read_spline_model, is_spline_model and GetTOAs read."""
+    import pickle
+    with open(outfile, "wb") as fh:
+        pickle.dump([model_name, source, datafile, mean_prof, eigvec, tck], fh, protocol=2)
+    if not quiet:
+        print("%s written." % outfile)
+
+
 # ---- simulated archives (pplib.py:3183-3378) --------------------------------------------------
 def read_ephemeris(ephemeris):
     """(F0 [Hz], F1 [Hz/s], PEPOCH [MJD], DM, source) from a .par file (F0, optional F1 and PEPOCH, DM, PSRJ / PSR)
