@@ -406,6 +406,26 @@ typedef struct {
 int pp_fit_gaussian_portraits(pp_plan_t* plan, const pp_gfit_args_t* args,
                               const pp_gfit_out_t* out);
 
+/* Join parameters (ppgauss's multi-receiver fit): one evolving-Gaussian model fit to a portrait whose channels
+ * come from several archives, each archive after the first with its own phase and DM offset.  Channel n of group
+ * j = join_chan[n] is rotated as rotate_data(row, phi_j, DM_j, P, freqs, nu_ref) after scattering: harmonic k is
+ * multiplied by e^{2 pi i k theta_n}, theta_n = phi_j + Dconst DM_j / P (nu_n^-2 - nu_ref^-2), and the Nyquist term
+ * (irfft keeps its real part) by cos(2 pi N theta_n).  Channels with join_chan[n] = -1 are not rotated.  The
+ * parameter vector grows to P = 3 + 6*ngauss + 2*njoin:
+ *   [DC, tau, (loc, m_loc, wid, m_wid, amp, m_amp) x ngauss, alpha, (phi_j, DM_j) x njoin]
+ * and fit_flags, bounds, init and every output of pp_fit_gaussian_portraits_join cover all P entries.
+ * NULL join or njoin = 0: exactly pp_fit_gaussian_portraits.  data (and errs) may be NULL when max_iter < 0 and
+ * out->model is the only output: the model portraits at init (the device generator of joined models, FP64).
+ * Errors: njoin > 8, P <= 0, a join_chan entry outside [-1, njoin), a group with no channel. */
+typedef struct {
+  int32_t njoin;              /* 0..8 groups                                            */
+  const int32_t* join_chan;   /* HOST [nchan] group of each channel, -1 = none          */
+  double P;                   /* spin period [s] of the DM term, > 0                    */
+} pp_gfit_join_t;
+
+int pp_fit_gaussian_portraits_join(pp_plan_t* plan, const pp_gfit_args_t* args,
+                                   const pp_gfit_join_t* join, const pp_gfit_out_t* out);
+
 /* ---- simulated archives ---------------------------------------------------------
  * Replaces the data generation of pplib.make_fake_pulsar (pplib.py:3183-3378) for a batch of subints, without the
  * PSRFITS writing.  Row (s, n), m = model_index[s]:

@@ -26,6 +26,7 @@ SYMBOLS = ["pp_plan_create", "pp_plan_destroy", "pp_plan_set_stream",
            "pp_fit_phase_shift_batch", "pp_fit_phase_shift_batch_bounds", "pp_rotate_batch", "pp_rotate_full_batch", "pp_apply_response_batch",
            "pp_align_accumulate", "pp_gen_gaussian_portrait", "pp_gen_gaussian_portrait_f64", "pp_gen_spline_portrait",
            "pp_get_noise_batch", "pp_get_noise_cut_batch", "pp_get_noise_fit_batch", "pp_measure_fp64", "pp_fit_gaussian_portraits",
+           "pp_fit_gaussian_portraits_join",
            "pp_simulate_batch", "pp_pca_moments", "pp_pca_project", "pp_lowpass_rows",
            "pp_plan_enable_timing", "pp_get_stats", "pp_host_alloc",
            "pp_host_free", "pp_last_error",
@@ -126,6 +127,14 @@ class GfitOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in (
         "params", "param_errs", "cov", "chi2", "red_chi2", "nfeval", "return_code",
         "jtr", "jtj", "model")]
+
+
+class GfitJoin(C.Structure):
+    _fields_ = [
+        ("njoin", C.c_int32),
+        ("join_chan", C.c_void_p),
+        ("P", C.c_double),
+    ]
 
 
 class SimArgs(C.Structure):
@@ -230,6 +239,8 @@ def lib():
     L.pp_measure_fp64.restype = C.c_int
     L.pp_fit_gaussian_portraits.argtypes = [vp, C.POINTER(GfitArgs), C.POINTER(GfitOut)]
     L.pp_fit_gaussian_portraits.restype = C.c_int
+    L.pp_fit_gaussian_portraits_join.argtypes = [vp, C.POINTER(GfitArgs), C.POINTER(GfitJoin), C.POINTER(GfitOut)]
+    L.pp_fit_gaussian_portraits_join.restype = C.c_int
     L.pp_simulate_batch.argtypes = [vp, C.POINTER(SimArgs), C.POINTER(SimOut)]
     L.pp_simulate_batch.restype = C.c_int
     L.pp_pca_moments.argtypes = [vp, vp, vp, i32, vp, vp]

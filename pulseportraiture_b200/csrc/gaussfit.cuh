@@ -3,30 +3,41 @@
 //
 //   k_gfit_pass<N>   one (portrait, channel) row at a time: the model row g_n and its analytic
 //                    local derivative rows are transformed with the double row FFT of fft.cuh,
-//                    scattered in the Fourier domain, and the channel's local normal matrix,
-//                    J^T r and chi^2 are summed over harmonics in a fixed order
+//                    scattered (and rotated, with join parameters) in the Fourier domain, and the
+//                    channel's local normal matrix, J^T r and chi^2 are summed over harmonics in a
+//                    fixed order
 //   k_gfit_reduce    chain rule: local sums of every channel -> the global P x P system, summed
 //                    over channels in channel order (one thread per entry)
 //   k_gfit_update    Levenberg-Marquardt with Marquardt scaling, an active set for the bounds,
 //                    damped Cholesky, accept / reject by chi^2, and the epilogue (errors, cov)
 //
-// Parameter vector (P = 3 + 6 ngauss): [DC, tau [bin at nu_ref], (loc, m_loc, wid, m_wid, amp,
-// m_amp) x ngauss, alpha].  Local columns of channel n (L = 2 + 3 ngauss): 0 = DC, 1 + 3g + q with
-// q = 0 loc_n, 1 wid_n, 2 amp_n of component g, and L - 1 = tau_n.
+// Parameter vector (P = 3 + 6 ngauss + 2 njoin): [DC, tau [bin at nu_ref], (loc, m_loc, wid, m_wid, amp,
+// m_amp) x ngauss, alpha, (phi_j, DM_j) x njoin]; alpha is entry ia = 2 + 6 ngauss.  Local columns of
+// channel n (L = 2 + 3 ngauss, plus 1 with joins): 0 = DC, 1 + 3g + q with q = 0 loc_n, 1 wid_n, 2 amp_n
+// of component g, 1 + 3 ngauss = tau_n and, with joins, 2 + 3 ngauss = theta_n.
 //
 // Objective (Parseval, N = nbin/2): chi^2 = sum_n (R_0^2 + 2 sum_{0<k<N} |R_k|^2 + R_N^2) / (nbin sigma_n^2)
-// with R = rfft(d) - M, M_0 = G_0, M_k = B_k G_k, M_N = Re(B_N) G_N, B_k = 1 / (1 + 2 pi i k tau_n):
-// what irfft(B rfft(g)) of gen_gaussian_portrait (pplib.py:921-927) does with each harmonic.
+// with R = rfft(d) - M, M_0 = G_0, M_k = E_k B_k G_k, M_N = cos(2 pi N theta_n) Re(B_N) G_N,
+// B_k = 1 / (1 + 2 pi i k tau_n), E_k = e^{2 pi i k theta_n}: what irfft(B rfft(g)) of gen_gaussian_portrait
+// (pplib.py:921-927) does with each harmonic, followed by rotate_data(., phi_j, DM_j, P, freqs, nu_ref) on the
+// channels of join group j.  theta_n = phi_j + Dconst DM_j / P (nu_n^-2 - nu_ref^-2) for a channel of group j
+// (join_chan[n] = j) and 0 for a channel in no group; dM_k/dtheta_n = 2 pi i k M_k, and at the Nyquist term
+// -2 pi N sin(2 pi N theta_n) Re(B_N) G_N.  The restatement is tests/test_cpu_gaussjoin.py.
+//
+// Size caps: ngauss <= 16, njoin <= 8, so P <= kGfitMaxP = 3 + 6 * 16 + 2 * 8 = 115.  k_gfit_update holds two
+// P x P double matrices in dynamic shared memory (2 * 115^2 * 8 = 211600 bytes at the cap) next to its static
+// arrays (idx, D, g, dx and flags: 3248 bytes): within the 227 KB a block may opt in to.
 #pragma once
 #include "kernels.cuh"
 
 namespace ppb {
 
 constexpr int kGfitMaxGauss = 16;
-constexpr int kGfitMaxP = 3 + 6 * kGfitMaxGauss;   // 99
+constexpr int kGfitMaxJoin = 8;
+constexpr int kGfitMaxP = 3 + 6 * kGfitMaxGauss + 2 * kGfitMaxJoin;   // 115
 
 struct GfitArgs {
-  const double* data;    // [nc, nchan, nbin]
+  const double* data;    // [nc, nchan, nbin], or null when only the model is written
   const double* errs;    // [nc, nchan]
   const double* freqs;   // [nchan]
   const double* xt;      // [nc, P] point to evaluate
@@ -37,24 +48,32 @@ struct GfitArgs {
   double* model;         // [nc, nchan, nbin] or null: write the model portrait at xt instead of sums
   const void* twN;
   const void* tw2N;
+  const int* join_chan;  // [nchan] join group of each channel, -1 = none (null when njoin = 0)
   double nu_ref;
+  double P_period;       // spin period [s] of the DM chain (njoin > 0)
   int nc, nchan, ngauss, P, L, S;
+  int ia;                // index of alpha: 2 + 6 ngauss; the join pairs follow it
+  int njoin;
   int code[3];           // loc, wid, amp: 0 power law, 1 linear
 };
 
 // index of (u, v), u <= v, in the packed upper triangle of an n x n symmetric matrix
 __host__ __device__ __forceinline__ int tri_index(int u, int v, int n) { return u * n - u * (u - 1) / 2 + (v - u); }
 
-// the local column global parameter i maps to (P = 3 + 6 ngauss)
-__device__ __forceinline__ int gfit_local(int i, int P, int L) {
+// the local column global parameter i maps to (ia = index of alpha = 2 + 6 ngauss; tau_n is local column
+// ia / 2 = 1 + 3 ngauss, theta_n the one after it)
+__device__ __forceinline__ int gfit_local(int i, int ia) {
   if (i == 0) return 0;
-  if (i == 1 || i == P - 1) return L - 1;
+  if (i == 1 || i == ia) return ia / 2;
+  if (i > ia) return ia / 2 + 1;           // phi_j, DM_j: through theta_n
   const int j = i - 2;                      // (g, q, e) = component, quantity, evolution term
   return 1 + 3 * (j / 6) + (j % 6) / 2;
 }
 
-template <int N>
-__global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
+// kJoin: a.njoin > 0 (a separate instance, so that the unjoined fit carries no join code).  Two CTAs per SM:
+// without the bound ptxas caps some instances at 80 registers and spills.
+template <int N, bool kJoin>
+__global__ void __launch_bounds__(256, 2) k_gfit_pass(GfitArgs a) {
   using G = RowGeom<N>;
   constexpr int nbin = 2 * N;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -64,7 +83,7 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
   __shared__ double p[kGfitMaxP];
   __shared__ GaussComp comp[kGfitMaxGauss];
   __shared__ double cval[kGfitMaxGauss][3];   // loc_n, wid_n, amp_n
-  __shared__ double sh_tau;
+  __shared__ double sh_tau, sh_theta;
   const int tid = threadIdx.x, r = tid / G::kTRow, t_row = tid % G::kTRow;
   const int lane = tid & 31, warp = tid >> 5;
   {
@@ -75,7 +94,9 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
   }
   cx<double>* bufA = bufs + (size_t)r * 2 * N;
   cx<double>* bufB = bufA + N;
-  const int P = a.P, L = a.L, ng = a.ngauss;
+  const int P = a.P, L = a.L, ng = a.ngauss, ia = a.ia;
+  const int Lt = ia / 2 + 1;   // slab row of the tau_n column (L without joins)
+  constexpr bool join = kJoin;
   const BinCentres xbin(nbin);
   cx<double>* slab = reinterpret_cast<cx<double>*>(a.slab) + (size_t)blockIdx.x * (L + 1) * (N + 1);
   const long nunits = (long)a.nc * a.nchan;
@@ -83,6 +104,8 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
     const int s = (int)(unit / a.nchan), ch = (int)(unit % a.nchan);
     if (a.done && a.done[s]) continue;
     const double f = a.freqs[ch];
+    const int jg = join ? a.join_chan[ch] : -1;                      // join group of the channel
+    const double kdm = join ? kDconst / a.P_period * (1.0 / (f * f) - 1.0 / (a.nu_ref * a.nu_ref)) : 0.0;
     __syncthreads();   // the previous unit is finished with p, comp and the slab
     for (int i = tid; i < P; i += 256) p[i] = a.xt[(size_t)s * P + i];
     __syncthreads();
@@ -94,17 +117,23 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
       comp[g] = gauss_comp(loc, wid, amp, xbin);
       cval[g][0] = loc; cval[g][1] = wid; cval[g][2] = amp;
     }
-    if (tid == 0) sh_tau = (p[1] / (double)nbin) * pow(f / a.nu_ref, p[P - 1]);   // pplib.py:4049-4053
+    if (tid == 0) {
+      sh_tau = (p[1] / (double)nbin) * pow(f / a.nu_ref, p[ia]);   // pplib.py:4049-4053
+      double th = 0.0;
+      if (jg >= 0) { th = p[ia + 1 + 2 * jg] + p[ia + 2 + 2 * jg] * kdm; th -= rint(th); }
+      sh_theta = th;
+    }
     __syncthreads();
     // time-domain rows, transformed kRows at a time: j = 0 data -> slab row 0, j = 1 model g -> row L
-    // (replaced by the tau_n column below), j = 2 + 3g + q -> row 2 + 3g + q (local column 1 + 3g + q)
+    // (replaced by the tau_n column, or with joins the theta_n column, below), j = 2 + 3g + q -> row
+    // 2 + 3g + q (local column 1 + 3g + q)
     const int nfft = 2 + 3 * ng;
-    const double* drow = a.data + ((size_t)s * a.nchan + ch) * nbin;
+    const double* drow = a.data ? a.data + ((size_t)s * a.nchan + ch) * nbin : nullptr;
     for (int base = 0; base < nfft; base += G::kRows) {
       const int j = base + r;
       auto sample = [&](int t) -> double {
         if (j >= nfft) return 0.0;
-        if (j == 0) return drow[t];
+        if (j == 0) return drow ? drow[t] : 0.0;
         const double x = xbin(t);
         if (j == 1) {
           double v = p[0];
@@ -144,9 +173,9 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
       }
       __syncthreads();
     }
-    // scattering, residual and weights, harmonic by harmonic
-    const double tau_n = sh_tau;
-    const double sig = a.errs[(size_t)s * a.nchan + ch];
+    // scattering, rotation, residual and weights, harmonic by harmonic
+    const double tau_n = sh_tau, theta_n = sh_theta;
+    const double sig = a.errs ? a.errs[(size_t)s * a.nchan + ch] : 1.0;   // null: model only
     const double s_mid = sqrt(2.0 / (double)nbin) / sig, s_end = sqrt(1.0 / (double)nbin) / sig;
     for (int k = tid; k <= N; k += 256) {
       cx<double> fB = mk<double>(1.0, 0.0), fT = mk<double>(0.0, 0.0);   // M_k / G_k and dM_k/dtau_n / G_k
@@ -157,6 +186,20 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
         fT = mk<double>(kTwoPi * (double)k * B2.y, -kTwoPi * (double)k * B2.x);   // -2 pi i k B^2
         if (k == N) { fB.y = 0.0; fT.y = 0.0; }                            // irfft keeps Re of the Nyquist term
       }
+      cx<double> fH = mk<double>(0.0, 0.0);                                // dM_k/dtheta_n / G_k
+      if (join) {   // E_k = e^{2 pi i k theta_n}; the rotated real row keeps cos(2 pi N theta_n) at the Nyquist term
+        double c, sn;
+        cis2pi((double)k * theta_n, c, sn);
+        const double w = kTwoPi * (double)k;
+        if (k == N) {
+          fH = mk<double>(-w * sn * fB.x, 0.0);
+          fB.x *= c; fT.x *= c;
+        } else {
+          const cx<double> E = mk<double>(c, sn);
+          fB = cmul(fB, E); fT = cmul(fT, E);
+          fH = mk<double>(-w * fB.y, w * fB.x);                            // 2 pi i k E_k B_k
+        }
+      }
       const double sc = (k == 0 || k == N) ? s_end : s_mid;
       const cx<double> Gk = slab[(size_t)L * (N + 1) + k];
       const cx<double> M = cmul(fB, Gk);
@@ -164,9 +207,13 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
       const cx<double> D = slab[k];
       slab[k] = mk<double>((D.x - M.x) * sc, (D.y - M.y) * sc);
       const cx<double> T = cmul(fT, Gk);
-      slab[(size_t)L * (N + 1) + k] = mk<double>(T.x * sc, T.y * sc);
+      slab[(size_t)Lt * (N + 1) + k] = mk<double>(T.x * sc, T.y * sc);
+      if (join) {
+        const cx<double> H = cmul(fH, Gk);
+        slab[(size_t)L * (N + 1) + k] = mk<double>(H.x * sc, H.y * sc);
+      }
       slab[(size_t)(N + 1) + k] = mk<double>(k == 0 ? (double)nbin * sc : 0.0, 0.0);   // DC: rfft(1) = nbin at k = 0
-      for (int c = 1; c < L - 1; ++c) {
+      for (int c = 1; c < Lt - 1; ++c) {
         const cx<double> J = cmul(fB, slab[(size_t)(c + 1) * (N + 1) + k]);
         slab[(size_t)(c + 1) * (N + 1) + k] = mk<double>(J.x * sc, J.y * sc);
       }
@@ -213,9 +260,12 @@ __global__ void __launch_bounds__(256) k_gfit_pass(GfitArgs a) {
       const double lr = log(f) - log(a.nu_ref);
       double c;
       if (i == 0) c = 1.0;
-      else if (i == 1) c = pow(f / a.nu_ref, p[P - 1]) / (double)nbin;
-      else if (i == P - 1) c = tau_n * lr;
-      else {
+      else if (i == 1) c = pow(f / a.nu_ref, p[ia]) / (double)nbin;
+      else if (i == ia) c = tau_n * lr;
+      else if (i > ia) {   // phi_j, DM_j: d theta_n on the channels of group j, 0 elsewhere
+        const int jj = (i - ia - 1) / 2;
+        c = jg != jj ? 0.0 : ((i - ia - 1) % 2 == 0 ? 1.0 : kdm);
+      } else {
         const int j = i - 2, g = j / 6, q = (j % 6) / 2, ev = j % 2;
         if (a.code[q] == 1) c = ev ? f - a.nu_ref : 1.0;
         else c = ev ? cval[g][q] * lr : exp(lr * p[i + 1]);   // (nu/nu_ref)^m, x_n ln(nu/nu_ref)
@@ -258,7 +308,7 @@ __global__ void __launch_bounds__(256) k_gfit_reduce(GfitArgs a, GfitState st, c
   if (e >= npair) {
     const int i = e - npair;
     if (free_[i]) {
-      const int t = tri_index(0, 1 + gfit_local(i, P, L), L + 1);
+      const int t = tri_index(0, 1 + gfit_local(i, a.ia), L + 1);
       for (int n = 0; n < a.nchan; ++n) { const double* rn = rec + (size_t)n * a.S; acc += rn[nsum + i] * rn[t]; }
     }
     st.jtr_t[(size_t)s * P + i] = acc;
@@ -268,7 +318,7 @@ __global__ void __launch_bounds__(256) k_gfit_reduce(GfitArgs a, GfitState st, c
   while (rem >= P - i) { rem -= P - i; ++i; }
   const int j = i + rem;
   if (free_[i] && free_[j]) {
-    const int u = 1 + gfit_local(i, P, L), v = 1 + gfit_local(j, P, L);
+    const int u = 1 + gfit_local(i, a.ia), v = 1 + gfit_local(j, a.ia);
     const int t = u <= v ? tri_index(u, v, L + 1) : tri_index(v, u, L + 1);
     for (int n = 0; n < a.nchan; ++n) {
       const double* rn = rec + (size_t)n * a.S;
@@ -349,7 +399,8 @@ struct GfitUpdateArgs {
 constexpr double kGfitLam0 = 1e-3;
 constexpr double kGfitChi2Slack = 1e-12;
 
-__global__ void __launch_bounds__(256) k_gfit_update(GfitState st, GfitUpdateArgs u) {
+// one CTA per SM (up to 211600 bytes of dynamic shared memory); the bound lets ptxas keep it free of spills
+__global__ void __launch_bounds__(256, 1) k_gfit_update(GfitState st, GfitUpdateArgs u) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int s = blockIdx.x, P = u.P, tid = threadIdx.x;
   if (st.done[s]) return;

@@ -126,7 +126,7 @@ struct pp_plan {
   // chunk-sized
   DBuf X, Xlo, partial, data_stage[2], data_stage64[2], Dspec, Ddc, al_acc, al_wparts, al_dc;
   // evolving-Gaussian portrait fit (pp_fit_gaussian_portraits): per-chunk state and outputs, per-CTA slabs
-  DBuf gf_data, gf_errs, gf_rec, gf_slab, gf_state, gf_out, gf_model, gf_par;
+  DBuf gf_data, gf_errs, gf_rec, gf_slab, gf_state, gf_out, gf_model, gf_par, gf_join;
   // simulated archives (pp_simulate_batch): the call's models, spectra and tables, staged inputs, chunk scratch
   DBuf sim_models, sim_freqs, sim_nu2, sim_mspec, sim_mdc, sim_index, sim_par[9], sim_scales, sim_sigma, sim_spec, sim_dc,
       sim_rows, sim_out, sim_raw, sim_scl, sim_offs;
@@ -1978,11 +1978,12 @@ extern "C" int pp_get_noise_cut_batch(pp_plan_t* pl, const float* data, int32_t 
 // 65535), or is pp_plan_set_chunk's count: the scratch does not grow with nport.
 static const size_t kGfitChunkBytes = 256u << 20;
 
-template <int N> static int gfit_slabs(pp_plan* pl, int* nslab) {
+template <int N> static int gfit_slabs(pp_plan* pl, bool join, int* nslab) {
   const size_t smem = fft_smem_bytes<N, double>();
-  CK(cudaFuncSetAttribute(k_gfit_pass<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kern = join ? k_gfit_pass<N, true> : k_gfit_pass<N, false>;
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_gfit_pass<N>, 256, smem));
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, smem));
   *nslab = std::max(1, per_sm) * pl->sm_count;
   return 0;
 }
@@ -1990,7 +1991,8 @@ template <int N> static int gfit_slabs(pp_plan* pl, int* nslab) {
 template <int N> static int gfit_pass(pp_plan* pl, const GfitArgs& a, int nslab) {
   const long units = (long)a.nc * a.nchan;
   const unsigned grid = (unsigned)std::min<long>(units, nslab);
-  k_gfit_pass<N><<<grid, 256, fft_smem_bytes<N, double>(), pl->stream>>>(a);
+  if (a.njoin > 0) k_gfit_pass<N, true><<<grid, 256, fft_smem_bytes<N, double>(), pl->stream>>>(a);
+  else k_gfit_pass<N, false><<<grid, 256, fft_smem_bytes<N, double>(), pl->stream>>>(a);
   pl->stats.launches++;
   pl->stats.pass_launches++;
   CK(cudaGetLastError());
@@ -1998,10 +2000,20 @@ template <int N> static int gfit_pass(pp_plan* pl, const GfitArgs& a, int nslab)
 }
 
 extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* args, const pp_gfit_out_t* out) {
+  return pp_fit_gaussian_portraits_join(pl, args, nullptr, out);
+}
+
+extern "C" int pp_fit_gaussian_portraits_join(pp_plan_t* pl, const pp_gfit_args_t* args, const pp_gfit_join_t* join,
+                                              const pp_gfit_out_t* out) {
   if (!pl || !args || !out) return fail(-1, "NULL argument");
   const pp_gfit_args_t& A = *args;
   if (A.nport < 1) return fail(-1, "nport must be >= 1");
-  if (!A.data || !A.errs || !A.init || !A.model_code || !A.fit_flags) return fail(-1, "NULL input array");
+  // data = NULL: the model portraits at init only (the generator of joined models)
+  const bool gen = A.data == nullptr;
+  if (gen && (A.max_iter >= 0 || !out->model || out->params || out->param_errs || out->cov || out->chi2 ||
+              out->red_chi2 || out->nfeval || out->return_code || out->jtr || out->jtj))
+    return fail(-1, "data may be NULL only with max_iter < 0 and out->model the only output");
+  if ((!gen && !A.errs) || !A.init || !A.model_code || !A.fit_flags) return fail(-1, "NULL input array");
   if (A.ngauss < 1 || A.ngauss > kGfitMaxGauss) return fail(-1, "ngauss must be in [1, %d] (got %d)", kGfitMaxGauss, A.ngauss);
   if (strlen(A.model_code) < 3) return fail(-1, "model_code needs three characters (loc, wid, amp)");
   for (int i = 0; i < 3; ++i)
@@ -2010,13 +2022,28 @@ extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* ar
   if (pl->anyn) return fail(-1, "the Gaussian portrait fit needs nbin a power of two in [64, 4096] (got %d)", pl->nbin);
   if (!pl->freqs_set) return fail(-1, "pp_set_freqs must be called before pp_fit_gaussian_portraits");
   if (is_device_ptr(A.fit_flags) || (A.bounds && is_device_ptr(A.bounds))) return fail(-1, "fit_flags and bounds must be host arrays");
+  const int njoin = join ? join->njoin : 0;
+  if (njoin < 0 || njoin > kGfitMaxJoin) return fail(-1, "njoin must be in [0, %d] (got %d)", kGfitMaxJoin, njoin);
+  if (njoin > 0) {
+    if (!join->join_chan) return fail(-1, "NULL join_chan");
+    if (is_device_ptr(join->join_chan)) return fail(-1, "join_chan must be a host array");
+    if (!(join->P > 0.0) || !std::isfinite(join->P)) return fail(-1, "the join period P must be positive (got %g)", join->P);
+    std::vector<int> count(njoin, 0);
+    for (int n = 0; n < pl->nchan; ++n) {
+      const int j = join->join_chan[n];
+      if (j < -1 || j >= njoin) return fail(-1, "join_chan[%d] = %d is not a group in [-1, %d)", n, j, njoin);
+      if (j >= 0) ++count[j];
+    }
+    for (int j = 0; j < njoin; ++j)
+      if (!count[j]) return fail(-1, "join group %d has no channel", j);
+  }
   CK(cudaSetDevice(pl->device));
   stats_begin(pl);
   const int N = pl->N, nbin = pl->nbin, nchan = pl->nchan, ng = A.ngauss;
-  const int P = 3 + 6 * ng, L = 2 + 3 * ng, S = (L + 1) * (L + 2) / 2 + P;
+  const int P = 3 + 6 * ng + 2 * njoin, L = 2 + 3 * ng + (njoin > 0 ? 1 : 0), S = (L + 1) * (L + 2) / 2 + P;
   const int nport = A.nport;
   // host checks of sigma (a device array is read back once)
-  {
+  if (!gen) {
     std::vector<double> e((size_t)nport * nchan);
     CK(cudaMemcpy(e.data(), A.errs, sizeof(double) * e.size(), cudaMemcpyDefault));
     for (size_t i = 0; i < e.size(); ++i)
@@ -2041,12 +2068,18 @@ extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* ar
   // the chunk's portraits are gridDim.y of k_gfit_reduce (<= 65535)
   const int chunk = (int)std::min<size_t>(std::min<size_t>(want, 65535), (size_t)nport);
   int nslab = 0;
-  DISPATCH_N(N, if (gfit_slabs<NN>(pl, &nslab)) return -2);
+  DISPATCH_N(N, if (gfit_slabs<NN>(pl, njoin > 0, &nslab)) return -2);
   nslab = (int)std::min<long>(nslab, (long)chunk * nchan);
   CK(pl->gf_slab.need(sizeof(double2) * (size_t)nslab * (L + 1) * (N + 1)));
   CK(pl->gf_rec.need(sizeof(double) * (size_t)chunk * nchan * S));
-  CK(pl->gf_data.need(sizeof(double) * (size_t)chunk * nchan * nbin));
-  CK(pl->gf_errs.need(sizeof(double) * (size_t)chunk * nchan));
+  if (!gen) {
+    CK(pl->gf_data.need(sizeof(double) * (size_t)chunk * nchan * nbin));
+    CK(pl->gf_errs.need(sizeof(double) * (size_t)chunk * nchan));
+  }
+  if (njoin > 0) {
+    CK(pl->gf_join.need(sizeof(int32_t) * nchan));
+    CK(cudaMemcpyAsync(pl->gf_join.p, join->join_chan, sizeof(int32_t) * nchan, cudaMemcpyHostToDevice, pl->stream));
+  }
   if (out->model) CK(pl->gf_model.need(sizeof(double) * (size_t)chunk * nchan * nbin));
   // parameter tables: free flags (as bytes after lo, hi)
   CK(pl->gf_par.need(sizeof(double) * 2 * P + P));
@@ -2105,31 +2138,34 @@ extern "C" int pp_fit_gaussian_portraits(pp_plan_t* pl, const pp_gfit_args_t* ar
   GfitArgs g;
   g.freqs = pl->freqs.as<double>(); g.rec = pl->gf_rec.as<double>(); g.slab = pl->gf_slab.as<double2>();
   g.twN = pl->twN64.p; g.tw2N = pl->tw2N64.p; g.nu_ref = A.nu_ref; g.nchan = nchan; g.ngauss = ng;
-  g.P = P; g.L = L; g.S = S;
+  g.P = P; g.L = L; g.S = S; g.ia = 2 + 6 * ng; g.njoin = njoin;
+  g.join_chan = njoin > 0 ? pl->gf_join.as<int>() : nullptr; g.P_period = njoin > 0 ? join->P : 0.0;
   for (int i = 0; i < 3; ++i) g.code[i] = A.model_code[i] - '0';
   const int npair_all = P * (P + 1) / 2 + P + 1;
   std::vector<double> x0((size_t)chunk * P);
   for (int s0 = 0; s0 < nport; s0 += chunk) {
     const int nc = std::min(chunk, nport - s0);
     const size_t rows = (size_t)nc * nchan;
-    CK(cudaMemcpyAsync(pl->gf_data.p, A.data + (size_t)s0 * nchan * nbin, sizeof(double) * rows * nbin,
-                       cudaMemcpyDefault, pl->stream));
-    CK(cudaMemcpyAsync(pl->gf_errs.p, A.errs + (size_t)s0 * nchan, sizeof(double) * rows, cudaMemcpyDefault, pl->stream));
+    if (!gen) {
+      CK(cudaMemcpyAsync(pl->gf_data.p, A.data + (size_t)s0 * nchan * nbin, sizeof(double) * rows * nbin,
+                         cudaMemcpyDefault, pl->stream));
+      CK(cudaMemcpyAsync(pl->gf_errs.p, A.errs + (size_t)s0 * nchan, sizeof(double) * rows, cudaMemcpyDefault, pl->stream));
+    }
     // start values moved into the box
     CK(cudaMemcpyAsync(x0.data(), A.init + (size_t)s0 * P, sizeof(double) * nc * P, cudaMemcpyDefault, pl->stream));
     CK(cudaStreamSynchronize(pl->stream));
     for (int s = 0; s < nc; ++s)
       for (int i = 0; i < P; ++i) x0[(size_t)s * P + i] = std::min(std::max(x0[(size_t)s * P + i], lo[i]), hi[i]);
-    CK(cudaMemcpyAsync(st.xt, x0.data(), sizeof(double) * nc * P, cudaMemcpyHostToDevice, pl->stream));
+    CK(cudaMemcpyAsync(gen ? st.x : st.xt, x0.data(), sizeof(double) * nc * P, cudaMemcpyHostToDevice, pl->stream));
     {
       std::vector<double> lam(nc, kGfitLam0);
       CK(cudaMemcpyAsync(st.lam, lam.data(), sizeof(double) * nc, cudaMemcpyHostToDevice, pl->stream));
       CK(cudaMemsetAsync(st.nfev, 0, sizeof(int) * 2 * chunk, pl->stream));   // nfev and done
       CK(cudaStreamSynchronize(pl->stream));
     }
-    g.data = pl->gf_data.as<double>(); g.errs = pl->gf_errs.as<double>(); g.nc = nc;
+    g.data = gen ? nullptr : pl->gf_data.as<double>(); g.errs = gen ? nullptr : pl->gf_errs.as<double>(); g.nc = nc;
     // passes are launched while some portrait of the chunk is still running
-    for (;;) {
+    while (!gen) {
       g.xt = st.xt; g.done = st.done; g.model = nullptr;
       DISPATCH_N(N, if (gfit_pass<NN>(pl, g, nslab)) return -2);
       k_gfit_reduce<<<dim3((npair_all + 255) / 256, nc), 256, 0, pl->stream>>>(g, st, d_free);

@@ -320,23 +320,43 @@ class WidebandPlan(object):
 
     # ---- evolving-Gaussian model fit ----------------------------------------------------
     def fit_gaussian_portraits(self, data, errs, model_code, init, fit_flags, nu_ref, bounds=None,
-                               max_iter=0, tol=0, want_model=False, want_sums=False):
+                               max_iter=0, tol=0, want_model=False, want_sums=False, join_chan=None, P=None):
         """Fit evolving-Gaussian portraits (pplib.py:1924-2052) to ``data`` [nport, nchan, nbin] float64
         with per-channel sigma ``errs`` [nport, nchan], on the plan's frequencies (set_freqs first).
         ``init`` [nport, P] and ``fit_flags`` [P] use the layout [DC, tau [bin], (loc, m_loc, wid, m_wid,
-        amp, m_amp) * ngauss, alpha], P = 3 + 6 ngauss; ``bounds`` [P, 2] with NaN (or None) for open
-        ends.  ``max_iter`` < 0 evaluates chi2, J^T r and J^T J at the start point only (0: default 200);
-        ``tol`` 0 = 1e-4.  numpy arrays or CUDA tensors.  Returns a dict of numpy arrays: params,
-        param_errs, cov, chi2, red_chi2, dof, nfeval, return_code, and with ``want_model`` the model
-        portraits [nport, nchan, nbin], with ``want_sums`` jtr [nport, P] and jtj [nport, P, P]."""
+        amp, m_amp) * ngauss, alpha, (phi_j, DM_j) * njoin], P = 3 + 6 ngauss + 2 njoin; ``bounds`` [P, 2]
+        with NaN (or None) for open ends.  ``max_iter`` < 0 evaluates chi2, J^T r and J^T J at the start
+        point only (0: default 200); ``tol`` 0 = 1e-4.  numpy arrays or CUDA tensors.
+
+        Join parameters (pp_fit_gaussian_portraits_join): ``join_chan`` [nchan] int gives the join group of
+        each channel (-1: none; njoin = max + 1) and ``P`` the spin period [s]; channel n of group j is rotated
+        by phi_j + Dconst DM_j / P (nu_n^-2 - nu_ref^-2) turns after scattering (rotate_data's convention).
+
+        Returns a dict of numpy arrays: params, param_errs, cov, chi2, red_chi2, dof, nfeval, return_code,
+        and with ``want_model`` the model portraits [nport, nchan, nbin], with ``want_sums`` jtr [nport, P]
+        and jtj [nport, P, P].  ``data=None`` (with ``errs=None`` and max_iter < 0) returns only the model
+        portraits at ``init``."""
         fit_flags = np.ascontiguousarray(np.asarray(fit_flags) != 0, dtype=np.uint8).ravel()
-        P = fit_flags.size
-        if P < 9 or (P - 3) % 6:
-            raise ValueError("fit_flags must have 3 + 6*ngauss entries")
-        ngauss = (P - 3) // 6
-        nport = int(data.shape[0])
         nchan, nbin = self.nchan, self.nbin
-        keep = []
+        jn = None
+        if join_chan is not None:
+            jc = np.ascontiguousarray(join_chan, dtype=np.int32).ravel()
+            if jc.size != nchan:
+                raise ValueError("join_chan must have nchan = %d entries" % nchan)
+            jn = _ffi.GfitJoin()
+            jn.njoin = int(jc.max()) + 1 if jc.size and jc.max() >= 0 else 0
+            jn.join_chan = jc.ctypes.data
+            jn.P = float("nan") if P is None else float(P)
+        njoin = jn.njoin if jn is not None else 0
+        nP = fit_flags.size
+        if nP < 9 + 2 * njoin or (nP - 3 - 2 * njoin) % 6:
+            raise ValueError("fit_flags must have 3 + 6*ngauss + 2*njoin entries (njoin = %d)" % njoin)
+        ngauss = (nP - 3 - 2 * njoin) // 6
+        gen = data is None
+        if gen and (errs is not None or max_iter >= 0):
+            raise ValueError("data=None evaluates the model at init only: errs=None and max_iter < 0")
+        nport = int(init.shape[0]) if gen else int(data.shape[0])
+        keep = [jn, jc] if jn is not None else []
         a = _ffi.GfitArgs()
         a.nport = nport
         a.data = _ptr(data, np.float64, keep, "data", (nport, nchan, nbin))
@@ -344,32 +364,38 @@ class WidebandPlan(object):
         a.model_code = str(model_code).encode("ascii")
         a.ngauss = ngauss
         a.nu_ref = float(nu_ref)
-        a.init = _ptr(init, np.float64, keep, "init", (nport, P))
+        a.init = _ptr(init, np.float64, keep, "init", (nport, nP))
         a.fit_flags = fit_flags.ctypes.data
         if bounds is not None:
             b = np.array([[np.nan if v is None else v for v in pair] for pair in bounds], dtype=np.float64)
-            if b.shape != (P, 2):
+            if b.shape != (nP, 2):
                 raise ValueError("bounds must be [P, 2]")
             a.bounds = _ptr(b, np.float64, keep, "bounds")
         a.max_iter = int(max_iter)
         a.tol = float(tol)
-        spec = {"params": ((nport, P), np.float64), "param_errs": ((nport, P), np.float64),
-                "cov": ((nport, P, P), np.float64), "chi2": ((nport,), np.float64),
-                "red_chi2": ((nport,), np.float64), "nfeval": ((nport,), np.int32),
-                "return_code": ((nport,), np.int32)}
-        if want_model:
+        spec = {} if gen else {
+            "params": ((nport, nP), np.float64), "param_errs": ((nport, nP), np.float64),
+            "cov": ((nport, nP, nP), np.float64), "chi2": ((nport,), np.float64),
+            "red_chi2": ((nport,), np.float64), "nfeval": ((nport,), np.int32),
+            "return_code": ((nport,), np.int32)}
+        if want_model or gen:
             spec["model"] = ((nport, nchan, nbin), np.float64)
-        if want_sums:
-            spec["jtr"] = ((nport, P), np.float64)
-            spec["jtj"] = ((nport, P, P), np.float64)
+        if want_sums and not gen:
+            spec["jtr"] = ((nport, nP), np.float64)
+            spec["jtj"] = ((nport, nP, nP), np.float64)
         res = {k: np.empty(sh, dtype=dt) for k, (sh, dt) in spec.items()}
         o = _ffi.GfitOut()
         for k, v in res.items():
             setattr(o, k, v.ctypes.data)
-        _ffi.check(self._lib.pp_fit_gaussian_portraits(self._h, C.byref(a), C.byref(o)),
-                   "pp_fit_gaussian_portraits")
+        if jn is None:
+            _ffi.check(self._lib.pp_fit_gaussian_portraits(self._h, C.byref(a), C.byref(o)),
+                       "pp_fit_gaussian_portraits")
+        else:
+            _ffi.check(self._lib.pp_fit_gaussian_portraits_join(self._h, C.byref(a), C.byref(jn), C.byref(o)),
+                       "pp_fit_gaussian_portraits_join")
         del keep
-        res["dof"] = np.full(nport, nchan * nbin - int(fit_flags.sum()), dtype=np.int64)
+        if not gen:
+            res["dof"] = np.full(nport, nchan * nbin - int(fit_flags.sum()), dtype=np.int64)
         return res
 
     # ---- batched 1-D FFTFIT --------------------------------------------------------
@@ -421,12 +447,29 @@ class WidebandPlan(object):
         return out
 
     def gen_gaussian_portrait(self, model_code, params, scattering_index, nu_ref, out=None, device_out=False,
-                              dtype=np.float32):
+                              dtype=np.float32, join_chan=None, P=None):
         """Evolving-Gaussian model portrait on the device (pplib.py:853-930) for the plan's
         frequencies (set_freqs first).  ``params`` = [DC, tau_bin, (loc, m_loc, wid, m_wid, amp,
         m_amp) * ngauss].  Returns [nchan, nbin] of ``dtype`` (float32, or float64: evaluated and stored in
         double): a numpy array, or a torch CUDA tensor with ``device_out=True`` (ready for set_model without a
-        host round trip)."""
+        host round trip).
+
+        With ``join_chan`` ([nchan] join group per channel, -1 = none; njoin = max + 1) and the period ``P`` [s],
+        ``params`` ends with (phi_j, DM_j) * njoin and the channels of group j are rotated after scattering, as
+        fit_gaussian_portraits defines it: the model output of pp_fit_gaussian_portraits_join, float64 numpy
+        (ngauss >= 1, nbin a power of two)."""
+        if join_chan is not None:
+            if out is not None or device_out:
+                raise ValueError("a joined model is returned as a new float64 numpy array")
+            jc = np.asarray(join_chan, dtype=np.int32).ravel()
+            njoin = int(jc.max()) + 1 if jc.size and jc.max() >= 0 else 0
+            params = np.asarray(params, dtype=np.float64).ravel()
+            nc = params.size - 2 * njoin
+            if nc < 8 or (nc - 2) % 6:
+                raise ValueError("params must have 2 + 6*ngauss + 2*njoin entries (njoin = %d)" % njoin)
+            x = np.concatenate([params[:nc], [float(scattering_index)], params[nc:]])
+            return self.fit_gaussian_portraits(None, None, model_code, x[None], np.zeros(x.size, bool), nu_ref,
+                                               max_iter=-1, join_chan=jc, P=P)["model"][0]
         params = np.ascontiguousarray(params, dtype=np.float64)
         if params.ndim != 1 or (params.size - 2) % 6:
             raise ValueError("params must have 2 + 6*ngauss entries")

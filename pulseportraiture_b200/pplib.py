@@ -11,6 +11,7 @@ generation from ``.gmodel`` files and scalar reference-frequency transforms.
 """
 from __future__ import annotations
 
+import os
 import sys
 import time
 
@@ -438,15 +439,48 @@ def evolve_parameter(freqs, nu_ref, parameter, evol_parameter, code):
     raise KeyError(code)
 
 
+_gauss_max_join = 8
+
+
+def _join_table(join_ichans, nchan, P):
+    """int32 [nchan] join group of each channel (-1: none) from join_ichans, a sequence of channel-index lists
+    (one per archive after the first).  Groups must be non-empty, disjoint and in range, at most 8, and P > 0."""
+    njoin = len(join_ichans)
+    if njoin > _gauss_max_join:
+        raise ValueError("at most %d join groups (got %d)" % (_gauss_max_join, njoin))
+    if P is None or not float(P) > 0.0:
+        raise ValueError("join parameters need the period P > 0 (got %r)" % (P,))
+    table = np.full(nchan, -1, dtype=np.int32)
+    for j, ich in enumerate(join_ichans):
+        ich = np.atleast_1d(np.asarray(ich))
+        if not ich.size:
+            raise ValueError("join group %d is empty" % j)
+        if ich.dtype.kind not in "iu":
+            raise ValueError("join group %d: channel indices must be integers" % j)
+        if ich.min() < 0 or ich.max() >= nchan:
+            raise ValueError("join group %d: channel index out of range [0, %d)" % (j, nchan))
+        if (table[ich] >= 0).any() or len(np.unique(ich)) != ich.size:
+            raise ValueError("join group %d overlaps another group" % j)
+        table[ich] = j
+    return table
+
+
 def gen_gaussian_portrait(model_code, params, scattering_index, phases, freqs,
                           nu_ref, join_ichans=[], P=None):
     """Evolving-Gaussian model portrait (pplib.py:853-930).  params =
-    [DC, tau_bin, (loc, m_loc, wid, m_wid, amp, m_amp) * ngauss]."""
-    if len(join_ichans):
-        raise NotImplementedError("join parameters are a ppgauss feature")
+    [DC, tau_bin, (loc, m_loc, wid, m_wid, amp, m_amp) * ngauss, (phi_j, DM_j) * len(join_ichans)].
+
+    Join parameters: after scattering, the channels join_ichans[j] are rotated as rotate_data(rows, phi_j, DM_j,
+    P, freqs, nu_ref) does, here in float64 numpy: harmonic k times e^{2 pi i k theta_n}, theta_n = phi_j +
+    Dconst DM_j / P (nu_n^-2 - nu_ref^-2), the Nyquist term keeping its real part (irfft).  P [s] is required with
+    joins; the groups must be disjoint, non-empty and in range (ValueError)."""
     params = np.asarray(params, dtype=np.float64)
     freqs = np.asarray(freqs, dtype=np.float64)
     nbin, nchan = len(phases), len(freqs)
+    njoin = len(join_ichans)
+    if njoin:
+        table = _join_table(join_ichans, nchan, P)
+        params, jvals = params[:len(params) - 2 * njoin], params[len(params) - 2 * njoin:]
     locs = evolve_parameter(freqs, nu_ref, params[2::6], params[3::6], model_code[0])
     wids = evolve_parameter(freqs, nu_ref, params[4::6], params[5::6], model_code[1])
     amps = evolve_parameter(freqs, nu_ref, params[6::6], params[7::6], model_code[2])
@@ -461,6 +495,12 @@ def gen_gaussian_portrait(model_code, params, scattering_index, phases, freqs,
         taus = scattering_times(float(tau) / nbin, scattering_index, freqs, nu_ref)
         gport = np.fft.irfft(scattering_portrait_FT(taus, nbin) *
                              np.fft.rfft(gport, axis=-1), axis=-1)
+    if njoin:
+        rows = np.where(table >= 0)[0]
+        j = table[rows]
+        theta = jvals[2 * j] + Dconst * jvals[2 * j + 1] / float(P) * (freqs[rows] ** -2.0 - nu_ref ** -2.0)
+        ph = np.exp(2j * np.pi * np.outer(theta, np.arange(nbin // 2 + 1)))
+        gport[rows] = np.fft.irfft(ph * np.fft.rfft(gport[rows], axis=-1), n=nbin, axis=-1)
     return gport
 
 
@@ -470,14 +510,19 @@ def gen_gaussian_portrait_device(model_code, params, scattering_index, phases, f
     ``k_gauss_model`` (+ the scattering multiply of ``k_rotate``): the per-archive /
     per-subint model build of pptoas.py:356-379.  ``phases`` must be the bin centres
     of get_bin_centers(nbin).  Returns float64 [nchan, nbin], evaluated in double (a scattered model,
-    tau != 0, passes through float32 rows)."""
-    if len(join_ichans):
-        raise NotImplementedError("join parameters are a ppgauss feature")
+    tau != 0, passes through float32 rows).
+
+    With join_ichans (and P) the joined model of gen_gaussian_portrait is evaluated in FP64 by the model output
+    of the fit's kernel (WidebandPlan.gen_gaussian_portrait with join_chan): ngauss >= 1 and nbin a power of
+    two."""
     nbin, nchan = len(phases), len(freqs)
     if not np.allclose(phases, get_bin_centers(nbin), rtol=0, atol=1e-12):
         raise ValueError("the device generator works on get_bin_centers(nbin)")
+    table = _join_table(join_ichans, nchan, P) if len(join_ichans) else None
     pl = get_plan(nchan, nbin)
     pl.set_freqs(np.asarray(freqs, dtype=np.float64))
+    if table is not None:
+        return pl.gen_gaussian_portrait(model_code, params, scattering_index, nu_ref, join_chan=table, P=P)
     return pl.gen_gaussian_portrait(model_code, params, scattering_index, nu_ref, dtype=np.float64)
 
 
@@ -630,16 +675,33 @@ def fit_gaussian_portrait(model_code, data, init_params, scattering_index, errs,
     Bounds, the policy of this facade: tau >= 0, 0 < wid <= wid_max (wid_max = 0.25 in this module's
     settings; the lower edge is wid = 1e-6 rot, far below one bin), amp >= 0, and loc >= 0 when its
     evolution code is a power law.  A free parameter that cannot move the model at the fitted point (alpha
-    while tau = 0, for example) gets fit_err 0 and a zero covariance row, MINPACK's convention.  Join
-    parameters (multi-receiver offsets) are not supported.
+    while tau = 0, for example) gets fit_err 0 and a zero covariance row, MINPACK's convention.
+
+    Join parameters fit one model to the portraits of several archives (receivers or bands) joined along the
+    channel axis (join_archives makes such a portrait): join_params = [join_ichans, join_values,
+    join_fit_flags] with join_ichans one list of channel indices per archive after the first, join_values
+    [phi_1, DM_1, ..., phi_J, DM_J] (start values) and join_fit_flags one flag per value; P [s] is the period
+    of the DM term.  The channels join_ichans[j] of the model are rotated by phi_j and DM_j about nu_ref after
+    scattering, as gen_gaussian_portrait(..., join_ichans, P) defines it; the other channels are the reference.
+    Up to 8 groups, disjoint, non-empty and in range (ValueError otherwise); join_params that is not a
+    three-part sequence raises NotImplementedError.  phi_j and DM_j are not bounded.
 
     Returns a DataBunch with fitted_params (layout of init_params, tau in bins), fit_errs,
-    scattering_index, scattering_index_err, chi2, dof, red_chi2, nfeval, return_code (0 converged,
-    1 iteration limit, 3 non-finite), duration, and the extras covariance ([P, P] in the layout
-    [params..., alpha], scaled by red_chi2 as lmfit's scale_covar) and model (the fitted portrait,
-    float64).  The reference's lm_results (the lmfit object) cannot be provided."""
+    scattering_index, scattering_index_err, join_params and join_param_errs ([phi_1, DM_1, ...]; empty
+    without joins), chi2, dof, red_chi2, nfeval, return_code (0 converged, 1 iteration limit, 3 non-finite),
+    duration, and the extras covariance ([P, P] in the layout [params..., alpha, phi_1, DM_1, ...], scaled by
+    red_chi2 as lmfit's scale_covar) and model (the fitted portrait, float64).  The reference's lm_results
+    (the lmfit object) cannot be provided."""
+    table, jvals, jflags = None, np.zeros(0), np.zeros(0, bool)
     if len(join_params):
-        raise NotImplementedError("join parameters are a ppgauss feature")
+        if isinstance(join_params, (str, bytes)) or len(join_params) != 3:
+            raise NotImplementedError("join_params must be [join_ichans, join_values, join_fit_flags]")
+        join_ichans, jvals, jflags = join_params
+        table = _join_table(join_ichans, np.shape(data)[0], P)
+        jvals = np.asarray(jvals, dtype=np.float64).ravel()
+        jflags = np.asarray(jflags, dtype=bool).ravel()
+        if jvals.size != 2 * len(join_ichans) or jflags.size != jvals.size:
+            raise ValueError("join_values and join_fit_flags need 2 entries (phi, DM) per join group")
     start = time.time()
     data = np.asarray(data, dtype=np.float64)
     nchan, nbin = data.shape
@@ -649,23 +711,56 @@ def fit_gaussian_portrait(model_code, data, init_params, scattering_index, errs,
     if init_params.ndim != 1 or (init_params.size - 2) % 6 or init_params.size < 8:
         raise ValueError("init_params must have 2 + 6*ngauss entries")
     ngauss = (init_params.size - 2) // 6
-    x0 = np.append(init_params, float(scattering_index))
-    flags = np.append(np.asarray(fit_flags, dtype=bool), bool(fit_scattering_index))
+    x0 = np.concatenate([init_params, [float(scattering_index)], jvals])
+    flags = np.concatenate([np.asarray(fit_flags, dtype=bool), [bool(fit_scattering_index)], jflags])
+    bounds = np.concatenate([_gauss_default_bounds(model_code, ngauss), np.full((jvals.size, 2), np.nan)])
     pl = get_plan(nchan, nbin)
     pl.set_freqs(np.asarray(freqs, dtype=np.float64))
     r = pl.fit_gaussian_portraits(data[None], np.asarray(errs, dtype=np.float64).reshape(1, nchan), model_code,
-                                  x0[None], flags, nu_ref, bounds=_gauss_default_bounds(model_code, ngauss),
-                                  want_model=True)
+                                  x0[None], flags, nu_ref, bounds=bounds, want_model=True, join_chan=table, P=P)
     params, perrs = r["params"][0], r["param_errs"][0]
+    ia = init_params.size
     rc = int(r["return_code"][0])
     if not quiet:
         print("Fit %d-component model: chi2 %.3f, red_chi2 %.5f, %d evaluations (%s)"
               % (ngauss, r["chi2"][0], r["red_chi2"][0], r["nfeval"][0], DEVICE_RCSTRINGS.get(str(rc), rc)))
-    return DataBunch(fitted_params=params[:-1].copy(), fit_errs=perrs[:-1].copy(),
-                     scattering_index=params[-1], scattering_index_err=perrs[-1],
+    return DataBunch(fitted_params=params[:ia].copy(), fit_errs=perrs[:ia].copy(),
+                     scattering_index=params[ia], scattering_index_err=perrs[ia],
+                     join_params=params[ia + 1:].copy(), join_param_errs=perrs[ia + 1:].copy(),
                      chi2=r["chi2"][0], dof=int(r["dof"][0]), red_chi2=r["red_chi2"][0],
                      nfeval=int(r["nfeval"][0]), return_code=rc, duration=time.time() - start,
                      covariance=r["cov"][0], model=r["model"][0])
+
+
+def join_archives(archives, ref=0):
+    """One portrait of several archives of one pulsar (DataBunches or .npz paths that pptoas.load_data reads, all
+    with the same nbin), for a joined fit_gaussian_portrait: each archive is averaged over its subints
+    (pptoas.tscrunch_databunch, total intensity), and the usable channels of every archive are concatenated in the
+    order given.  Archives are used as stored (dispersed unless stored dedispersed).
+
+    Returns a DataBunch with port [nchan, nbin], freqs [nchan], noise_stds [nchan] (get_noise of each averaged
+    channel), P (the period of archive ``ref``), join_ichans (the channel indices of every archive but ``ref``, in
+    order: the join_ichans of fit_gaussian_portrait), archive_ichans (those of every archive) and nbin."""
+    from .pptoas import load_data, tscrunch_databunch
+    if not len(archives):
+        raise ValueError("no archives")
+    if not 0 <= ref < len(archives):
+        raise ValueError("ref must index one of the %d archives" % len(archives))
+    ds = [tscrunch_databunch(load_data(a) if isinstance(a, (str, os.PathLike)) else a) for a in archives]
+    nbins = {int(d.nbin) for d in ds}
+    if len(nbins) != 1:
+        raise ValueError("the archives must have one nbin (got %s)" % sorted(nbins))
+    ports, freqs, noise, ichans, n0 = [], [], [], [], 0
+    for d in ds:
+        ok = np.asarray(d.ok_ichans[0], dtype=int)
+        ports.append(np.asarray(d.subints, dtype=np.float64)[0, 0, ok])
+        freqs.append(np.asarray(d.freqs, dtype=np.float64)[0, ok])
+        noise.append(np.asarray(d.noise_stds, dtype=np.float64)[0, 0, ok])
+        ichans.append(np.arange(n0, n0 + len(ok)))
+        n0 += len(ok)
+    return DataBunch(port=np.concatenate(ports), freqs=np.concatenate(freqs), noise_stds=np.concatenate(noise),
+                     P=float(np.asarray(ds[ref].Ps)[0]), join_ichans=[ichans[i] for i in range(len(ds)) if i != ref],
+                     archive_ichans=ichans, nbin=nbins.pop())
 
 
 def write_model(filenm, name, model_code, nu_ref, model_params, fit_flags, alpha, fit_alpha,
